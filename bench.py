@@ -95,7 +95,14 @@ def parse():
     ap.add_argument("--solve-scenarios", type=int, default=4,
                     help="also solve this many dispersed scenarios of the shipped example per GPU to convergence "
                          "(batched NLP solves per hour, BASELINE.json metric iii; 0 = skip)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned to its caller for rank 0's scenarios "
+                         "(residuals.npy: scenarios x residual rows; jacobian_packed.npy: scenarios x packed Jacobian "
+                         "values) as float64 arrays under DIR, at most 64 MB in all (beyond that, the columns of a "
+                         "fixed seeded sample), so that two builds can be compared output for output")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != "gelato":
+        ap.error("--dump-outputs: only the GPU arm (--impl gelato) returns its outputs to this process")
     variant, factor, scen = WORKLOADS[a.workload]
     a.variant = variant
     a.factor = a.factor or factor
@@ -198,6 +205,28 @@ def ncu_traffic(kernel, grid_blocks):
     except (OSError, KeyError, ValueError):
         pass
     return None, None
+
+
+DUMP_BYTES = 64 * 1000 * 1000  # files, .npy headers included
+DUMP_SEED = 20260119
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each (scenarios x n) device tensor of `arrays` as out_dir/<name>.npy in float64.  If together they pass
+    DUMP_BYTES, the larger ones keep only the columns of a sample drawn with DUMP_SEED (sorted, the same in every
+    run) so that the total fits; the smaller ones are written whole."""
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    left, todo = DUMP_BYTES, sorted(arrays.items(), key=lambda kv: kv[1].numel())
+    for i, (name, a) in enumerate(todo):
+        keep = min(a.shape[1], (left // (len(todo) - i) - 4096) // (8 * a.shape[0]))
+        if keep < a.shape[1]:
+            cols = np.sort(np.random.default_rng(DUMP_SEED).choice(a.shape[1], keep, replace=False))
+            a = a.index_select(1, torch.from_numpy(cols).to(a.device))
+        path = os.path.join(out_dir, name + ".npy")
+        np.save(path, a.to(torch.float64).cpu().numpy())
+        left -= os.path.getsize(path)
 
 
 def measured_peaks():
@@ -455,6 +484,8 @@ def run_gelato(args):
     launches = (E.launches - launches0) * args.steps // (args.steps + W)
     clocks = sampler.summary(t_dev0 + 0.1, t_dev1 + 0.05)
     clocks["window"] = "0.5 s of the timed launches run immediately before the timed steps, and the timed steps"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"residuals": gd, "jacobian_packed": pd})
 
     # ---- each kernel alone (CUDA events around the single launch, L2 flushed): the roofline's kernel is the heavy one ----
     vd = torch.empty((B, P.n_vals), dtype=torch.float64, device="cuda")

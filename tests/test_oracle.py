@@ -62,6 +62,19 @@ def test_oracle_libm_matches_reference_golden(name):
     _check_against_npz(npz, name, f, s, exact=False)
 
 
+def test_oracle_libm_matches_reference_golden_at_the_bench_workload():
+    """The same at the workload bench.py times (example x15 in sections of <= 20 nodes, N = 990): the reference's
+    own outputs in tests/golden/bench_reference.npz."""
+    npz = np.load(os.path.join(helpers.GOLDEN, "bench_reference.npz"))
+    p, u, c, x0 = helpers.example_problem(factor=15, max_nodes=20)
+    O = helpers.oracle_nlp(p, u, c, "libm", "numpy")
+    x = problem.vector_to_xdict(npz["x1/x"].copy(), p["M"], p["N"], p["num_sections"])
+    f, fail = O.objfunc(x)
+    assert fail is False
+    s, fail = O.sens(x)
+    _check_against_npz(npz, "x1", f, s, exact=False)
+
+
 @pytest.mark.parametrize("name", ["x0", "x1"])
 def test_oracle_gmath_matches_golden_bitwise(name):
     npz = np.load(GOLD_GM)
