@@ -22,7 +22,7 @@ from .plan import GROUPS, ORBIT_QUANTITIES, VAR_ORDER, CompiledPlan, OrbitAtEven
 
 class GelatoProblem:
     def __init__(self, pdict, unitdict, condition, user_eq=None, user_ineq=None, device=0, coord=None,
-                 engine_factory=None, reuse_output=True, fuse_pair=False):
+                 engine_factory=None, reuse_output=True, fuse_pair=False, derivative="forward", fd_step=None):
         """engine_factory(plan) -> object with eval_residuals / eval_jacobian / close / launches;
         default: the CUDA engine on `device` (the CPU test tier passes the host emulator of the
         kernels, tests/emu_binding.py, to exercise this host logic without a GPU).
@@ -36,9 +36,17 @@ class GelatoProblem:
         that also writes objfunc's rows -- and keeps the Jacobian; a `sens` call at the same decision vector (what a
         solver does after it accepts a point) then returns it without touching the GPU.  Same values bit for bit;
         one call of ~0.07 ms instead of two for the shipped example, at the price of a Jacobian download for every
-        objfunc call that no sens follows (line-search trial points)."""
+        objfunc call that no sens follows (line-search trial points).
+
+        derivative="forward" (default): the reference's forward-difference Jacobian, bit for bit.  "central": central
+        differences with step fd_step (None: engine.DEFAULT_FD_STEP) -- 100-1000x closer to the derivative on most
+        blocks for about twice the Jacobian's GPU time; same sparsity, same objfunc (DESIGN.md H6).  `sens`,
+        `jacobian_csr` and the fused pair follow it; `engine.set_fd` switches it later."""
+        _engine.fd_args(derivative, fd_step)  # a bad mode or step fails before anything is built
         self.plan = CompiledPlan(pdict, unitdict, condition, user_eq=user_eq, user_ineq=user_ineq, coord=coord)
         self.engine = engine_factory(self.plan) if engine_factory else _engine.Engine(self.plan, device=device)
+        if derivative != "forward":
+            self.engine.set_fd(derivative, fd_step)
         self.reuse_output = bool(reuse_output) and hasattr(self.engine, "eval_jacobian_update")
         self._vals = None
         self._csr = None

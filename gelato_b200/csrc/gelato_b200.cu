@@ -199,6 +199,27 @@ __global__ void k_scatter_xdep_host(const double* __restrict__ vals_all, const i
   }
 }
 
+// Central differences (DESIGN.md H6): `out` holds the +h pass in its own layout, `minus` the -h pass packed
+// ([n_scen][n_pack]).  Packed output (full == NULL): out[scen][i] = fd_central(out[scen][i], minus[scen][i]), i < n_ent
+// = n_pack.  COO output: the packed map, vals[scen][full[i]] = fd_central(vals[scen][full[i]], sgn[i] * minus[scen][src[i]]),
+// i < n_ent = n_xdep.
+__global__ void k_fd_central(double* __restrict__ out_all, long long out_stride, const double* __restrict__ minus_all,
+                             long long n_pack, int n_scen, const int64_t* __restrict__ full, const int64_t* __restrict__ src,
+                             const double* __restrict__ sgn, long long n_ent) {
+  for (int scen = blockIdx.y; scen < n_scen; scen += gridDim.y) {
+    double* out = out_all + (size_t)scen * out_stride;
+    const double* minus = minus_all + (size_t)scen * n_pack;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n_ent; i += (long long)gridDim.x * blockDim.x) {
+      if (full) {
+        const long long k = full[i];
+        out[k] = fd_central(out[k], sgn[i] * minus[src[i]]);
+      } else {
+        out[i] = fd_central(out[i], minus[i]);
+      }
+    }
+  }
+}
+
 // probe: is a*b+c left unfused?  (1 + 2^-30)(1 - 2^-30) - 1 is 0 unfused, -2^-60 fused
 __global__ void k_unfused_probe(double a, double b, double c, double* out) { *out = a * b + c; }
 
@@ -310,6 +331,13 @@ struct GelatoPlan {
   std::vector<Lane> lanes;
   int update_slices = 0;  // 0 = choose from the batch size
   int32_t* d_iota = nullptr;  // 0, 1, 2 ...: a slice's scenario ids
+  // finite-difference mode (gelato_plan_set_fd); central: the -h pass of batch slot s goes to d_fd + s * n_pack
+  int fd_mode = GELATO_FD_FORWARD;
+  double fd_step = 0.0;
+  double* d_fd = nullptr;
+  size_t cap_fd = 0;
+  const int64_t *d_pk_full = nullptr, *d_pk_src = nullptr;  // the packed map on the device (uploaded on first use)
+  const double* d_pk_sgn = nullptr;
   long long launches = 0;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
 };
@@ -339,11 +367,13 @@ static int upload(GelatoPlan* p, const T* src, size_t count, const T** dst) {
 struct JacRange {
   int b0 = 0, nb = -1, v0 = 0, nv = 0;
 };
-static int launch_jacobian(GelatoPlan* p, const double* x_dev, double* out_dev, double* g_dev, int n_scen, cudaStream_t st,
-                           cudaStream_t aux, cudaEvent_t ev_fork, cudaEvent_t ev_join, const int32_t* ids_dev, bool packed,
-                           JacRange rg = JacRange()) {
+// dx: the step of the finite-difference protocol (the plan's dx for forward differences).
+static int launch_jacobian_pass(GelatoPlan* p, double dx, const double* x_dev, double* out_dev, double* g_dev, int n_scen,
+                                cudaStream_t st, cudaStream_t aux, cudaEvent_t ev_fork, cudaEvent_t ev_join,
+                                const int32_t* ids_dev, bool packed, JacRange rg = JacRange()) {
   PlanView v = p->view;
   v.packed = packed ? 1 : 0;
+  v.un.dx = dx;
   const bool all = rg.nb < 0;
   const int nb = all ? (g_dev ? p->n_jac_blocks : p->n_jac_main) : rg.nb;
   const int nv = all ? p->n_vac : rg.nv;
@@ -369,6 +399,53 @@ static int launch_jacobian(GelatoPlan* p, const double* x_dev, double* out_dev, 
     CU(cudaEventRecord(ev_join, aux));
     CU(cudaStreamWaitEvent(st, ev_join, 0));
   }
+  return GELATO_OK;
+}
+
+// The central-difference scratch for batch slots [0, n_scen) and the packed map on the device; nothing in forward mode.
+// Every entry point that evaluates the Jacobian calls it before its first launch.
+static int ensure_fd_scratch(GelatoPlan* p, size_t n_scen) {
+  if (p->fd_mode != GELATO_FD_CENTRAL) return GELATO_OK;
+  CU(cudaSetDevice(p->device));
+  if (!p->d_pk_full && !p->pk_full.empty()) {
+    int rc;
+    if ((rc = upload(p, p->pk_full.data(), p->pk_full.size(), &p->d_pk_full)) != GELATO_OK) return rc;
+    if ((rc = upload(p, p->pk_src.data(), p->pk_src.size(), &p->d_pk_src)) != GELATO_OK) return rc;
+    if ((rc = upload(p, p->pk_sgn.data(), p->pk_sgn.size(), &p->d_pk_sgn)) != GELATO_OK) return rc;
+  }
+  if (n_scen <= p->cap_fd) return GELATO_OK;
+  if (p->d_fd) CU(cudaFree(p->d_fd));  // synchronises: no launch still reads the old region
+  p->d_fd = nullptr;
+  p->cap_fd = 0;
+  CU(cudaMalloc(&p->d_fd, std::max<size_t>(1, n_scen * (size_t)p->n_pack) * sizeof(double)));
+  p->cap_fd = n_scen;
+  return GELATO_OK;
+}
+
+// One Jacobian evaluation in the plan's finite-difference mode (DESIGN.md H6).  Forward: one pass with the plan's dx.
+// Central: the +h pass writes the caller's output (and g of a pair evaluation), the -h pass (Jacobian only) writes the
+// packed scratch of batch slots [s0, s0 + n_scen) -- slices of one batch in flight on several streams use disjoint
+// regions -- and k_fd_central averages the two into the caller's output.
+static int launch_jacobian(GelatoPlan* p, const double* x_dev, double* out_dev, double* g_dev, int n_scen, cudaStream_t st,
+                           cudaStream_t aux, cudaEvent_t ev_fork, cudaEvent_t ev_join, const int32_t* ids_dev, bool packed,
+                           int s0 = 0) {
+  if (p->fd_mode != GELATO_FD_CENTRAL)
+    return launch_jacobian_pass(p, p->view.un.dx, x_dev, out_dev, g_dev, n_scen, st, aux, ev_fork, ev_join, ids_dev, packed);
+  if ((size_t)s0 + (size_t)n_scen > p->cap_fd) return fail(GELATO_ERR_ARG, "central-difference scratch not allocated");
+  const double h = p->fd_step;
+  double* minus = p->d_fd + (size_t)s0 * p->n_pack;
+  int rc = launch_jacobian_pass(p, h, x_dev, out_dev, g_dev, n_scen, st, aux, ev_fork, ev_join, ids_dev, packed);
+  if (rc) return rc;
+  if ((rc = launch_jacobian_pass(p, -h, x_dev, minus, nullptr, n_scen, st, aux, ev_fork, ev_join, ids_dev, true))) return rc;
+  const long long n_ent = packed ? p->n_pack : (long long)p->pk_full.size();
+  if (n_ent == 0) return GELATO_OK;
+  const int threads = 256;
+  const unsigned bx = (unsigned)std::min<long long>((n_ent + threads - 1) / threads, 4096);
+  const unsigned by = (unsigned)std::min(n_scen, 65535);
+  k_fd_central<<<dim3(bx, by), threads, 0, st>>>(out_dev, packed ? p->n_pack : p->view.n_vals, minus, p->n_pack, n_scen,
+                                                 packed ? nullptr : p->d_pk_full, p->d_pk_src, p->d_pk_sgn, n_ent);
+  p->launches++;
+  CU(cudaGetLastError());
   return GELATO_OK;
 }
 
@@ -589,6 +666,7 @@ int gelato_plan_destroy(GelatoPlan* p) {
     for (cudaEvent_t e : {L.ev_h2d, L.ev_g, L.ev_gdone})
       if (e) cudaEventDestroy(e);
   if (p->d_iota) cudaFree(p->d_iota);
+  if (p->d_fd) cudaFree(p->d_fd);
   if (p->ev0) cudaEventDestroy(p->ev0);
   if (p->ev1) cudaEventDestroy(p->ev1);
   if (p->ev_kernel) cudaEventDestroy(p->ev_kernel);
@@ -599,6 +677,26 @@ int gelato_plan_destroy(GelatoPlan* p) {
   if (p->pair_stream) cudaStreamDestroy(p->pair_stream);
   if (p->stream) cudaStreamDestroy(p->stream);
   delete p;
+  return GELATO_OK;
+}
+
+int gelato_plan_set_fd(GelatoPlan* p, int32_t mode, double step) {
+  if (!p) return fail(GELATO_ERR_ARG, "null plan");
+  if (mode == GELATO_FD_FORWARD) {
+    p->fd_mode = mode;
+    return GELATO_OK;
+  }
+  if (mode != GELATO_FD_CENTRAL) return fail(GELATO_ERR_ARG, "unknown finite-difference mode");
+  if (!(step > 0.0 && step <= 1e-3)) return fail(GELATO_ERR_ARG, "the central-difference step must be finite and in (0, 1e-3]");
+  p->fd_mode = mode;
+  p->fd_step = step;
+  return GELATO_OK;
+}
+
+int gelato_plan_get_fd(const GelatoPlan* p, int32_t* mode, double* step) {
+  if (!p || !mode || !step) return fail(GELATO_ERR_ARG, "null argument");
+  *mode = p->fd_mode;
+  *step = p->fd_mode == GELATO_FD_CENTRAL ? p->fd_step : p->view.un.dx;
   return GELATO_OK;
 }
 
@@ -650,6 +748,7 @@ int gelato_eval_pair_dev(GelatoPlan* p, const double* x_dev, double* g_dev, doub
   // objfunc's rows come out of the Jacobian launch: the dynamics blocks hold the right-hand side of the pristine
   // x as their centre column and subtract it from the D.X products; aero and event blocks carry one more column
   // at the pristine state; the linear rows are blocks of their own (no second pass over the physics)
+  if ((rc = ensure_fd_scratch(p, n_scen))) return rc;
   return launch_jacobian(p, x_dev, vals_dev, g_dev, n_scen, st, p->pair_stream, p->ev_fork, p->ev_join, nullptr, false);
 }
 
@@ -659,6 +758,7 @@ int gelato_eval_pair_packed_dev(GelatoPlan* p, const double* x_dev, double* g_de
   if (rc) return rc;
   CU(cudaSetDevice(p->device));
   cudaStream_t st = stream ? (cudaStream_t)stream : p->stream;
+  if ((rc = ensure_fd_scratch(p, n_scen))) return rc;
   return launch_jacobian(p, x_dev, packed_dev, g_dev, n_scen, st, p->pair_stream, p->ev_fork, p->ev_join, nullptr, true);
 }
 
@@ -672,6 +772,7 @@ int gelato_eval_pair_packed_range_dev(GelatoPlan* p, const double* x_dev, double
   int rc = check_scen(p, n_scen);
   if (rc) return rc;
   if (!g_dev || !packed_dev) return fail(GELATO_ERR_ARG, "null buffer");
+  if (p->fd_mode != GELATO_FD_FORWARD) return fail(GELATO_ERR_ARG, "the range evaluation supports forward differences only");
   if (block_first < 0 || block_count < 0 || block_first + block_count > p->n_jac_blocks || vac_first < 0 || vac_count < 0 ||
       vac_first + vac_count > p->n_vac)
     return fail(GELATO_ERR_ARG, "block or vacuum-node range outside the plan");
@@ -679,7 +780,8 @@ int gelato_eval_pair_packed_range_dev(GelatoPlan* p, const double* x_dev, double
   cudaStream_t st = stream ? (cudaStream_t)stream : p->stream;
   JacRange rg;
   rg.b0 = block_first; rg.nb = block_count; rg.v0 = vac_first; rg.nv = vac_count;
-  return launch_jacobian(p, x_dev, packed_dev, g_dev, n_scen, st, p->pair_stream, p->ev_fork, p->ev_join, nullptr, true, rg);
+  return launch_jacobian_pass(p, p->view.un.dx, x_dev, packed_dev, g_dev, n_scen, st, p->pair_stream, p->ev_fork, p->ev_join,
+                              nullptr, true, rg);
 }
 
 int gelato_fill_template(GelatoPlan* p, double* vals_dev, int32_t n_scen, void* stream) {
@@ -705,6 +807,7 @@ int gelato_eval_jacobian_dev(GelatoPlan* p, const double* x_dev, double* vals_de
   cudaStream_t st = stream ? (cudaStream_t)stream : p->stream;
   // the constants and D entries of vals_dev were put there once by gelato_fill_template;
   // the kernels rewrite every x-dependent slot and never touch the rest
+  if ((rc = ensure_fd_scratch(p, n_scen))) return rc;
   return launch_jacobian(p, x_dev, vals_dev, nullptr, n_scen, st, p->pair_stream, p->ev_fork, p->ev_join, nullptr, false);
 }
 
@@ -762,6 +865,7 @@ static int eval_host(GelatoPlan* p, int which, const double* x, double* out, int
   if (rc) return rc;
   if (!x || !out) return fail(GELATO_ERR_ARG, "null buffer");
   if ((rc = ensure_staging(p, n_scen))) return rc;
+  if (which == 1 && (rc = ensure_fd_scratch(p, n_scen))) return rc;
   const PlanView& v = p->view;
   const size_t nx = (size_t)n_scen * v.n_vars;
   const size_t no = (size_t)n_scen * (which == 0 ? (size_t)v.n_rows : (size_t)v.n_vals);
@@ -945,6 +1049,7 @@ static int eval_update(GelatoPlan* p, const double* x, double* g, double* vals, 
   if (!p->d_xdep) return fail(GELATO_ERR_ARG, "the plan was created without xdep_idx");
   if (n_scen > 65535) return fail(GELATO_ERR_ARG, "n_scen > 65535 in update mode (gridDim.y)");
   if ((rc = ensure_staging(p, n_scen))) return rc;
+  if ((rc = ensure_fd_scratch(p, n_scen))) return rc;
   const PlanView& v = p->view;
   if ((size_t)n_scen > p->cap_pack) {
     if (p->d_pack) cudaFree(p->d_pack);
@@ -1037,7 +1142,8 @@ static int eval_update(GelatoPlan* p, const double* x, double* g, double* vals, 
     CU(cudaMemcpyAsync(dx, hx + (size_t)s0 * v.n_vars, (size_t)ns * v.n_vars * sizeof(double), cudaMemcpyHostToDevice, L.stream));
     CU(cudaEventRecord(L.ev_h2d, L.stream));
     // g != NULL: pair evaluation, the residual rows come out of the same launches
-    if ((rc = launch_jacobian(p, dx, dvals, g ? dg : nullptr, ns, L.stream, L.pair_stream, L.ev_fork, L.ev_join, ids, false)))
+    if ((rc = launch_jacobian(p, dx, dvals, g ? dg : nullptr, ns, L.stream, L.pair_stream, L.ev_fork, L.ev_join, ids, false,
+                              s0)))
       return rc;
     if (g) {  // its copy travels on the side stream, next to the Jacobian's transfers
       CU(cudaEventRecord(L.ev_g, L.stream));
@@ -1111,6 +1217,7 @@ static int eval_packed(GelatoPlan* p, const double* x, double* g, double* packed
     for (int k = 0; k < n_scen; k++)
       if (scen_ids[k] < 0 || scen_ids[k] >= p->n_scen_cfg) return fail(GELATO_ERR_ARG, "scenario id outside the configured scenarios");
   CU(cudaSetDevice(p->device));
+  if ((rc = ensure_fd_scratch(p, n_scen))) return rc;
   const size_t np = (size_t)p->n_pack;
   if ((size_t)n_scen > p->cap_packed) {
     if (p->d_packed) cudaFree(p->d_packed);
@@ -1169,7 +1276,7 @@ static int eval_packed(GelatoPlan* p, const double* x, double* g, double* packed
     CU(cudaMemcpyAsync(dx, hx + (size_t)s0 * v.n_vars, (size_t)ns * v.n_vars * sizeof(double), cudaMemcpyHostToDevice, L.stream));
     CU(cudaEventRecord(L.ev_h2d, L.stream));
     if ((rc = launch_jacobian(p, dx, dpk, g ? dg : nullptr, ns, L.stream, L.pair_stream, L.ev_fork, L.ev_join,
-                              need_ids ? p->d_pids + s0 : nullptr, true)))
+                              need_ids ? p->d_pids + s0 : nullptr, true, s0)))
       return rc;
     // both results on the lane's copy stream, after everything of the slice has been computed
     CU(cudaEventRecord(L.ev_kernel, L.stream));
@@ -1304,7 +1411,8 @@ int gelato_launch_kernel_dev(GelatoPlan* p, int which, const double* x_dev, doub
   if (which == 0) {
     k_residuals<<<(unsigned)p->n_res_blocks * n_scen, GR_THREADS, 0, st>>>(v, p->res_blocks, n_scen, nullptr, x_dev, out_dev);
   } else if (which == 1) {
-    return launch_jacobian(p, x_dev, out_dev, g_dev, n_scen, st, p->pair_stream, p->ev_fork, p->ev_join, nullptr, packed != 0);
+    return launch_jacobian_pass(p, p->view.un.dx, x_dev, out_dev, g_dev, n_scen, st, p->pair_stream, p->ev_fork, p->ev_join,
+                                nullptr, packed != 0);
   } else if (which == 2) {
     if (p->n_jac_heavy == 0) return fail(GELATO_ERR_ARG, "the plan has no heavy blocks");
     k_jacobian_heavy<<<(unsigned)p->n_jac_heavy * n_scen, GJ_THREADS, 0, st>>>(v, p->jac_heavy, n_scen, nullptr, x_dev, out_dev, g_dev);
@@ -1339,8 +1447,8 @@ int gelato_time_kernel(GelatoPlan* p, int which, const double* x_dev, double* ou
     if (which == 0) {
       k_residuals<<<(unsigned)p->n_res_blocks * n_scen, GR_THREADS, 0, p->stream>>>(p->view, p->res_blocks, n_scen, nullptr, x_dev, out_dev);
     } else if (which == 1) {  // the whole Jacobian evaluation (heavy and light kernels)
-      if ((rc = launch_jacobian(p, x_dev, out_dev, nullptr, n_scen, p->stream, p->pair_stream, p->ev_fork, p->ev_join, nullptr,
-                                false)))
+      if ((rc = launch_jacobian_pass(p, p->view.un.dx, x_dev, out_dev, nullptr, n_scen, p->stream, p->pair_stream, p->ev_fork,
+                                     p->ev_join, nullptr, false)))
         return rc;
       continue;
     } else if (which == 2) {  // the heavy roles' blocks alone (air dynamics + aero rows)

@@ -196,13 +196,16 @@ P_HD double residue_n(double x, double dx, int n) {
   return x;
 }
 
-/* num / dx for the finite-difference quotients (dx > 0, checked at plan creation).  Many
- * quotients have an exactly zero numerator (a column that does not move an output); IEEE gives
- * 0/dx = 0 with the numerator's sign, and saying so skips the division's slow path, which the
- * GPU's software FP64 division takes for zero numerators (ncu r01b: 8 % of all instructions). */
+/* num / dx for the finite-difference quotients (the plan's dx > 0, checked at plan creation; the -h pass of
+ * central differences runs with dx < 0).  Many quotients have an exactly zero numerator (a column that does not
+ * move an output); IEEE gives 0/dx = 0 with the numerator's sign for dx > 0, and saying so skips the division's
+ * slow path, which the GPU's software FP64 division takes for zero numerators (ncu r01b: 8 % of all instructions).
+ * For dx < 0 the zero keeps the numerator's sign too, unlike IEEE's 0/dx: DESIGN.md H6 makes that the rule. */
 P_HD double fd_div(double num, double dx) { return num == 0.0 ? num : gm_div(num, dx); }
 /* the same with the reciprocal of dx computed once by the caller (gmath.h: gm_div_by is the IEEE quotient) */
 P_HD double fd_div_by(double num, const GmRcp Rdx) { return num == 0.0 ? num : gm_div_by(num, Rdx); }
+/* a central-difference value from the forward protocol's values with steps +h and -h (DESIGN.md H6) */
+P_HD double fd_central(double q_plus, double q_minus) { return (q_plus + q_minus) * 0.5; }
 
 P_HD Units scen_units(const PlanView& P, int scen) {
   Units u = P.un;

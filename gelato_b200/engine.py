@@ -25,6 +25,11 @@ NVCC_FLAGS = [
     "-Xcompiler", "-fPIC", "-shared",
 ]
 
+# Finite-difference modes of the Jacobian (include/gelato_b200.h: gelato_plan_set_fd; DESIGN.md H6)
+FD_MODES = {"forward": 0, "central": 1}
+# default step of central differences: the step sweep of profiles/r03a_fd_step_sweep.txt (DESIGN.md H6)
+DEFAULT_FD_STEP = 1e-6
+
 _c_d = ctypes.c_double
 _pd = ctypes.POINTER(ctypes.c_double)
 _pi32 = ctypes.POINTER(ctypes.c_int32)
@@ -206,6 +211,8 @@ def load_library():
     L.gelato_plan_n_vals.restype = ctypes.c_int64
     L.gelato_plan_launch_count.argtypes = [vp]
     L.gelato_plan_launch_count.restype = ctypes.c_int64
+    L.gelato_plan_set_fd.argtypes = [vp, ctypes.c_int32, _c_d]
+    L.gelato_plan_get_fd.argtypes = [vp, _pi32, _pd]
     L.gelato_eval_residuals.argtypes = [vp, _pd, _pd, ctypes.c_int32]
     L.gelato_eval_jacobian.argtypes = [vp, _pd, _pd, ctypes.c_int32]
     L.gelato_eval_residuals_ids.argtypes = [vp, _pd, _pd, ctypes.c_int32, _pi32]
@@ -270,8 +277,21 @@ EXPORTS = (
     "gelato_pack_xdep_dev gelato_leaf_dynamics_velocity gelato_leaf_dynamics_velocity_noair "
     "gelato_leaf_dynamics_quaternion gelato_leaf_aero gelato_leaf_eci2geodetic gelato_leaf_gravity gelato_leaf_iip "
     "gelato_leaf_atmosphere gelato_leaf_output_table gelato_init_rocket_simulation gelato_leaf_coordinate "
-    "gelato_eval_pair_packed_range_dev"
+    "gelato_eval_pair_packed_range_dev gelato_plan_set_fd gelato_plan_get_fd"
 ).split()
+
+
+def fd_args(mode, step=None):
+    """("forward" | "central", step or None) -> (C mode code, step): what gelato_plan_set_fd accepts, else ValueError.
+    The step of forward mode is the plan's dx and is ignored."""
+    if mode not in FD_MODES:
+        raise ValueError("derivative mode must be one of %s, not %r" % (sorted(FD_MODES), mode))
+    if mode == "forward":
+        return FD_MODES[mode], 0.0
+    step = DEFAULT_FD_STEP if step is None else step
+    if isinstance(step, bool) or not isinstance(step, (int, float)) or not 0.0 < float(step) <= 1e-3:
+        raise ValueError("the central-difference step must be a number in (0, 1e-3], not %r" % (step,))
+    return FD_MODES[mode], float(step)
 
 
 def _check(L, rc, what):
@@ -325,6 +345,19 @@ class Engine:
     @property
     def launches(self):
         return int(self.L.gelato_plan_launch_count(self.h))
+
+    def set_fd(self, mode, step=None):
+        """Finite-difference mode of every Jacobian this handle returns: "forward" (default; the plan's dx, the
+        reference's values bit for bit) or "central" with step `step` (None: DEFAULT_FD_STEP).  DESIGN.md H6."""
+        code, step = fd_args(mode, step)
+        _check(self.L, self.L.gelato_plan_set_fd(self.h, code, step), "gelato_plan_set_fd")
+
+    @property
+    def fd(self):
+        """(mode, step): the current finite-difference mode and its step (forward: the plan's dx)."""
+        m, h = ctypes.c_int32(0), ctypes.c_double(0.0)
+        _check(self.L, self.L.gelato_plan_get_fd(self.h, ctypes.byref(m), ctypes.byref(h)), "gelato_plan_get_fd")
+        return {v: k for k, v in FD_MODES.items()}[m.value], h.value
 
     # ---- host-buffer calls (what objfunc / sens use) --------------------
     def _x(self, x, n_scen):

@@ -196,6 +196,25 @@ int32_t gelato_plan_n_blocks(const GelatoPlan* plan, int which);
 /* kernels launched by this plan so far (bench.py's gpu_launches) */
 int64_t gelato_plan_launch_count(const GelatoPlan* plan);
 
+/* How the Jacobian's finite-difference values are formed (DESIGN.md H3, H6).
+ *   GELATO_FD_FORWARD (default)  the reference's forward differences with the plan's dx, bit for bit;
+ *   GELATO_FD_CENTRAL            central differences with step h: every finite-difference value is
+ *                                (q(+h) + q(-h)) * 0.5, q(+-h) being the forward protocol run with step +-h.
+ *                                Analytic and constant slots, sparsity, COO order and the packed layout do not
+ *                                change; objfunc values do not depend on the mode.  It costs a second Jacobian
+ *                                launch and one averaging pass (DESIGN.md H6 gives the measured cost), plus
+ *                                n_scen x n_pack doubles of plan-owned device scratch.
+ * gelato_plan_set_fd: mode and step (`step` is ignored for FORWARD, which always uses the plan's dx); a bad mode, or a
+ * central step that is not finite and in (0, 1e-3], returns GELATO_ERR_ARG and leaves the plan unchanged.  Every entry
+ * point that returns Jacobian values honours the mode (host, update, packed, _ids and _dev calls), except
+ * gelato_eval_pair_packed_range_dev, which refuses central mode, and the measurement helpers gelato_time_kernel and
+ * gelato_launch_kernel_dev, which always launch the forward kernels once.  Central _dev calls use the plan's scratch:
+ * calls on one plan must not overlap on different streams.
+ * gelato_plan_get_fd: the current mode and step (FORWARD: the plan's dx). */
+enum { GELATO_FD_FORWARD = 0, GELATO_FD_CENTRAL = 1 };
+int gelato_plan_set_fd(GelatoPlan* plan, int32_t mode, double step);
+int gelato_plan_get_fd(const GelatoPlan* plan, int32_t* mode, double* step);
+
 /* Host-buffer entry points (what the drop-in objfunc / sens call): copy x to the
  * device, run ONE fused kernel, copy the result back.  n_scen = 1 for a single NLP;
  * x is [n_scen][n_vars], g [n_scen][n_rows], vals [n_scen][n_vals].  Buffers obtained
@@ -291,7 +310,8 @@ int gelato_eval_pair_packed_dev(GelatoPlan* plan, const double* x_dev, double* g
  * linear rows) and vacuum dynamics nodes [vac_first, vac_first + vac_count) (gelato_plan_n_blocks(plan, 5) nodes).
  * Every packed slot and residual row is written by exactly one block or node: ranks with disjoint covering ranges
  * fill disjoint parts of packed[] and g[] (gelato_b200/batch.py: ShardedProblem finds each rank's part once and
- * gathers).  Device pointers, caller's stream, not synchronised. */
+ * gathers).  Device pointers, caller's stream, not synchronised.  Forward differences only: in central mode it returns
+ * GELATO_ERR_ARG. */
 int gelato_eval_pair_packed_range_dev(GelatoPlan* plan, const double* x_dev, double* g_dev, double* packed_dev, int32_t n_scen,
                                       int32_t block_first, int32_t block_count, int32_t vac_first, int32_t vac_count,
                                       void* stream);
@@ -303,7 +323,8 @@ int gelato_pack_xdep_dev(GelatoPlan* plan, const double* vals_dev, double* packe
 /* Timing helper for benchmarks: runs `reps` back-to-back launches of the chosen kernel on device-resident
  * buffers and returns the average duration in milliseconds measured with CUDA events on the launch stream.
  * which: 0 residual kernel | 1 the Jacobian kernel | 2 the heavy roles' blocks alone (air dynamics + aero rows)
- * | 3 the light roles' blocks alone (vacuum dynamics, fallback, event rows). */
+ * | 3 the light roles' blocks alone (vacuum dynamics, fallback, event rows).  Always forward differences with the
+ * plan's dx, whatever gelato_plan_set_fd chose (this and gelato_launch_kernel_dev time the kernels themselves). */
 int gelato_time_kernel(GelatoPlan* plan, int which, const double* x_dev, double* out_dev, int32_t n_scen, int reps,
                        float* avg_ms);
 /* Measurement helper: enqueue exactly one kernel on `stream`, not synchronised -- for benchmarks that bracket single
