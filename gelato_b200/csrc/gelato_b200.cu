@@ -15,11 +15,13 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <string>
 #include <thread>
 #include <utility>
 #include <vector>
 
+#include "cuda_owned.h"
 #include "host_pool.h"
 #include "plan_host.h"
 
@@ -262,10 +264,17 @@ static int fail(int code, const std::string& msg) {
       return fail(GELATO_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e_));           \
   } while (0)
 
+using gelato_host::DeviceBuf;
+using gelato_host::Event;
+using gelato_host::GraphExec;
+using gelato_host::PinnedBuf;
+using gelato_host::Stream;
+
 struct GelatoPlan {
   int device = 0;
-  PlanView view{};  // device pointers
-  std::vector<void*> owned;
+  PlanView view{};         // device pointers
+  PlanView shared_view{};  // the view as created, with the blocks every scenario shares (gelato_plan_set_scenarios)
+  std::vector<DeviceBuf<char>> owned;
   int32_t* jac_blocks = nullptr;  // n_jac_main dynamics / aero / event blocks (roles interleaved), then the linear-row blocks
   int n_jac_blocks = 0, n_jac_main = 0;
   int32_t *jac_heavy = nullptr, *jac_light = nullptr;  // the same blocks by role group (measurements)
@@ -277,37 +286,35 @@ struct GelatoPlan {
   long long n_pack = 0;
   std::vector<int64_t> pk_full, pk_src;
   std::vector<double> pk_sgn;
-  std::vector<void*> scen_owned;  // uploads of gelato_plan_set_scenarios (replaced by the next call)
-  double *d_packed = nullptr, *h_packed = nullptr;  // staging of the packed host entry points
-  size_t cap_packed = 0;
-  double *d_px = nullptr, *d_pg = nullptr, *h_px = nullptr;
-  int32_t* d_pids = nullptr;
-  bool pids_iota = false;
-  size_t cap_px = 0;
-  double* vals_template = nullptr;       // [n_vals] (or [n_scen][n_vals])
+  std::vector<DeviceBuf<char>> scen_owned;  // uploads of gelato_plan_set_scenarios (replaced by the next call)
+  const double* vals_template = nullptr;    // [n_vals] (or [n_scen][n_vals])
+  const double* shared_template = nullptr;  // the plan's own [n_vals]
   long long vals_template_sstride = 0;
   int n_scen_cfg = 1;
-  cudaStream_t stream = nullptr;
-  // staging for the host-buffer entry points
-  double *d_x = nullptr, *d_g = nullptr, *d_vals = nullptr;
-  double *h_x = nullptr, *h_out = nullptr;  // pinned
-  size_t cap_scen = 0;
+  // staging of every host-buffer entry point: x, g and the scenario ids of the batch slots, which hold either the
+  // caller's ids or 0, 1, 2 ... (ids_iota)
+  DeviceBuf<double> d_x, d_g;
+  PinnedBuf<double> h_x, h_g;
+  DeviceBuf<int32_t> d_ids;
+  bool ids_iota = false;
+  // COO Jacobian of the host entry points: slot k of d_vals holds scenario k's constants for k < vals_filled (written
+  // once, the kernels only rewrite x-dependent slots); d_vals_ids holds those of the slots of an _ids call
+  DeviceBuf<double> d_vals, d_vals_ids;
+  size_t vals_filled = 0;
+  PinnedBuf<double> h_vals;
+  // packed host entry points
+  DeviceBuf<double> d_packed;
+  PinnedBuf<double> h_packed;
   // small host-buffer objfunc calls: upload, kernel and download as ONE captured graph launch (the staging pointers
   // and the plan view are baked into it: rebuilt whenever either changes)
-  cudaGraphExec_t res_graph = nullptr;
+  GraphExec res_graph;
   int res_graph_n = 0;
-  double* h_small_out = nullptr;  // pinned staging of the small-problem path of update mode
-  size_t cap_small_out = 0;
-  // subset batches (gelato_eval_*_ids)
-  int32_t* d_ids = nullptr;
-  double* d_vals_ids = nullptr;
-  size_t cap_ids = 0;
   // update mode
   const int64_t* d_xdep = nullptr;
   std::vector<int64_t> h_xdep;
   long long n_xdep = 0;
-  double *d_pack = nullptr, *h_pack = nullptr;  // [cap_pack][n_xdep], h_pack pinned
-  size_t cap_pack = 0;
+  DeviceBuf<double> d_pack;  // [n_scen][n_xdep]
+  PinnedBuf<double> h_pack;
   int host_threads = 0;
   // scattered slots of a page-locked caller buffer: packed + host pool (0) or written from the device (1).
   // With 8+ host threads the pool is 1.6x faster end to end (profiles/r01v_e2e.txt); few cores: zero-copy.
@@ -316,46 +323,53 @@ struct GelatoPlan {
   const int64_t* d_xdep_small = nullptr;              // the slots outside those runs
   std::vector<int64_t> h_small;
   long long n_small = 0;
-  cudaStream_t copy_stream = nullptr;
-  cudaEvent_t ev_kernel = nullptr, ev_copy = nullptr;
-  cudaStream_t pair_stream = nullptr;  // residual kernel of a pair evaluation, concurrent with the Jacobian kernel
-  cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
-  // update mode pipelined over slices of the batch: slice k's upload and kernels overlap slice k-1's copies.
-  // Slice 0 runs on the streams above, the others on lanes created on first use.
+  // The plan's streams.  Lane 0 is created with the plan and serves every call (a device-pointer call launches on the
+  // caller's stream with lane 0's side stream and events); the host-buffer entry points pipeline a batch over slices,
+  // slice k's upload and kernels overlapping slice k-1's copies on lane k (created on first use).
   struct Lane {
-    cudaStream_t stream = nullptr, copy_stream = nullptr, pair_stream = nullptr;
-    cudaEvent_t ev_kernel = nullptr, ev_copy = nullptr, ev_fork = nullptr, ev_join = nullptr, ev_h2d = nullptr;
-    cudaEvent_t ev_g = nullptr, ev_gdone = nullptr;
-    std::vector<cudaEvent_t> chunk_ev;
+    Stream stream, copy_stream;
+    Stream pair_stream;  // the vacuum-node kernel of a Jacobian evaluation, concurrent with the block kernel
+    Event ev_kernel, ev_copy, ev_fork, ev_join, ev_h2d, ev_g, ev_gdone;
+    std::vector<Event> chunk_ev;
   };
   std::vector<Lane> lanes;
   int update_slices = 0;  // 0 = choose from the batch size
-  int32_t* d_iota = nullptr;  // 0, 1, 2 ...: a slice's scenario ids
   // finite-difference mode (gelato_plan_set_fd); central: the -h pass of batch slot s goes to d_fd + s * n_pack
   int fd_mode = GELATO_FD_FORWARD;
   double fd_step = 0.0;
-  double* d_fd = nullptr;
-  size_t cap_fd = 0;
+  DeviceBuf<double> d_fd;
   const int64_t *d_pk_full = nullptr, *d_pk_src = nullptr;  // the packed map on the device (uploaded on first use)
   const double* d_pk_sgn = nullptr;
   long long launches = 0;
-  cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+  Event ev0, ev1;
 };
+typedef GelatoPlan::Lane Lane;
 
 template <typename T>
-static int upload(GelatoPlan* p, const T* src, size_t count, const T** dst) {
+static int upload(std::vector<DeviceBuf<char>>& owner, const T* src, size_t count, const T** dst) {
   *dst = nullptr;
   if (count == 0 || src == nullptr) return GELATO_OK;
-  void* d = nullptr;
-  CU(cudaMalloc(&d, count * sizeof(T)));
-  p->owned.push_back(d);
-  CU(cudaMemcpy(d, src, count * sizeof(T), cudaMemcpyHostToDevice));
-  *dst = static_cast<const T*>(d);
+  owner.emplace_back();
+  CU(owner.back().reserve(count * sizeof(T)));
+  CU(cudaMemcpy(owner.back().get(), src, count * sizeof(T), cudaMemcpyHostToDevice));
+  *dst = reinterpret_cast<const T*>(owner.back().get());
+  return GELATO_OK;
+}
+
+static int add_lane(GelatoPlan* p) {
+  p->lanes.emplace_back();
+  Lane& L = p->lanes.back();
+  for (cudaStream_t* st : {L.stream.out(), L.copy_stream.out(), L.pair_stream.out()})
+    CU(cudaStreamCreateWithFlags(st, cudaStreamNonBlocking));
+  for (cudaEvent_t* e : {L.ev_kernel.out(), L.ev_copy.out(), L.ev_fork.out(), L.ev_join.out(), L.ev_h2d.out(), L.ev_g.out(),
+                         L.ev_gdone.out()})
+    CU(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
   return GELATO_OK;
 }
 
 // One Jacobian evaluation: the block kernel (air dynamics nodes, aero rows, fallback nodes, event rows) on `st` and the
-// one-thread-per-node kernel of the vacuum nodes on `aux`, forked from and joined back into `st` with the two events.
+// one-thread-per-node kernel of the vacuum nodes on the lane's pair stream, forked from and joined back into `st` with
+// the lane's two events.
 // g_dev != NULL: pair evaluation -- both also write objfunc's rows (collocation defects of their nodes, aero / event
 // rows at the pristine state) and the linear-row blocks at the end of the block table are launched too.
 // packed: output layout.
@@ -369,8 +383,7 @@ struct JacRange {
 };
 // dx: the step of the finite-difference protocol (the plan's dx for forward differences).
 static int launch_jacobian_pass(GelatoPlan* p, double dx, const double* x_dev, double* out_dev, double* g_dev, int n_scen,
-                                cudaStream_t st, cudaStream_t aux, cudaEvent_t ev_fork, cudaEvent_t ev_join,
-                                const int32_t* ids_dev, bool packed, JacRange rg = JacRange()) {
+                                cudaStream_t st, const Lane& L, const int32_t* ids_dev, bool packed, JacRange rg = JacRange()) {
   PlanView v = p->view;
   v.packed = packed ? 1 : 0;
   v.un.dx = dx;
@@ -379,10 +392,11 @@ static int launch_jacobian_pass(GelatoPlan* p, double dx, const double* x_dev, d
   const int nv = all ? p->n_vac : rg.nv;
   const int v_first = p->vac_first + (all ? 0 : rg.v0);
   const int32_t* table = p->jac_blocks + (size_t)(all ? 0 : rg.b0) * BT_COLS;
+  const cudaStream_t aux = L.pair_stream;
   const bool side = nv > 0 && nb > 0 && aux != st;
   if (side) {
-    CU(cudaEventRecord(ev_fork, st));
-    CU(cudaStreamWaitEvent(aux, ev_fork, 0));
+    CU(cudaEventRecord(L.ev_fork, st));
+    CU(cudaStreamWaitEvent(aux, L.ev_fork, 0));
   }
   if (nv > 0) {
     const int per = (nv + 31) / 32;
@@ -396,8 +410,8 @@ static int launch_jacobian_pass(GelatoPlan* p, double dx, const double* x_dev, d
   }
   CU(cudaGetLastError());
   if (side) {
-    CU(cudaEventRecord(ev_join, aux));
-    CU(cudaStreamWaitEvent(st, ev_join, 0));
+    CU(cudaEventRecord(L.ev_join, aux));
+    CU(cudaStreamWaitEvent(st, L.ev_join, 0));
   }
   return GELATO_OK;
 }
@@ -409,16 +423,11 @@ static int ensure_fd_scratch(GelatoPlan* p, size_t n_scen) {
   CU(cudaSetDevice(p->device));
   if (!p->d_pk_full && !p->pk_full.empty()) {
     int rc;
-    if ((rc = upload(p, p->pk_full.data(), p->pk_full.size(), &p->d_pk_full)) != GELATO_OK) return rc;
-    if ((rc = upload(p, p->pk_src.data(), p->pk_src.size(), &p->d_pk_src)) != GELATO_OK) return rc;
-    if ((rc = upload(p, p->pk_sgn.data(), p->pk_sgn.size(), &p->d_pk_sgn)) != GELATO_OK) return rc;
+    if ((rc = upload(p->owned, p->pk_full.data(), p->pk_full.size(), &p->d_pk_full)) != GELATO_OK) return rc;
+    if ((rc = upload(p->owned, p->pk_src.data(), p->pk_src.size(), &p->d_pk_src)) != GELATO_OK) return rc;
+    if ((rc = upload(p->owned, p->pk_sgn.data(), p->pk_sgn.size(), &p->d_pk_sgn)) != GELATO_OK) return rc;
   }
-  if (n_scen <= p->cap_fd) return GELATO_OK;
-  if (p->d_fd) CU(cudaFree(p->d_fd));  // synchronises: no launch still reads the old region
-  p->d_fd = nullptr;
-  p->cap_fd = 0;
-  CU(cudaMalloc(&p->d_fd, std::max<size_t>(1, n_scen * (size_t)p->n_pack) * sizeof(double)));
-  p->cap_fd = n_scen;
+  CU(p->d_fd.reserve(std::max<size_t>(1, n_scen * (size_t)p->n_pack)));  // synchronises: no launch still reads the old region
   return GELATO_OK;
 }
 
@@ -427,16 +436,16 @@ static int ensure_fd_scratch(GelatoPlan* p, size_t n_scen) {
 // packed scratch of batch slots [s0, s0 + n_scen) -- slices of one batch in flight on several streams use disjoint
 // regions -- and k_fd_central averages the two into the caller's output.
 static int launch_jacobian(GelatoPlan* p, const double* x_dev, double* out_dev, double* g_dev, int n_scen, cudaStream_t st,
-                           cudaStream_t aux, cudaEvent_t ev_fork, cudaEvent_t ev_join, const int32_t* ids_dev, bool packed,
-                           int s0 = 0) {
+                           const Lane& L, const int32_t* ids_dev, bool packed, int s0 = 0) {
   if (p->fd_mode != GELATO_FD_CENTRAL)
-    return launch_jacobian_pass(p, p->view.un.dx, x_dev, out_dev, g_dev, n_scen, st, aux, ev_fork, ev_join, ids_dev, packed);
-  if ((size_t)s0 + (size_t)n_scen > p->cap_fd) return fail(GELATO_ERR_ARG, "central-difference scratch not allocated");
+    return launch_jacobian_pass(p, p->view.un.dx, x_dev, out_dev, g_dev, n_scen, st, L, ids_dev, packed);
+  if (((size_t)s0 + (size_t)n_scen) * p->n_pack > p->d_fd.size())
+    return fail(GELATO_ERR_ARG, "central-difference scratch not allocated");
   const double h = p->fd_step;
-  double* minus = p->d_fd + (size_t)s0 * p->n_pack;
-  int rc = launch_jacobian_pass(p, h, x_dev, out_dev, g_dev, n_scen, st, aux, ev_fork, ev_join, ids_dev, packed);
+  double* minus = p->d_fd.get() + (size_t)s0 * p->n_pack;
+  int rc = launch_jacobian_pass(p, h, x_dev, out_dev, g_dev, n_scen, st, L, ids_dev, packed);
   if (rc) return rc;
-  if ((rc = launch_jacobian_pass(p, -h, x_dev, minus, nullptr, n_scen, st, aux, ev_fork, ev_join, ids_dev, true))) return rc;
+  if ((rc = launch_jacobian_pass(p, -h, x_dev, minus, nullptr, n_scen, st, L, ids_dev, true))) return rc;
   const long long n_ent = packed ? p->n_pack : (long long)p->pk_full.size();
   if (n_ent == 0) return GELATO_OK;
   const int threads = 256;
@@ -447,6 +456,19 @@ static int launch_jacobian(GelatoPlan* p, const double* x_dev, double* out_dev, 
   p->launches++;
   CU(cudaGetLastError());
   return GELATO_OK;
+}
+
+static int launch_residuals(GelatoPlan* p, const double* x_dev, double* g_dev, int n_scen, const int32_t* ids_dev,
+                            cudaStream_t st) {
+  k_residuals<<<(unsigned)p->n_res_blocks * n_scen, GR_THREADS, 0, st>>>(p->view, p->res_blocks, n_scen, ids_dev, x_dev, g_dev);
+  p->launches++;
+  CU(cudaGetLastError());
+  return GELATO_OK;
+}
+
+static void drop_graph(GelatoPlan* p) {
+  p->res_graph.reset();
+  p->res_graph_n = 0;
 }
 
 extern "C" {
@@ -468,40 +490,36 @@ int gelato_plan_create(const GelatoPlanDesc* d, int device, GelatoPlan** out) {
   if (e != cudaSuccess || ndev == 0)
     return fail(GELATO_ERR_CUDA, "no CUDA device: the B200 kernels are the only evaluation path (no CPU fallback)");
   CU(cudaSetDevice(device));
-  GelatoPlan* p = new GelatoPlan();
+  std::unique_ptr<GelatoPlan> p(new GelatoPlan());
   p->device = device;
   PlanView& v = p->view;
   planview_scalars(d, v);
   const int S = v.S;
   int rc;
-#define UP(field, src, count) if ((rc = upload(p, src, (size_t)(count), &v.field)) != GELATO_OK) { gelato_plan_destroy(p); return rc; }
-  UP(sec_i32, d->sec_i32, (size_t)S * GS_I32_COLS)
-  UP(sec_i64, d->sec_i64, (size_t)S * GS_I64_COLS)
-  UP(sec_f64, d->sec_f64, (size_t)S * GS_F64_COLS)
-  UP(d_pool, d->d_pool, d->d_pool_len)
-  UP(tau_pool, d->tau_pool, d->tau_pool_len)
-  UP(wind, d->wind, (size_t)d->n_wind * 3)
-  UP(ca, d->ca, (size_t)d->n_ca * 2)
-  UP(lin_i32, d->lin_i32, (size_t)d->n_lin * GL_I32_COLS)
-  UP(lin_f64, d->lin_f64, (size_t)d->n_lin * GL_F64_COLS)
-  UP(aero_i32, d->aero_i32, (size_t)d->n_aero * GA_I32_COLS)
-  UP(aero_i64, d->aero_i64, (size_t)d->n_aero * GA_I64_COLS)
-  UP(aero_f64, d->aero_f64, (size_t)d->n_aero * GA_F64_COLS)
-  UP(rc_aero, d->rc_aero, d->rc_aero ? (size_t)v.n_vars : 0)
-  UP(evt_i32, d->evt_i32, (size_t)d->n_evt * GE_I32_COLS)
-  UP(evt_i64, d->evt_i64, (size_t)d->n_evt * GE_I64_COLS)
-  UP(evt_f64, d->evt_f64, (size_t)d->n_evt * GE_F64_COLS)
+#define UP(dst, src, count) if ((rc = upload(p->owned, src, (size_t)(count), &(dst))) != GELATO_OK) return rc;
+  UP(v.sec_i32, d->sec_i32, (size_t)S * GS_I32_COLS)
+  UP(v.sec_i64, d->sec_i64, (size_t)S * GS_I64_COLS)
+  UP(v.sec_f64, d->sec_f64, (size_t)S * GS_F64_COLS)
+  UP(v.d_pool, d->d_pool, d->d_pool_len)
+  UP(v.tau_pool, d->tau_pool, d->tau_pool_len)
+  UP(v.wind, d->wind, (size_t)d->n_wind * 3)
+  UP(v.ca, d->ca, (size_t)d->n_ca * 2)
+  UP(v.lin_i32, d->lin_i32, (size_t)d->n_lin * GL_I32_COLS)
+  UP(v.lin_f64, d->lin_f64, (size_t)d->n_lin * GL_F64_COLS)
+  UP(v.aero_i32, d->aero_i32, (size_t)d->n_aero * GA_I32_COLS)
+  UP(v.aero_i64, d->aero_i64, (size_t)d->n_aero * GA_I64_COLS)
+  UP(v.aero_f64, d->aero_f64, (size_t)d->n_aero * GA_F64_COLS)
+  UP(v.rc_aero, d->rc_aero, d->rc_aero ? (size_t)v.n_vars : 0)
+  UP(v.evt_i32, d->evt_i32, (size_t)d->n_evt * GE_I32_COLS)
+  UP(v.evt_i64, d->evt_i64, (size_t)d->n_evt * GE_I64_COLS)
+  UP(v.evt_f64, d->evt_f64, (size_t)d->n_evt * GE_F64_COLS)
   if (d->xdep_idx && d->n_xdep > 0) {
     for (int64_t i = 0; i < d->n_xdep; i++)
-      if (d->xdep_idx[i] < 0 || d->xdep_idx[i] >= d->n_vals || (i > 0 && d->xdep_idx[i] <= d->xdep_idx[i - 1])) {
-        gelato_plan_destroy(p);
+      if (d->xdep_idx[i] < 0 || d->xdep_idx[i] >= d->n_vals || (i > 0 && d->xdep_idx[i] <= d->xdep_idx[i - 1]))
         return fail(GELATO_ERR_ARG, "xdep_idx must be strictly ascending and inside [0, n_vals)");
-      }
     p->h_xdep.assign(d->xdep_idx, d->xdep_idx + d->n_xdep);
     p->n_xdep = d->n_xdep;
-    const int64_t* dx = nullptr;
-    if ((rc = upload(p, d->xdep_idx, (size_t)d->n_xdep, &dx)) != GELATO_OK) { gelato_plan_destroy(p); return rc; }
-    p->d_xdep = dx;
+    UP(p->d_xdep, d->xdep_idx, d->n_xdep)
     // split for the zero-copy route: long runs of consecutive slots go through the copy engine (one strided
     // 2-D copy per run covers every scenario), the scattered rest is written by a kernel
     std::vector<int64_t> small;
@@ -514,18 +532,14 @@ int gelato_plan_create(const GelatoPlanDesc* d, int device, GelatoPlan** out) {
     }
     p->n_small = (long long)small.size();
     p->h_small = small;
-    if ((rc = upload(p, small.data(), small.size(), &dx)) != GELATO_OK) { gelato_plan_destroy(p); return rc; }
-    p->d_xdep_small = dx;
+    UP(p->d_xdep_small, small.data(), small.size())
   }
-  const double* tmpl = nullptr;
-  if ((rc = upload(p, d->vals_template, (size_t)d->n_vals, &tmpl)) != GELATO_OK) { gelato_plan_destroy(p); return rc; }
-  p->vals_template = const_cast<double*>(tmpl);
-#undef UP
+  UP(p->vals_template, d->vals_template, d->n_vals)
+  p->shared_template = p->vals_template;
 
   // block tables
   HostTables ht;
   build_host_tables(d, ht);
-  const int32_t* tb = nullptr;
   p->n_jac_blocks = (int)(ht.jac_blocks.size() / BT_COLS);
   p->n_res_blocks = (int)(ht.res_blocks.size() / BT_COLS);
   p->n_jac_main = ht.n_jac_main;
@@ -533,50 +547,41 @@ int gelato_plan_create(const GelatoPlanDesc* d, int device, GelatoPlan** out) {
   p->n_vac = ht.n_vac;
   p->n_jac_heavy = (int)(ht.jac_heavy.size() / BT_COLS);
   p->n_jac_light = (int)(ht.jac_light.size() / BT_COLS);
-  if ((rc = upload(p, ht.jac_heavy.data(), ht.jac_heavy.size(), &tb)) != GELATO_OK) { gelato_plan_destroy(p); return rc; }
+  const int32_t* tb = nullptr;
+  UP(tb, ht.jac_heavy.data(), ht.jac_heavy.size())
   p->jac_heavy = const_cast<int32_t*>(tb);
-  if ((rc = upload(p, ht.jac_light.data(), ht.jac_light.size(), &tb)) != GELATO_OK) { gelato_plan_destroy(p); return rc; }
+  UP(tb, ht.jac_light.data(), ht.jac_light.size())
   p->jac_light = const_cast<int32_t*>(tb);
   {
     PackedLayout L;
     build_packed_layout(d, L);
     if (d->xdep_idx && d->n_xdep > 0 &&
-        ((size_t)d->n_xdep != L.full_slot.size() || !std::equal(L.full_slot.begin(), L.full_slot.end(), d->xdep_idx))) {
-      gelato_plan_destroy(p);
+        ((size_t)d->n_xdep != L.full_slot.size() || !std::equal(L.full_slot.begin(), L.full_slot.end(), d->xdep_idx)))
       return fail(GELATO_ERR_ARG, "xdep_idx is not the set of slots the Jacobian kernel writes for this plan");
-    }
     p->n_pack = L.n_pack;
     v.n_pack = L.n_pack;
-    if ((rc = upload(p, L.sec_pk.data(), L.sec_pk.size(), &v.sec_pk)) != GELATO_OK) { gelato_plan_destroy(p); return rc; }
-    if ((rc = upload(p, L.aero_pk.data(), L.aero_pk.size(), &v.aero_pk)) != GELATO_OK) { gelato_plan_destroy(p); return rc; }
-    if ((rc = upload(p, L.evt_pk.data(), L.evt_pk.size(), &v.evt_pk)) != GELATO_OK) { gelato_plan_destroy(p); return rc; }
+    UP(v.sec_pk, L.sec_pk.data(), L.sec_pk.size())
+    UP(v.aero_pk, L.aero_pk.data(), L.aero_pk.size())
+    UP(v.evt_pk, L.evt_pk.data(), L.evt_pk.size())
     p->pk_full.swap(L.full_slot);
     p->pk_src.swap(L.src);
     p->pk_sgn.swap(L.sgn);
   }
-  if ((rc = upload(p, ht.jac_blocks.data(), ht.jac_blocks.size(), &tb)) != GELATO_OK) { gelato_plan_destroy(p); return rc; }
+  UP(tb, ht.jac_blocks.data(), ht.jac_blocks.size())
   p->jac_blocks = const_cast<int32_t*>(tb);
-  if ((rc = upload(p, ht.res_blocks.data(), ht.res_blocks.size(), &tb)) != GELATO_OK) { gelato_plan_destroy(p); return rc; }
+  UP(tb, ht.res_blocks.data(), ht.res_blocks.size())
   p->res_blocks = const_cast<int32_t*>(tb);
-  if ((rc = upload(p, ht.node_rec.data(), ht.node_rec.size(), &v.node_rec)) != GELATO_OK) { gelato_plan_destroy(p); return rc; }
-  if ((rc = upload(p, ht.jac_rec.data(), ht.jac_rec.size(), &v.jac_rec)) != GELATO_OK) { gelato_plan_destroy(p); return rc; }
-  if ((rc = upload(p, ht.aero_rows.data(), ht.aero_rows.size(), &v.aero_rows)) != GELATO_OK) { gelato_plan_destroy(p); return rc; }
+  UP(v.node_rec, ht.node_rec.data(), ht.node_rec.size())
+  UP(v.jac_rec, ht.jac_rec.data(), ht.jac_rec.size())
+  UP(v.aero_rows, ht.aero_rows.data(), ht.aero_rows.size())
+#undef UP
   v.n_aero_rows = (int)ht.aero_rows.size();
+  p->shared_view = v;
 
-  cudaError_t ce = cudaStreamCreateWithFlags(&p->stream, cudaStreamNonBlocking);
-  if (ce == cudaSuccess) ce = cudaStreamCreateWithFlags(&p->copy_stream, cudaStreamNonBlocking);
-  if (ce == cudaSuccess) ce = cudaEventCreateWithFlags(&p->ev_kernel, cudaEventDisableTiming);
-  if (ce == cudaSuccess) ce = cudaEventCreateWithFlags(&p->ev_copy, cudaEventDisableTiming);
-  if (ce == cudaSuccess) ce = cudaStreamCreateWithFlags(&p->pair_stream, cudaStreamNonBlocking);
-  if (ce == cudaSuccess) ce = cudaEventCreateWithFlags(&p->ev_fork, cudaEventDisableTiming);
-  if (ce == cudaSuccess) ce = cudaEventCreateWithFlags(&p->ev_join, cudaEventDisableTiming);
-  if (ce == cudaSuccess) ce = cudaEventCreate(&p->ev0);
-  if (ce == cudaSuccess) ce = cudaEventCreate(&p->ev1);
-  if (ce != cudaSuccess) {
-    gelato_plan_destroy(p);
-    return fail(GELATO_ERR_CUDA, std::string("stream / event creation: ") + cudaGetErrorString(ce));
-  }
-  *out = p;
+  if ((rc = add_lane(p.get()))) return rc;
+  CU(cudaEventCreate(p->ev0.out()));
+  CU(cudaEventCreate(p->ev1.out()));
+  *out = p.release();
   return GELATO_OK;
 }
 
@@ -584,98 +589,39 @@ int gelato_plan_set_scenarios(GelatoPlan* p, const GelatoScenarioDesc* sc) {
   if (!p || !sc || sc->n_scen <= 0) return fail(GELATO_ERR_ARG, "bad scenario descriptor");
   CU(cudaSetDevice(p->device));
   CU(cudaDeviceSynchronize());  // nothing in flight may still read the blocks being replaced
+  // Every call starts from the plan's own blocks, so a NULL member means the block every scenario shares.  The blocks
+  // of an earlier call are superseded as a whole.
   PlanView& v = p->view;
-  // the blocks of an earlier call are superseded as a whole
-  for (void* d : p->scen_owned) cudaFree(d);
+  v = p->shared_view;
+  p->vals_template = p->shared_template;
+  p->vals_template_sstride = 0;
   p->scen_owned.clear();
-  auto up = [&](const double* src, size_t count, const double** dst) -> int {
-    void* d = nullptr;
-    CU(cudaMalloc(&d, count * sizeof(double)));
-    p->scen_owned.push_back(d);
-    CU(cudaMemcpy(d, src, count * sizeof(double), cudaMemcpyHostToDevice));
-    *dst = static_cast<const double*>(d);
-    return GELATO_OK;
-  };
+  p->n_scen_cfg = sc->n_scen;
+  // the staging Jacobian buffer holds the constants of the PREVIOUS scenarios: have it refilled on the next call
+  p->vals_filled = 0;
+  drop_graph(p);
+  const size_t n = (size_t)sc->n_scen;
   int rc;
-  const double* dptr;
   if (sc->sec_f64) {
-    if ((rc = up(sc->sec_f64, (size_t)sc->n_scen * v.S * GS_F64_COLS, &dptr)) != GELATO_OK) return rc;
-    v.sec_f64 = dptr;
+    if ((rc = upload(p->scen_owned, sc->sec_f64, n * v.S * GS_F64_COLS, &v.sec_f64))) return rc;
     v.sec_f64_sstride = (long long)v.S * GS_F64_COLS;
   }
   if (sc->wind) {
-    if ((rc = up(sc->wind, (size_t)sc->n_scen * v.n_wind * 3, &dptr)) != GELATO_OK) return rc;
-    v.wind = dptr;
+    if ((rc = upload(p->scen_owned, sc->wind, n * v.n_wind * 3, &v.wind))) return rc;
     v.wind_sstride = (long long)v.n_wind * 3;
   }
-  if (sc->unit_mass) {
-    if ((rc = up(sc->unit_mass, (size_t)sc->n_scen, &dptr)) != GELATO_OK) return rc;
-    v.unit_mass_scen = dptr;
-  }
-  if (sc->lin_const) {
-    if ((rc = up(sc->lin_const, (size_t)sc->n_scen * v.n_lin, &dptr)) != GELATO_OK) return rc;
-    v.lin_const_scen = dptr;
-  }
+  if (sc->unit_mass && (rc = upload(p->scen_owned, sc->unit_mass, n, &v.unit_mass_scen))) return rc;
+  if (sc->lin_const && (rc = upload(p->scen_owned, sc->lin_const, n * v.n_lin, &v.lin_const_scen))) return rc;
   if (sc->vals_template) {
-    if ((rc = up(sc->vals_template, (size_t)sc->n_scen * v.n_vals, &dptr)) != GELATO_OK) return rc;
-    p->vals_template = const_cast<double*>(dptr);
+    if ((rc = upload(p->scen_owned, sc->vals_template, n * v.n_vals, &p->vals_template))) return rc;
     p->vals_template_sstride = v.n_vals;
   }
-  p->n_scen_cfg = sc->n_scen;
-  // the staging Jacobian buffer holds the constants of the PREVIOUS scenarios: have it rebuilt on the next call
-  p->cap_scen = 0;
-  p->cap_ids = 0;
-  if (p->res_graph) cudaGraphExecDestroy(p->res_graph);
-  p->res_graph = nullptr;
-  p->res_graph_n = 0;
   return GELATO_OK;
 }
 
 int gelato_plan_destroy(GelatoPlan* p) {
   if (!p) return GELATO_OK;
   cudaSetDevice(p->device);
-  if (p->res_graph) cudaGraphExecDestroy(p->res_graph);
-  if (p->h_small_out) cudaFreeHost(p->h_small_out);
-  for (void* d : p->owned) cudaFree(d);
-  for (void* d : p->scen_owned) cudaFree(d);
-  if (p->d_packed) cudaFree(p->d_packed);
-  if (p->h_packed) cudaFreeHost(p->h_packed);
-  if (p->d_px) cudaFree(p->d_px);
-  if (p->d_pg) cudaFree(p->d_pg);
-  if (p->d_pids) cudaFree(p->d_pids);
-  if (p->h_px) cudaFreeHost(p->h_px);
-  if (p->d_x) cudaFree(p->d_x);
-  if (p->d_g) cudaFree(p->d_g);
-  if (p->d_vals) cudaFree(p->d_vals);
-  if (p->h_x) cudaFreeHost(p->h_x);
-  if (p->h_out) cudaFreeHost(p->h_out);
-  if (p->d_pack) cudaFree(p->d_pack);
-  if (p->h_pack) cudaFreeHost(p->h_pack);
-  if (p->d_ids) cudaFree(p->d_ids);
-  if (p->d_vals_ids) cudaFree(p->d_vals_ids);
-  for (size_t k = 0; k < p->lanes.size(); k++) {
-    GelatoPlan::Lane& L = p->lanes[k];
-    for (cudaEvent_t e : L.chunk_ev) cudaEventDestroy(e);
-    if (k == 0) continue;  // lane 0 borrows the plan's own streams and events
-    for (cudaEvent_t e : {L.ev_kernel, L.ev_copy, L.ev_fork, L.ev_join})
-      if (e) cudaEventDestroy(e);
-    for (cudaStream_t st : {L.stream, L.copy_stream, L.pair_stream})
-      if (st) cudaStreamDestroy(st);
-  }
-  for (GelatoPlan::Lane& L : p->lanes)
-    for (cudaEvent_t e : {L.ev_h2d, L.ev_g, L.ev_gdone})
-      if (e) cudaEventDestroy(e);
-  if (p->d_iota) cudaFree(p->d_iota);
-  if (p->d_fd) cudaFree(p->d_fd);
-  if (p->ev0) cudaEventDestroy(p->ev0);
-  if (p->ev1) cudaEventDestroy(p->ev1);
-  if (p->ev_kernel) cudaEventDestroy(p->ev_kernel);
-  if (p->ev_copy) cudaEventDestroy(p->ev_copy);
-  if (p->copy_stream) cudaStreamDestroy(p->copy_stream);
-  if (p->ev_fork) cudaEventDestroy(p->ev_fork);
-  if (p->ev_join) cudaEventDestroy(p->ev_join);
-  if (p->pair_stream) cudaStreamDestroy(p->pair_stream);
-  if (p->stream) cudaStreamDestroy(p->stream);
   delete p;
   return GELATO_OK;
 }
@@ -729,37 +675,41 @@ static int check_scen(GelatoPlan* p, int n_scen) {
   return GELATO_OK;
 }
 
-int gelato_eval_residuals_dev(GelatoPlan* p, const double* x_dev, double* g_dev, int32_t n_scen, void* stream) {
+// The start of every device-pointer entry point: the batch checked, the plan's device made current, and the stream to
+// launch on (the caller's, else the plan's own).
+static int begin_dev(GelatoPlan* p, int n_scen, void* stream, cudaStream_t* st) {
   int rc = check_scen(p, n_scen);
   if (rc) return rc;
   CU(cudaSetDevice(p->device));
-  cudaStream_t st = stream ? (cudaStream_t)stream : p->stream;
-  k_residuals<<<(unsigned)p->n_res_blocks * n_scen, GR_THREADS, 0, st>>>(p->view, p->res_blocks, n_scen, nullptr, x_dev, g_dev);
-  p->launches++;
-  CU(cudaGetLastError());
+  *st = stream ? (cudaStream_t)stream : p->lanes[0].stream;
   return GELATO_OK;
 }
 
-int gelato_eval_pair_dev(GelatoPlan* p, const double* x_dev, double* g_dev, double* vals_dev, int32_t n_scen, void* stream) {
-  int rc = check_scen(p, n_scen);
+int gelato_eval_residuals_dev(GelatoPlan* p, const double* x_dev, double* g_dev, int32_t n_scen, void* stream) {
+  cudaStream_t st;
+  int rc = begin_dev(p, n_scen, stream, &st);
   if (rc) return rc;
-  CU(cudaSetDevice(p->device));
-  cudaStream_t st = stream ? (cudaStream_t)stream : p->stream;
+  return launch_residuals(p, x_dev, g_dev, n_scen, nullptr, st);
+}
+
+int gelato_eval_pair_dev(GelatoPlan* p, const double* x_dev, double* g_dev, double* vals_dev, int32_t n_scen, void* stream) {
+  cudaStream_t st;
+  int rc = begin_dev(p, n_scen, stream, &st);
+  if (rc) return rc;
   // objfunc's rows come out of the Jacobian launch: the dynamics blocks hold the right-hand side of the pristine
   // x as their centre column and subtract it from the D.X products; aero and event blocks carry one more column
   // at the pristine state; the linear rows are blocks of their own (no second pass over the physics)
   if ((rc = ensure_fd_scratch(p, n_scen))) return rc;
-  return launch_jacobian(p, x_dev, vals_dev, g_dev, n_scen, st, p->pair_stream, p->ev_fork, p->ev_join, nullptr, false);
+  return launch_jacobian(p, x_dev, vals_dev, g_dev, n_scen, st, p->lanes[0], nullptr, false);
 }
 
 int gelato_eval_pair_packed_dev(GelatoPlan* p, const double* x_dev, double* g_dev, double* packed_dev, int32_t n_scen,
                                 void* stream) {
-  int rc = check_scen(p, n_scen);
+  cudaStream_t st;
+  int rc = begin_dev(p, n_scen, stream, &st);
   if (rc) return rc;
-  CU(cudaSetDevice(p->device));
-  cudaStream_t st = stream ? (cudaStream_t)stream : p->stream;
   if ((rc = ensure_fd_scratch(p, n_scen))) return rc;
-  return launch_jacobian(p, x_dev, packed_dev, g_dev, n_scen, st, p->pair_stream, p->ev_fork, p->ev_join, nullptr, true);
+  return launch_jacobian(p, x_dev, packed_dev, g_dev, n_scen, st, p->lanes[0], nullptr, true);
 }
 
 // ONE problem sharded over GPUs (SURVEY.md 8(e)-2): the pair evaluation restricted to blocks
@@ -769,26 +719,23 @@ int gelato_eval_pair_packed_dev(GelatoPlan* p, const double* x_dev, double* g_de
 int gelato_eval_pair_packed_range_dev(GelatoPlan* p, const double* x_dev, double* g_dev, double* packed_dev, int32_t n_scen,
                                       int32_t block_first, int32_t block_count, int32_t vac_first, int32_t vac_count,
                                       void* stream) {
-  int rc = check_scen(p, n_scen);
+  cudaStream_t st;
+  int rc = begin_dev(p, n_scen, stream, &st);
   if (rc) return rc;
   if (!g_dev || !packed_dev) return fail(GELATO_ERR_ARG, "null buffer");
   if (p->fd_mode != GELATO_FD_FORWARD) return fail(GELATO_ERR_ARG, "the range evaluation supports forward differences only");
   if (block_first < 0 || block_count < 0 || block_first + block_count > p->n_jac_blocks || vac_first < 0 || vac_count < 0 ||
       vac_first + vac_count > p->n_vac)
     return fail(GELATO_ERR_ARG, "block or vacuum-node range outside the plan");
-  CU(cudaSetDevice(p->device));
-  cudaStream_t st = stream ? (cudaStream_t)stream : p->stream;
   JacRange rg;
   rg.b0 = block_first; rg.nb = block_count; rg.v0 = vac_first; rg.nv = vac_count;
-  return launch_jacobian_pass(p, p->view.un.dx, x_dev, packed_dev, g_dev, n_scen, st, p->pair_stream, p->ev_fork, p->ev_join,
-                              nullptr, true, rg);
+  return launch_jacobian_pass(p, p->view.un.dx, x_dev, packed_dev, g_dev, n_scen, st, p->lanes[0], nullptr, true, rg);
 }
 
 int gelato_fill_template(GelatoPlan* p, double* vals_dev, int32_t n_scen, void* stream) {
-  int rc = check_scen(p, n_scen);
+  cudaStream_t st;
+  int rc = begin_dev(p, n_scen, stream, &st);
   if (rc) return rc;
-  CU(cudaSetDevice(p->device));
-  cudaStream_t st = stream ? (cudaStream_t)stream : p->stream;
   if (p->vals_template_sstride) {
     CU(cudaMemcpyAsync(vals_dev, p->vals_template, (size_t)n_scen * p->view.n_vals * sizeof(double),
                        cudaMemcpyDeviceToDevice, st));
@@ -801,51 +748,59 @@ int gelato_fill_template(GelatoPlan* p, double* vals_dev, int32_t n_scen, void* 
 }
 
 int gelato_eval_jacobian_dev(GelatoPlan* p, const double* x_dev, double* vals_dev, int32_t n_scen, void* stream) {
-  int rc = check_scen(p, n_scen);
+  cudaStream_t st;
+  int rc = begin_dev(p, n_scen, stream, &st);
   if (rc) return rc;
-  CU(cudaSetDevice(p->device));
-  cudaStream_t st = stream ? (cudaStream_t)stream : p->stream;
   // the constants and D entries of vals_dev were put there once by gelato_fill_template;
   // the kernels rewrite every x-dependent slot and never touch the rest
   if ((rc = ensure_fd_scratch(p, n_scen))) return rc;
-  return launch_jacobian(p, x_dev, vals_dev, nullptr, n_scen, st, p->pair_stream, p->ev_fork, p->ev_join, nullptr, false);
+  return launch_jacobian(p, x_dev, vals_dev, nullptr, n_scen, st, p->lanes[0], nullptr, false);
 }
 
-static void drop_graphs(GelatoPlan* p) {
-  if (p->res_graph) cudaGraphExecDestroy(p->res_graph);
-  p->res_graph = nullptr;
-  p->res_graph_n = 0;
-}
-
+// x, g and ids staging of the host-buffer entry points for n_scen batch slots.  They grow together, and the captured
+// residual graph bakes in their pointers: growing them drops it.
 static int ensure_staging(GelatoPlan* p, size_t n_scen) {
-  if (n_scen <= p->cap_scen) return GELATO_OK;
-  CU(cudaSetDevice(p->device));
-  drop_graphs(p);
-  if (p->d_x) cudaFree(p->d_x);
-  if (p->d_g) cudaFree(p->d_g);
-  if (p->d_vals) cudaFree(p->d_vals);
-  if (p->h_x) cudaFreeHost(p->h_x);
-  if (p->h_out) cudaFreeHost(p->h_out);
-  if (p->d_iota) cudaFree(p->d_iota);
-  p->d_x = p->d_g = p->d_vals = p->h_x = p->h_out = nullptr;
-  p->d_iota = nullptr;
-  p->cap_scen = 0;
   const PlanView& v = p->view;
-  const size_t nout = std::max<size_t>((size_t)v.n_rows, (size_t)v.n_vals);
-  CU(cudaMalloc(&p->d_x, n_scen * v.n_vars * sizeof(double)));
-  CU(cudaMalloc(&p->d_g, n_scen * v.n_rows * sizeof(double)));
-  CU(cudaMalloc(&p->d_vals, n_scen * (size_t)v.n_vals * sizeof(double)));
-  CU(cudaMallocHost(&p->h_x, n_scen * v.n_vars * sizeof(double)));
-  CU(cudaMallocHost(&p->h_out, n_scen * nout * sizeof(double)));
-  CU(cudaMalloc(&p->d_iota, n_scen * sizeof(int32_t)));
-  std::vector<int32_t> iota(n_scen);
-  for (size_t k = 0; k < n_scen; k++) iota[k] = (int32_t)k;
-  CU(cudaMemcpy(p->d_iota, iota.data(), n_scen * sizeof(int32_t), cudaMemcpyHostToDevice));
-  p->cap_scen = n_scen;
-  // constants of the Jacobian: written once, the kernel only rewrites x-dependent slots
-  int rc = gelato_fill_template(p, p->d_vals, (int)n_scen, p->stream);
+  if (n_scen <= p->d_ids.size()) return GELATO_OK;
+  drop_graph(p);
+  CU(p->d_x.reserve(n_scen * v.n_vars));
+  CU(p->h_x.reserve(n_scen * v.n_vars));
+  CU(p->d_g.reserve(n_scen * v.n_rows));
+  CU(p->h_g.reserve(n_scen * v.n_rows));
+  CU(p->d_ids.reserve(n_scen));
+  p->ids_iota = false;
+  return GELATO_OK;
+}
+
+// The COO Jacobian staging with the constants of batch slots [0, n_scen) in place.
+static int ensure_vals(GelatoPlan* p, size_t n_scen) {
+  if (n_scen <= p->vals_filled) return GELATO_OK;
+  CU(p->d_vals.reserve(n_scen * (size_t)p->view.n_vals));
+  int rc = gelato_fill_template(p, p->d_vals.get(), (int)n_scen, p->lanes[0].stream);
   if (rc) return rc;
-  CU(cudaStreamSynchronize(p->stream));  // the other lanes' kernels write into it too
+  CU(cudaStreamSynchronize(p->lanes[0].stream));  // the other lanes' kernels write into it too
+  p->vals_filled = n_scen;
+  return GELATO_OK;
+}
+
+// The scenario ids of the batch slots in d_ids, uploaded on `st`: the caller's `ids` (each checked against the
+// configured scenarios), else 0, 1, 2 ... when `sliced` (a slice of a batch names its scenarios), else none (*out = NULL).
+static int stage_ids(GelatoPlan* p, const int32_t* ids, int n_scen, bool sliced, cudaStream_t st, const int32_t** out) {
+  *out = nullptr;
+  if (ids) {
+    for (int k = 0; k < n_scen; k++)
+      if (ids[k] < 0 || ids[k] >= p->n_scen_cfg) return fail(GELATO_ERR_ARG, "scenario id outside the configured scenarios");
+    CU(cudaMemcpyAsync(p->d_ids.get(), ids, (size_t)n_scen * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    p->ids_iota = false;
+  } else if (!sliced) {
+    return GELATO_OK;
+  } else if (!p->ids_iota) {
+    std::vector<int32_t> iota(p->d_ids.size());
+    for (size_t k = 0; k < iota.size(); k++) iota[k] = (int32_t)k;
+    CU(cudaMemcpyAsync(p->d_ids.get(), iota.data(), iota.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    p->ids_iota = true;
+  }
+  *out = p->d_ids.get();
   return GELATO_OK;
 }
 
@@ -859,91 +814,90 @@ static bool is_pinned(const void* ptr) {
   return a.type == cudaMemoryTypeHost;
 }
 
+// The source of the upload of a caller's x[n]: x itself when it is page-locked, else `stage` with a copy of it.
+static const double* host_src(const double* x, double* stage, size_t n) {
+  if (is_pinned(x)) return x;
+  memcpy(stage, x, n * sizeof(double));
+  return stage;
+}
+
+// The destination of the download of a caller's out[n] (out == NULL: none): out itself when it is page-locked, else
+// `stage`, grown as needed; land() copies it over once the download is complete.
+static int host_dst(double* out, PinnedBuf<double>& stage, size_t n, double** dst) {
+  *dst = out;
+  if (!out || is_pinned(out)) return GELATO_OK;
+  CU(stage.reserve(n));
+  *dst = stage.get();
+  return GELATO_OK;
+}
+
+static void land(double* out, const double* dst, size_t n) {
+  if (dst != out) memcpy(out, dst, n * sizeof(double));
+}
+
 static int eval_host(GelatoPlan* p, int which, const double* x, double* out, int32_t n_scen,
                      const int32_t* ids = nullptr) {
   int rc = check_scen(p, n_scen);
   if (rc) return rc;
   if (!x || !out) return fail(GELATO_ERR_ARG, "null buffer");
+  CU(cudaSetDevice(p->device));
   if ((rc = ensure_staging(p, n_scen))) return rc;
-  if (which == 1 && (rc = ensure_fd_scratch(p, n_scen))) return rc;
   const PlanView& v = p->view;
+  const Lane& L = p->lanes[0];
   const size_t nx = (size_t)n_scen * v.n_vars;
   const size_t no = (size_t)n_scen * (which == 0 ? (size_t)v.n_rows : (size_t)v.n_vals);
-  double* d_out = which == 0 ? p->d_g : p->d_vals;
-  if (ids) {  // batch slot k evaluates configured scenario ids[k]
-    for (int k = 0; k < n_scen; k++)
-      if (ids[k] < 0 || ids[k] >= p->n_scen_cfg) return fail(GELATO_ERR_ARG, "scenario id outside the configured scenarios");
-    if ((size_t)n_scen > p->cap_ids) {
-      if (p->d_ids) cudaFree(p->d_ids);
-      if (p->d_vals_ids) cudaFree(p->d_vals_ids);
-      p->d_ids = nullptr;
-      p->d_vals_ids = nullptr;
-      p->cap_ids = 0;
-      CU(cudaMalloc(&p->d_ids, (size_t)n_scen * sizeof(int32_t)));
-      CU(cudaMalloc(&p->d_vals_ids, (size_t)n_scen * v.n_vals * sizeof(double)));
-      p->cap_ids = n_scen;
-    }
-    CU(cudaMemcpyAsync(p->d_ids, ids, (size_t)n_scen * sizeof(int32_t), cudaMemcpyHostToDevice, p->stream));
-    if (which == 1) {  // constants of each slot's scenario
-      d_out = p->d_vals_ids;
-      for (int k = 0; k < n_scen; k++)
-        CU(cudaMemcpyAsync(d_out + (size_t)k * v.n_vals, p->vals_template + (size_t)ids[k] * p->vals_template_sstride,
-                           (size_t)v.n_vals * sizeof(double), cudaMemcpyDeviceToDevice, p->stream));
-    }
-  }
   // a small objfunc call (one NLP, a few scenarios) is launch-latency bound: upload + kernel + download go out as one
   // graph launch through the pinned staging buffers (GELATO_B200_NO_GRAPH=1 keeps the three separate submissions)
   static const bool use_graph = !getenv("GELATO_B200_NO_GRAPH");
   if (which == 0 && !ids && use_graph && (nx + no) * sizeof(double) <= (size_t)64 * 1024) {
-    if (p->res_graph && p->res_graph_n != n_scen) drop_graphs(p);
+    if (p->res_graph && p->res_graph_n != n_scen) drop_graph(p);
     if (!p->res_graph) {
       cudaGraph_t graph = nullptr;
-      CU(cudaStreamBeginCapture(p->stream, cudaStreamCaptureModeThreadLocal));
-      cudaMemcpyAsync(p->d_x, p->h_x, nx * sizeof(double), cudaMemcpyHostToDevice, p->stream);
-      k_residuals<<<(unsigned)p->n_res_blocks * n_scen, GR_THREADS, 0, p->stream>>>(p->view, p->res_blocks, n_scen, nullptr, p->d_x,
-                                                                                p->d_g);
-      cudaMemcpyAsync(p->h_out, p->d_g, no * sizeof(double), cudaMemcpyDeviceToHost, p->stream);
-      CU(cudaStreamEndCapture(p->stream, &graph));
-      cudaError_t ge = cudaGraphInstantiate(&p->res_graph, graph, 0);
+      CU(cudaStreamBeginCapture(L.stream, cudaStreamCaptureModeThreadLocal));
+      cudaMemcpyAsync(p->d_x.get(), p->h_x.get(), nx * sizeof(double), cudaMemcpyHostToDevice, L.stream);
+      k_residuals<<<(unsigned)p->n_res_blocks * n_scen, GR_THREADS, 0, L.stream>>>(p->view, p->res_blocks, n_scen, nullptr,
+                                                                                  p->d_x.get(), p->d_g.get());
+      cudaMemcpyAsync(p->h_g.get(), p->d_g.get(), no * sizeof(double), cudaMemcpyDeviceToHost, L.stream);
+      CU(cudaStreamEndCapture(L.stream, &graph));
+      cudaGraphExec_t exec = nullptr;
+      cudaError_t ge = cudaGraphInstantiate(&exec, graph, 0);
       cudaGraphDestroy(graph);
-      if (ge != cudaSuccess) {
-        p->res_graph = nullptr;
-        return fail(GELATO_ERR_CUDA, std::string("cudaGraphInstantiate: ") + cudaGetErrorString(ge));
-      }
+      if (ge != cudaSuccess) return fail(GELATO_ERR_CUDA, std::string("cudaGraphInstantiate: ") + cudaGetErrorString(ge));
+      p->res_graph = GraphExec(exec);
       p->res_graph_n = n_scen;
     }
-    memcpy(p->h_x, x, nx * sizeof(double));
-    CU(cudaGraphLaunch(p->res_graph, p->stream));
+    memcpy(p->h_x.get(), x, nx * sizeof(double));
+    CU(cudaGraphLaunch(p->res_graph, L.stream));
     p->launches++;
-    CU(cudaStreamSynchronize(p->stream));
-    memcpy(out, p->h_out, no * sizeof(double));
+    CU(cudaStreamSynchronize(L.stream));
+    memcpy(out, p->h_g.get(), no * sizeof(double));
     return GELATO_OK;
   }
-  const double* hx = x;
-  if (!is_pinned(x)) {
-    memcpy(p->h_x, x, nx * sizeof(double));
-    hx = p->h_x;
-  }
-  CU(cudaMemcpyAsync(p->d_x, hx, nx * sizeof(double), cudaMemcpyHostToDevice, p->stream));
-  if (!ids) {
-    if (which == 0) rc = gelato_eval_residuals_dev(p, p->d_x, p->d_g, n_scen, p->stream);
-    else rc = gelato_eval_jacobian_dev(p, p->d_x, p->d_vals, n_scen, p->stream);
-    if (rc) return rc;
-  } else {
-    if (which == 0) {
-      k_residuals<<<(unsigned)p->n_res_blocks * n_scen, GR_THREADS, 0, p->stream>>>(p->view, p->res_blocks, n_scen, p->d_ids,
-                                                                                p->d_x, p->d_g);
-      p->launches++;
-    } else if ((rc = launch_jacobian(p, p->d_x, d_out, nullptr, n_scen, p->stream, p->pair_stream, p->ev_fork, p->ev_join,
-                                     p->d_ids, false))) {
-      return rc;
+  const int32_t* d_ids = nullptr;  // batch slot k evaluates configured scenario ids[k]
+  if ((rc = stage_ids(p, ids, n_scen, false, L.stream, &d_ids))) return rc;
+  double* d_out = p->d_g.get();
+  if (which == 1) {
+    if ((rc = ensure_fd_scratch(p, n_scen))) return rc;
+    if (!ids) {
+      if ((rc = ensure_vals(p, n_scen))) return rc;
+      d_out = p->d_vals.get();
+    } else {  // constants of each slot's scenario
+      CU(p->d_vals_ids.reserve(no));
+      d_out = p->d_vals_ids.get();
+      for (int k = 0; k < n_scen; k++)
+        CU(cudaMemcpyAsync(d_out + (size_t)k * v.n_vals, p->vals_template + (size_t)ids[k] * p->vals_template_sstride,
+                           (size_t)v.n_vals * sizeof(double), cudaMemcpyDeviceToDevice, L.stream));
     }
-    CU(cudaGetLastError());
   }
-  const bool direct = is_pinned(out);
-  CU(cudaMemcpyAsync(direct ? out : p->h_out, d_out, no * sizeof(double), cudaMemcpyDeviceToHost, p->stream));
-  CU(cudaStreamSynchronize(p->stream));
-  if (!direct) memcpy(out, p->h_out, no * sizeof(double));
+  CU(cudaMemcpyAsync(p->d_x.get(), host_src(x, p->h_x.get(), nx), nx * sizeof(double), cudaMemcpyHostToDevice, L.stream));
+  if (which == 0) rc = launch_residuals(p, p->d_x.get(), d_out, n_scen, d_ids, L.stream);
+  else rc = launch_jacobian(p, p->d_x.get(), d_out, nullptr, n_scen, L.stream, L, d_ids, false);
+  if (rc) return rc;
+  double* dst;
+  if ((rc = host_dst(out, which == 0 ? p->h_g : p->h_vals, no, &dst))) return rc;
+  CU(cudaMemcpyAsync(dst, d_out, no * sizeof(double), cudaMemcpyDeviceToHost, L.stream));
+  CU(cudaStreamSynchronize(L.stream));
+  land(out, dst, no);
   return GELATO_OK;
 }
 
@@ -966,12 +920,11 @@ int gelato_eval_jacobian_ids(GelatoPlan* p, const double* x, double* vals, int32
 }
 
 int gelato_pack_xdep_dev(GelatoPlan* p, const double* vals_dev, double* packed_dev, int32_t n_scen, void* stream) {
-  int rc = check_scen(p, n_scen);
+  cudaStream_t st;
+  int rc = begin_dev(p, n_scen, stream, &st);
   if (rc) return rc;
   if (!p->d_xdep) return fail(GELATO_ERR_ARG, "the plan was created without xdep_idx");
   if (n_scen > 65535) return fail(GELATO_ERR_ARG, "n_scen > 65535 in update mode (gridDim.y)");
-  CU(cudaSetDevice(p->device));
-  cudaStream_t st = stream ? (cudaStream_t)stream : p->stream;
   const int threads = 256;
   const int bx = (int)std::min<long long>((p->n_xdep + threads - 1) / threads, 4096);
   k_pack_xdep<<<dim3(bx, n_scen), threads, 0, st>>>(vals_dev, p->d_xdep, p->n_xdep, p->view.n_vals, packed_dev);
@@ -1009,89 +962,83 @@ int gelato_set_host_threads(GelatoPlan* p, int32_t n) {
 
 using gelato_host::scatter_parallel;
 
-static int ensure_lanes(GelatoPlan* p, int n) {
-  if (p->lanes.empty()) {
-    GelatoPlan::Lane L;
-    L.stream = p->stream; L.copy_stream = p->copy_stream; L.pair_stream = p->pair_stream;
-    L.ev_kernel = p->ev_kernel; L.ev_copy = p->ev_copy; L.ev_fork = p->ev_fork; L.ev_join = p->ev_join;
-    p->lanes.push_back(L);
-  }
-  while ((int)p->lanes.size() < n) {
-    p->lanes.emplace_back();
-    GelatoPlan::Lane& L = p->lanes.back();  // registered first: gelato_plan_destroy releases whatever exists
-    for (cudaStream_t* st : {&L.stream, &L.copy_stream, &L.pair_stream}) CU(cudaStreamCreateWithFlags(st, cudaStreamNonBlocking));
-    for (cudaEvent_t* e : {&L.ev_kernel, &L.ev_copy, &L.ev_fork, &L.ev_join}) CU(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
-  }
-  for (GelatoPlan::Lane& L : p->lanes)
-    for (cudaEvent_t* e : {&L.ev_h2d, &L.ev_g, &L.ev_gdone})
-      if (!*e) CU(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
+// The slices a host-buffer call cuts its batch into, each on a lane of its own (measured: profiles/r01v_e2e.txt).
+struct Slices {
+  int n_scen, n;
+  int lo(int k) const { return (int)((long long)n_scen * k / n); }
+};
+static Slices slices_for(const GelatoPlan* p, int n_scen) {
+  const int n = p->update_slices > 0 ? p->update_slices : n_scen / 16;
+  return Slices{n_scen, std::max(1, std::min(n, std::min(n_scen, 8)))};
+}
+
+// lanes [0, n), each with n_chunks chunk events
+static int ensure_lanes(GelatoPlan* p, int n, int n_chunks) {
+  int rc;
+  while ((int)p->lanes.size() < n)
+    if ((rc = add_lane(p))) return rc;
+  for (int k = 0; k < n; k++)
+    while ((int)p->lanes[k].chunk_ev.size() < n_chunks) {
+      p->lanes[k].chunk_ev.emplace_back();
+      CU(cudaEventCreateWithFlags(p->lanes[k].chunk_ev.back().out(), cudaEventDisableTiming));
+    }
   return GELATO_OK;
+}
+
+// Slice k of a batch on lane k: after slice k-1's upload (uploads go one after the other), the slice's x goes up from
+// hx and one Jacobian evaluation of its scenarios writes out_dev (and g_dev), both offset to the slice already.
+static int launch_slice(GelatoPlan* p, const Slices& sl, int k, const double* hx, double* out_dev, double* g_dev,
+                        const int32_t* ids, bool packed) {
+  const Lane& L = p->lanes[k];
+  const int s0 = sl.lo(k), ns = sl.lo(k + 1) - s0;
+  const size_t nx = (size_t)p->view.n_vars;
+  double* const dx = p->d_x.get() + (size_t)s0 * nx;
+  if (k > 0) CU(cudaStreamWaitEvent(L.stream, p->lanes[k - 1].ev_h2d, 0));
+  CU(cudaMemcpyAsync(dx, hx + (size_t)s0 * nx, (size_t)ns * nx * sizeof(double), cudaMemcpyHostToDevice, L.stream));
+  CU(cudaEventRecord(L.ev_h2d, L.stream));
+  return launch_jacobian(p, dx, out_dev, g_dev, ns, L.stream, L, ids ? ids + s0 : nullptr, packed, s0);
 }
 
 // shared body of gelato_eval_jacobian_update / gelato_eval_pair_update; g == NULL: Jacobian only.
 // The batch is cut into slices of scenarios, each on its own lane of streams: slice k's upload and kernels
 // overlap slice k-1's device->host traffic (PCIe is full duplex), and the host threads scatter slice k-1's
 // packed slots meanwhile.  Per slice: upload x -> { residual kernel -> copy g | Jacobian kernel -> transfers }.
-static int ensure_small_out(GelatoPlan* p, size_t n_doubles) {
-  if (n_doubles <= p->cap_small_out) return GELATO_OK;
-  if (p->h_small_out) cudaFreeHost(p->h_small_out);
-  p->h_small_out = nullptr;
-  p->cap_small_out = 0;
-  CU(cudaMallocHost(&p->h_small_out, n_doubles * sizeof(double)));
-  p->cap_small_out = n_doubles;
-  return GELATO_OK;
-}
-
 static int eval_update(GelatoPlan* p, const double* x, double* g, double* vals, int32_t n_scen) {
   int rc = check_scen(p, n_scen);
   if (rc) return rc;
   if (!x || !vals) return fail(GELATO_ERR_ARG, "null buffer");
   if (!p->d_xdep) return fail(GELATO_ERR_ARG, "the plan was created without xdep_idx");
   if (n_scen > 65535) return fail(GELATO_ERR_ARG, "n_scen > 65535 in update mode (gridDim.y)");
+  CU(cudaSetDevice(p->device));
   if ((rc = ensure_staging(p, n_scen))) return rc;
+  if ((rc = ensure_vals(p, n_scen))) return rc;
   if ((rc = ensure_fd_scratch(p, n_scen))) return rc;
   const PlanView& v = p->view;
-  if ((size_t)n_scen > p->cap_pack) {
-    if (p->d_pack) cudaFree(p->d_pack);
-    if (p->h_pack) cudaFreeHost(p->h_pack);
-    p->d_pack = p->h_pack = nullptr;
-    p->cap_pack = 0;
-    CU(cudaMalloc(&p->d_pack, (size_t)n_scen * p->n_xdep * sizeof(double)));
-    CU(cudaMallocHost(&p->h_pack, (size_t)n_scen * p->n_xdep * sizeof(double)));
-    p->cap_pack = n_scen;
-  }
-  const double* hx = x;
-  if (!is_pinned(x)) {
-    memcpy(p->h_x, x, (size_t)n_scen * v.n_vars * sizeof(double));
-    hx = p->h_x;
-  }
+  CU(p->d_pack.reserve((size_t)n_scen * p->n_xdep));
+  CU(p->h_pack.reserve((size_t)n_scen * p->n_xdep));
+  const double* hx = host_src(x, p->h_x.get(), (size_t)n_scen * v.n_vars);
+  const size_t nv = (size_t)n_scen * (size_t)v.n_vals, ng = (size_t)n_scen * v.n_rows;
+  double* g_dst;
+  if ((rc = host_dst(g, p->h_g, ng, &g_dst))) return rc;
   // A small Jacobian (one NLP of a few hundred nodes) is cheaper to bring down whole than through the gather / strided
   // copies / host scatter below: the staging copy on the device always holds the complete value vector (constants
   // filled once, x-dependent slots rewritten by every launch), so one contiguous copy refreshes the caller's buffer
   // to the same bits.
-  if ((size_t)n_scen * (size_t)v.n_vals * sizeof(double) <= (size_t)512 * 1024) {
-    CU(cudaMemcpyAsync(p->d_x, hx, (size_t)n_scen * v.n_vars * sizeof(double), cudaMemcpyHostToDevice, p->stream));
-    if ((rc = launch_jacobian(p, p->d_x, p->d_vals, g ? p->d_g : nullptr, n_scen, p->stream, p->pair_stream, p->ev_fork,
-                              p->ev_join, nullptr, false)))
+  if (nv * sizeof(double) <= (size_t)512 * 1024) {
+    const Lane& L = p->lanes[0];
+    CU(cudaMemcpyAsync(p->d_x.get(), hx, (size_t)n_scen * v.n_vars * sizeof(double), cudaMemcpyHostToDevice, L.stream));
+    if ((rc = launch_jacobian(p, p->d_x.get(), p->d_vals.get(), g ? p->d_g.get() : nullptr, n_scen, L.stream, L, nullptr,
+                              false)))
       return rc;
-    const size_t nv = (size_t)n_scen * (size_t)v.n_vals, ng = (size_t)n_scen * v.n_rows;
-    const bool v_direct = is_pinned(vals), gd = g && is_pinned(g);
-    double* v_dst = vals;
-    double* g_dst = g;
-    if (!v_direct || (g && !gd)) {  // pageable: through one pinned staging block laid out [vals | g]
-      if ((rc = ensure_small_out(p, nv + ng))) return rc;
-      if (!v_direct) v_dst = p->h_small_out;
-      if (g && !gd) g_dst = p->h_small_out + nv;
-    }
-    CU(cudaMemcpyAsync(v_dst, p->d_vals, nv * sizeof(double), cudaMemcpyDeviceToHost, p->stream));
-    if (g) CU(cudaMemcpyAsync(g_dst, p->d_g, ng * sizeof(double), cudaMemcpyDeviceToHost, p->stream));
-    CU(cudaStreamSynchronize(p->stream));
-    if (v_dst != vals) memcpy(vals, v_dst, nv * sizeof(double));
-    if (g && g_dst != g) memcpy(g, g_dst, ng * sizeof(double));
+    double* v_dst;
+    if ((rc = host_dst(vals, p->h_vals, nv, &v_dst))) return rc;
+    CU(cudaMemcpyAsync(v_dst, p->d_vals.get(), nv * sizeof(double), cudaMemcpyDeviceToHost, L.stream));
+    if (g) CU(cudaMemcpyAsync(g_dst, p->d_g.get(), ng * sizeof(double), cudaMemcpyDeviceToHost, L.stream));
+    CU(cudaStreamSynchronize(L.stream));
+    land(vals, v_dst, nv);
+    if (g) land(g, g_dst, ng);
     return GELATO_OK;
   }
-  const bool g_direct = g && is_pinned(g);
-  double* const g_dst = g_direct ? g : p->h_out;
 
   // Which slots travel packed (gathered on the device, copied, scattered by the host pool) and which go
   // straight to their place: a page-locked `vals` takes the long runs of consecutive slots through the copy
@@ -1113,38 +1060,25 @@ static int eval_update(GelatoPlan* p, const double* x, double* g, double* vals, 
   int threads = p->host_threads > 0 ? p->host_threads : (int)std::min(16u, std::max(1u, std::thread::hardware_concurrency()));
   if ((long long)n_scen * n_pack < (1LL << 18)) threads = 1;
   threads = std::min(threads, (int)n_scen);
-  int n_slices = p->update_slices > 0 ? p->update_slices : n_scen / 16;  // measured: profiles/r01v_e2e.txt
-  n_slices = std::max(1, std::min(n_slices, std::min((int)n_scen, 8)));
+  const Slices sl = slices_for(p, n_scen);
   // one slice: the packed slots come down in chunks so the scatter of chunk k overlaps the copy of chunk k+1
-  const int n_chunks = (n_slices == 1 && n_scen >= 4 * threads && threads > 1) ? 4 : 1;
-  if ((rc = ensure_lanes(p, n_slices))) return rc;
-  for (int k = 0; k < n_slices; k++)
-    while ((int)p->lanes[k].chunk_ev.size() < n_chunks) {
-      cudaEvent_t e;
-      CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-      p->lanes[k].chunk_ev.push_back(e);
-    }
-  auto slice_lo = [&](int k) { return (int)((long long)n_scen * k / n_slices); };
+  const int n_chunks = (sl.n == 1 && n_scen >= 4 * threads && threads > 1) ? 4 : 1;
+  if ((rc = ensure_lanes(p, sl.n, n_chunks))) return rc;
+  const int32_t* ids;  // the slices' scenario parameter blocks
+  if ((rc = stage_ids(p, nullptr, n_scen, sl.n > 1, p->lanes[0].stream, &ids))) return rc;
   auto chunk_lo = [&](int k, int c) {
-    const int s0 = slice_lo(k), s1 = slice_lo(k + 1);
+    const int s0 = sl.lo(k), s1 = sl.lo(k + 1);
     return s0 + (int)((long long)(s1 - s0) * c / n_chunks);
   };
 
-  for (int k = 0; k < n_slices; k++) {
-    GelatoPlan::Lane& L = p->lanes[k];
-    const int s0 = slice_lo(k), ns = slice_lo(k + 1) - s0;
-    const int32_t* ids = n_slices > 1 ? p->d_iota + s0 : nullptr;  // the slice's scenario parameter blocks
-    double* const dx = p->d_x + (size_t)s0 * v.n_vars;
-    double* const dg = p->d_g + (size_t)s0 * v.n_rows;
-    double* const dvals = p->d_vals + (size_t)s0 * v.n_vals;
+  for (int k = 0; k < sl.n; k++) {
+    const Lane& L = p->lanes[k];
+    const int s0 = sl.lo(k), ns = sl.lo(k + 1) - s0;
+    double* const dg = p->d_g.get() + (size_t)s0 * v.n_rows;
+    double* const dvals = p->d_vals.get() + (size_t)s0 * v.n_vals;
     double* const hvals = vals + (size_t)s0 * v.n_vals;
-    if (k > 0) CU(cudaStreamWaitEvent(L.stream, p->lanes[k - 1].ev_h2d, 0));  // uploads one after the other
-    CU(cudaMemcpyAsync(dx, hx + (size_t)s0 * v.n_vars, (size_t)ns * v.n_vars * sizeof(double), cudaMemcpyHostToDevice, L.stream));
-    CU(cudaEventRecord(L.ev_h2d, L.stream));
     // g != NULL: pair evaluation, the residual rows come out of the same launches
-    if ((rc = launch_jacobian(p, dx, dvals, g ? dg : nullptr, ns, L.stream, L.pair_stream, L.ev_fork, L.ev_join, ids, false,
-                              s0)))
-      return rc;
+    if ((rc = launch_slice(p, sl, k, hx, dvals, g ? dg : nullptr, ids, false))) return rc;
     if (g) {  // its copy travels on the side stream, next to the Jacobian's transfers
       CU(cudaEventRecord(L.ev_g, L.stream));
       CU(cudaStreamWaitEvent(L.pair_stream, L.ev_g, 0));
@@ -1176,12 +1110,13 @@ static int eval_update(GelatoPlan* p, const double* x, double* g, double* vals, 
       if ((rc = issue_runs(L.ev_kernel))) return rc;
     } else if (n_pack > 0) {
       k_pack_xdep<<<dim3(bx, ns), gpu_threads, 0, L.stream>>>(dvals, pack_idx_dev, n_pack, v.n_vals,
-                                                             p->d_pack + (size_t)s0 * n_pack);
+                                                             p->d_pack.get() + (size_t)s0 * n_pack);
       p->launches++;
       CU(cudaGetLastError());
       for (int c = 0; c < n_chunks; c++) {
         const size_t off = (size_t)chunk_lo(k, c) * n_pack, cnt = (size_t)(chunk_lo(k, c + 1) - chunk_lo(k, c)) * n_pack;
-        CU(cudaMemcpyAsync(p->h_pack + off, p->d_pack + off, cnt * sizeof(double), cudaMemcpyDeviceToHost, L.stream));
+        CU(cudaMemcpyAsync(p->h_pack.get() + off, p->d_pack.get() + off, cnt * sizeof(double), cudaMemcpyDeviceToHost,
+                           L.stream));
         CU(cudaEventRecord(L.chunk_ev[c], L.stream));
       }
       // the packed slots cross PCIe first: the host threads scatter them while the long runs follow
@@ -1189,18 +1124,18 @@ static int eval_update(GelatoPlan* p, const double* x, double* g, double* vals, 
     }
   }
   if (!zero_copy && n_pack > 0)
-    for (int k = 0; k < n_slices; k++)
+    for (int k = 0; k < sl.n; k++)
       for (int c = 0; c < n_chunks; c++) {
         CU(cudaEventSynchronize(p->lanes[k].chunk_ev[c]));
-        scatter_parallel(pack_idx_host, n_pack, p->h_pack, vals, v.n_vals, chunk_lo(k, c), chunk_lo(k, c + 1), threads);
+        scatter_parallel(pack_idx_host, n_pack, p->h_pack.get(), vals, v.n_vals, chunk_lo(k, c), chunk_lo(k, c + 1), threads);
       }
-  for (int k = 0; k < n_slices; k++) {
-    GelatoPlan::Lane& L = p->lanes[k];
+  for (int k = 0; k < sl.n; k++) {
+    const Lane& L = p->lanes[k];
     if (direct) CU(cudaStreamWaitEvent(L.stream, L.ev_copy, 0));
     if (g) CU(cudaStreamWaitEvent(L.stream, L.ev_gdone, 0));
     CU(cudaStreamSynchronize(L.stream));
   }
-  if (g && !g_direct) memcpy(g, p->h_out, (size_t)n_scen * v.n_rows * sizeof(double));
+  if (g) land(g, g_dst, ng);
   return GELATO_OK;
 }
 
@@ -1213,71 +1148,27 @@ static int eval_packed(GelatoPlan* p, const double* x, double* g, double* packed
   if (rc) return rc;
   if (!x || !packed) return fail(GELATO_ERR_ARG, "null buffer");
   const PlanView& v = p->view;
-  if (scen_ids)
-    for (int k = 0; k < n_scen; k++)
-      if (scen_ids[k] < 0 || scen_ids[k] >= p->n_scen_cfg) return fail(GELATO_ERR_ARG, "scenario id outside the configured scenarios");
   CU(cudaSetDevice(p->device));
+  if ((rc = ensure_staging(p, n_scen))) return rc;
   if ((rc = ensure_fd_scratch(p, n_scen))) return rc;
   const size_t np = (size_t)p->n_pack;
-  if ((size_t)n_scen > p->cap_packed) {
-    if (p->d_packed) cudaFree(p->d_packed);
-    if (p->h_packed) cudaFreeHost(p->h_packed);
-    p->d_packed = p->h_packed = nullptr;
-    p->cap_packed = 0;
-    CU(cudaMalloc(&p->d_packed, (size_t)n_scen * np * sizeof(double)));
-    CU(cudaMallocHost(&p->h_packed, (size_t)n_scen * np * sizeof(double)));
-    p->cap_packed = n_scen;
-  }
-  // device x / g / ids: shared with the COO entry points when those were used, else allocated here
-  if ((size_t)n_scen > p->cap_px) {
-    for (void* d : {(void*)p->d_px, (void*)p->d_pg, (void*)p->d_pids}) if (d) cudaFree(d);
-    if (p->h_px) cudaFreeHost(p->h_px);
-    p->d_px = p->d_pg = nullptr; p->d_pids = nullptr; p->h_px = nullptr;
-    p->cap_px = 0;
-    CU(cudaMalloc(&p->d_px, (size_t)n_scen * v.n_vars * sizeof(double)));
-    CU(cudaMalloc(&p->d_pg, (size_t)n_scen * v.n_rows * sizeof(double)));
-    CU(cudaMalloc(&p->d_pids, (size_t)n_scen * sizeof(int32_t)));
-    CU(cudaMallocHost(&p->h_px, (size_t)n_scen * ((size_t)v.n_vars + (size_t)v.n_rows) * sizeof(double)));
-    p->cap_px = n_scen;
-    p->pids_iota = false;
-  }
-  const double* hx = x;
-  if (!is_pinned(x)) {
-    memcpy(p->h_px, x, (size_t)n_scen * v.n_vars * sizeof(double));
-    hx = p->h_px;
-  }
-  double* const h_g_stage = p->h_px + (size_t)n_scen * v.n_vars;
-  const bool g_direct = g && is_pinned(g), pk_direct = is_pinned(packed);
-  double* const g_dst = g_direct ? g : h_g_stage;
-  double* const pk_dst = pk_direct ? packed : p->h_packed;
-
-  int n_slices = p->update_slices > 0 ? p->update_slices : n_scen / 16;
-  n_slices = std::max(1, std::min(n_slices, std::min((int)n_scen, 8)));
-  if ((rc = ensure_lanes(p, n_slices))) return rc;
-  // scenario ids of the batch slots: the caller's subset, or 0, 1, 2 ... when the batch is cut into slices
-  const bool need_ids = scen_ids || n_slices > 1;
-  if (scen_ids) {
-    CU(cudaMemcpyAsync(p->d_pids, scen_ids, (size_t)n_scen * sizeof(int32_t), cudaMemcpyHostToDevice, p->lanes[0].stream));
-    p->pids_iota = false;
-  } else if (need_ids && !p->pids_iota) {
-    std::vector<int32_t> iota(p->cap_px);
-    for (size_t k = 0; k < iota.size(); k++) iota[k] = (int32_t)k;
-    CU(cudaMemcpy(p->d_pids, iota.data(), iota.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
-    p->pids_iota = true;
-  }
-  auto slice_lo = [&](int k) { return (int)((long long)n_scen * k / n_slices); };
-  for (int k = 0; k < n_slices; k++) {
-    GelatoPlan::Lane& L = p->lanes[k];
-    const int s0 = slice_lo(k), ns = slice_lo(k + 1) - s0;
-    double* const dx = p->d_px + (size_t)s0 * v.n_vars;
-    double* const dg = p->d_pg + (size_t)s0 * v.n_rows;
-    double* const dpk = p->d_packed + (size_t)s0 * np;
-    if (k > 0) CU(cudaStreamWaitEvent(L.stream, p->lanes[k - 1].ev_h2d, 0));  // uploads one after the other (and after the ids)
-    CU(cudaMemcpyAsync(dx, hx + (size_t)s0 * v.n_vars, (size_t)ns * v.n_vars * sizeof(double), cudaMemcpyHostToDevice, L.stream));
-    CU(cudaEventRecord(L.ev_h2d, L.stream));
-    if ((rc = launch_jacobian(p, dx, dpk, g ? dg : nullptr, ns, L.stream, L.pair_stream, L.ev_fork, L.ev_join,
-                              need_ids ? p->d_pids + s0 : nullptr, true, s0)))
-      return rc;
+  CU(p->d_packed.reserve((size_t)n_scen * np));
+  const Slices sl = slices_for(p, n_scen);
+  if ((rc = ensure_lanes(p, sl.n, 0))) return rc;
+  // scenario ids of the batch slots: the caller's subset, or 0, 1, 2 ... when the batch is cut into slices; the first
+  // upload waits for them
+  const int32_t* ids;
+  if ((rc = stage_ids(p, scen_ids, n_scen, sl.n > 1, p->lanes[0].stream, &ids))) return rc;
+  const double* hx = host_src(x, p->h_x.get(), (size_t)n_scen * v.n_vars);
+  double *g_dst, *pk_dst;
+  if ((rc = host_dst(g, p->h_g, (size_t)n_scen * v.n_rows, &g_dst))) return rc;
+  if ((rc = host_dst(packed, p->h_packed, (size_t)n_scen * np, &pk_dst))) return rc;
+  for (int k = 0; k < sl.n; k++) {
+    const Lane& L = p->lanes[k];
+    const int s0 = sl.lo(k), ns = sl.lo(k + 1) - s0;
+    double* const dg = p->d_g.get() + (size_t)s0 * v.n_rows;
+    double* const dpk = p->d_packed.get() + (size_t)s0 * np;
+    if ((rc = launch_slice(p, sl, k, hx, dpk, g ? dg : nullptr, ids, true))) return rc;
     // both results on the lane's copy stream, after everything of the slice has been computed
     CU(cudaEventRecord(L.ev_kernel, L.stream));
     CU(cudaStreamWaitEvent(L.copy_stream, L.ev_kernel, 0));
@@ -1287,9 +1178,9 @@ static int eval_packed(GelatoPlan* p, const double* x, double* g, double* packed
     CU(cudaMemcpyAsync(pk_dst + (size_t)s0 * np, dpk, (size_t)ns * np * sizeof(double), cudaMemcpyDeviceToHost, L.copy_stream));
     CU(cudaEventRecord(L.ev_copy, L.copy_stream));
   }
-  for (int k = 0; k < n_slices; k++) CU(cudaEventSynchronize(p->lanes[k].ev_copy));
-  if (g && !g_direct) memcpy(g, h_g_stage, (size_t)n_scen * v.n_rows * sizeof(double));
-  if (!pk_direct) memcpy(packed, p->h_packed, (size_t)n_scen * np * sizeof(double));
+  for (int k = 0; k < sl.n; k++) CU(cudaEventSynchronize(p->lanes[k].ev_copy));
+  if (g) land(g, g_dst, (size_t)n_scen * v.n_rows);
+  land(packed, pk_dst, (size_t)n_scen * np);
   return GELATO_OK;
 }
 
@@ -1341,8 +1232,10 @@ int gelato_probe_update(GelatoPlan* p, double* vals, int32_t n_scen, int reps, f
   int rc = check_scen(p, n_scen);
   if (rc) return rc;
   if (!vals || !out_ms || reps <= 0 || !is_pinned(vals)) return fail(GELATO_ERR_ARG, "page-locked vals required");
-  if (!p->d_xdep || (size_t)n_scen > p->cap_pack) return fail(GELATO_ERR_ARG, "call gelato_eval_jacobian_update first");
+  if (!p->d_xdep || (size_t)n_scen * p->n_xdep > p->d_pack.size())
+    return fail(GELATO_ERR_ARG, "call gelato_eval_jacobian_update first");
   const PlanView& v = p->view;
+  const Lane& L = p->lanes[0];
   double* dev_view = nullptr;
   CU(cudaHostGetDevicePointer((void**)&dev_view, vals, 0));
   const size_t pitch = (size_t)v.n_vals * sizeof(double);
@@ -1350,32 +1243,36 @@ int gelato_probe_update(GelatoPlan* p, double* vals, int32_t n_scen, int reps, f
   const int bx = (int)std::min<long long>((p->n_small + threads - 1) / threads, 4096);
   auto copies = [&]() {
     for (const auto& run : p->big_runs)
-      cudaMemcpy2DAsync(vals + run.first, pitch, p->d_vals + run.first, pitch, (size_t)run.second * sizeof(double),
-                        (size_t)n_scen, cudaMemcpyDeviceToHost, p->copy_stream);
+      cudaMemcpy2DAsync(vals + run.first, pitch, p->d_vals.get() + run.first, pitch, (size_t)run.second * sizeof(double),
+                        (size_t)n_scen, cudaMemcpyDeviceToHost, L.copy_stream);
   };
   auto zero_copy = [&]() {
     if (p->n_small > 0)
-      k_scatter_xdep_host<<<dim3(bx, n_scen), threads, 0, p->stream>>>(p->d_vals, p->d_xdep_small, p->n_small, v.n_vals, dev_view);
+      k_scatter_xdep_host<<<dim3(bx, n_scen), threads, 0, L.stream>>>(p->d_vals.get(), p->d_xdep_small, p->n_small, v.n_vals,
+                                                                       dev_view);
   };
   for (int piece = 0; piece < 6; piece++) {
     CU(cudaDeviceSynchronize());
-    CU(cudaEventRecord(p->ev0, p->stream));
-    CU(cudaStreamWaitEvent(p->copy_stream, p->ev0, 0));
+    CU(cudaEventRecord(p->ev0, L.stream));
+    CU(cudaStreamWaitEvent(L.copy_stream, p->ev0, 0));
     for (int r = 0; r < reps; r++) {
       if (piece == 0 || piece == 2) copies();
       if (piece == 1 || piece == 2) zero_copy();
       if (piece == 3 && p->n_small > 0) {
-        k_pack_xdep<<<dim3(bx, n_scen), threads, 0, p->stream>>>(p->d_vals, p->d_xdep_small, p->n_small, v.n_vals, p->d_pack);
-        cudaMemcpyAsync(p->h_pack, p->d_pack, (size_t)n_scen * p->n_small * sizeof(double), cudaMemcpyDeviceToHost, p->stream);
+        k_pack_xdep<<<dim3(bx, n_scen), threads, 0, L.stream>>>(p->d_vals.get(), p->d_xdep_small, p->n_small, v.n_vals,
+                                                               p->d_pack.get());
+        cudaMemcpyAsync(p->h_pack.get(), p->d_pack.get(), (size_t)n_scen * p->n_small * sizeof(double), cudaMemcpyDeviceToHost,
+                        L.stream);
       }
       if (piece == 4)
-        cudaMemcpyAsync(p->h_pack, p->d_pack, (size_t)n_scen * p->n_xdep * sizeof(double), cudaMemcpyDeviceToHost, p->stream);
+        cudaMemcpyAsync(p->h_pack.get(), p->d_pack.get(), (size_t)n_scen * p->n_xdep * sizeof(double), cudaMemcpyDeviceToHost,
+                        L.stream);
       if (piece == 5)
-        cudaMemcpyAsync(p->h_out, p->d_g, (size_t)n_scen * v.n_rows * sizeof(double), cudaMemcpyDeviceToHost, p->stream);
+        cudaMemcpyAsync(p->h_g.get(), p->d_g.get(), (size_t)n_scen * v.n_rows * sizeof(double), cudaMemcpyDeviceToHost, L.stream);
     }
-    CU(cudaEventRecord(p->ev_copy, p->copy_stream));
-    CU(cudaStreamWaitEvent(p->stream, p->ev_copy, 0));
-    CU(cudaEventRecord(p->ev1, p->stream));
+    CU(cudaEventRecord(L.ev_copy, L.copy_stream));
+    CU(cudaStreamWaitEvent(L.stream, L.ev_copy, 0));
+    CU(cudaEventRecord(p->ev1, L.stream));
     CU(cudaEventSynchronize(p->ev1));
     CU(cudaGetLastError());
     float ms = 0.f;
@@ -1402,17 +1299,15 @@ int gelato_host_free(void* ptr) {
 // CUDA events.
 int gelato_launch_kernel_dev(GelatoPlan* p, int which, const double* x_dev, double* out_dev, double* g_dev, int32_t n_scen,
                              int32_t packed, void* stream) {
-  int rc = check_scen(p, n_scen);
+  cudaStream_t st;
+  int rc = begin_dev(p, n_scen, stream, &st);
   if (rc) return rc;
-  CU(cudaSetDevice(p->device));
-  cudaStream_t st = stream ? (cudaStream_t)stream : p->stream;
   PlanView v = p->view;
   v.packed = packed ? 1 : 0;
   if (which == 0) {
     k_residuals<<<(unsigned)p->n_res_blocks * n_scen, GR_THREADS, 0, st>>>(v, p->res_blocks, n_scen, nullptr, x_dev, out_dev);
   } else if (which == 1) {
-    return launch_jacobian_pass(p, p->view.un.dx, x_dev, out_dev, g_dev, n_scen, st, p->pair_stream, p->ev_fork, p->ev_join,
-                                nullptr, packed != 0);
+    return launch_jacobian_pass(p, p->view.un.dx, x_dev, out_dev, g_dev, n_scen, st, p->lanes[0], nullptr, packed != 0);
   } else if (which == 2) {
     if (p->n_jac_heavy == 0) return fail(GELATO_ERR_ARG, "the plan has no heavy blocks");
     k_jacobian_heavy<<<(unsigned)p->n_jac_heavy * n_scen, GJ_THREADS, 0, st>>>(v, p->jac_heavy, n_scen, nullptr, x_dev, out_dev, g_dev);
@@ -1441,28 +1336,28 @@ int gelato_time_kernel(GelatoPlan* p, int which, const double* x_dev, double* ou
   if (rc) return rc;
   if (reps <= 0 || !avg_ms) return fail(GELATO_ERR_ARG, "bad reps");
   CU(cudaSetDevice(p->device));
-  CU(cudaStreamSynchronize(p->stream));
-  CU(cudaEventRecord(p->ev0, p->stream));
+  const Lane& L = p->lanes[0];
+  CU(cudaStreamSynchronize(L.stream));
+  CU(cudaEventRecord(p->ev0, L.stream));
   for (int i = 0; i < reps; i++) {
     if (which == 0) {
-      k_residuals<<<(unsigned)p->n_res_blocks * n_scen, GR_THREADS, 0, p->stream>>>(p->view, p->res_blocks, n_scen, nullptr, x_dev, out_dev);
+      k_residuals<<<(unsigned)p->n_res_blocks * n_scen, GR_THREADS, 0, L.stream>>>(p->view, p->res_blocks, n_scen, nullptr, x_dev, out_dev);
     } else if (which == 1) {  // the whole Jacobian evaluation (heavy and light kernels)
-      if ((rc = launch_jacobian_pass(p, p->view.un.dx, x_dev, out_dev, nullptr, n_scen, p->stream, p->pair_stream, p->ev_fork,
-                                     p->ev_join, nullptr, false)))
+      if ((rc = launch_jacobian_pass(p, p->view.un.dx, x_dev, out_dev, nullptr, n_scen, L.stream, L, nullptr, false)))
         return rc;
       continue;
     } else if (which == 2) {  // the heavy roles' blocks alone (air dynamics + aero rows)
       if (p->n_jac_heavy > 0)
-        k_jacobian_heavy<<<(unsigned)p->n_jac_heavy * n_scen, GJ_THREADS, 0, p->stream>>>(p->view, p->jac_heavy, n_scen, nullptr,
+        k_jacobian_heavy<<<(unsigned)p->n_jac_heavy * n_scen, GJ_THREADS, 0, L.stream>>>(p->view, p->jac_heavy, n_scen, nullptr,
                                                                                         x_dev, out_dev, nullptr);
     } else {  // the light roles' blocks alone
       if (p->n_jac_light > 0)
-        k_jacobian_light<<<(unsigned)p->n_jac_light * n_scen, GJ_THREADS, 0, p->stream>>>(p->view, p->jac_light, n_scen, nullptr,
+        k_jacobian_light<<<(unsigned)p->n_jac_light * n_scen, GJ_THREADS, 0, L.stream>>>(p->view, p->jac_light, n_scen, nullptr,
                                                                                         x_dev, out_dev, nullptr);
     }
     p->launches++;
   }
-  CU(cudaEventRecord(p->ev1, p->stream));
+  CU(cudaEventRecord(p->ev1, L.stream));
   CU(cudaEventSynchronize(p->ev1));
   CU(cudaGetLastError());
   float ms = 0.f;
@@ -1474,12 +1369,11 @@ int gelato_time_kernel(GelatoPlan* p, int which, const double* x_dev, double* ou
 int gelato_selftest_unfused(int device, int* ok) {
   if (!ok) return fail(GELATO_ERR_ARG, "null");
   CU(cudaSetDevice(device));
-  double* d = nullptr;
-  CU(cudaMalloc(&d, sizeof(double)));
-  k_unfused_probe<<<1, 1>>>(1.0 + 0x1p-30, 1.0 - 0x1p-30, -1.0, d);
+  DeviceBuf<double> d;
+  CU(d.reserve(1));
+  k_unfused_probe<<<1, 1>>>(1.0 + 0x1p-30, 1.0 - 0x1p-30, -1.0, d.get());
   double h = 1.0;
-  CU(cudaMemcpy(&h, d, sizeof(double), cudaMemcpyDeviceToHost));
-  cudaFree(d);
+  CU(cudaMemcpy(&h, d.get(), sizeof(double), cudaMemcpyDeviceToHost));
   *ok = (h == 0.0);
   return GELATO_OK;
 }
@@ -1489,11 +1383,12 @@ int gelato_fp64_peak(int device, double* tflops_fma, double* tflops_nofma) {
   cudaDeviceProp prop;
   CU(cudaGetDeviceProperties(&prop, device));
   const int blocks = prop.multiProcessorCount * 8, threads = 256, iters = 1 << 14;
-  double* d = nullptr;
-  CU(cudaMalloc(&d, (size_t)blocks * threads * sizeof(double)));
-  cudaEvent_t e0, e1;
-  CU(cudaEventCreate(&e0));
-  CU(cudaEventCreate(&e1));
+  DeviceBuf<double> buf;
+  CU(buf.reserve((size_t)blocks * threads));
+  double* const d = buf.get();
+  Event e0, e1;
+  CU(cudaEventCreate(e0.out()));
+  CU(cudaEventCreate(e1.out()));
   float ms;
   for (int pass = 0; pass < 2; pass++) {
     k_fp64_fma<<<blocks, threads>>>(d, iters);  // warm-up on pass 0
@@ -1513,9 +1408,6 @@ int gelato_fp64_peak(int device, double* tflops_fma, double* tflops_nofma) {
     CU(cudaEventElapsedTime(&ms, e0, e1));
     if (tflops_nofma) *tflops_nofma = 2.0 * 8.0 * iters * (double)blocks * threads / (ms * 1e-3) / 1e12;
   }
-  cudaEventDestroy(e0);
-  cudaEventDestroy(e1);
-  cudaFree(d);
   return GELATO_OK;
 }
 
