@@ -56,6 +56,7 @@ class GelatoProblem:
         self.fuse_pair = bool(fuse_pair) and self.reuse_output and hasattr(self.engine, "eval_pair_update")
         self._x_pair = None  # the decision vector the kept Jacobian belongs to
         self._pair_fresh = False
+        self._mesh_grid = False
 
     # -- helpers ---------------------------------------------------------
     def pack(self, xdict):
@@ -133,6 +134,18 @@ class GelatoProblem:
         vals = self.engine.eval_jacobian(self.pack(xdict))
         data = np.append(vals, 0.0)[m["src"]]
         return sp.csr_matrix((data, m["indices"], m["indptr"]), shape=m["shape"])
+
+    def mesh_error(self, xdict):
+        """{event name: err[11]}: the collocation error estimate of each section between its nodes, per state component
+        (mass | position 3 | velocity 3 | quaternion 4), on the default test grid (n + 1 points, set on first use).
+        gelato_b200.mesh.refine_nodes takes the result as it is (DESIGN.md section 11)."""
+        if not self._mesh_grid:
+            from . import mesh
+
+            self.engine.set_mesh_grid(mesh.grid_tables(self.plan.ps))
+            self._mesh_grid = True
+        err = self.engine.mesh_error(self.pack(xdict))
+        return {prm["name"]: err[i] for i, prm in enumerate(self.plan.p["params"][: self.plan.S])}
 
     # -- flat-vector variants (no dictionaries), used by benchmarks / batched drivers
     def residuals(self, x, n_scen=1):

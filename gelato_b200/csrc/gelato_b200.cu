@@ -12,6 +12,7 @@
 // gelato_selftest_unfused() verifies the flag at run time).
 #include <cuda_runtime.h>
 
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -23,6 +24,7 @@
 
 #include "cuda_owned.h"
 #include "host_pool.h"
+#include "mesh_error.h"
 #include "plan_host.h"
 
 // ---------------------------------------------------------------------------
@@ -222,6 +224,36 @@ __global__ void k_fd_central(double* __restrict__ out_all, long long out_stride,
   }
 }
 
+// Mesh error estimate (mesh_error.h; DESIGN.md section 11), two launches.  First one thread per (scenario, test point):
+// the interpolated state and the right-hand side there, MESH_PT doubles per point into pts[n_scen][n_pts][MESH_PT].
+// Then one thread per (scenario, section, state component): the integral and the two maxima, err[n_scen][S][11].
+#define GM_THREADS 128
+__global__ void __launch_bounds__(GM_THREADS)
+k_mesh_points(const __grid_constant__ PlanView P, const MeshPt* __restrict__ pt, const MeshSec* __restrict__ ms,
+              const double* __restrict__ pool, int n_pts, int n_scen, const double* __restrict__ x_all,
+              double* __restrict__ pts_all) {
+  const long long i = (long long)blockIdx.x * GM_THREADS + threadIdx.x;
+  if (i >= (long long)n_pts * n_scen) return;
+  const int scen = (int)(i / n_pts), k = (int)(i - (long long)scen * n_pts);
+  const MeshPt q = pt[k];
+  const MeshTabs tb = mesh_tabs(pool, ms[q.sec], P.sec_i32[q.sec * GS_I32_COLS + GS_N]);
+  double* out = pts_all + (size_t)i * MESH_PT;
+  mesh_point(P, scen, x_all + (size_t)scen * P.n_vars, q.sec, tb, q.l, out, out + MESH_STATE);
+}
+__global__ void __launch_bounds__(GM_THREADS)
+k_mesh_error(const __grid_constant__ PlanView P, const MeshSec* __restrict__ ms, const double* __restrict__ pool, int n_pts,
+             int n_scen, const double* __restrict__ x_all, const double* __restrict__ pts_all, double* __restrict__ err_all) {
+  const long long i = (long long)blockIdx.x * GM_THREADS + threadIdx.x;
+  const int per = P.S * MESH_STATE;
+  if (i >= (long long)per * n_scen) return;
+  const int scen = (int)(i / per), r = (int)(i - (long long)scen * per);
+  const int sec = r / MESH_STATE, c = r - sec * MESH_STATE;
+  const MeshSec s = ms[sec];
+  const MeshTabs tb = mesh_tabs(pool, s, P.sec_i32[sec * GS_I32_COLS + GS_N]);
+  const double* pts = pts_all + ((size_t)scen * n_pts + s.pt0) * MESH_PT;
+  err_all[i] = mesh_component(P, x_all + (size_t)scen * P.n_vars, sec, tb, s.m, pts, c);
+}
+
 // probe: is a*b+c left unfused?  (1 + 2^-30)(1 - 2^-30) - 1 is 0 unfused, -2^-60 fused
 __global__ void k_unfused_probe(double a, double b, double c, double* out) { *out = a * b + c; }
 
@@ -340,6 +372,14 @@ struct GelatoPlan {
   DeviceBuf<double> d_fd;
   const int64_t *d_pk_full = nullptr, *d_pk_src = nullptr;  // the packed map on the device (uploaded on first use)
   const double* d_pk_sgn = nullptr;
+  // mesh error estimate (gelato_plan_set_mesh_grid): the grid's sections, test points and table pool on the device,
+  // n_mesh_pts = 0 until a grid is set; d_mesh_pts is the per-point scratch, d_err / h_err the host entry's staging
+  std::vector<int32_t> sec_n;  // LGR nodes of each section
+  DeviceBuf<MeshSec> d_mesh_sec;
+  DeviceBuf<MeshPt> d_mesh_pt;
+  DeviceBuf<double> d_mesh_pool, d_mesh_pts, d_err;
+  PinnedBuf<double> h_err;
+  int n_mesh_pts = 0;
   long long launches = 0;
   Event ev0, ev1;
 };
@@ -497,6 +537,7 @@ int gelato_plan_create(const GelatoPlanDesc* d, int device, GelatoPlan** out) {
   const int S = v.S;
   int rc;
 #define UP(dst, src, count) if ((rc = upload(p->owned, src, (size_t)(count), &(dst))) != GELATO_OK) return rc;
+  for (int i = 0; i < S; i++) p->sec_n.push_back(d->sec_i32[i * GS_I32_COLS + GS_N]);
   UP(v.sec_i32, d->sec_i32, (size_t)S * GS_I32_COLS)
   UP(v.sec_i64, d->sec_i64, (size_t)S * GS_I64_COLS)
   UP(v.sec_f64, d->sec_f64, (size_t)S * GS_F64_COLS)
@@ -917,6 +958,83 @@ int gelato_eval_residuals_ids(GelatoPlan* p, const double* x, double* g, int32_t
 int gelato_eval_jacobian_ids(GelatoPlan* p, const double* x, double* vals, int32_t n_scen, const int32_t* scen_ids) {
   if (!scen_ids) return fail(GELATO_ERR_ARG, "null scen_ids");
   return eval_host(p, 1, x, vals, n_scen, scen_ids);
+}
+
+// ---- mesh error estimate (mesh_error.h) ----
+int gelato_plan_set_mesh_grid(GelatoPlan* p, const GelatoMeshGridDesc* g) {
+  if (!p || !g || !g->m || !g->off || !g->pool) return fail(GELATO_ERR_ARG, "null argument");
+  const int S = p->view.S;
+  std::vector<MeshSec> secs(S);
+  std::vector<MeshPt> pts;
+  for (int i = 0; i < S; i++) {
+    const long long m = g->m[i], n = p->sec_n[i], off = g->off[i];
+    if (m < 1) return fail(GELATO_ERR_ARG, "every section needs at least one test point");
+    if (off < 0 || off > g->pool_len || m > (g->pool_len - off) / (m + 2 * n + 2))
+      return fail(GELATO_ERR_ARG, "a section's tables lie outside the pool");
+    if ((long long)pts.size() + m > 0x7fffffffLL / MESH_PT) return fail(GELATO_ERR_ARG, "too many test points");
+    secs[i].m = (int32_t)m;
+    secs[i].pt0 = (int32_t)pts.size();
+    secs[i].off = off;
+    for (int l = 0; l < m; l++) pts.push_back(MeshPt{i, l});
+  }
+  for (int64_t k = 0; k < g->pool_len; k++)
+    if (!std::isfinite(g->pool[k])) return fail(GELATO_ERR_ARG, "the table pool holds a value that is not finite");
+  CU(cudaSetDevice(p->device));
+  CU(cudaDeviceSynchronize());  // nothing in flight may still read the grid being replaced
+  CU(p->d_mesh_sec.reserve(secs.size()));
+  CU(p->d_mesh_pt.reserve(pts.size()));
+  CU(p->d_mesh_pool.reserve((size_t)g->pool_len));
+  const cudaStream_t st = p->lanes[0].stream;
+  CU(cudaMemcpyAsync(p->d_mesh_sec.get(), secs.data(), secs.size() * sizeof(MeshSec), cudaMemcpyHostToDevice, st));
+  CU(cudaMemcpyAsync(p->d_mesh_pt.get(), pts.data(), pts.size() * sizeof(MeshPt), cudaMemcpyHostToDevice, st));
+  CU(cudaMemcpyAsync(p->d_mesh_pool.get(), g->pool, (size_t)g->pool_len * sizeof(double), cudaMemcpyHostToDevice, st));
+  CU(cudaStreamSynchronize(st));
+  p->n_mesh_pts = (int)pts.size();
+  return GELATO_OK;
+}
+
+// The two launches of one estimate on `st`; the point scratch grows to the batch (DeviceBuf::reserve synchronises).
+static int launch_mesh_error(GelatoPlan* p, const double* x_dev, double* err_dev, int n_scen, cudaStream_t st) {
+  const long long n1 = (long long)n_scen * p->n_mesh_pts, n2 = (long long)n_scen * p->view.S * MESH_STATE;
+  if ((std::max(n1, n2) + GM_THREADS - 1) / GM_THREADS > 0x7fffffffLL)
+    return fail(GELATO_ERR_ARG, "test points x n_scen exceeds the grid limit");
+  CU(p->d_mesh_pts.reserve((size_t)n1 * MESH_PT));
+  k_mesh_points<<<(unsigned)((n1 + GM_THREADS - 1) / GM_THREADS), GM_THREADS, 0, st>>>(
+      p->view, p->d_mesh_pt.get(), p->d_mesh_sec.get(), p->d_mesh_pool.get(), p->n_mesh_pts, n_scen, x_dev, p->d_mesh_pts.get());
+  k_mesh_error<<<(unsigned)((n2 + GM_THREADS - 1) / GM_THREADS), GM_THREADS, 0, st>>>(
+      p->view, p->d_mesh_sec.get(), p->d_mesh_pool.get(), p->n_mesh_pts, n_scen, x_dev, p->d_mesh_pts.get(), err_dev);
+  p->launches += 2;
+  CU(cudaGetLastError());
+  return GELATO_OK;
+}
+
+int gelato_eval_mesh_error_dev(GelatoPlan* p, const double* x_dev, double* err_dev, int32_t n_scen, void* stream) {
+  cudaStream_t st;
+  int rc = begin_dev(p, n_scen, stream, &st);
+  if (rc) return rc;
+  if (!p->n_mesh_pts) return fail(GELATO_ERR_ARG, "no mesh grid set (gelato_plan_set_mesh_grid)");
+  if (!x_dev || !err_dev) return fail(GELATO_ERR_ARG, "null buffer");
+  return launch_mesh_error(p, x_dev, err_dev, n_scen, st);
+}
+
+int gelato_eval_mesh_error(GelatoPlan* p, const double* x, double* err, int32_t n_scen) {
+  int rc = check_scen(p, n_scen);
+  if (rc) return rc;
+  if (!p->n_mesh_pts) return fail(GELATO_ERR_ARG, "no mesh grid set (gelato_plan_set_mesh_grid)");
+  if (!x || !err) return fail(GELATO_ERR_ARG, "null buffer");
+  CU(cudaSetDevice(p->device));
+  if ((rc = ensure_staging(p, n_scen))) return rc;
+  const cudaStream_t st = p->lanes[0].stream;
+  const size_t nx = (size_t)n_scen * p->view.n_vars, ne = (size_t)n_scen * p->view.S * MESH_STATE;
+  CU(p->d_err.reserve(ne));
+  CU(cudaMemcpyAsync(p->d_x.get(), host_src(x, p->h_x.get(), nx), nx * sizeof(double), cudaMemcpyHostToDevice, st));
+  if ((rc = launch_mesh_error(p, p->d_x.get(), p->d_err.get(), n_scen, st))) return rc;
+  double* dst;
+  if ((rc = host_dst(err, p->h_err, ne, &dst))) return rc;
+  CU(cudaMemcpyAsync(dst, p->d_err.get(), ne * sizeof(double), cudaMemcpyDeviceToHost, st));
+  CU(cudaStreamSynchronize(st));
+  land(err, dst, ne);
+  return GELATO_OK;
 }
 
 int gelato_pack_xdep_dev(GelatoPlan* p, const double* vals_dev, double* packed_dev, int32_t n_scen, void* stream) {

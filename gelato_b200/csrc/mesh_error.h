@@ -1,0 +1,115 @@
+/* mesh_error.h -- the integral-form collocation error estimate of each section (Patterson, Hager & Rao 2015; DESIGN.md
+ * section 11), as per-thread functions.
+ *
+ * Section i has n LGR nodes over the support points s = {-1, tau_1 .. tau_n}.  Its test grid has M points tau'_l with
+ * four host-built tables (include/gelato_b200.h: GelatoMeshGridDesc): tau_t[M], the Lagrange basis P[M][n+1] over s
+ * (states), the basis Q[M][n] over tau_1 .. tau_n (controls) and the integration matrix I[M][M] of the test grid.  Per
+ * test point l the state X_l and controls U_l are interpolated and rh_l, the right-hand-side term of dyn_res_finish,
+ * is evaluated there (mesh_point).  Per state component c the estimate is then
+ *     err = max_l |X_0 + sum_k I[l][k] rh_k - X_l| / (1 + max_l |X_l|)
+ * with X_0 the section's first state row (mesh_component).  Every sum is a fused multiply-add chain with ascending
+ * index from 0.0, and max and division are exact, so the result has one value: the kernels, the host emulator
+ * (tests/emu/emu_mesh.cpp) and the oracle (tests/mesh_oracle.py) agree bit for bit.
+ */
+#ifndef GELATO_B200_MESH_ERROR_H_
+#define GELATO_B200_MESH_ERROR_H_
+
+#include "jobs.h"
+
+#define MESH_STATE 11            /* mass | position 3 | velocity 3 | quaternion 4 */
+#define MESH_PT (2 * MESH_STATE) /* doubles per test point in the scratch: X_l, then rh_l */
+
+/* one section of a test grid: M test points, the first one's index in the plan's list of test points, and the offset
+ * of the section's tables in the pool */
+struct MeshSec {
+  int32_t m, pt0;
+  int64_t off;
+};
+/* one test point: its section and its index inside the section */
+struct MeshPt {
+  int32_t sec, l;
+};
+
+struct MeshTabs {
+  const double *tau, *P, *Q, *I;
+};
+/* the pool is laid out tau_t[M] | P[M][n+1] | Q[M][n] | I[M][M] from the section's offset */
+P_HD MeshTabs mesh_tabs(const double* pool, const MeshSec& ms, int n) {
+  MeshTabs t;
+  t.tau = pool + ms.off;
+  t.P = t.tau + ms.m;
+  t.Q = t.P + (long long)ms.m * (n + 1);
+  t.I = t.Q + (long long)ms.m * n;
+  return t;
+}
+
+/* component c of state row `row` */
+P_HD double mesh_state(const PlanView& P, const double* x, int row, int c) {
+  if (c == 0) return x[row];
+  if (c < 4) return x[P.off_pos + 3 * row + c - 1];
+  if (c < 7) return x[P.off_vel + 3 * row + c - 4];
+  return x[P.off_quat + 4 * row + c - 7];
+}
+
+/* Test point l of section `sec`: xl[11] = the interpolated state, rh[11] = the right-hand-side term of each state
+ * component there, with the operations of dyn_res_finish (engine-off mass and held attitude: 0). */
+P_HD void mesh_point(const PlanView& P, int scen, const double* x, int sec, const MeshTabs& tb, int l, double* xl,
+                     double* rh) {
+  const int32_t* si = P.sec_i32 + sec * GS_I32_COLS;
+  const int n = si[GS_N], ua = si[GS_UA], xa = si[GS_XA], flags = si[GS_FLAGS];
+  const double* Prow = tb.P + (long long)l * (n + 1);
+  const double* Qrow = tb.Q + (long long)l * n;
+  dx_dot<1>(Prow, x + xa, n + 1, xl);
+  dx_dot<3>(Prow, x + P.off_pos + 3 * xa, n + 1, xl + 1);
+  dx_dot<3>(Prow, x + P.off_vel + 3 * xa, n + 1, xl + 4);
+  dx_dot<4>(Prow, x + P.off_quat + 4 * xa, n + 1, xl + 7);
+  double ul[2];
+  dx_dot<2>(Qrow, x + P.off_u + 2 * ua, n, ul);
+
+  const Units un = scen_units(P, scen);
+  const SecParam sp = sec_param(P, scen, sec);
+  const double ut = un.t;
+  const double to = x[P.off_t + sec], tf = x[P.off_t + sec + 1];
+  const double dt = tf - to;
+  rh[0] = (flags & GSF_ENGINE_ON) ? gm_div(-sp.massflow, un.mass) * dt * ut / 2.0 : 0.0;
+  const GmRcp Rp = gm_rcp(un.pos);
+  for (int k = 0; k < 3; k++) rh[1 + k] = gm_div_by(xl[4 + k] * un.vel * dt * ut / 2.0, Rp);
+  const Vec3 p = v3(xl[1], xl[2], xl[3]), v = v3(xl[4], xl[5], xl[6]);
+  const Quat q = q4(xl[7], xl[8], xl[9], xl[10]);
+  Vec3 f;
+  if (flags & GSF_AIR) f = rhs_velocity_air(xl[0], p, v, q, time_node(tb.tau, l + 1, to, tf), sp, un, scen_tables(P, scen));
+  else f = rhs_velocity_noair(xl[0], p, q, sp, un);
+  rh[4] = f.x * dt * ut / 2.0;
+  rh[5] = f.y * dt * ut / 2.0;
+  rh[6] = f.z * dt * ut / 2.0;
+  if (flags & GSF_HOLD) {
+    for (int k = 0; k < 4; k++) rh[7 + k] = 0.0;
+  } else {
+    const Quat d = rhs_quaternion(q, ul[0], ul[1], un.u);
+    rh[7] = d.w * dt * ut / 2.0;
+    rh[8] = d.x * dt * ut / 2.0;
+    rh[9] = d.y * dt * ut / 2.0;
+    rh[10] = d.z * dt * ut / 2.0;
+  }
+}
+
+/* max as numpy's: a NaN operand makes the result NaN */
+P_HD double mesh_max(double a, double b) { return (b > a || b != b) ? b : a; }
+
+/* The estimate of state component c of section `sec`: pts = the section's M test points as mesh_point left them,
+ * MESH_PT doubles each. */
+P_HD double mesh_component(const PlanView& P, const double* x, int sec, const MeshTabs& tb, int M, const double* pts, int c) {
+  const double x0 = mesh_state(P, x, P.sec_i32[sec * GS_I32_COLS + GS_XA], c);
+  double emax = 0.0, xmax = 0.0;
+  for (int l = 0; l < M; l++) {
+    const double* Irow = tb.I + (long long)l * M;
+    double acc = 0.0;
+    for (int k = 0; k < M; k++) acc = gm_fma(Irow[k], pts[(long long)k * MESH_PT + MESH_STATE + c], acc);
+    const double xl = pts[(long long)l * MESH_PT + c];
+    emax = mesh_max(emax, gm_fabs((x0 + acc) - xl));
+    xmax = mesh_max(xmax, gm_fabs(xl));
+  }
+  return gm_div(emax, 1.0 + xmax);
+}
+
+#endif /* GELATO_B200_MESH_ERROR_H_ */

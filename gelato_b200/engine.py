@@ -66,6 +66,12 @@ class ScenarioDesc(ctypes.Structure):
                 ("vals_template", _pd)]
 
 
+class MeshGridDesc(ctypes.Structure):
+    """GelatoMeshGridDesc (include/gelato_b200.h)."""
+
+    _fields_ = [("m", _pi32), ("off", _pi64), ("pool", _pd), ("pool_len", ctypes.c_int64)]
+
+
 def _ptr(arr, typ):
     if arr is None or arr.size == 0:
         return ctypes.cast(None, typ)
@@ -167,6 +173,16 @@ def make_scenario_desc(plans):
     return sc, keep
 
 
+def make_mesh_grid_desc(tables):
+    """{"m", "off", "pool"} (gelato_b200/mesh.py: grid_tables) -> (MeshGridDesc, keepalive list)."""
+    m = np.ascontiguousarray(tables["m"], dtype=np.int32)
+    off = np.ascontiguousarray(tables["off"], dtype=np.int64)
+    pool = np.ascontiguousarray(tables["pool"], dtype=np.float64)
+    d = MeshGridDesc()
+    d.m, d.off, d.pool, d.pool_len = _ptr(m, _pi32), _ptr(off, _pi64), _ptr(pool, _pd), pool.size
+    return d, [m, off, pool]
+
+
 def build_library(force=False, verbose=False, out=None, extra=()):
     """Compile csrc/gelato_b200.cu for sm_100a into csrc/libgelato_b200.so (in tree).
     `out` / `extra`: another output path and extra nvcc flags (tuning variants)."""
@@ -214,6 +230,9 @@ def load_library():
     L.gelato_plan_set_fd.argtypes = [vp, ctypes.c_int32, _c_d]
     L.gelato_plan_get_fd.argtypes = [vp, _pi32, _pd]
     L.gelato_eval_residuals.argtypes = [vp, _pd, _pd, ctypes.c_int32]
+    L.gelato_plan_set_mesh_grid.argtypes = [vp, ctypes.POINTER(MeshGridDesc)]
+    L.gelato_eval_mesh_error.argtypes = [vp, _pd, _pd, ctypes.c_int32]
+    L.gelato_eval_mesh_error_dev.argtypes = [vp, vp, vp, ctypes.c_int32, vp]
     L.gelato_eval_jacobian.argtypes = [vp, _pd, _pd, ctypes.c_int32]
     L.gelato_eval_residuals_ids.argtypes = [vp, _pd, _pd, ctypes.c_int32, _pi32]
     L.gelato_eval_jacobian_ids.argtypes = [vp, _pd, _pd, ctypes.c_int32, _pi32]
@@ -277,7 +296,8 @@ EXPORTS = (
     "gelato_pack_xdep_dev gelato_leaf_dynamics_velocity gelato_leaf_dynamics_velocity_noair "
     "gelato_leaf_dynamics_quaternion gelato_leaf_aero gelato_leaf_eci2geodetic gelato_leaf_gravity gelato_leaf_iip "
     "gelato_leaf_atmosphere gelato_leaf_output_table gelato_init_rocket_simulation gelato_leaf_coordinate "
-    "gelato_eval_pair_packed_range_dev gelato_plan_set_fd gelato_plan_get_fd"
+    "gelato_eval_pair_packed_range_dev gelato_plan_set_fd gelato_plan_get_fd "
+    "gelato_plan_set_mesh_grid gelato_eval_mesh_error gelato_eval_mesh_error_dev"
 ).split()
 
 
@@ -358,6 +378,25 @@ class Engine:
         m, h = ctypes.c_int32(0), ctypes.c_double(0.0)
         _check(self.L, self.L.gelato_plan_get_fd(self.h, ctypes.byref(m), ctypes.byref(h)), "gelato_plan_get_fd")
         return {v: k for k, v in FD_MODES.items()}[m.value], h.value
+
+    # ---- mesh error estimate (DESIGN.md section 11) ----
+    def set_mesh_grid(self, tables):
+        """The test grid of the mesh error estimate: {"m", "off", "pool"} as gelato_b200.mesh.grid_tables builds it."""
+        desc, _keep = make_mesh_grid_desc(tables)
+        _check(self.L, self.L.gelato_plan_set_mesh_grid(self.h, ctypes.byref(desc)), "gelato_plan_set_mesh_grid")
+
+    def mesh_error(self, x, n_scen=1, out=None):
+        """err[S][11] (n_scen > 1: [n_scen][S][11]) of the decision vectors x[n_scen][n_vars]: per section and state
+        component (mass | position 3 | velocity 3 | quaternion 4) the collocation error estimate between the nodes."""
+        x = self._x(x, n_scen)
+        self.calls += 1
+        n = n_scen * self.plan.S * 11
+        err = _out(out, n, "out") if out is not None else np.empty(n)
+        _check(self.L, self.L.gelato_eval_mesh_error(self.h, _ptr(x, _pd), _ptr(err, _pd), n_scen), "gelato_eval_mesh_error")
+        return err.reshape(self.plan.S, 11) if n_scen == 1 else err.reshape(n_scen, self.plan.S, 11)
+
+    def mesh_error_dev(self, x_ptr, err_ptr, n_scen=1, stream=None):
+        _check(self.L, self.L.gelato_eval_mesh_error_dev(self.h, x_ptr, err_ptr, n_scen, stream), "gelato_eval_mesh_error_dev")
 
     # ---- host-buffer calls (what objfunc / sens use) --------------------
     def _x(self, x, n_scen):

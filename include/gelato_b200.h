@@ -285,6 +285,35 @@ int gelato_eval_jacobian_packed(GelatoPlan* plan, const double* x, double* packe
 int gelato_eval_pair_packed_ids(GelatoPlan* plan, const double* x, double* g, double* packed, int32_t n_scen,
                                 const int32_t* scen_ids);
 
+/* Mesh error estimate (DESIGN.md section 11): how well the dynamics hold BETWEEN the collocation nodes.  For each section
+ * the state and controls are interpolated at M test points tau'_l, the right-hand side of the collocation defects is
+ * evaluated there, integrated with the test grid's integration matrix from the section's first state row, and compared
+ * with the interpolated state:
+ *     err[s][i][c] = max_l |X_0,c + sum_k I[l][k] rh_k,c - X_l,c| / (1 + max_l |X_l,c|)
+ * for scenario s, section i and state component c (mass | position 3 | velocity 3 | quaternion 4).  Engine-off mass
+ * and held attitude have no right-hand side: their estimate is the spread of the interpolated state around X_0.
+ * gelato_plan_set_mesh_grid: the test grid, copied to the device.  m[i] (>= 1) test points of section i, whose tables
+ * lie in `pool` from offset off[i] on, laid out
+ *     tau_t[M] | P[M][n+1] | Q[M][n] | I[M][M]
+ * (n = the section's LGR nodes): the test points in [-1, 1], the Lagrange basis over {-1, tau_1 .. tau_n} (states) and
+ * over tau_1 .. tau_n (controls) at the test points, and the inverse of the test grid's LGR differentiation matrix
+ * without its first column (gelato_b200/mesh.py: grid_tables builds them with M = n + 1).  M < 1, a table outside the
+ * pool or a value in the pool that is not finite returns GELATO_ERR_ARG and leaves the plan unchanged.
+ * gelato_eval_mesh_error: host buffers, x [n_scen][n_vars], err [n_scen][S][11] (page-locked buffers are DMA'd
+ * directly, others staged).  _dev: device pointers, enqueued on `stream` (NULL = the plan's own), not synchronised.
+ * Both use the scenario blocks of gelato_plan_set_scenarios, refuse an n_scen beyond them as every entry point does, and
+ * refuse calls before a grid is set.  Two launches per call (DESIGN.md section 11 gives the measured cost); the _dev call
+ * uses plan-owned scratch (n_scen x sum(M) x 22 doubles): calls on one plan must not overlap on different streams. */
+typedef struct GelatoMeshGridDesc {
+  const int32_t* m;   /* [S] test points of each section */
+  const int64_t* off; /* [S] offset (doubles) of each section's tables in pool */
+  const double* pool;
+  int64_t pool_len;
+} GelatoMeshGridDesc;
+int gelato_plan_set_mesh_grid(GelatoPlan* plan, const GelatoMeshGridDesc* grid);
+int gelato_eval_mesh_error(GelatoPlan* plan, const double* x, double* err, int32_t n_scen);
+int gelato_eval_mesh_error_dev(GelatoPlan* plan, const double* x_dev, double* err_dev, int32_t n_scen, void* stream);
+
 int gelato_host_alloc(size_t bytes, void** out);
 int gelato_host_free(void* ptr);
 
