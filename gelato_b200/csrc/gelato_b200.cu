@@ -963,22 +963,9 @@ int gelato_eval_jacobian_ids(GelatoPlan* p, const double* x, double* vals, int32
 // ---- mesh error estimate (mesh_error.h) ----
 int gelato_plan_set_mesh_grid(GelatoPlan* p, const GelatoMeshGridDesc* g) {
   if (!p || !g || !g->m || !g->off || !g->pool) return fail(GELATO_ERR_ARG, "null argument");
-  const int S = p->view.S;
-  std::vector<MeshSec> secs(S);
+  std::vector<MeshSec> secs;
   std::vector<MeshPt> pts;
-  for (int i = 0; i < S; i++) {
-    const long long m = g->m[i], n = p->sec_n[i], off = g->off[i];
-    if (m < 1) return fail(GELATO_ERR_ARG, "every section needs at least one test point");
-    if (off < 0 || off > g->pool_len || m > (g->pool_len - off) / (m + 2 * n + 2))
-      return fail(GELATO_ERR_ARG, "a section's tables lie outside the pool");
-    if ((long long)pts.size() + m > 0x7fffffffLL / MESH_PT) return fail(GELATO_ERR_ARG, "too many test points");
-    secs[i].m = (int32_t)m;
-    secs[i].pt0 = (int32_t)pts.size();
-    secs[i].off = off;
-    for (int l = 0; l < m; l++) pts.push_back(MeshPt{i, l});
-  }
-  for (int64_t k = 0; k < g->pool_len; k++)
-    if (!std::isfinite(g->pool[k])) return fail(GELATO_ERR_ARG, "the table pool holds a value that is not finite");
+  if (const char* why = build_mesh_grid(g, p->sec_n.data(), p->view.S, secs, pts)) return fail(GELATO_ERR_ARG, why);
   CU(cudaSetDevice(p->device));
   CU(cudaDeviceSynchronize());  // nothing in flight may still read the grid being replaced
   CU(p->d_mesh_sec.reserve(secs.size()));

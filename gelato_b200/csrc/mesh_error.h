@@ -9,7 +9,7 @@
  *     err = max_l |X_0 + sum_k I[l][k] rh_k - X_l| / (1 + max_l |X_l|)
  * with X_0 the section's first state row (mesh_component).  Every sum is a fused multiply-add chain with ascending
  * index from 0.0, and max and division are exact, so the result has one value: the kernels, the host emulator
- * (tests/emu/emu_mesh.cpp) and the oracle (tests/mesh_oracle.py) agree bit for bit.
+ * (tests/emu/emu.cpp) and the oracle (tests/mesh_oracle.py) agree bit for bit.
  */
 #ifndef GELATO_B200_MESH_ERROR_H_
 #define GELATO_B200_MESH_ERROR_H_

@@ -1,13 +1,16 @@
 /* plan_host.h -- host-side helpers shared by the CUDA library and the test
  * emulator: PlanView scalar fields from a GelatoPlanDesc, the node / row lists
- * and the block tables of the two kernels. */
+ * and the block tables of the two kernels, and the test grid of the mesh error
+ * estimate. */
 #ifndef GELATO_B200_PLAN_HOST_H_
 #define GELATO_B200_PLAN_HOST_H_
 
 #include <algorithm>
+#include <cmath>
 #include <vector>
 
 #include "jobs.h"
+#include "mesh_error.h"
 
 /* fills every non-pointer field of the view; pointer fields are left untouched */
 static inline void planview_scalars(const GelatoPlanDesc* d, PlanView& v) {
@@ -312,6 +315,29 @@ static inline void build_host_tables(const GelatoPlanDesc* d, HostTables& h) {
   push_chunks(rb, BR_AERO, 0, n_aero_rows, GR_THREADS);
   push_chunks(rb, BR_EVT, 0, d->n_evt, GR_THREADS);
   push_chunks(rb, BR_LIN, 0, d->n_lin, GR_THREADS);
+}
+
+/* The test grid of the mesh error estimate (include/gelato_b200.h: GelatoMeshGridDesc) over S sections of n[i] LGR
+ * nodes: its sections and the list of its test points.  Returns NULL or why the grid is refused.  The kernels trust
+ * the grid, so one that fails here is not uploaded. */
+static inline const char* build_mesh_grid(const GelatoMeshGridDesc* g, const int32_t* n, int S, std::vector<MeshSec>& secs,
+                                          std::vector<MeshPt>& pts) {
+  secs.assign(S, MeshSec());
+  pts.clear();
+  for (int i = 0; i < S; i++) {
+    const long long m = g->m[i], ni = n[i], off = g->off[i];
+    if (m < 1) return "every section needs at least one test point";
+    if (off < 0 || off > g->pool_len || m > (g->pool_len - off) / (m + 2 * ni + 2))
+      return "a section's tables lie outside the pool";
+    if ((long long)pts.size() + m > 0x7fffffffLL / MESH_PT) return "too many test points";
+    secs[i].m = (int32_t)m;
+    secs[i].pt0 = (int32_t)pts.size();
+    secs[i].off = off;
+    for (int l = 0; l < m; l++) pts.push_back(MeshPt{i, l});
+  }
+  for (int64_t k = 0; k < g->pool_len; k++)
+    if (!std::isfinite(g->pool[k])) return "the table pool holds a value that is not finite";
+  return nullptr;
 }
 
 #endif

@@ -1,10 +1,11 @@
-// emu.cpp -- host emulator of the two fused CUDA kernels (TEST HARNESS ONLY).
+// emu.cpp -- host emulator of the CUDA kernels (TEST HARNESS ONLY).
 //
 // Compiles gelato_b200/csrc/jobs.h (the per-thread job functions the kernels
 // run) with g++ and steps through every block and thread serially: phase 1 for
 // all threads of a block, then phase 2 -- the same order the block barrier
 // enforces on the GPU (the Jacobian kernel has GJ_PHASES phases, the residual kernel two).  It lets the CPU-only test tier check the plan compiler
-// and the kernels' index arithmetic against the oracle bit for bit.  It is not
+// and the kernels' index arithmetic against the oracle bit for bit, in both
+// finite-difference modes, and the mesh error estimate (mesh_error.h).  It is not
 // part of the product: libgelato_b200.so has no CPU path and bench.py never
 // loads this file.
 #include <cstring>
@@ -76,14 +77,20 @@ extern "C" int emu_eval_residuals(const GelatoPlanDesc* d, const GelatoScenarioD
   return 0;
 }
 
-// packed: out_all is [n_scen][n_pack] and nothing is pre-filled;  g_all != NULL: pair evaluation -- objfunc's
-// rows come out of the Jacobian blocks (what gelato_eval_pair_* launches).
-static int g_range[4] = {0, -1, 0, 0}; /* block first / count (-1: all), vacuum first / count */
-static int emu_jacobian(const GelatoPlanDesc* d, const GelatoScenarioDesc* sc, const double* x_all, double* g_all,
-                        double* out_all, int n_scen, const int32_t* ids, int packed) {
+// One pass of the Jacobian blocks and vacuum nodes with finite-difference step `dx`: what launch_jacobian_pass launches.
+// packed: out_all is [n_scen][n_pack] and nothing is pre-filled, else [n_scen][n_vals] from the template;  g_all != NULL:
+// pair evaluation -- objfunc's rows come out of the Jacobian blocks and the linear-row blocks run too.  A sub-range (one
+// problem sharded over ranks): blocks [b0, b0 + nb) and vacuum nodes [v0, v0 + nv); nb < 0: everything.
+struct JacRange {
+  int b0 = 0, nb = -1, v0 = 0, nv = 0;
+};
+static int emu_jacobian_pass(const GelatoPlanDesc* d, const GelatoScenarioDesc* sc, double dx, const double* x_all,
+                             double* g_all, double* out_all, int n_scen, const int32_t* ids, int packed,
+                             JacRange rg = JacRange()) {
   if (validate_desc(d)) return -1;
   PlanView P = host_view(d);
   apply_scen(P, sc);
+  P.un.dx = dx;
   HostTables h;
   build_host_tables(d, h);
   attach_tables(P, h);
@@ -93,6 +100,10 @@ static int emu_jacobian(const GelatoPlanDesc* d, const GelatoScenarioDesc* sc, c
   P.n_pack = L.n_pack;
   P.sec_pk = L.sec_pk.data(); P.aero_pk = L.aero_pk.data(); P.evt_pk = L.evt_pk.data();
   const std::vector<int32_t>& jb = h.jac_blocks;
+  const bool all = rg.nb < 0;
+  const size_t b_lo = all ? 0 : (size_t)rg.b0;
+  const size_t b_hi = b_lo + (all ? (g_all ? jb.size() / BT_COLS : (size_t)h.n_jac_main) : (size_t)rg.nb);
+  const int v_lo = all ? 0 : rg.v0, v_hi = v_lo + (all ? h.n_vac : rg.nv);
   JacStore store;
   const JacScratch sm = jac_scratch(store);
   const size_t stride = packed ? (size_t)L.n_pack : (size_t)P.n_vals;
@@ -105,10 +116,7 @@ static int emu_jacobian(const GelatoPlanDesc* d, const GelatoScenarioDesc* sc, c
       const double* tmpl = (sc && sc->vals_template) ? sc->vals_template + (size_t)sid * P.n_vals : d->vals_template;
       memcpy(vals, tmpl, (size_t)P.n_vals * sizeof(double));
     }
-    const size_t nb_all = g ? jb.size() / BT_COLS : (size_t)h.n_jac_main;  /* the linear-row blocks: pair evaluations only */
-    const size_t b_lo = g_range[1] < 0 ? 0 : (size_t)g_range[0], nb = g_range[1] < 0 ? nb_all : (size_t)(g_range[0] + g_range[1]);
-    const int v_lo = g_range[1] < 0 ? 0 : g_range[2], v_hi = g_range[1] < 0 ? h.n_vac : g_range[2] + g_range[3];
-    for (size_t b = b_lo; b < nb; b++) {
+    for (size_t b = b_lo; b < b_hi; b++) {
       const int32_t* bt = jb.data() + b * BT_COLS;
       /* poison the scratch so a phase that reads what no thread wrote shows up as NaN */
       memset(&store, 0xff, sizeof store);
@@ -121,18 +129,38 @@ static int emu_jacobian(const GelatoPlanDesc* d, const GelatoScenarioDesc* sc, c
   return 0;
 }
 
-extern "C" int emu_eval_jacobian(const GelatoPlanDesc* d, const GelatoScenarioDesc* sc, const double* x_all,
-                                 double* vals_all, int n_scen, const int32_t* ids) {
-  return emu_jacobian(d, sc, x_all, nullptr, vals_all, n_scen, ids, 0);
+// One Jacobian evaluation in finite-difference mode fd_mode (DESIGN.md H6): what launch_jacobian does.  Forward: one
+// pass with the plan's dx.  Central: the +step pass into the caller's output (and g), the -step pass packed into
+// scratch, then fd_central per x-dependent value (COO output through the packed map).  g_all == NULL: Jacobian only.
+extern "C" int emu_eval_jacobian(const GelatoPlanDesc* d, const GelatoScenarioDesc* sc, const double* x_all, double* g_all,
+                                 double* out_all, int n_scen, const int32_t* ids, int packed, int32_t fd_mode, double step) {
+  const bool central = fd_mode == GELATO_FD_CENTRAL;
+  if (central && !(step > 0.0)) return -1;
+  int rc = emu_jacobian_pass(d, sc, central ? step : d->dx, x_all, g_all, out_all, n_scen, ids, packed);
+  if (rc || !central) return rc;
+  PackedLayout L;
+  build_packed_layout(d, L);
+  std::vector<double> minus((size_t)n_scen * (size_t)L.n_pack);
+  emu_jacobian_pass(d, sc, -step, x_all, nullptr, minus.data(), n_scen, ids, 1);
+  for (int scen = 0; scen < n_scen; scen++) {
+    const double* m = minus.data() + (size_t)scen * L.n_pack;
+    if (packed) {
+      double* out = out_all + (size_t)scen * L.n_pack;
+      for (long long i = 0; i < L.n_pack; i++) out[i] = fd_central(out[i], m[i]);
+    } else {
+      double* out = out_all + (size_t)scen * d->n_vals;
+      for (size_t i = 0; i < L.full_slot.size(); i++)
+        out[L.full_slot[i]] = fd_central(out[L.full_slot[i]], L.sgn[i] * m[L.src[i]]);
+    }
+  }
+  return 0;
 }
 
-// one problem sharded over ranks: the pair evaluation restricted to a block range and a vacuum-node range
+// one problem sharded over ranks: the packed pair evaluation restricted to a block range and a vacuum-node range
+// (forward differences only, as gelato_eval_pair_packed_range_dev)
 extern "C" int emu_eval_pair_range(const GelatoPlanDesc* d, const GelatoScenarioDesc* sc, const double* x_all, double* g_all,
                                    double* out_all, int n_scen, int b0, int nb, int v0, int nv) {
-  g_range[0] = b0; g_range[1] = nb; g_range[2] = v0; g_range[3] = nv;
-  const int rc = emu_jacobian(d, sc, x_all, g_all, out_all, n_scen, nullptr, 1);
-  g_range[1] = -1;
-  return rc;
+  return emu_jacobian_pass(d, sc, d->dx, x_all, g_all, out_all, n_scen, nullptr, 1, JacRange{b0, nb, v0, nv});
 }
 extern "C" void emu_block_counts(const GelatoPlanDesc* d, int* n_blocks_pair, int* n_vac) {
   HostTables h;
@@ -141,9 +169,45 @@ extern "C" void emu_block_counts(const GelatoPlanDesc* d, int* n_blocks_pair, in
   *n_vac = h.n_vac;
 }
 
-extern "C" int emu_eval_pair(const GelatoPlanDesc* d, const GelatoScenarioDesc* sc, const double* x_all, double* g_all,
-                             double* out_all, int n_scen, const int32_t* ids, int packed) {
-  return emu_jacobian(d, sc, x_all, g_all, out_all, n_scen, ids, packed);
+// ---- mesh error estimate (mesh_error.h; DESIGN.md section 11) ----
+static std::vector<int32_t> sec_nodes(const GelatoPlanDesc* d) {
+  std::vector<int32_t> n(d->n_sections);
+  for (int i = 0; i < d->n_sections; i++) n[i] = d->sec_i32[i * GS_I32_COLS + GS_N];
+  return n;
+}
+
+// NULL or why gelato_plan_set_mesh_grid refuses the grid (plan_host.h: build_mesh_grid)
+extern "C" const char* emu_check_mesh_grid(const GelatoPlanDesc* d, const GelatoMeshGridDesc* g) {
+  std::vector<MeshSec> secs;
+  std::vector<MeshPt> pts;
+  return build_mesh_grid(g, sec_nodes(d).data(), d->n_sections, secs, pts);
+}
+
+// err_all: [n_scen][S][11]; what k_mesh_points (every test point) and then k_mesh_error (every section and state
+// component) compute
+extern "C" int emu_eval_mesh_error(const GelatoPlanDesc* d, const GelatoScenarioDesc* sc, const GelatoMeshGridDesc* g,
+                                   const double* x_all, double* err_all, int n_scen) {
+  if (validate_desc(d)) return -1;
+  PlanView P = host_view(d);
+  apply_scen(P, sc);
+  const std::vector<int32_t> n = sec_nodes(d);
+  std::vector<MeshSec> ms;
+  std::vector<MeshPt> mp;
+  if (build_mesh_grid(g, n.data(), P.S, ms, mp)) return -1;
+  std::vector<double> pts(mp.size() * MESH_PT);
+  for (int scen = 0; scen < n_scen; scen++) {
+    const double* x = x_all + (size_t)scen * P.n_vars;
+    for (size_t k = 0; k < mp.size(); k++) {
+      const MeshPt q = mp[k];
+      double* out = pts.data() + k * MESH_PT;
+      mesh_point(P, scen, x, q.sec, mesh_tabs(g->pool, ms[q.sec], n[q.sec]), q.l, out, out + MESH_STATE);
+    }
+    for (int i = 0; i < P.S; i++)
+      for (int c = 0; c < MESH_STATE; c++)
+        err_all[((size_t)scen * P.S + i) * MESH_STATE + c] = mesh_component(
+            P, x, i, mesh_tabs(g->pool, ms[i], n[i]), ms[i].m, pts.data() + (size_t)ms[i].pt0 * MESH_PT, c);
+  }
+  return 0;
 }
 
 // packed layout of a plan: returns n_pack; with non-NULL arrays also the map of the n_xdep COO slots

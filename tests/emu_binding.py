@@ -1,7 +1,8 @@
 """ctypes front-end of tests/emu (the host emulator of the CUDA kernels).
 
 TEST HARNESS ONLY: lets the CPU test tier run the kernels' per-thread code
-(gelato_b200/csrc/jobs.h) through the same GelatoPlanDesc the GPU library gets.
+(gelato_b200/csrc/jobs.h, mesh_error.h) through the same GelatoPlanDesc the GPU library gets, with the settings
+gelato_b200.engine.Engine has: the finite-difference mode (DESIGN.md H6) and the mesh grid (DESIGN.md section 11).
 """
 import ctypes
 import os
@@ -16,6 +17,8 @@ ROOT = os.path.dirname(_HERE)
 BUILD = os.path.join(_HERE, "_build")
 LIB = os.path.join(BUILD, "libgelato_emu.so")
 _pd = ctypes.POINTER(ctypes.c_double)
+_pi32 = ctypes.POINTER(ctypes.c_int32)
+_pi64 = ctypes.POINTER(ctypes.c_int64)
 
 
 def build(force=False):
@@ -33,25 +36,30 @@ def build(force=False):
 class Emulator:
     def __init__(self, plan, scenario_plans=None):
         build()
-        self.L = ctypes.CDLL(LIB)
-        assert self.L.emu_unfused_check() == 1
+        self.L = L = ctypes.CDLL(LIB)
+        assert L.emu_unfused_check() == 1
         self.plan = plan
         self.desc, self._keep = engine.make_desc(plan)
         self.sc = None
         if scenario_plans is not None:
             self.sc, keep = engine.make_scenario_desc(scenario_plans)
             self._keep += keep
-        for fn in (self.L.emu_eval_residuals, self.L.emu_eval_jacobian):
-            fn.argtypes = [ctypes.POINTER(engine.PlanDesc), ctypes.POINTER(engine.ScenarioDesc), _pd, _pd, ctypes.c_int,
-                           ctypes.POINTER(ctypes.c_int32)]
-        self.L.emu_eval_pair.argtypes = [ctypes.POINTER(engine.PlanDesc), ctypes.POINTER(engine.ScenarioDesc), _pd, _pd, _pd,
-                                         ctypes.c_int, ctypes.POINTER(ctypes.c_int32), ctypes.c_int]
-        _pi64 = ctypes.POINTER(ctypes.c_int64)
-        self.L.emu_packed_map.argtypes = [ctypes.POINTER(engine.PlanDesc), _pi64, _pi64, _pd]
-        self.L.emu_packed_map.restype = ctypes.c_longlong
-        self.L.emu_n_xdep.argtypes = [ctypes.POINTER(engine.PlanDesc)]
-        self.L.emu_n_xdep.restype = ctypes.c_longlong
-        self.n_pack = int(self.L.emu_packed_map(ctypes.byref(self.desc), None, None, None))
+        pdesc, psc, pgrid, c_int = (ctypes.POINTER(engine.PlanDesc), ctypes.POINTER(engine.ScenarioDesc),
+                                    ctypes.POINTER(engine.MeshGridDesc), ctypes.c_int)
+        L.emu_eval_residuals.argtypes = [pdesc, psc, _pd, _pd, c_int, _pi32]
+        L.emu_eval_jacobian.argtypes = [pdesc, psc, _pd, _pd, _pd, c_int, _pi32, c_int, ctypes.c_int32, ctypes.c_double]
+        L.emu_eval_pair_range.argtypes = [pdesc, psc, _pd, _pd, _pd] + [c_int] * 5
+        L.emu_block_counts.argtypes = [pdesc, ctypes.POINTER(c_int), ctypes.POINTER(c_int)]
+        L.emu_packed_map.argtypes = [pdesc, _pi64, _pi64, _pd]
+        L.emu_packed_map.restype = ctypes.c_longlong
+        L.emu_n_xdep.argtypes = [pdesc]
+        L.emu_n_xdep.restype = ctypes.c_longlong
+        L.emu_check_mesh_grid.argtypes = [pdesc, pgrid]
+        L.emu_check_mesh_grid.restype = ctypes.c_char_p
+        L.emu_eval_mesh_error.argtypes = [pdesc, psc, pgrid, _pd, _pd, c_int]
+        self.n_pack = int(L.emu_packed_map(ctypes.byref(self.desc), None, None, None))
+        self._fd = engine.fd_args("forward")  # (C mode code, step) as gelato_plan_set_fd takes them
+        self._grid = None
 
     def _sc(self):
         return ctypes.byref(self.sc) if self.sc is not None else None
@@ -61,8 +69,29 @@ class Emulator:
         if scen_ids is None:
             return None, None
         ids = np.ascontiguousarray(scen_ids, dtype=np.int32)
-        return ids, ids.ctypes.data_as(ctypes.POINTER(ctypes.c_int32))
+        return ids, ids.ctypes.data_as(_pi32)
 
+    # ---- settings, as engine.Engine has them ----
+    def set_fd(self, mode, step=None):
+        """engine.Engine.set_fd: "forward" or "central" with step `step` (None: engine.DEFAULT_FD_STEP)."""
+        self._fd = engine.fd_args(mode, step)
+
+    @property
+    def fd(self):
+        """engine.Engine.fd: (mode, step), forward's step being the plan's dx."""
+        code, step = self._fd
+        return ("central", step) if code == engine.FD_MODES["central"] else ("forward", float(self.plan.units[5]))
+
+    def set_mesh_grid(self, tables):
+        """engine.Engine.set_mesh_grid: a grid gelato_plan_set_mesh_grid refuses raises ValueError(<its reason>) and
+        the previous grid stays."""
+        grid = engine.make_mesh_grid_desc(tables)
+        why = self.L.emu_check_mesh_grid(ctypes.byref(self.desc), ctypes.byref(grid[0]))
+        if why is not None:
+            raise ValueError(why.decode())
+        self._grid = grid
+
+    # ---- evaluations ----
     def eval_residuals(self, x, n_scen=1, scen_ids=None):
         x = np.ascontiguousarray(x, dtype=np.float64)
         g = np.full(n_scen * self.plan.n_rows, np.nan)
@@ -71,55 +100,65 @@ class Emulator:
         assert rc == 0, "the plan description failed validate_desc (plan_host.h)"
         return g if n_scen == 1 else g.reshape(n_scen, -1)
 
-    def eval_jacobian(self, x, n_scen=1, scen_ids=None):
+    def _jacobian(self, x, n_scen, scen_ids, packed, pair):
+        """(g or None, COO or packed values) of one evaluation in the current finite-difference mode."""
         x = np.ascontiguousarray(x, dtype=np.float64)
-        v = np.full(n_scen * self.plan.n_vals, np.nan)
+        g = np.full(n_scen * self.plan.n_rows, np.nan) if pair else None
+        v = np.full(n_scen * (self.n_pack if packed else self.plan.n_vals), np.nan)
         ids, pids = self._ids(scen_ids)
-        rc = self.L.emu_eval_jacobian(ctypes.byref(self.desc), self._sc(), x.ctypes.data_as(_pd), v.ctypes.data_as(_pd), n_scen, pids)
+        rc = self.L.emu_eval_jacobian(ctypes.byref(self.desc), self._sc(), x.ctypes.data_as(_pd),
+                                      None if g is None else g.ctypes.data_as(_pd), v.ctypes.data_as(_pd), n_scen, pids,
+                                      1 if packed else 0, *self._fd)
         assert rc == 0, "the plan description failed validate_desc (plan_host.h)"
-        return v if n_scen == 1 else v.reshape(n_scen, -1)
+        if n_scen > 1:
+            v = v.reshape(n_scen, -1)
+            g = None if g is None else g.reshape(n_scen, -1)
+        return g, v
 
+    def eval_jacobian(self, x, n_scen=1, scen_ids=None):
+        return self._jacobian(x, n_scen, scen_ids, False, False)[1]
+
+    def eval_jacobian_packed(self, x, n_scen=1, scen_ids=None):
+        """packed[n_scen][n_pack] of a Jacobian-only evaluation."""
+        return self._jacobian(x, n_scen, scen_ids, True, False)[1]
+
+    def eval_pair(self, x, n_scen=1, scen_ids=None, packed=False):
+        """(g, vals or packed) of a pair evaluation: defects from the Jacobian blocks' centre columns."""
+        return self._jacobian(x, n_scen, scen_ids, packed, True)
 
     def packed_map(self):
         """(full_slot, src, sgn): vals[full_slot] = sgn * packed[src] (plan_host.h: build_packed_layout)."""
         n = int(self.L.emu_n_xdep(ctypes.byref(self.desc)))
         full, src, sgn = np.empty(n, dtype=np.int64), np.empty(n, dtype=np.int64), np.empty(n)
-        _pi64 = ctypes.POINTER(ctypes.c_int64)
         self.L.emu_packed_map(ctypes.byref(self.desc), full.ctypes.data_as(_pi64), src.ctypes.data_as(_pi64),
                               sgn.ctypes.data_as(_pd))
         return full, src, sgn
 
-    def eval_pair(self, x, n_scen=1, scen_ids=None, packed=False):
-        """(g, vals or packed) of a pair evaluation: defects from the Jacobian blocks' centre columns."""
+    def mesh_error(self, x, n_scen=1):
+        """engine.Engine.mesh_error."""
+        assert self._grid is not None, "no mesh grid set"
         x = np.ascontiguousarray(x, dtype=np.float64)
-        g = np.full(n_scen * self.plan.n_rows, np.nan)
-        width = self.n_pack if packed else self.plan.n_vals
-        v = np.full(n_scen * width, np.nan)
-        ids, pids = self._ids(scen_ids)
-        rc = self.L.emu_eval_pair(ctypes.byref(self.desc), self._sc(), x.ctypes.data_as(_pd), g.ctypes.data_as(_pd),
-                                  v.ctypes.data_as(_pd), n_scen, pids, 1 if packed else 0)
-        assert rc == 0
-        if n_scen == 1:
-            return g, v
-        return g.reshape(n_scen, -1), v.reshape(n_scen, -1)
-
+        err = np.full(n_scen * self.plan.S * 11, np.nan)
+        rc = self.L.emu_eval_mesh_error(ctypes.byref(self.desc), self._sc(), ctypes.byref(self._grid[0]),
+                                        x.ctypes.data_as(_pd), err.ctypes.data_as(_pd), n_scen)
+        assert rc == 0, "the plan description failed validate_desc (plan_host.h)"
+        return err.reshape(self.plan.S, 11) if n_scen == 1 else err.reshape(n_scen, self.plan.S, 11)
 
     # ---- one problem sharded over ranks (gelato_b200/batch.py: ShardedProblem) ----
     def block_counts(self):
         """(blocks of a pair evaluation, vacuum dynamics nodes): the two ranges a rank's share is cut from."""
         nb, nv = ctypes.c_int(0), ctypes.c_int(0)
-        self.L.emu_block_counts.argtypes = [ctypes.POINTER(engine.PlanDesc), ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_int)]
         self.L.emu_block_counts(ctypes.byref(self.desc), ctypes.byref(nb), ctypes.byref(nv))
         return nb.value, nv.value
 
     def eval_pair_range(self, x, g, packed, blocks, vacuum):
         """The packed pair evaluation restricted to blocks [b0, b1) and vacuum nodes [v0, v1), written into the
         caller's g[n_rows] / packed[n_pack] (what gelato_eval_pair_packed_range_dev launches)."""
+        if self.fd[0] != "forward":
+            raise ValueError("the range evaluation supports forward differences only")
         x = np.ascontiguousarray(x, dtype=np.float64)
         assert g.dtype == np.float64 and g.flags.c_contiguous and g.size == self.plan.n_rows
         assert packed.dtype == np.float64 and packed.flags.c_contiguous and packed.size == self.n_pack
-        self.L.emu_eval_pair_range.argtypes = [ctypes.POINTER(engine.PlanDesc), ctypes.POINTER(engine.ScenarioDesc), _pd, _pd, _pd,
-                                               ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_int]
         rc = self.L.emu_eval_pair_range(ctypes.byref(self.desc), self._sc(), x.ctypes.data_as(_pd), g.ctypes.data_as(_pd),
                                         packed.ctypes.data_as(_pd), 1, blocks[0], blocks[1] - blocks[0], vacuum[0],
                                         vacuum[1] - vacuum[0])
@@ -161,9 +200,7 @@ class EmuEngine(Emulator):
 
     def eval_jacobian_update(self, x, out, n_scen=1):
         assert n_scen == 1
-        self.launches += 1
-        self.calls += 1
-        v = super().eval_jacobian(x, 1, None)
+        v = self.eval_jacobian(x)
         idx = self.plan.xdep_index()
         out[idx] = v[idx]  # only the x-dependent slots move, as on the device
         return out
@@ -172,7 +209,7 @@ class EmuEngine(Emulator):
         assert n_scen == 1
         self.launches += 1
         self.calls += 1
-        g, v = super().eval_pair(x, 1, None, packed=False)
+        g, v = self.eval_pair(x)
         g_out[:] = g
         idx = self.plan.xdep_index()
         vals_out[idx] = v[idx]

@@ -13,9 +13,9 @@ import subprocess
 import numpy as np
 import pytest
 
+import emu_binding
 import helpers
 from central_oracle import CentralOracleNLP, Step, fd_quotient
-from emu_central import FdEmuEngine
 from gelato_b200 import callbacks, engine, problem, scenarios
 from oracle import leaves, user_builtin
 
@@ -166,9 +166,9 @@ def test_zero_quotient_keeps_the_numerator_sign():
 @pytest.mark.parametrize("variant,factor,user", VARIANTS)
 def test_emulated_central_matches_oracle_bitwise(variant, factor, user):
     p, u, c, x0, O, P = _case(variant, factor, user)
-    E = FdEmuEngine(P)
+    E = emu_binding.EmuEngine(P)
     E.set_fd("central", H)
-    F = FdEmuEngine(P)
+    F = emu_binding.EmuEngine(P)
     full, src, sgn = E.packed_map()
     for x in (x0, helpers.perturbed(x0)):
         xv = problem.xdict_to_vector(x)
@@ -199,7 +199,7 @@ def test_emulated_central_dispersed_scenarios_with_ids():
         plans.append(helpers.compiled_plan(p, u, c, coord=Lg.coordinate_c))
         oracles.append(_oracle(p, u, c))
         xs.append(helpers.perturbed(x0, seed=len(xs)))
-    E = FdEmuEngine(plans[0], scenario_plans=plans)
+    E = emu_binding.EmuEngine(plans[0], scenario_plans=plans)
     E.set_fd("central")
     ids = [2, 0, 2, 1]
     X = np.stack([problem.xdict_to_vector(xs[i]) for i in ids])
@@ -219,7 +219,7 @@ def _problem_on_emulator(derivative="forward", fd_step=None, **kw):
     Lg = leaves.get("gmath")
     p, u, c, x0 = helpers.example_problem(coord=Lg.coordinate_c)
     prob = callbacks.GelatoProblem(p, u, c, user_eq=callbacks.PerigeeAtEvent(helpers.USER_EVENT), coord=Lg.coordinate_c,
-                                   engine_factory=FdEmuEngine, derivative=derivative, fd_step=fd_step, **kw)
+                                   engine_factory=emu_binding.EmuEngine, derivative=derivative, fd_step=fd_step, **kw)
     return prob, p, u, c, x0
 
 
@@ -238,7 +238,7 @@ def test_gelato_problem_central_on_the_emulator(kw):
     # jacobian_csr follows the mode too
     x = helpers.perturbed(x0, seed=3)
     csr = prob.jacobian_csr(x)
-    vals = FdEmuEngine(prob.plan)
+    vals = emu_binding.EmuEngine(prob.plan)
     vals.set_fd("central")
     m = prob.plan.csr_map(key_order=tuple(x.keys()))
     assert_bits_equal(csr.data, np.append(vals.eval_jacobian(problem.xdict_to_vector(x)), 0.0)[m["src"]])
@@ -438,7 +438,7 @@ def test_capi_central_at_the_bench_workload_against_the_emulator():
     torch.cuda.synchronize()
     E.eval_pair_packed_dev(xd.data_ptr(), gd.data_ptr(), pd.data_ptr(), n)
     torch.cuda.synchronize()
-    Em = FdEmuEngine(P)
+    Em = emu_binding.EmuEngine(P)
     Em.set_fd("central", H)
     g_emu, pk_emu = Em.eval_pair(X, n_scen=n, packed=True)
     assert_bits_equal(pd.cpu().numpy(), pk_emu)

@@ -3,17 +3,18 @@
 CPU tier: the tables of gelato_b200.mesh, the oracle's estimate on each section's own grid against -A^-1 g (g =
 objfunc's collocation defect), the kernels' code in the host emulator against the oracle bit for bit, the convergence
 of the estimate on the example's vacuum coast sections for a state integrated to high accuracy, refine_nodes,
-transfer and GelatoProblem.mesh_error on the emulator.  GPU tier: the C ABI against the oracle bit for bit (variants,
-a dispersed batch with per-scenario blocks, the benchmark workload), the square grid against the GPU's own defects,
-host / device entry points and buffers, argument errors and the independence from the finite-difference mode."""
+transfer, GelatoProblem.mesh_error on the emulator and the grid checks the emulator shares with the C ABI.  GPU tier:
+the C ABI against the oracle bit for bit (variants, a dispersed batch with per-scenario blocks, the benchmark
+workload), the square grid against the GPU's own defects, host / device entry points and buffers, argument errors and
+the independence from the finite-difference mode."""
 import ctypes
 
 import numpy as np
 import pytest
 
+import emu_binding
 import helpers
 import mesh_oracle
-from emu_mesh import MeshEmuEngine
 from gelato_b200 import callbacks, engine, mesh, problem, scenarios
 from gelato_b200.psparams import PSparams, lgr_diff_matrix, lgr_nodes
 from oracle import leaves
@@ -128,7 +129,7 @@ def test_oracle_square_grid_is_the_integrated_defect(variant, factor):
 @pytest.mark.parametrize("variant,factor", VARIANTS)
 def test_emulator_equals_oracle_bit_for_bit(variant, factor):
     p, u, c, x0, O, P = _setup(variant, factor)
-    E = MeshEmuEngine(P)
+    E = emu_binding.EmuEngine(P)
     xs = [x0, helpers.perturbed(x0)] + ([_solution(P)] if (variant, factor) == ("example", 1) else [])
     for tabs in (mesh.grid_tables(O.ps), _square_grid(O.ps)):
         E.set_mesh_grid(tabs)
@@ -275,7 +276,7 @@ def test_transfer_polynomials_identity_and_refined_plan():
     p2, u2, c2, _ = problem.problem_from_inputs(inp, coord=Lg.coordinate_c)
     x2 = mesh.transfer(x_sol, p["ps_params"], p2["ps_params"])
     P2 = helpers.compiled_plan(p2, u2, c2, coord=Lg.coordinate_c)
-    E = MeshEmuEngine(P2)
+    E = emu_binding.EmuEngine(P2)
     g = E.eval_residuals(problem.xdict_to_vector(x2))
     assert g.shape == (P2.n_rows,) and np.isfinite(g).all()
     O2 = helpers.oracle_nlp(p2, u2, c2, "gmath", "seqfma")
@@ -288,7 +289,7 @@ def test_gelato_problem_mesh_error_on_the_emulator():
     Lg = leaves.get("gmath")
     p, u, c, x0 = helpers.example_problem(coord=Lg.coordinate_c)
     prob = callbacks.GelatoProblem(p, u, c, user_eq=callbacks.PerigeeAtEvent(helpers.USER_EVENT), coord=Lg.coordinate_c,
-                                   engine_factory=MeshEmuEngine)
+                                   engine_factory=emu_binding.EmuEngine)
     x = helpers.perturbed(x0)
     got = prob.mesh_error(x)
     want = mesh_oracle.mesh_error(helpers.oracle_nlp(p, u, c, "gmath", "seqfma"), x, mesh.grid_tables(p["ps_params"]))
@@ -297,6 +298,39 @@ def test_gelato_problem_mesh_error_on_the_emulator():
     assert _same_bits(np.stack([got[k] for k in names]), want)
     assert _same_bits(np.stack(list(prob.mesh_error(x).values())), want)  # the grid is set once, the result repeats
     prob.close()
+
+
+def _malformed_grids(tabs):
+    """(grid, why it is refused): copies of `tabs` with one defect each (plan_host.h: build_mesh_grid)."""
+    out = []
+    for key, i, value, why in (("m", 3, 0, "at least one test point"),
+                               ("off", -1, tabs["pool"].size - 1, "outside the pool"),
+                               ("off", 0, -1, "outside the pool"),
+                               ("pool", 7, np.nan, "not finite"),
+                               ("pool", -1, np.inf, "not finite"),
+                               ("m", 0, 2 ** 31 - 1, "outside the pool")):
+        t = {k: v.copy() for k, v in tabs.items()}
+        t[key][i] = value
+        out.append((t, why))
+    return out
+
+
+def test_emulator_refused_grids_keep_the_previous_grid_and_fd_mode_is_irrelevant():
+    """The grid checks gelato_plan_set_mesh_grid runs, on the CPU: every malformed grid is refused with its reason and
+    the previous grid stays; central differences do not change the estimate."""
+    p, u, c, x0, O, P = _setup("example", 1)
+    E = emu_binding.EmuEngine(P)
+    x = problem.xdict_to_vector(helpers.perturbed(x0))
+    tabs = mesh.grid_tables(O.ps)
+    E.set_mesh_grid(tabs)
+    ref = E.mesh_error(x)
+    for t, why in _malformed_grids(tabs):
+        with pytest.raises(ValueError, match=why):
+            E.set_mesh_grid(t)
+        assert _same_bits(E.mesh_error(x), ref)
+    E.set_fd("central")
+    E.eval_jacobian(x)
+    assert _same_bits(E.mesh_error(x), ref)
 
 
 # ------------------------------------------------------------------------------------------------ GPU tier
@@ -405,27 +439,8 @@ def test_gpu_argument_errors_leave_the_plan_usable_and_fd_mode_is_irrelevant():
     tabs = mesh.grid_tables(O.ps)
     E.set_mesh_grid(tabs)
     ref = E.mesh_error(x)
-    bad = []
-    t = {k: v.copy() for k, v in tabs.items()}
-    t["m"][3] = 0
-    bad.append(t)
-    t = {k: v.copy() for k, v in tabs.items()}
-    t["off"][-1] = tabs["pool"].size - 1
-    bad.append(t)
-    t = {k: v.copy() for k, v in tabs.items()}
-    t["off"][0] = -1
-    bad.append(t)
-    t = {k: v.copy() for k, v in tabs.items()}
-    t["pool"][7] = np.nan
-    bad.append(t)
-    t = {k: v.copy() for k, v in tabs.items()}
-    t["pool"][-1] = np.inf
-    bad.append(t)
-    t = {k: v.copy() for k, v in tabs.items()}
-    t["m"][0] = 2 ** 31 - 1
-    bad.append(t)
-    for t in bad:
-        with pytest.raises(engine.GelatoError, match="gelato_plan_set_mesh_grid"):
+    for t, why in _malformed_grids(tabs):
+        with pytest.raises(engine.GelatoError, match="gelato_plan_set_mesh_grid.*" + why):
             E.set_mesh_grid(t)
         assert _same_bits(E.mesh_error(x), ref)
     L = E.L
