@@ -127,11 +127,11 @@ k_jacobian_light(const __grid_constant__ PlanView P, const int32_t* __restrict__
   jacobian_body<JR_LIGHT>(P, block_table, n_scen, scen_ids, x_all, out_all, g_all);
 }
 
-// Vacuum dynamics nodes: GV_PARTS threads per node, a warp per part (jobs.h: dyn_noair_part); no shared memory, no
-// barrier.  A block is GV_PARTS warps = 32 nodes.
+// Vacuum dynamics nodes: GV_PARTS threads per node, a warp per part (jobs.h: dyn_noair_part).  A block is GV_PARTS
+// warps = 32 nodes; phase A stages each node's shared values in shared memory, one barrier, phase B.
 #define GV_THREADS (32 * GV_PARTS)
 #ifndef GV_MIN_BLOCKS
-#define GV_MIN_BLOCKS 5 /* the 158 registers ptxas would take leave 12 warps per SM; measured best of 1, 4, 5, 6, 8 */
+#define GV_MIN_BLOCKS 5 /* 96 registers, no spills; 4 (113 registers) measured slower, 6 spills (profiles/r05b_ab.txt) */
 #endif
 __global__ void __launch_bounds__(GV_THREADS, GV_MIN_BLOCKS)
 k_jacobian_noair(const __grid_constant__ PlanView P, const int first, const int count, const int n_scen,
@@ -141,7 +141,7 @@ k_jacobian_noair(const __grid_constant__ PlanView P, const int first, const int 
   const int scen = blockIdx.x / per;
   const int lane = threadIdx.x & 31, part = threadIdx.x >> 5;
   const int k = (blockIdx.x - scen * per) * 32 + lane;
-  __shared__ double grav[32][NPV * 3];  // the node's five gravity vectors, shared by the four parts
+  __shared__ NoairStage stage[32];  // per node: what its four parts share
   const double* x = x_all + (size_t)scen * P.n_vars;
   double* out = out_all + (size_t)scen * (size_t)(P.packed ? P.n_pack : P.n_vals);
   double* g = g_all ? g_all + (size_t)scen * P.n_rows : nullptr;
@@ -150,10 +150,10 @@ k_jacobian_noair(const __grid_constant__ PlanView P, const int first, const int 
   NodeRef nr;
   if (live) {
     nr = jac_node(P, first + k);
-    for (int pv = part; pv < NPV; pv += GV_PARTS) dyn_noair_gravity(P, sid, x, nr, pv, grav[lane] + 3 * pv);
+    dyn_noair_stage(P, sid, x, nr, part, stage[lane]);
   }
   __syncthreads();
-  if (live) dyn_noair_part(P, sid, x, out, g, nr, part, grav[lane]);
+  if (live) dyn_noair_part(P, sid, x, out, g, nr, part, stage[lane]);
 }
 
 #ifndef GR_MIN_BLOCKS

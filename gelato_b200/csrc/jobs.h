@@ -654,10 +654,10 @@ GM_HD_INL void dyn_noair_phase(const PlanView& P, int scen, const double* x, dou
 /* right-hand side is ~70 flops, so sharing gravity among its columns through   */
 /* shared memory and two block barriers cost more than it saved -- the blocks   */
 /* were latency bound with most threads idle (ncu r02b: 0.084 ms for 2 % of the */
-/* arithmetic).  Here a thread walks its node's columns in registers and stores */
-/* each quotient as soon as it has it; no shared memory, no barrier, and enough */
-/* resident threads to hide the chain.  Same per-(node, lane) functions, same   */
-/* bits.                                                                        */
+/* arithmetic).  Here a thread walks its share of a node's columns in registers */
+/* and stores each quotient as soon as it has it; one barrier (after the values */
+/* a node's threads share are staged) and enough resident threads to hide the  */
+/* chain.  Same per-(node, lane) formulas, same bits.                          */
 /* ========================================================================= */
 /* One node's columns in GV_PARTS independent parts (a warp per part in k_jacobian_noair: the parts differ in code
  * path, so they must not share a warp).  Every value is a pure function of (node, lane): each part recomputes the
@@ -669,67 +669,256 @@ GM_HD_INL void dyn_noair_phase(const PlanView& P, int scen, const double* x, dou
  * (The defects as a fifth part, 160-thread blocks, measured slower: 0.075 against 0.062 ms.)
  * The J2 gravity vector -- the expensive piece of a vacuum column -- has only NPV = 5 distinct arguments per node
  * (pristine, x / y / z perturbed, all restored); the parts would evaluate 10 of them between themselves.  Phase A
- * (dyn_noair_gravity, one variant per warp, the fourth warp two) puts the five into shared memory, phase B
- * (dyn_noair_part) reads them. */
+ * (dyn_noair_stage, one variant per warp, the first warp two) puts the five into shared memory, phase B
+ * (dyn_noair_part) reads them.  Phase A also stages what every part reads of the node -- its pristine mass,
+ * quaternion, velocity and controls, the section's times, thrust and output offsets -- so that phase B loads none
+ * of it from global memory, where every output store before a load would force that load to be issued again. */
 #define GV_PARTS 4
-P_HD void dyn_noair_gravity(const PlanView& P, int scen, const double* x, const NodeRef& nr, int pv, double* out3) {
+struct NoairStage {
+  double m, q[4], u[2], vel[3], to, tf, thrust;
+  double grav[NPV * 3]; /* [pv][3] */
+  int64_t sj[GS_I64_COLS]; /* the section's row of sec_pk (packed output) or sec_i64 (COO) */
+  double pad; /* an odd number of 8-byte words: an array of these, one per lane, is free of shared-memory bank conflicts */
+};
+static_assert(sizeof(NoairStage) % 16 == 8, "NoairStage: odd number of 8-byte words");
+
+/* phase A, warp `part`: its share of the node's stage */
+P_HD void dyn_noair_stage(const PlanView& P, int scen, const double* x, const NodeRef& nr, int part, NoairStage& s) {
   const Units un = scen_units(P, scen);
-  double p[3];
-  pos_variant(x + P.off_pos + 3 * nr.row, pv, un.dx, p);
-  const Vec3 gr = gravity_eci(v3(p[0] * un.pos, p[1] * un.pos, p[2] * un.pos));
-  out3[0] = gr.x; out3[1] = gr.y; out3[2] = gr.z;
+  const int row = nr.row;
+  for (int pv = part; pv < NPV; pv += GV_PARTS) {
+    double p[3];
+    pos_variant(x + P.off_pos + 3 * row, pv, un.dx, p);
+    const Vec3 gr = gravity_eci(v3(p[0] * un.pos, p[1] * un.pos, p[2] * un.pos));
+    s.grav[3 * pv] = gr.x; s.grav[3 * pv + 1] = gr.y; s.grav[3 * pv + 2] = gr.z;
+  }
+  if (part == 1) {
+    s.m = x[row];
+    for (int k = 0; k < 4; k++) s.q[k] = x[P.off_quat + 4 * row + k];
+    for (int k = 0; k < 2; k++) s.u[k] = (nr.flags & GSF_HOLD) ? 0.0 : x[P.off_u + 2 * (nr.ua + nr.j) + k];
+  } else if (part == 2) {
+    for (int k = 0; k < 3; k++) s.vel[k] = x[P.off_vel + 3 * row + k];
+    s.to = x[P.off_t + nr.sec];
+    s.tf = x[P.off_t + nr.sec + 1];
+  } else if (part == 3) {
+    s.thrust = sec_param(P, scen, nr.sec).thrust;
+    const int64_t* sj = (P.packed ? P.sec_pk : P.sec_i64) + nr.sec * GS_I64_COLS;
+    for (int c = 0; c < GS_I64_COLS; c++) s.sj[c] = sj[c];
+  }
 }
-/* grav: the node's NPV gravity vectors, [pv][3] */
-P_HD void dyn_noair_part(const PlanView& P, int scen, const double* x, double* vals, double* g, const NodeRef& nr, int part,
-                         const double* grav) {
-  const Units un = scen_units(P, scen);
+
+/* gm_div_by, with the zero numerator answered directly: a signed zero over a normal d is the zero with the sign
+ * a / d has.  The coast arcs' thrust is zero, and the division routine reaches that quotient only through its slow
+ * path.  Same bits as a / d. */
+P_HD double noair_div_by(double a, const GmRcp R) {
+  if (a == 0.0 && R.ok) return gm_u2d((gm_d2u(a) ^ gm_d2u(R.d)) & GM_SIGN_MASK);
+  return gm_div_by(a, R);
+}
+/* vacuum column `lane`: rhs_velocity_noair_col on the mass and quaternion dyn_col_state gives the lane and on the
+ * staged gravity of its position; Rv = gm_rcp(un.vel), shared by every column */
+P_HD void noair_col(const NoairStage& s, int lane, const Units& un, const GmRcp Rv, double* f) {
   const double dx = un.dx;
-  const SecParam sp = sec_param(P, scen, nr.sec);
+  double m = s.m;
+  if (lane == 1) m = m + dx;
+  else if (lane >= 2) m = residue(m, dx);
+  const int pidx = lane <= 11 ? lane - 1 : 11;
+  double q[4];
+#pragma unroll
+  for (int k = 0; k < 4; k++) {
+    double a = s.q[k];
+    if (lane != 0) {
+      if (7 + k < pidx) a = residue(a, dx);
+      else if (7 + k == pidx) a = a + dx;
+    }
+    q[k] = a;
+  }
+  const double mass = m * un.mass;
+  const Vec3 tdir = quatrot(quatconj(q4(q[0], q[1], q[2], q[3])), v3(1.0, 0.0, 0.0));
+  const Vec3 thr = scale3(s.thrust, tdir);
+  const GmRcp Rm = gm_rcp(mass);
+  const double* gv = s.grav + 3 * lane_pv(lane);
+  f[0] = noair_div_by(noair_div_by(thr.x, Rm) + gv[0], Rv);
+  f[1] = noair_div_by(noair_div_by(thr.y, Rm) + gv[1], Rv);
+  f[2] = noair_div_by(noair_div_by(thr.z, Rm) + gv[2], Rv);
+}
+/* dyn_quat_variant on the staged quaternion and controls, every index a constant (the variant is a loop variable
+ * of dyn_noair_part: indexing by it put qv / uv on the stack) */
+P_HD void noair_quat_variant(const NoairStage& s, int var, const Units& un, double* out) {
+  const double dx = un.dx;
+  double qv[4], uv[2];
+#pragma unroll
+  for (int k = 0; k < 4; k++) {
+    double a = s.q[k];
+    if (var != 7) a = residue(a, dx);
+    if (var >= 1 && var <= 4) {
+      if (k < var - 1) a = residue(a, dx);
+      else if (k == var - 1) a = a + dx;
+    } else if (var == 5 || var == 6) {
+      a = residue(a, dx);
+    }
+    qv[k] = a;
+  }
+#pragma unroll
+  for (int k = 0; k < 2; k++) {
+    double b = s.u[k];
+    if (var == 5 || var == 6) {
+      if (k < var - 5) b = residue(b, dx);
+      else if (k == var - 5) b = b + dx;
+    }
+    uv[k] = b;
+  }
+  const Quat d = rhs_quaternion(q4(qv[0], qv[1], qv[2], qv[3]), uv[0], uv[1], un.u);
+  out[0] = d.w; out[1] = d.x; out[2] = d.y; out[3] = d.z;
+}
+/* dyn_scatter for a vacuum node (no velocity / time finite differences), on the staged values; Rdx = gm_rcp(un.dx) */
+P_HD void dyn_noair_scatter(const PlanView& P, double* vals, const NodeRef& nr, const NoairStage& s, const Units& un,
+                            const GmRcp Rdx, int lane, const double* fc, const double* fl, const double* qc, const double* ql) {
+  const bool pk = P.packed != 0;
+  const int64_t* sj = s.sj;
+  const int n = nr.n, j = nr.j;
+  const double ut = un.t;
+  const double dt = s.tf - s.to;
+  const long long n3 = 3LL * n, n4 = 4LL * n;
+  if (lane >= 1 && lane <= 11 && !(lane >= 5 && lane <= 7)) {
+    double rh[3];
+    for (int k = 0; k < 3; k++) rh[k] = fd_div_by(-(fl[k] - fc[k]), Rdx) * dt * ut / 2.0;
+    const long long at = lane == 1 ? sj[GS_JV_MASS] : lane <= 4 ? sj[GS_JV_POS] + (lane - 2) * n3 : sj[GS_JV_QUAT] + (lane - 8) * n3;
+    for (int k = 0; k < 3; k++) vals[at + 3LL * j + k] = rh[k];
+  }
+  if (lane == 12) {
+    for (int k = 0; k < 3; k++) {
+      const double rh_to = fc[k] * ut / 2.0;
+      vals[sj[GS_JV_T] + 3LL * j + k] = rh_to;
+      if (!pk) vals[sj[GS_JV_T] + n3 + 3LL * j + k] = -rh_to;
+    }
+  }
+  if (lane == 14) {
+    const GmRcp Rp = gm_rcp(un.pos);
+    const double rh_vel = gm_div_by(-un.vel * dt * ut / 2.0, Rp);
+    if (pk) {
+      if (j == 0) vals[sj[GS_JP_VEL]] = rh_vel;
+    } else {
+      for (int k = 0; k < 3; k++) vals[sj[GS_JP_VEL] + 3LL * j + k] = rh_vel;
+    }
+    for (int k = 0; k < 3; k++) {
+      const double rh_to = gm_div_by(s.vel[k] * un.vel * ut / 2.0, Rp);
+      vals[sj[GS_JP_T] + 3LL * j + k] = rh_to;
+      if (!pk) vals[sj[GS_JP_T] + n3 + 3LL * j + k] = -rh_to;
+    }
+  }
+  if (!(nr.flags & GSF_HOLD)) {
+    if (lane >= 1 && lane <= 6) {
+      double rh[4];
+      for (int a = 0; a < 4; a++) rh[a] = fd_div_by(-(ql[a] - qc[a]), Rdx) * dt * ut / 2.0;
+      if (lane <= 4) {
+        const int kk = lane - 1;
+        const double d_diag = P.d_pool[nr.d_off + (long long)j * (n + 1) + (j + 1)];
+        for (int a = 0; a < 4; a++) {
+          const double base = (a == kk) ? d_diag : 0.0;
+          const long long at = pk ? (4LL * j + a) * 4 + kk : (4LL * j + a) * (4LL * (n + 1)) + 4LL * (j + 1) + kk;
+          vals[sj[GS_JQ_QUAT] + at] = base + rh[a];
+        }
+      } else {
+        for (int a = 0; a < 4; a++) vals[sj[GS_JQ_U] + (lane - 5) * n4 + 4LL * j + a] = rh[a];
+      }
+    } else if (lane == 0) {
+      for (int a = 0; a < 4; a++) {
+        const double rh_to = qc[a] * ut / 2.0;
+        vals[sj[GS_JQ_T] + 4LL * j + a] = rh_to;
+        if (!pk) vals[sj[GS_JQ_T] + n4 + 4LL * j + a] = -rh_to;
+      }
+    }
+  }
+}
+/* dx_dot<W> with the loads of four steps issued together, and optionally a one-column chain (the mass) in the same
+ * loop: every chain still accumulates m ascending from 0.0 (DESIGN.md H2), so the bits are dx_dot's, but a part of the
+ * vacuum kernel waits for loads (n + 1) / 4 times instead of (n + 1) / 2 times per array. */
+template <int W, bool MASS>
+P_HD void noair_dx_dot(const double* Drow, const double* xrows, const double* xmass, int n1, double* acc, double* acc_m) {
+  double am = 0.0;
+  for (int w = 0; w < W; w++) acc[w] = 0.0;
+  int m = 0;
+  for (; m + 4 <= n1; m += 4) {
+    double d[4], xv[4][W], xm[4];
+#pragma unroll
+    for (int t = 0; t < 4; t++) {
+      d[t] = Drow[m + t];
+      for (int w = 0; w < W; w++) xv[t][w] = xrows[(long long)(m + t) * W + w];
+      if (MASS) xm[t] = xmass[m + t];
+    }
+#pragma unroll
+    for (int t = 0; t < 4; t++) {
+      for (int w = 0; w < W; w++) acc[w] = gm_fma(d[t], xv[t][w], acc[w]);
+      if (MASS) am = gm_fma(d[t], xm[t], am);
+    }
+  }
+  for (; m < n1; m++) {
+    const double d0 = Drow[m];
+    for (int w = 0; w < W; w++) acc[w] = gm_fma(d0, xrows[(long long)m * W + w], acc[w]);
+    if (MASS) am = gm_fma(d0, xmass[m], am);
+  }
+  if (MASS) *acc_m = am;
+}
+/* dyn_lh_item of the groups part 1 (velocity), 2 (position) or 3 (quaternion and mass) of a vacuum node computes */
+P_HD void noair_lh(const PlanView& P, const double* x, const NodeRef& nr, int part, double* lh) {
+  const int n1 = nr.n + 1, xa = nr.si[GS_XA], row = nr.row;
+  const double* Drow = P.d_pool + nr.d_off + (long long)nr.j * n1;
+  if (part == 1) {
+    noair_dx_dot<3, false>(Drow, x + P.off_vel + 3 * xa, nullptr, n1, lh + 7, nullptr);
+  } else if (part == 2) {
+    noair_dx_dot<3, false>(Drow, x + P.off_pos + 3 * xa, nullptr, n1, lh, nullptr);
+  } else {
+    const bool qdot = !(nr.flags & GSF_HOLD), mdot = nr.flags & GSF_ENGINE_ON;
+    if (qdot && mdot) {
+      noair_dx_dot<4, true>(Drow, x + P.off_quat + 4 * xa, x + xa, n1, lh + 3, lh + 10);
+      return;
+    }
+    if (qdot) noair_dx_dot<4, false>(Drow, x + P.off_quat + 4 * xa, nullptr, n1, lh + 3, nullptr);
+    else
+      for (int k = 0; k < 4; k++) lh[3 + k] = x[P.off_quat + 4 * row + k] - x[P.off_quat + 4 * xa + k];
+    if (mdot) noair_dx_dot<1, false>(Drow, x + xa, nullptr, n1, lh + 10, nullptr);
+    else lh[10] = x[row] - x[xa];
+  }
+}
+/* phase B, warp `part` */
+P_HD void dyn_noair_part(const PlanView& P, int scen, const double* x, double* vals, double* g, const NodeRef& nr, int part,
+                         const NoairStage& s) {
+  const Units un = scen_units(P, scen);
+  const GmRcp Rv = gm_rcp(un.vel), Rdx = gm_rcp(un.dx);
   const bool hold = nr.flags & GSF_HOLD;
   double fc[3], fl[3], qc[4] = {0.0, 0.0, 0.0, 0.0}, ql[4] = {0.0, 0.0, 0.0, 0.0};
-  double v[11];
   /* centre column: pristine state, gravity at the pristine position */
-  dyn_col_state(P, x, nr.row, 0, false, dx, v);
-  Vec3 f = rhs_velocity_noair_col(v[0], q4(v[7], v[8], v[9], v[10]), v3(grav[0], grav[1], grav[2]), sp, un);
-  fc[0] = f.x; fc[1] = f.y; fc[2] = f.z;
-  if (!hold && part < 3) dyn_quat_variant(P, x, nr, un, 0, qc);
+  noair_col(s, 0, un, Rv, fc);
+  if (!hold && part < 3) noair_quat_variant(s, 0, un, qc);
   if (part == 0) {
-    dyn_scatter(P, scen, x, vals, nr, 0, fc, fc, qc, qc);   /* eqcon_dyn_quat / t */
-    dyn_scatter(P, scen, x, vals, nr, 12, fc, fc, qc, qc);  /* eqcon_dyn_vel / t (analytic in vacuum) */
-    dyn_scatter(P, scen, x, vals, nr, 14, fc, fc, qc, qc);  /* eqcon_dyn_pos / velocity, t */
+    dyn_noair_scatter(P, vals, nr, s, un, Rdx, 0, fc, fc, qc, qc);   /* eqcon_dyn_quat / t */
+    dyn_noair_scatter(P, vals, nr, s, un, Rdx, 12, fc, fc, qc, qc);  /* eqcon_dyn_vel / t (analytic in vacuum) */
+    dyn_noair_scatter(P, vals, nr, s, un, Rdx, 14, fc, fc, qc, qc);  /* eqcon_dyn_pos / velocity, t */
   }
   const int first = part == 0 ? 1 : part == 1 ? 3 : part == 2 ? 6 : 10;
   const int last = part == 0 ? 2 : part == 1 ? 5 : part == 2 ? 9 : 11;
   for (int lane = first; lane <= last; lane++) {
     if (lane == 7) continue;
     const bool vel_lane = lane >= 5 && lane <= 7;
-    if (!vel_lane) {
-      dyn_col_state(P, x, nr.row, lane, false, dx, v);
-      /* the position changes with lanes 2-4 and is fully restored from lane 5 on: lanes 8-11 share variant 4 */
-      const double* gv = grav + 3 * lane_pv(lane);
-      f = rhs_velocity_noair_col(v[0], q4(v[7], v[8], v[9], v[10]), v3(gv[0], gv[1], gv[2]), sp, un);
-      fl[0] = f.x; fl[1] = f.y; fl[2] = f.z;
-    }
-    if (!hold && lane <= 6) dyn_quat_variant(P, x, nr, un, lane, ql);
-    dyn_scatter(P, scen, x, vals, nr, lane, fc, fl, qc, ql);
+    /* the position changes with lanes 2-4 and is fully restored from lane 5 on: lanes 8-11 share variant 4 */
+    if (!vel_lane) noair_col(s, lane, un, Rv, fl);
+    if (!hold && lane <= 6) noair_quat_variant(s, lane, un, ql);
+    dyn_noair_scatter(P, vals, nr, s, un, Rdx, lane, fc, fl, qc, ql);
   }
   if (g && part > 0) { /* pair evaluation: the node's collocation defects, spread over the three lighter parts --
                           position | velocity | quaternion and mass (groups 0 | 2 | 1, 3 of dyn_lh_item) */
     double lh[11], qp[4] = {0.0, 0.0, 0.0, 0.0};
-    if (part == 3 && !hold) dyn_quat_variant(P, x, nr, un, 7, qp);
+    if (part == 3 && !hold) noair_quat_variant(s, 7, un, qp);
     const int g0 = part == 2 ? 0 : part == 1 ? 2 : 1;
-    dyn_lh_item(P, x, nr, g0, lh);
+    noair_lh(P, x, nr, part, lh);
     dyn_res_finish(P, scen, x, g, nr, g0, lh, fc, qp);
-    if (part == 3) {
-      dyn_lh_item(P, x, nr, 3, lh);
-      dyn_res_finish(P, scen, x, g, nr, 3, lh, fc, qp);
-    }
+    if (part == 3) dyn_res_finish(P, scen, x, g, nr, 3, lh, fc, qp);
   }
 }
 P_HD void dyn_noair_node(const PlanView& P, int scen, const double* x, double* vals, double* g, const NodeRef& nr) {
-  double grav[NPV * 3];
-  for (int pv = 0; pv < NPV; pv++) dyn_noair_gravity(P, scen, x, nr, pv, grav + 3 * pv);
-  for (int part = 0; part < GV_PARTS; part++) dyn_noair_part(P, scen, x, vals, g, nr, part, grav);
+  NoairStage s;
+  for (int part = 0; part < GV_PARTS; part++) dyn_noair_stage(P, scen, x, nr, part, s);
+  for (int part = 0; part < GV_PARTS; part++) dyn_noair_part(P, scen, x, vals, g, nr, part, s);
 }
 
 /* ========================================================================= */
