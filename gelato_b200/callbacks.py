@@ -56,7 +56,7 @@ class GelatoProblem:
         self.fuse_pair = bool(fuse_pair) and self.reuse_output and hasattr(self.engine, "eval_pair_update")
         self._x_pair = None  # the decision vector the kept Jacobian belongs to
         self._pair_fresh = False
-        self._mesh_grid = False
+        self._mesh_grid = None  # the tables of the engine's mesh grid (mesh.grid_tables), once set
 
     # -- helpers ---------------------------------------------------------
     def pack(self, xdict):
@@ -139,13 +139,41 @@ class GelatoProblem:
         """{event name: err[11]}: the collocation error estimate of each section between its nodes, per state component
         (mass | position 3 | velocity 3 | quaternion 4), on the default test grid (n + 1 points, set on first use).
         gelato_b200.mesh.refine_nodes takes the result as it is (DESIGN.md section 11)."""
-        if not self._mesh_grid:
-            from . import mesh
-
-            self.engine.set_mesh_grid(mesh.grid_tables(self.plan.ps))
-            self._mesh_grid = True
+        self._default_mesh_grid()
         err = self.engine.mesh_error(self.pack(xdict))
         return {prm["name"]: err[i] for i, prm in enumerate(self.plan.p["params"][: self.plan.S])}
+
+    _AERO_KEYS = ("ineqcon_alpha", "ineqcon_q", "ineqcon_qalpha")
+
+    def path_check(self, xdict):
+        """{(funcs key, event name): (residual, time_s)}: for each aero constraint over a whole section (range "all"),
+        the smallest value of its row's expression 1 - f / limit between the nodes -- on the default test grid (n + 1
+        points, set on first use and shared with mesh_error) -- and the flight time [s] of the test point where it
+        occurs.  The NLP only holds the rows at the nodes; a negative residual is a violation in between.
+        gelato_b200.mesh.refine_nodes takes the result as its `path` argument (DESIGN.md section 11)."""
+        tables = self._default_mesh_grid()
+        x = self.pack(xdict)
+        res, at = self.engine.path_check(x)
+        t = x[-(self.plan.S + 1):]
+        out = {}
+        for j, (kind, i, nk, _) in enumerate(self.plan.aero_i32):
+            if nk == 1:  # "initial": a point constraint, nothing between nodes
+                continue
+            to, tf = t[i], t[i + 1]
+            tau = tables["pool"][tables["off"][i] + at[j]]  # tau_t[at] of section i
+            out[(self._AERO_KEYS[kind], self.plan.p["params"][i]["name"])] = (
+                float(res[j]), float((tau * (tf - to) / 2 + (tf + to) / 2) * self.plan.units[4]))
+        return out
+
+    def _default_mesh_grid(self):
+        """The grid of mesh_error and path_check (n + 1 test points per section): set on the engine on first use."""
+        if self._mesh_grid is None:
+            from . import mesh
+
+            tables = mesh.grid_tables(self.plan.ps)
+            self.engine.set_mesh_grid(tables)
+            self._mesh_grid = tables
+        return self._mesh_grid
 
     # -- flat-vector variants (no dictionaries), used by benchmarks / batched drivers
     def residuals(self, x, n_scen=1):

@@ -254,6 +254,31 @@ k_mesh_error(const __grid_constant__ PlanView P, const MeshSec* __restrict__ ms,
   err_all[i] = mesh_component(P, x_all + (size_t)scen * P.n_vars, sec, tb, s.m, pts, c);
 }
 
+// Path check (mesh_error.h; DESIGN.md section 11), two launches on the same grid.  First one thread per (scenario, test
+// point of an aero job over a whole section): the residual 1 - f there into r[n_scen][n_pts].  Then one thread per
+// (scenario, aero job): its minimum and the test point of the minimum, res / at [n_scen][n_aero].
+__global__ void __launch_bounds__(GM_THREADS)
+k_path_points(const __grid_constant__ PlanView P, const PathPt* __restrict__ pt, const MeshSec* __restrict__ ms,
+              const double* __restrict__ pool, int n_pts, int n_scen, const double* __restrict__ x_all,
+              double* __restrict__ r_all) {
+  const long long i = (long long)blockIdx.x * GM_THREADS + threadIdx.x;
+  if (i >= (long long)n_pts * n_scen) return;
+  const int scen = (int)(i / n_pts), k = (int)(i - (long long)scen * n_pts);
+  const PathPt q = pt[k];
+  const int sec = P.aero_i32[q.job * GA_I32_COLS + GA_SECTION];
+  const MeshTabs tb = mesh_tabs(pool, ms[sec], P.sec_i32[sec * GS_I32_COLS + GS_N]);
+  r_all[i] = mesh_path_point(P, scen, x_all + (size_t)scen * P.n_vars, q.job, tb, q.l);
+}
+__global__ void __launch_bounds__(GM_THREADS)
+k_path_min(int n_aero, const int32_t* __restrict__ job0, int n_pts, int n_scen, const double* __restrict__ r_all,
+           double* __restrict__ res_all, int32_t* __restrict__ at_all) {
+  const long long i = (long long)blockIdx.x * GM_THREADS + threadIdx.x;
+  if (i >= (long long)n_aero * n_scen) return;
+  const int scen = (int)(i / n_aero), j = (int)(i - (long long)scen * n_aero);
+  const int p0 = job0[j];
+  mesh_path_min(r_all + (size_t)scen * n_pts + p0, job0[j + 1] - p0, res_all + i, at_all + i);
+}
+
 // probe: is a*b+c left unfused?  (1 + 2^-30)(1 - 2^-30) - 1 is 0 unfused, -2^-60 fused
 __global__ void k_unfused_probe(double a, double b, double c, double* out) { *out = a * b + c; }
 
@@ -380,6 +405,15 @@ struct GelatoPlan {
   DeviceBuf<double> d_mesh_pool, d_mesh_pts, d_err;
   PinnedBuf<double> h_err;
   int n_mesh_pts = 0;
+  // path check on the same grid: the test points of the aero jobs over a whole section and each job's first one
+  // (plan_host.h: build_path_points, rebuilt with the grid), the per-point scratch d_path_r, the host entry's staging
+  std::vector<int32_t> aero_i32;  // the aero jobs, as the plan description gave them
+  DeviceBuf<PathPt> d_path_pt;
+  DeviceBuf<int32_t> d_path_job0, d_at;
+  DeviceBuf<double> d_path_r, d_res;
+  PinnedBuf<double> h_res;
+  PinnedBuf<int32_t> h_at;
+  int n_path_pts = 0;
   long long launches = 0;
   Event ev0, ev1;
 };
@@ -538,6 +572,7 @@ int gelato_plan_create(const GelatoPlanDesc* d, int device, GelatoPlan** out) {
   int rc;
 #define UP(dst, src, count) if ((rc = upload(p->owned, src, (size_t)(count), &(dst))) != GELATO_OK) return rc;
   for (int i = 0; i < S; i++) p->sec_n.push_back(d->sec_i32[i * GS_I32_COLS + GS_N]);
+  if (d->n_aero > 0) p->aero_i32.assign(d->aero_i32, d->aero_i32 + (size_t)d->n_aero * GA_I32_COLS);
   UP(v.sec_i32, d->sec_i32, (size_t)S * GS_I32_COLS)
   UP(v.sec_i64, d->sec_i64, (size_t)S * GS_I64_COLS)
   UP(v.sec_f64, d->sec_f64, (size_t)S * GS_F64_COLS)
@@ -863,8 +898,10 @@ static const double* host_src(const double* x, double* stage, size_t n) {
 }
 
 // The destination of the download of a caller's out[n] (out == NULL: none): out itself when it is page-locked, else
-// `stage`, grown as needed; land() copies it over once the download is complete.
-static int host_dst(double* out, PinnedBuf<double>& stage, size_t n, double** dst) {
+// `stage`, grown as needed; land() copies it over once the download is complete.  (Templates: C++ linkage.)
+extern "C++" {
+template <typename T>
+static int host_dst(T* out, PinnedBuf<T>& stage, size_t n, T** dst) {
   *dst = out;
   if (!out || is_pinned(out)) return GELATO_OK;
   CU(stage.reserve(n));
@@ -872,8 +909,10 @@ static int host_dst(double* out, PinnedBuf<double>& stage, size_t n, double** ds
   return GELATO_OK;
 }
 
-static void land(double* out, const double* dst, size_t n) {
-  if (dst != out) memcpy(out, dst, n * sizeof(double));
+template <typename T>
+static void land(T* out, const T* dst, size_t n) {
+  if (dst != out) memcpy(out, dst, n * sizeof(T));
+}
 }
 
 static int eval_host(GelatoPlan* p, int which, const double* x, double* out, int32_t n_scen,
@@ -966,17 +1005,27 @@ int gelato_plan_set_mesh_grid(GelatoPlan* p, const GelatoMeshGridDesc* g) {
   std::vector<MeshSec> secs;
   std::vector<MeshPt> pts;
   if (const char* why = build_mesh_grid(g, p->sec_n.data(), p->view.S, secs, pts)) return fail(GELATO_ERR_ARG, why);
+  std::vector<PathPt> path_pts;
+  std::vector<int32_t> job0;
+  if (const char* why = build_path_points(p->aero_i32.data(), p->view.n_aero, secs, path_pts, job0))
+    return fail(GELATO_ERR_ARG, why);
   CU(cudaSetDevice(p->device));
   CU(cudaDeviceSynchronize());  // nothing in flight may still read the grid being replaced
   CU(p->d_mesh_sec.reserve(secs.size()));
   CU(p->d_mesh_pt.reserve(pts.size()));
   CU(p->d_mesh_pool.reserve((size_t)g->pool_len));
+  CU(p->d_path_pt.reserve(path_pts.size()));
+  CU(p->d_path_job0.reserve(job0.size()));
   const cudaStream_t st = p->lanes[0].stream;
   CU(cudaMemcpyAsync(p->d_mesh_sec.get(), secs.data(), secs.size() * sizeof(MeshSec), cudaMemcpyHostToDevice, st));
   CU(cudaMemcpyAsync(p->d_mesh_pt.get(), pts.data(), pts.size() * sizeof(MeshPt), cudaMemcpyHostToDevice, st));
   CU(cudaMemcpyAsync(p->d_mesh_pool.get(), g->pool, (size_t)g->pool_len * sizeof(double), cudaMemcpyHostToDevice, st));
+  if (!path_pts.empty())
+    CU(cudaMemcpyAsync(p->d_path_pt.get(), path_pts.data(), path_pts.size() * sizeof(PathPt), cudaMemcpyHostToDevice, st));
+  CU(cudaMemcpyAsync(p->d_path_job0.get(), job0.data(), job0.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
   CU(cudaStreamSynchronize(st));
   p->n_mesh_pts = (int)pts.size();
+  p->n_path_pts = (int)path_pts.size();
   return GELATO_OK;
 }
 
@@ -999,7 +1048,7 @@ int gelato_eval_mesh_error_dev(GelatoPlan* p, const double* x_dev, double* err_d
   cudaStream_t st;
   int rc = begin_dev(p, n_scen, stream, &st);
   if (rc) return rc;
-  if (!p->n_mesh_pts) return fail(GELATO_ERR_ARG, "no mesh grid set (gelato_plan_set_mesh_grid)");
+  if (!p->n_mesh_pts) return fail(GELATO_ERR_ARG, GELATO_NO_MESH_GRID);
   if (!x_dev || !err_dev) return fail(GELATO_ERR_ARG, "null buffer");
   return launch_mesh_error(p, x_dev, err_dev, n_scen, st);
 }
@@ -1007,7 +1056,7 @@ int gelato_eval_mesh_error_dev(GelatoPlan* p, const double* x_dev, double* err_d
 int gelato_eval_mesh_error(GelatoPlan* p, const double* x, double* err, int32_t n_scen) {
   int rc = check_scen(p, n_scen);
   if (rc) return rc;
-  if (!p->n_mesh_pts) return fail(GELATO_ERR_ARG, "no mesh grid set (gelato_plan_set_mesh_grid)");
+  if (!p->n_mesh_pts) return fail(GELATO_ERR_ARG, GELATO_NO_MESH_GRID);
   if (!x || !err) return fail(GELATO_ERR_ARG, "null buffer");
   CU(cudaSetDevice(p->device));
   if ((rc = ensure_staging(p, n_scen))) return rc;
@@ -1021,6 +1070,64 @@ int gelato_eval_mesh_error(GelatoPlan* p, const double* x, double* err, int32_t 
   CU(cudaMemcpyAsync(dst, p->d_err.get(), ne * sizeof(double), cudaMemcpyDeviceToHost, st));
   CU(cudaStreamSynchronize(st));
   land(err, dst, ne);
+  return GELATO_OK;
+}
+
+// ---- path check (mesh_error.h) ----
+// The launches of one check on `st`: none without aero jobs, k_path_points only when a job runs over a whole section;
+// the point scratch grows to the batch (DeviceBuf::reserve synchronises).
+static int launch_path_check(GelatoPlan* p, const double* x_dev, double* res_dev, int32_t* at_dev, int n_scen,
+                             cudaStream_t st) {
+  const int n_aero = p->view.n_aero, n_pts = p->n_path_pts;
+  if (!n_aero) return GELATO_OK;
+  const long long n1 = (long long)n_scen * n_pts, n2 = (long long)n_scen * n_aero;
+  if ((std::max(n1, n2) + GM_THREADS - 1) / GM_THREADS > 0x7fffffffLL)
+    return fail(GELATO_ERR_ARG, "test points x n_scen exceeds the grid limit");
+  CU(p->d_path_r.reserve((size_t)n1));
+  if (n1 > 0) {
+    k_path_points<<<(unsigned)((n1 + GM_THREADS - 1) / GM_THREADS), GM_THREADS, 0, st>>>(
+        p->view, p->d_path_pt.get(), p->d_mesh_sec.get(), p->d_mesh_pool.get(), n_pts, n_scen, x_dev, p->d_path_r.get());
+    p->launches++;
+  }
+  k_path_min<<<(unsigned)((n2 + GM_THREADS - 1) / GM_THREADS), GM_THREADS, 0, st>>>(
+      n_aero, p->d_path_job0.get(), n_pts, n_scen, p->d_path_r.get(), res_dev, at_dev);
+  p->launches++;
+  CU(cudaGetLastError());
+  return GELATO_OK;
+}
+
+int gelato_eval_path_check_dev(GelatoPlan* p, const double* x_dev, double* res_dev, int32_t* at_dev, int32_t n_scen,
+                               void* stream) {
+  cudaStream_t st;
+  int rc = begin_dev(p, n_scen, stream, &st);
+  if (rc) return rc;
+  if (!p->n_mesh_pts) return fail(GELATO_ERR_ARG, GELATO_NO_MESH_GRID);
+  if (!x_dev || (p->view.n_aero && (!res_dev || !at_dev))) return fail(GELATO_ERR_ARG, "null buffer");
+  return launch_path_check(p, x_dev, res_dev, at_dev, n_scen, st);
+}
+
+int gelato_eval_path_check(GelatoPlan* p, const double* x, double* res, int32_t* at, int32_t n_scen) {
+  int rc = check_scen(p, n_scen);
+  if (rc) return rc;
+  if (!p->n_mesh_pts) return fail(GELATO_ERR_ARG, GELATO_NO_MESH_GRID);
+  if (!x || (p->view.n_aero && (!res || !at))) return fail(GELATO_ERR_ARG, "null buffer");
+  if (!p->view.n_aero) return GELATO_OK;
+  CU(cudaSetDevice(p->device));
+  if ((rc = ensure_staging(p, n_scen))) return rc;
+  const cudaStream_t st = p->lanes[0].stream;
+  const size_t nx = (size_t)n_scen * p->view.n_vars, na = (size_t)n_scen * p->view.n_aero;
+  CU(p->d_res.reserve(na));
+  CU(p->d_at.reserve(na));
+  CU(cudaMemcpyAsync(p->d_x.get(), host_src(x, p->h_x.get(), nx), nx * sizeof(double), cudaMemcpyHostToDevice, st));
+  if ((rc = launch_path_check(p, p->d_x.get(), p->d_res.get(), p->d_at.get(), n_scen, st))) return rc;
+  double* res_dst;
+  int32_t* at_dst;
+  if ((rc = host_dst(res, p->h_res, na, &res_dst)) || (rc = host_dst(at, p->h_at, na, &at_dst))) return rc;
+  CU(cudaMemcpyAsync(res_dst, p->d_res.get(), na * sizeof(double), cudaMemcpyDeviceToHost, st));
+  CU(cudaMemcpyAsync(at_dst, p->d_at.get(), na * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+  CU(cudaStreamSynchronize(st));
+  land(res, res_dst, na);
+  land(at, at_dst, na);
   return GELATO_OK;
 }
 

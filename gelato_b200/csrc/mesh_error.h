@@ -10,6 +10,10 @@
  * with X_0 the section's first state row (mesh_component).  Every sum is a fused multiply-add chain with ascending
  * index from 0.0, and max and division are exact, so the result has one value: the kernels, the host emulator
  * (tests/emu/emu.cpp) and the oracle (tests/mesh_oracle.py) agree bit for bit.
+ *
+ * The path check runs on the same grid: the aero constraints' residual 1 - f at every test point of every aero job over
+ * a whole section (mesh_path_point), and its minimum per job (mesh_path_min).  Min and 1 - f are exact, so it too has
+ * one value.
  */
 #ifndef GELATO_B200_MESH_ERROR_H_
 #define GELATO_B200_MESH_ERROR_H_
@@ -28,6 +32,10 @@ struct MeshSec {
 /* one test point: its section and its index inside the section */
 struct MeshPt {
   int32_t sec, l;
+};
+/* one test point of the path check: an aero job over a whole section and the index of the test point in that section */
+struct PathPt {
+  int32_t job, l;
 };
 
 struct MeshTabs {
@@ -91,6 +99,40 @@ P_HD void mesh_point(const PlanView& P, int scen, const double* x, int sec, cons
     rh[9] = d.y * dt * ut / 2.0;
     rh[10] = d.z * dt * ut / 2.0;
   }
+}
+
+/* The path check (DESIGN.md section 11): one test point of an aero job.  The job's section is interpolated at test
+ * point l with the chains of mesh_point (v = its xl[1..10]: position | velocity | quaternion), and the residual is the
+ * expression aero_res gives objfunc's row at a node: pristine x, the time of the test point, the scenario's units and
+ * wind table.  At a test point that is a node it is that row's value, bit for bit. */
+P_HD double mesh_path_point(const PlanView& P, int scen, const double* x, int job, const MeshTabs& tb, int l) {
+  const int32_t* ai = P.aero_i32 + job * GA_I32_COLS;
+  const int sec = ai[GA_SECTION];
+  const int32_t* si = P.sec_i32 + sec * GS_I32_COLS;
+  const int n = si[GS_N], xa = si[GS_XA];
+  const double* Prow = tb.P + (long long)l * (n + 1);
+  double v[10];
+  dx_dot<3>(Prow, x + P.off_pos + 3 * xa, n + 1, v);
+  dx_dot<3>(Prow, x + P.off_vel + 3 * xa, n + 1, v + 3);
+  dx_dot<4>(Prow, x + P.off_quat + 4 * xa, n + 1, v + 6);
+  const double tn = time_node(tb.tau, l + 1, x[P.off_t + sec], x[P.off_t + sec + 1]);
+  return 1.0 - aero_value(P, scen, ai[GA_KIND], v, tn, P.aero_f64[job * GA_F64_COLS + GA_LIMIT]);
+}
+
+/* min and argmin of r[0 .. m) as numpy.min / numpy.argmin give them: ties go to the first, a NaN wins (the first NaN);
+ * m == 0 (an "initial" job, a point constraint with nothing between nodes): +inf at -1 */
+P_HD void mesh_path_min(const double* r, int m, double* res, int32_t* at) {
+  double best = gm_inf();
+  int32_t k_best = -1;
+  for (int k = 0; k < m; k++) {
+    const double v = r[k];
+    if (k == 0 || v < best || (v != v && best == best)) {
+      best = v;
+      k_best = k;
+    }
+  }
+  *res = best;
+  *at = k_best;
 }
 
 /* max as numpy's: a NaN operand makes the result NaN */

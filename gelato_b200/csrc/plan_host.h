@@ -1,7 +1,7 @@
 /* plan_host.h -- host-side helpers shared by the CUDA library and the test
  * emulator: PlanView scalar fields from a GelatoPlanDesc, the node / row lists
  * and the block tables of the two kernels, and the test grid of the mesh error
- * estimate. */
+ * estimate and of the path check. */
 #ifndef GELATO_B200_PLAN_HOST_H_
 #define GELATO_B200_PLAN_HOST_H_
 
@@ -317,6 +317,9 @@ static inline void build_host_tables(const GelatoPlanDesc* d, HostTables& h) {
   push_chunks(rb, BR_LIN, 0, d->n_lin, GR_THREADS);
 }
 
+/* why the mesh error estimate and the path check refuse a call before a grid is set */
+#define GELATO_NO_MESH_GRID "no mesh grid set (gelato_plan_set_mesh_grid)"
+
 /* The test grid of the mesh error estimate (include/gelato_b200.h: GelatoMeshGridDesc) over S sections of n[i] LGR
  * nodes: its sections and the list of its test points.  Returns NULL or why the grid is refused.  The kernels trust
  * the grid, so one that fails here is not uploaded. */
@@ -337,6 +340,25 @@ static inline const char* build_mesh_grid(const GelatoMeshGridDesc* g, const int
   }
   for (int64_t k = 0; k < g->pool_len; k++)
     if (!std::isfinite(g->pool[k])) return "the table pool holds a value that is not finite";
+  return nullptr;
+}
+
+/* The test points of the path check on the grid `secs` (build_mesh_grid): every test point of the section of every aero
+ * job over a whole section (GA_NK > 1), job by job in the plan's order, l ascending.  Job k's points are [job0[k],
+ * job0[k + 1]); an "initial" job (GA_NK == 1) has none.  Returns NULL or why the grid is refused. */
+static inline const char* build_path_points(const int32_t* aero_i32, int n_aero, const std::vector<MeshSec>& secs,
+                                            std::vector<PathPt>& pts, std::vector<int32_t>& job0) {
+  pts.clear();
+  job0.assign(1, 0);
+  for (int k = 0; k < n_aero; k++) {
+    const int32_t* ai = aero_i32 + (size_t)k * GA_I32_COLS;
+    if (ai[GA_NK] > 1) {
+      const int m = secs[ai[GA_SECTION]].m;
+      if ((long long)pts.size() + m > 0x7fffffffLL) return "too many test points";
+      for (int l = 0; l < m; l++) pts.push_back(PathPt{k, l});
+    }
+    job0.push_back((int32_t)pts.size());
+  }
   return nullptr;
 }
 

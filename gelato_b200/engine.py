@@ -233,6 +233,8 @@ def load_library():
     L.gelato_plan_set_mesh_grid.argtypes = [vp, ctypes.POINTER(MeshGridDesc)]
     L.gelato_eval_mesh_error.argtypes = [vp, _pd, _pd, ctypes.c_int32]
     L.gelato_eval_mesh_error_dev.argtypes = [vp, vp, vp, ctypes.c_int32, vp]
+    L.gelato_eval_path_check.argtypes = [vp, _pd, _pd, _pi32, ctypes.c_int32]
+    L.gelato_eval_path_check_dev.argtypes = [vp, vp, vp, vp, ctypes.c_int32, vp]
     L.gelato_eval_jacobian.argtypes = [vp, _pd, _pd, ctypes.c_int32]
     L.gelato_eval_residuals_ids.argtypes = [vp, _pd, _pd, ctypes.c_int32, _pi32]
     L.gelato_eval_jacobian_ids.argtypes = [vp, _pd, _pd, ctypes.c_int32, _pi32]
@@ -297,7 +299,8 @@ EXPORTS = (
     "gelato_leaf_dynamics_quaternion gelato_leaf_aero gelato_leaf_eci2geodetic gelato_leaf_gravity gelato_leaf_iip "
     "gelato_leaf_atmosphere gelato_leaf_output_table gelato_init_rocket_simulation gelato_leaf_coordinate "
     "gelato_eval_pair_packed_range_dev gelato_plan_set_fd gelato_plan_get_fd "
-    "gelato_plan_set_mesh_grid gelato_eval_mesh_error gelato_eval_mesh_error_dev"
+    "gelato_plan_set_mesh_grid gelato_eval_mesh_error gelato_eval_mesh_error_dev "
+    "gelato_eval_path_check gelato_eval_path_check_dev"
 ).split()
 
 
@@ -397,6 +400,28 @@ class Engine:
 
     def mesh_error_dev(self, x_ptr, err_ptr, n_scen=1, stream=None):
         _check(self.L, self.L.gelato_eval_mesh_error_dev(self.h, x_ptr, err_ptr, n_scen, stream), "gelato_eval_mesh_error_dev")
+
+    def path_check(self, x, n_scen=1, out=None):
+        """(res, at) of the decision vectors x[n_scen][n_vars], [n_aero] each (n_scen > 1: [n_scen][n_aero]), in the
+        plan's aero-job order: per aero job the smallest residual 1 - f / limit over the test points of its section on
+        the mesh grid, and the index of that test point (an "initial" job: +inf and -1).  out: (res float64, at int32)
+        buffers of n_scen * n_aero entries (page-locked ones are DMA'd directly)."""
+        x = self._x(x, n_scen)
+        self.calls += 1
+        n = n_scen * self.plan.n_aero
+        if out is not None:
+            res, at = _out(out[0], n, "out[0]"), out[1]
+            if not isinstance(at, np.ndarray) or at.dtype != np.int32 or not at.flags.c_contiguous or at.size != n:
+                raise ValueError("out[1] must be a C-contiguous int32 numpy array of %d entries" % n)
+        else:
+            res, at = np.empty(n), np.empty(n, dtype=np.int32)
+        _check(self.L, self.L.gelato_eval_path_check(self.h, _ptr(x, _pd), _ptr(res, _pd), _ptr(at, _pi32), n_scen),
+               "gelato_eval_path_check")
+        return (res, at) if n_scen == 1 else (res.reshape(n_scen, -1), at.reshape(n_scen, -1))
+
+    def path_check_dev(self, x_ptr, res_ptr, at_ptr, n_scen=1, stream=None):
+        _check(self.L, self.L.gelato_eval_path_check_dev(self.h, x_ptr, res_ptr, at_ptr, n_scen, stream),
+               "gelato_eval_path_check_dev")
 
     # ---- host-buffer calls (what objfunc / sens use) --------------------
     def _x(self, x, n_scen):

@@ -7,8 +7,12 @@ of the event mesh and the transfer of a solution onto the refined mesh.
     events2, report = mesh.refine_nodes(events, err, tol=1e-6, n_max=30)
     ... build the problem of events2, then x2 = mesh.transfer(xdict, ps, ps2) and re-solve from x2
 
-The estimate itself runs on the GPU (gelato_b200.cu: k_mesh_points, k_mesh_error); this module only builds its float64
-tables once per mesh and does the host-side bookkeeping of a refinement.
+With GelatoProblem, `prob.path_check(xdict)` (the aero constraints between the nodes, on the same grid) can drive the
+refinement too: refine_nodes(events, err, tol, n_max, path=prob.path_check(xdict)).
+
+The estimate and the path check run on the GPU (gelato_b200.cu: k_mesh_points, k_mesh_error, k_path_points,
+k_path_min); this module only builds their float64 tables once per mesh and does the host-side bookkeeping of a
+refinement.
 """
 import collections
 import copy
@@ -71,17 +75,38 @@ def grid_tables(ps, m=None):
     return {"m": np.array(ms, dtype=np.int32), "off": np.array(off, dtype=np.int64), "pool": np.concatenate(parts)}
 
 
-Refinement = collections.namedtuple("Refinement", "name n_old n_new err capped")
+Refinement = collections.namedtuple("Refinement", "name n_old n_new err capped path", defaults=(None,))
 
 
-def refine_nodes(events, err, tol, n_max):
+def _worst_path(events, path):
+    """[S] worst path residual per section from GelatoProblem.path_check's {(key, event name): (residual, time_s)} or
+    from [S] values; +inf for a section without an aero job over it."""
+    S = len(events) - 1
+    if isinstance(path, dict):
+        worst = {e["name"]: np.inf for e in events[:S]}
+        for (_, name), (r, _) in path.items():
+            worst[name] = r if r != r else min(worst[name], r)
+        path = [worst[e["name"]] for e in events[:S]]
+    path = np.asarray(path, dtype=np.float64).reshape(S)
+    if np.isnan(path).any() or np.isneginf(path).any():
+        raise ValueError("the path residual is not finite")
+    return path
+
+
+def refine_nodes(events, err, tol, n_max, path=None, path_tol=1e-3):
     """p-refinement: (new events, report).  `events` are the problem's event records (S + 1, the last one ends the
     flight), `err` the estimate per section ([S][11], or {event name: err[11]} as GelatoProblem.mesh_error returns it).
 
     A section whose largest component error e exceeds tol gets n + max(1, ceil(log(e / tol) / log(max(n, 2)))) nodes,
     at most n_max.  Only `num_nodes` changes: no event is added, so time_ref chains and attitude modes keep their
     meaning.  The report has one Refinement per section; `capped` marks a section that stays above tol because its
-    count would exceed n_max (it is reported, not split)."""
+    count would exceed n_max (it is reported, not split).
+
+    path: the aero path constraints between the nodes, as GelatoProblem.path_check returns them or as [S] worst
+    residuals per section.  A section whose worst residual r is below -path_tol also gets the increment above, with -r
+    and path_tol in place of e and tol; the section takes the larger of the two counts, at most n_max, and its report
+    carries r in `path` (None for a section without an aero job over it).  Without `path` the result is that of the
+    estimate alone."""
     if not tol > 0.0:
         raise ValueError("tol must be positive")
     S = len(events) - 1
@@ -90,6 +115,10 @@ def refine_nodes(events, err, tol, n_max):
     err = np.asarray(err, dtype=np.float64).reshape(S, -1)
     if not np.isfinite(err).all():
         raise ValueError("the error estimate is not finite")
+    if path is not None:
+        if not path_tol > 0.0:
+            raise ValueError("path_tol must be positive")
+        path = _worst_path(events, path)
     out = copy.deepcopy(events)
     report = []
     for i in range(S):
@@ -97,9 +126,14 @@ def refine_nodes(events, err, tol, n_max):
         want = n
         if e > tol:
             want = n + max(1, math.ceil(math.log(e / tol) / math.log(max(n, 2))))
+        r = None
+        if path is not None and np.isfinite(path[i]):
+            r = float(path[i])
+            if r < -path_tol:
+                want = max(want, n + max(1, math.ceil(math.log(-r / path_tol) / math.log(max(n, 2)))))
         n_new = min(want, max(n, int(n_max)))
         out[i]["num_nodes"] = n_new
-        report.append(Refinement(events[i]["name"], n, n_new, e, want > n_new))
+        report.append(Refinement(events[i]["name"], n, n_new, e, want > n_new, r))
     return out, report
 
 

@@ -314,6 +314,27 @@ int gelato_plan_set_mesh_grid(GelatoPlan* plan, const GelatoMeshGridDesc* grid);
 int gelato_eval_mesh_error(GelatoPlan* plan, const double* x, double* err, int32_t n_scen);
 int gelato_eval_mesh_error_dev(GelatoPlan* plan, const double* x_dev, double* err_dev, int32_t n_scen, void* stream);
 
+/* Path check (DESIGN.md section 11): do the aero constraints (ineqcon_alpha, ineqcon_q, ineqcon_qalpha) hold BETWEEN the
+ * nodes?  The NLP enforces them at the state nodes only.  On the grid of gelato_plan_set_mesh_grid, for scenario s and
+ * aero job j of the plan (section i, limit L), at each test point l of section i:
+ *     v_l = position | velocity | quaternion interpolated with the grid's P row (the chains of the mesh error estimate)
+ *     t_l = tau_t[l] (tf - to) / 2 + (tf + to) / 2,   to = t[i], tf = t[i + 1]
+ *     r_l = 1 - f(v_l, t_l) / L
+ * with f exactly the function objfunc's row of the job evaluates at a node (pristine x, the scenario's units and wind
+ * table); res[s][j] = min_l r_l and at[s][j] = the l of the minimum (ties: the smallest l; a NaN is the minimum, the
+ * first NaN's l, as numpy.min / numpy.argmin).  A job with range "initial" (one row) is a point constraint with
+ * nothing between nodes: res = +inf, at = -1.  Min and 1 - f are exact, so the result has one value.  At a test point
+ * that is an LGR node, r_l is objfunc's row for that node bit for bit.
+ * res and at are [n_scen][n_aero], in the plan's aero-job order; a plan without aero jobs writes nothing.
+ * gelato_eval_path_check: host buffers (page-locked ones are DMA'd directly, others staged).  _dev: device pointers,
+ * enqueued on `stream` (NULL = the plan's own), not synchronised.  Both use the scenario blocks, refuse an n_scen beyond
+ * them and refuse calls before a grid is set.  Two launches per call (DESIGN.md section 11 gives the measured cost); the
+ * _dev call uses plan-owned scratch (n_scen x the test points of the jobs over a whole section doubles): calls on one
+ * plan must not overlap on different streams. */
+int gelato_eval_path_check(GelatoPlan* plan, const double* x, double* res, int32_t* at, int32_t n_scen);
+int gelato_eval_path_check_dev(GelatoPlan* plan, const double* x_dev, double* res_dev, int32_t* at_dev, int32_t n_scen,
+                               void* stream);
+
 int gelato_host_alloc(size_t bytes, void** out);
 int gelato_host_free(void* ptr);
 
