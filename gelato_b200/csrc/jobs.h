@@ -1369,7 +1369,10 @@ P_HD void evt_res(const PlanView& P, int scen, const double* x, double* g, int j
  *   IIP       : 0 centre | 1 p0 2 v0 3 p1 4 v1 5 p2 6 v2 | 7 t   (:225-236, interleaved)
  *   TERM      : 0 centre | 1-3 pos j | 4-6 vel j                  (con_init_terminal_knot.py:391-399)
  *   USER_ORBIT: 0 base | 1-6 FD of p0 p1 p2 v0 v1 v2 | 7-12 background after k restores
- *               (jac_fd.py:54-60 restricted to the six variables the function reads) */
+ *               (jac_fd.py:54-60 restricted to the six variables the function reads).  Lane 7 holds k = 0, the
+ *               base state again: (g_base - g_base) / dx is what jac_fd gives every variable visited before the
+ *               first one the function reads -- +0, or NaN where g_base is not finite.  k = 1 is never needed
+ *               (the three position components are visited back to back), so the slot is free for it. */
 P_HD int evt_n_lanes(int type) {
   return type == GE_IIP ? 8 : (type == GE_TERM ? 7 : (type == GE_USER_ORBIT ? 13 : 5));
 }
@@ -1411,8 +1414,8 @@ P_HD void evt_jac_phase1(const PlanView& P, int scen, const double* x, int job, 
     if (lane <= nvar) { /* FD lane for variable order[lane-1] */
       n_restored = lane - 1;
       perturbed = order[lane - 1];
-    } else if (type == GE_USER_ORBIT) { /* background lanes 7..12: k = lane-6 restores done */
-      n_restored = lane - 6;
+    } else if (type == GE_USER_ORBIT) { /* background lanes 7..12: k = lane-6 restores done, except k = 0 on lane 7 */
+      n_restored = lane == 7 ? 0 : lane - 6;
     } else { /* the t lane: every variable already restored */
       n_restored = nvar;
       t_e = t_e + dx;
@@ -1481,7 +1484,10 @@ P_HD void lin_res(const PlanView& P, int scen, const double* x, double* g, int k
   const double a = (li[GL_IDX_PLUS] >= 0) ? x[li[GL_IDX_PLUS]] * lf[GL_SCALE_PLUS] : 0.0;
   const double b = (li[GL_IDX_MINUS] >= 0) ? x[li[GL_IDX_MINUS]] * lf[GL_SCALE_MINUS] : 0.0;
   const double c = P.lin_const_scen ? P.lin_const_scen[(long long)scen * P.n_lin + k] : lf[GL_CONST];
-  g[li[GL_ROW]] = (a - b) + c;
+  /* signed zeros as the reference's expressions give them: -u (the kick rows) and u_j - u_k are not 0 - u and
+   * (u_j - u_k) + 0, which turn -0 into +0 */
+  const double d = (li[GL_IDX_PLUS] >= 0) ? a - b : -b;
+  g[li[GL_ROW]] = (c != 0.0) ? d + c : d;
 }
 
 /* ========================================================================= */

@@ -193,11 +193,21 @@ extern "C" {
   cudaError_t err = cudaSetDevice(device);                                     \
   DevBuf buf;
 
+// interp_interval / np_interp (physics.h) read rows k and k + 1 of a table: one row is refused, as
+// gelato_plan_create refuses it (plan_host.h: validate_desc)
+#define LEAF_TABLE_ROWS(name, table, rows)                                              \
+  if (!(table) || (rows) < 2) {                                                        \
+    gelato_set_error_(name ": " #table " table needs at least two rows");               \
+    return GELATO_ERR_ARG;                                                             \
+  }
+
 int gelato_leaf_dynamics_velocity(int device, int32_t n, const double* mass_e, const double* pos_e,
                                   const double* vel_e, const double* quat, const double* t, const double* param5,
                                   const double* wind, int32_t n_wind, const double* ca, int32_t n_ca,
                                   const double* units3, double* out) {
   LEAF_PROLOGUE
+  LEAF_TABLE_ROWS("gelato_leaf_dynamics_velocity", wind, n_wind)
+  LEAF_TABLE_ROWS("gelato_leaf_dynamics_velocity", ca, n_ca)
   SecParam sp{param5[0], param5[1], param5[2], param5[4]};
   Units un{units3[0], units3[1], units3[2], 1.0, 1.0, 0.0};
   Tables tb;
@@ -240,7 +250,8 @@ int gelato_leaf_aero(int device, int32_t kind, int32_t n, const double* pos, con
                      const double* t, const double* wind, int32_t n_wind, double* out) {
   LEAF_PROLOGUE
   const bool state = kind != 4;  // kind 4 (wind_ned) reads the altitudes in t and the table only
-  if (kind < 0 || kind > 4 || !t || !wind || n_wind <= 0 || !out || (state && (!pos || !vel)) ||
+  LEAF_TABLE_ROWS("gelato_leaf_aero", wind, n_wind)
+  if (kind < 0 || kind > 4 || !t || !out || (state && (!pos || !vel)) ||
       ((kind == 0 || kind == 2 || kind == 3) && !quat)) {
     gelato_set_error_("gelato_leaf_aero: bad kind, missing quaternion or null buffer");
     return GELATO_ERR_ARG;
@@ -290,6 +301,8 @@ int gelato_leaf_output_table(int device, int32_t n, const double* mass, const do
                              const double* nozzle_area, const double* wind, int32_t n_wind, const double* ca, int32_t n_ca,
                              double launch_lat_deg, double launch_lon_deg, double* out) {
   LEAF_PROLOGUE
+  LEAF_TABLE_ROWS("gelato_leaf_output_table", wind, n_wind)
+  LEAF_TABLE_ROWS("gelato_leaf_output_table", ca, n_ca)
   Tables tb;
   tb.wind = buf.in(wind, (size_t)n_wind * 3, err); tb.n_wind = n_wind;
   tb.ca = buf.in(ca, (size_t)n_ca * 2, err); tb.n_ca = n_ca;
@@ -324,7 +337,9 @@ int gelato_init_rocket_simulation(int device, int32_t n, const double* x_init, c
     gelato_set_error_("rocket_simulation: null buffer");
     return GELATO_ERR_ARG;
   }
-  if (n_ev <= 0 || n_u <= 0 || n_wind <= 0 || n_ca <= 0 || n_out <= 0 || !(dt > 0.0) || !scenario_strides) {
+  LEAF_TABLE_ROWS("rocket_simulation", wind, n_wind)
+  LEAF_TABLE_ROWS("rocket_simulation", ca, n_ca)
+  if (n_ev <= 0 || n_u <= 0 || n_out <= 0 || !(dt > 0.0) || !scenario_strides) {
     gelato_set_error_("rocket_simulation: empty table, no output time or non-positive dt");
     return GELATO_ERR_ARG;
   }

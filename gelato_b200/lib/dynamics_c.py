@@ -10,7 +10,7 @@ def dynamics_velocity(mass_e, pos_eci_e, vel_eci_e, quat_eci2body, t, param, win
     n = m.size
     pos, vel, quat = arr(pos_eci_e, (n, 3)), arr(vel_eci_e, (n, 3)), arr(quat_eci2body, (n, 4))
     tt, prm, un = arr(t).ravel(), arr(param).ravel(), arr(units).ravel()
-    wind, ca = arr(wind_table), arr(CA_table)
+    wind, ca = arr(wind_table, (-1, 3)), arr(CA_table, (-1, 2))  # the row counts go to the C ABI
     out = np.empty((n, 3))
     call("gelato_leaf_dynamics_velocity", n, ptr(m), ptr(pos), ptr(vel), ptr(quat), ptr(tt), ptr(prm), ptr(wind),
          wind.shape[0], ptr(ca), ca.shape[0], ptr(un), ptr(out))

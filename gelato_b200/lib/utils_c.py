@@ -12,7 +12,7 @@ def _aero(kind, pos, vel, quat, t, wind):
     vel = arr(vel, (n, 3))
     q = arr(quat, (n, 4)) if quat is not None else None
     tt = arr(t).ravel()
-    w = arr(wind)
+    w = arr(wind, (-1, 3))
     out = np.empty(n)
     call("gelato_leaf_aero", kind, n, ptr(pos), ptr(vel), ptr(q), ptr(tt), ptr(w), w.shape[0], ptr(out))
     return out
@@ -46,7 +46,7 @@ def angle_of_attack_ab_array_rad(pos_eci, vel_eci, quat, t, wind):
     """wrapper_utils.hpp:150-161 -> (n, 2): pitch-plane and yaw-plane angles of the air-relative velocity in body axes."""
     pos = arr(pos_eci).reshape(-1, 3)
     n = pos.shape[0]
-    w = arr(wind)
+    w = arr(wind, (-1, 3))
     out = np.empty((n, 2))
     call("gelato_leaf_aero", 3, n, ptr(pos), ptr(arr(vel_eci, (n, 3))), ptr(arr(quat, (n, 4))), ptr(arr(t).ravel()), ptr(w),
          w.shape[0], ptr(out))
@@ -61,7 +61,7 @@ def angle_of_attack_ab_rad(pos_eci, vel_eci, quat, t, wind):
 def wind_ned(altitude_m, wind):
     """wrapper_utils.hpp:82-87 -> (north, east, 0) wind at an altitude (or (n, 3) for n altitudes)."""
     alt = arr(altitude_m).ravel()
-    w = arr(wind)
+    w = arr(wind, (-1, 3))
     out = np.empty((alt.size, 3))
     call("gelato_leaf_aero", 4, alt.size, ptr(None), ptr(None), ptr(None), ptr(alt), ptr(w), w.shape[0], ptr(out))
     return out[0] if np.ndim(altitude_m) == 0 else out

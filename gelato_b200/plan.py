@@ -1008,7 +1008,8 @@ class CompiledPlan:
         """Expand the 12 auxiliary quotients of every row into jac_fd's dense blocks
         (jac_fd.py:54-60): a variable the function does not read still gets
         (g(x after k restores) - g_base)/dx, k = how many of the six read
-        variables were visited before it.  `out`: the dictionary of an earlier call to refill in place (its arrays
+        variables were visited before it -- for k = 0 that is (g_base - g_base)/dx, +0 or NaN where g_base is not
+        finite.  `out`: the dictionary of an earlier call to refill in place (its arrays
         are column slices of one (rows, n_vars) buffer, filled by one gather per row)."""
         _, job, srow = spec
         nrow = job["i32"][GE_NROW]
@@ -1016,8 +1017,9 @@ class CompiledPlan:
         maps = self.__dict__.setdefault("_user_maps", {})
         idx = maps.get((order, srow))
         if idx is None:
-            # every entry of a row is one of 13 values: q = [0, background quotients after 1..6 restores, the six
-            # finite-difference quotients]; which one depends only on the variable's place in the perturbation order
+            # every entry of a row is one of 13 values: q = [background quotients after 0..6 restores, the six
+            # finite-difference quotients]; which one depends only on the variable's place in the perturbation order.
+            # Only k = 0, 3, 6 occur (position and velocity are visited three components at a time).
             if order.index("position") > order.index("velocity"):
                 raise NotImplementedError("xdict key order with velocity before position")
             parts, k = [], 0
@@ -1037,11 +1039,12 @@ class CompiledPlan:
                 out[key] = buf[:, o: o + self.sizes[key]]
                 o += self.sizes[key]
         buf = out.buffer
-        q = np.empty(13)
-        q[0] = 0.0
+        q = np.full(13, np.nan)  # q[1] (k = 1) is never indexed
         a0 = job["i64"][GE_J_POS]
         for r in range(nrow):
-            q[1:7] = vals[a0 + 6: a0 + 12]
+            # background slot 0 holds k = 0 (jobs.h: evt_jac_phase1, lane 7), slots 1..5 k = 2..6
+            q[0] = 0.0 * vals[a0 + 6]  # the same +0 / NaN; 0 for csr_map's probe, whose entries here stay structural zeros
+            q[2:7] = vals[a0 + 7: a0 + 12]
             q[7:13] = vals[a0: a0 + 6]
             np.take(q, idx, out=buf[r])
             a0 += AUX_PER_USER

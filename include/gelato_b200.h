@@ -91,7 +91,8 @@ enum { GE_LLH = 0, GE_IIP = 1, GE_ANT = 2, GE_TERM = 3, GE_USER_ORBIT = 4, GE_N_
  * quantities of the state at the first node of a named event, up to three rows: row r = q / scale - offset with the
  * quantity code in byte r of GE_COMP (GEQ_*) and scale / offset in GE_A0 + 2r, GE_A0 + 2r + 1.  It leaves GE_USER_AUX
  * values per row in the auxiliary tail of vals: 6 finite-difference quotients (position, velocity) and the 6
- * "background" quotients jac_fd's perturb / restore protocol gives every variable the function does not read. */
+ * "background" quotients jac_fd's perturb / restore protocol gives every variable the function does not read
+ * (after 0, 2, 3, 4, 5, 6 of the read variables are restored; the first is +0, or NaN where the row is not finite). */
 #define GE_USER_AUX 12
 enum {
   GEQ_PERIGEE_RADIUS = 0, /* a (1 - e)       Coordinate.cpp:197-245 orbital_elements */
