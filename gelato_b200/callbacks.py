@@ -22,7 +22,8 @@ from .plan import GROUPS, ORBIT_QUANTITIES, VAR_ORDER, CompiledPlan, OrbitAtEven
 
 class GelatoProblem:
     def __init__(self, pdict, unitdict, condition, user_eq=None, user_ineq=None, device=0, coord=None,
-                 engine_factory=None, reuse_output=True, fuse_pair=False, derivative="forward", fd_step=None):
+                 engine_factory=None, reuse_output=True, fuse_pair=False, derivative="forward", fd_step=None,
+                 path_grid=None):
         """engine_factory(plan) -> object with eval_residuals / eval_jacobian / close / launches;
         default: the CUDA engine on `device` (the CPU test tier passes the host emulator of the
         kernels, tests/emu_binding.py, to exercise this host logic without a GPU).
@@ -41,7 +42,14 @@ class GelatoProblem:
         derivative="forward" (default): the reference's forward-difference Jacobian, bit for bit.  "central": central
         differences with step fd_step (None: engine.DEFAULT_FD_STEP) -- 100-1000x closer to the derivative on most
         blocks for about twice the Jacobian's GPU time; same sparsity, same objfunc (DESIGN.md H6).  `sens`,
-        `jacobian_csr` and the fused pair follow it; `engine.set_fd` switches it later."""
+        `jacobian_csr` and the fused pair follow it; `engine.set_fd` switches it later.
+
+        path_grid=None (default): the NLP as the reference has it.  A test grid ({"m", "off", "pool"} as
+        gelato_b200.mesh.grid_tables builds it, e.g. mesh.grid_tables(plan.ps) for n + 1 points per section): the aero
+        constraints are also enforced between the nodes, as the inequality group "ineqcon_path" -- one row per test point
+        of every aero constraint over a whole section, except the points that are nodes (DESIGN.md section 11).
+        `objfunc`, `sens` and `jacobian_csr` add the group after the others; every other key is unchanged bit for bit.
+        path_rows_index() names the rows."""
         _engine.fd_args(derivative, fd_step)  # a bad mode or step fails before anything is built
         self.plan = CompiledPlan(pdict, unitdict, condition, user_eq=user_eq, user_ineq=user_ineq, coord=coord)
         self.engine = engine_factory(self.plan) if engine_factory else _engine.Engine(self.plan, device=device)
@@ -57,6 +65,13 @@ class GelatoProblem:
         self._x_pair = None  # the decision vector the kept Jacobian belongs to
         self._pair_fresh = False
         self._mesh_grid = None  # the tables of the engine's mesh grid (mesh.grid_tables), once set
+        # path rows: their layout (engine.path_rows_layout) and COO blocks (plan.path_rows_structure), and the Jacobian
+        # buffer funcsSens["ineqcon_path"] views (reuse_output; the fused pair fills it from objfunc)
+        self._path = self._path_vals = None
+        if path_grid is not None:
+            self.engine.set_path_rows(path_grid)
+            layout = self.engine.path_rows_layout()
+            self._path = (layout, self.plan.path_rows_structure(layout))
 
     # -- helpers ---------------------------------------------------------
     def pack(self, xdict):
@@ -96,34 +111,65 @@ class GelatoProblem:
                 self._x_pair = np.empty_like(x)
             self._x_pair[:] = x
             self._pair_fresh = True
-            return self.plan.split_residuals(g), False
+            return self._with_path(self.plan.split_residuals(g), x, self._path_buffer()), False
         g = self.engine.eval_residuals(x)
-        return self.plan.split_residuals(g), False
+        return self._with_path(self.plan.split_residuals(g), x, None), False
+
+    def _with_path(self, funcs, x, vals):
+        """funcs plus "ineqcon_path" (with path rows); vals: a buffer for the rows' Jacobian at x, or None."""
+        if self._path is not None:
+            funcs["ineqcon_path"] = self.engine.eval_path_rows(x, out=(np.empty(self._path[0]["n_rows"]), vals))[0]
+        return funcs
+
+    def _path_buffer(self):
+        """The one buffer of the path rows' Jacobian values kept across calls (reuse_output)."""
+        if self._path_vals is None and self._path is not None:
+            alloc = getattr(self.engine, "alloc_output", None)  # the CUDA engine: page-locked memory
+            self._path_vals = alloc(self._path[0]["n_vals"]) if alloc else _engine.PinnedArray(self._path[0]["n_vals"])
+        return None if self._path_vals is None else self._path_vals.array
+
+    def _path_sens(self, vals):
+        """funcsSens["ineqcon_path"]: the COO blocks with data arrays that are views of vals."""
+        return {var: {"coo": [b.rows, b.cols, vals[b.offset: b.offset + b.nnz]], "shape": b.shape}
+                for var, b in self._path[1].items()}
+
+    def _path_jacobian(self, x):
+        """The path rows' Jacobian values at x in a fresh array."""
+        return self.engine.eval_path_rows(x, out=(None, np.empty(self._path[0]["n_vals"])))[1]
 
     def sens(self, xdict, funcs=None):
         if self.reuse_output:
             x = self.pack(xdict)
             if self.fuse_pair and self._x_pair is not None and self._pair_fresh and np.array_equal(x, self._x_pair):
-                vals = self._output_buffer()  # already holds this point's Jacobian
+                vals = self._output_buffer()  # already holds this point's Jacobian (and the path rows')
             else:
                 vals = self.engine.eval_jacobian_update(x, self._output_buffer(), 1)
                 self._pair_fresh = False
+                if self._path is not None:
+                    self.engine.eval_path_rows(x, out=(None, self._path_buffer()))
             # the dictionary is built once per key order: its COO data arrays are views of the one buffer the engine
             # refreshes in place; only the dense user-constraint blocks are recomputed
             order = tuple(k for k in xdict.keys() if k in VAR_ORDER)
             if self._sens_dict is None or self._sens_dict[0] != order or self._sens_dict[2] is not vals:
                 self._sens_dict = (order, self.plan.split_jacobian(vals, key_order=list(order)), vals)
+                if self._path is not None:
+                    self._sens_dict[1]["ineqcon_path"] = self._path_sens(self._path_buffer())
             else:
                 self.plan.refresh_user_blocks(vals, self._sens_dict[1], order)
             return self._sens_dict[1], False
-        vals = self.engine.eval_jacobian(self.pack(xdict))
-        return self.plan.split_jacobian(vals, key_order=[k for k in xdict.keys() if k in VAR_ORDER]), False
+        x = self.pack(xdict)
+        vals = self.engine.eval_jacobian(x)
+        s = self.plan.split_jacobian(vals, key_order=[k for k in xdict.keys() if k in VAR_ORDER])
+        if self._path is not None:
+            s["ineqcon_path"] = self._path_sens(self._path_jacobian(x))
+        return s, False
 
     def jacobian_csr(self, xdict, wrt=None):
         """The constraint Jacobian of all registered groups as one scipy CSR matrix (rows in registration order,
         columns in `xdict` key order): the structure is compiled once (`plan.csr_map`), each call is one kernel
         launch and one gather -- no per-call COO sorting (what pyoptsparse does with the dictionaries of `sens`).
-        `wrt`: {group: [variables]} as in Trajectory_Optimization.py:358-384 (None = every block)."""
+        `wrt`: {group: [variables]} as in Trajectory_Optimization.py:358-384 (None = every block).  With path rows,
+        "ineqcon_path" comes last."""
         import scipy.sparse as sp
 
         order = tuple(k for k in xdict.keys() if k in VAR_ORDER)
@@ -131,9 +177,33 @@ class GelatoProblem:
         if self._csr is None or self._csr[0] != key:
             self._csr = (key, self.plan.csr_map(wrt=wrt, key_order=order))
         m = self._csr[1]
-        vals = self.engine.eval_jacobian(self.pack(xdict))
+        x = self.pack(xdict)
+        vals = self.engine.eval_jacobian(x)
         data = np.append(vals, 0.0)[m["src"]]
-        return sp.csr_matrix((data, m["indices"], m["indptr"]), shape=m["shape"])
+        J = sp.csr_matrix((data, m["indices"], m["indptr"]), shape=m["shape"])
+        if self._path is None:
+            return J
+        pv = self._path_jacobian(x)
+        col0 = dict(zip(order, np.cumsum([0] + [self.plan.sizes[k] for k in order])))
+        rows, cols, data = [], [], []
+        for var, b in self._path[1].items():
+            if wrt is not None and "ineqcon_path" in wrt and var not in wrt["ineqcon_path"]:
+                continue
+            rows.append(b.rows)
+            cols.append(b.cols.astype(np.int64) + col0[var])
+            data.append(pv[b.offset: b.offset + b.nnz])
+        Jp = sp.csr_matrix((np.concatenate(data), (np.concatenate(rows), np.concatenate(cols))),
+                           shape=(self._path[0]["n_rows"], J.shape[1]))
+        return sp.vstack([J, Jp], format="csr")
+
+    def path_rows_index(self):
+        """[(funcs key of the aero constraint, event name, test point l)] of the rows of funcs["ineqcon_path"], in
+        order (the test point is tau_t[l] of the path grid's section); [] without path rows."""
+        if self._path is None:
+            return []
+        lay = self._path[0]
+        return [(self._AERO_KEYS[self.plan.aero_i32[j, 0]], self.plan.p["params"][self.plan.aero_i32[j, 1]]["name"], int(l))
+                for j, l in zip(lay["job"], lay["l"])]
 
     def mesh_error(self, xdict):
         """{event name: err[11]}: the collocation error estimate of each section between its nodes, per state component
@@ -183,9 +253,10 @@ class GelatoProblem:
         return self.engine.eval_jacobian(x, n_scen)
 
     def close(self):
-        if self._vals is not None:
-            self._vals.free()
-            self._vals = None
+        for buf in (self._vals, self._path_vals):
+            if buf is not None:
+                buf.free()
+        self._vals = self._path_vals = None
         self.engine.close()
 
 

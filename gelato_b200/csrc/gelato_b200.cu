@@ -279,6 +279,39 @@ k_path_min(int n_aero, const int32_t* __restrict__ job0, int n_pts, int n_scen, 
   mesh_path_min(r_all + (size_t)scen * n_pts + p0, job0[j + 1] - p0, res_all + i, at_all + i);
 }
 
+// Path rows (mesh_error.h; DESIGN.md section 11): `lanes` threads per (scenario, row).  lanes == PATH_LANES: lane 0
+// evaluates the centre f and writes g = 1 - f (g_all != NULL); it reaches lanes 1-12 by a half-warp shuffle, and each
+// of those writes its quotient's entries into vals[n_scen][n_vals].  lanes == 1 (residual only): the centres alone.
+#define GP_THREADS 128
+__global__ void __launch_bounds__(GP_THREADS)
+k_path_rows(const __grid_constant__ PlanView P, const PathRow* __restrict__ rows, const MeshSec* __restrict__ ms,
+            const double* __restrict__ pool, int n_rows, long long n_vals, int n_scen, int lanes, int central, double step,
+            const double* __restrict__ x_all, double* __restrict__ g_all, double* __restrict__ vals_all) {
+  const long long i = (long long)blockIdx.x * GP_THREADS + threadIdx.x;
+  const long long item = i / lanes;
+  const int lane = (int)(i - item * lanes);
+  const bool live = item < (long long)n_rows * n_scen;
+  const int scen = live ? (int)(item / n_rows) : 0;
+  const int k = live ? (int)(item - (long long)scen * n_rows) : 0;
+  const PathRow pr = rows[k];
+  const int sec = P.aero_i32[pr.job * GA_I32_COLS + GA_SECTION], n = P.sec_i32[sec * GS_I32_COLS + GS_N];
+  const MeshTabs tb = mesh_tabs(pool, ms[sec], n);
+  const double* x = x_all + (size_t)scen * P.n_vars;
+  double v[10];
+  mesh_path_state(P, x, sec, tb, pr.l, v);
+  double f0 = 0.0;
+  if (live && lane == 0) f0 = path_lane_f(P, scen, x, pr.job, tb, pr.l, v, 0, 0.0);
+  if (lanes > 1) f0 = __shfl_sync(0xffffffffu, f0, 0, PATH_LANES);  // every thread of the warp is here
+  if (!live) return;
+  if (lane == 0) {
+    if (g_all) g_all[item] = 1.0 - f0;
+    return;
+  }
+  if (lane > 12 || (pr.off[PR_QUAT] < 0 && lane >= 7 && lane <= 10)) return;
+  const double q = path_lane_quot(P, scen, x, pr.job, tb, pr.l, v, lane, f0, central, step);
+  path_lane_store(pr, tb.P + (long long)pr.l * (n + 1), n, lane, q, vals_all + (size_t)scen * n_vals);
+}
+
 // probe: is a*b+c left unfused?  (1 + 2^-30)(1 - 2^-30) - 1 is 0 unfused, -2^-60 fused
 __global__ void k_unfused_probe(double a, double b, double c, double* out) { *out = a * b + c; }
 
@@ -414,6 +447,15 @@ struct GelatoPlan {
   PinnedBuf<double> h_res;
   PinnedBuf<int32_t> h_at;
   int n_path_pts = 0;
+  // path rows (gelato_plan_set_path_rows) on a grid of their own: its sections and pool, the row list (plan_host.h:
+  // build_path_rows) on the host and the device, the values per scenario, and the host entry's staging
+  bool prow_set = false;
+  std::vector<PathRow> prow;
+  long long prow_vals = 0;
+  DeviceBuf<MeshSec> d_prow_sec;
+  DeviceBuf<double> d_prow_pool, d_prow_g, d_prow_v;
+  DeviceBuf<PathRow> d_prow;
+  PinnedBuf<double> h_prow_g, h_prow_v;
   long long launches = 0;
   Event ev0, ev1;
 };
@@ -1128,6 +1170,101 @@ int gelato_eval_path_check(GelatoPlan* p, const double* x, double* res, int32_t*
   CU(cudaStreamSynchronize(st));
   land(res, res_dst, na);
   land(at, at_dst, na);
+  return GELATO_OK;
+}
+
+// ---- path rows (mesh_error.h) ----
+int gelato_plan_set_path_rows(GelatoPlan* p, const GelatoMeshGridDesc* g) {
+  if (!p || !g || !g->m || !g->off || !g->pool) return fail(GELATO_ERR_ARG, "null argument");
+  std::vector<MeshSec> secs;
+  std::vector<MeshPt> pts;
+  if (const char* why = build_mesh_grid(g, p->sec_n.data(), p->view.S, secs, pts)) return fail(GELATO_ERR_ARG, why);
+  std::vector<PathRow> rows;
+  long long n_vals = 0;
+  if (const char* why = build_path_rows(p->aero_i32.data(), p->view.n_aero, p->sec_n.data(), secs, g->pool, rows, &n_vals))
+    return fail(GELATO_ERR_ARG, why);
+  CU(cudaSetDevice(p->device));
+  CU(cudaDeviceSynchronize());  // nothing in flight may still read the rows being replaced
+  CU(p->d_prow_sec.reserve(secs.size()));
+  CU(p->d_prow_pool.reserve((size_t)g->pool_len));
+  CU(p->d_prow.reserve(rows.size()));
+  const cudaStream_t st = p->lanes[0].stream;
+  CU(cudaMemcpyAsync(p->d_prow_sec.get(), secs.data(), secs.size() * sizeof(MeshSec), cudaMemcpyHostToDevice, st));
+  CU(cudaMemcpyAsync(p->d_prow_pool.get(), g->pool, (size_t)g->pool_len * sizeof(double), cudaMemcpyHostToDevice, st));
+  if (!rows.empty())
+    CU(cudaMemcpyAsync(p->d_prow.get(), rows.data(), rows.size() * sizeof(PathRow), cudaMemcpyHostToDevice, st));
+  CU(cudaStreamSynchronize(st));
+  p->prow.swap(rows);
+  p->prow_vals = n_vals;
+  p->prow_set = true;
+  return GELATO_OK;
+}
+
+int gelato_plan_path_rows(const GelatoPlan* p, int32_t* n_rows, int64_t* n_vals, int32_t* job, int32_t* l, int64_t* off) {
+  if (!p || !n_rows || !n_vals) return fail(GELATO_ERR_ARG, "null argument");
+  if (!p->prow_set) return fail(GELATO_ERR_ARG, GELATO_NO_PATH_ROWS);
+  *n_rows = (int32_t)p->prow.size();
+  *n_vals = p->prow_vals;
+  for (size_t k = 0; k < p->prow.size(); k++) {
+    if (job) job[k] = p->prow[k].job;
+    if (l) l[k] = p->prow[k].l;
+    if (off)
+      for (int c = 0; c < PR_OFFS; c++) off[k * PR_OFFS + c] = p->prow[k].off[c];
+  }
+  return GELATO_OK;
+}
+
+// The launch of one evaluation on `st` in the plan's finite-difference mode: PATH_LANES threads per row with a Jacobian,
+// one without.  Nothing without rows or outputs.
+static int launch_path_rows(GelatoPlan* p, const double* x_dev, double* g_dev, double* vals_dev, int n_scen, cudaStream_t st) {
+  const int n_rows = (int)p->prow.size();
+  if (!n_rows || (!g_dev && !vals_dev)) return GELATO_OK;
+  const int lanes = vals_dev ? PATH_LANES : 1;
+  const long long nt = (long long)n_scen * n_rows * lanes;
+  if ((nt + GP_THREADS - 1) / GP_THREADS > 0x7fffffffLL) return fail(GELATO_ERR_ARG, "path rows x n_scen exceeds the grid limit");
+  const int central = p->fd_mode == GELATO_FD_CENTRAL;
+  k_path_rows<<<(unsigned)((nt + GP_THREADS - 1) / GP_THREADS), GP_THREADS, 0, st>>>(
+      p->view, p->d_prow.get(), p->d_prow_sec.get(), p->d_prow_pool.get(), n_rows, p->prow_vals, n_scen, lanes, central,
+      central ? p->fd_step : p->view.un.dx, x_dev, g_dev, vals_dev);
+  p->launches++;
+  CU(cudaGetLastError());
+  return GELATO_OK;
+}
+
+int gelato_eval_path_rows_dev(GelatoPlan* p, const double* x_dev, double* g_dev, double* vals_dev, int32_t n_scen,
+                              void* stream) {
+  cudaStream_t st;
+  int rc = begin_dev(p, n_scen, stream, &st);
+  if (rc) return rc;
+  if (!p->prow_set) return fail(GELATO_ERR_ARG, GELATO_NO_PATH_ROWS);
+  if (!x_dev) return fail(GELATO_ERR_ARG, "null buffer");
+  return launch_path_rows(p, x_dev, g_dev, vals_dev, n_scen, st);
+}
+
+int gelato_eval_path_rows(GelatoPlan* p, const double* x, double* g_path, double* vals_path, int32_t n_scen) {
+  int rc = check_scen(p, n_scen);
+  if (rc) return rc;
+  if (!p->prow_set) return fail(GELATO_ERR_ARG, GELATO_NO_PATH_ROWS);
+  if (!x) return fail(GELATO_ERR_ARG, "null buffer");
+  if (p->prow.empty() || (!g_path && !vals_path)) return GELATO_OK;
+  CU(cudaSetDevice(p->device));
+  if ((rc = ensure_staging(p, n_scen))) return rc;
+  const cudaStream_t st = p->lanes[0].stream;
+  const size_t nx = (size_t)n_scen * p->view.n_vars, ng = (size_t)n_scen * p->prow.size(),
+               nv = (size_t)n_scen * (size_t)p->prow_vals;
+  if (g_path) CU(p->d_prow_g.reserve(ng));
+  if (vals_path) CU(p->d_prow_v.reserve(nv));
+  CU(cudaMemcpyAsync(p->d_x.get(), host_src(x, p->h_x.get(), nx), nx * sizeof(double), cudaMemcpyHostToDevice, st));
+  if ((rc = launch_path_rows(p, p->d_x.get(), g_path ? p->d_prow_g.get() : nullptr, vals_path ? p->d_prow_v.get() : nullptr,
+                             n_scen, st)))
+    return rc;
+  double *g_dst, *v_dst;
+  if ((rc = host_dst(g_path, p->h_prow_g, ng, &g_dst)) || (rc = host_dst(vals_path, p->h_prow_v, nv, &v_dst))) return rc;
+  if (g_path) CU(cudaMemcpyAsync(g_dst, p->d_prow_g.get(), ng * sizeof(double), cudaMemcpyDeviceToHost, st));
+  if (vals_path) CU(cudaMemcpyAsync(v_dst, p->d_prow_v.get(), nv * sizeof(double), cudaMemcpyDeviceToHost, st));
+  CU(cudaStreamSynchronize(st));
+  if (g_path) land(g_path, g_dst, ng);
+  if (vals_path) land(vals_path, v_dst, nv);
   return GELATO_OK;
 }
 

@@ -14,6 +14,10 @@
  * The path check runs on the same grid: the aero constraints' residual 1 - f at every test point of every aero job over
  * a whole section (mesh_path_point), and its minimum per job (mesh_path_min).  Min and 1 - f are exact, so it too has
  * one value.
+ *
+ * The path rows put those residuals into the NLP as inequality rows, on a grid of their own (gelato_plan_set_path_rows),
+ * with their Jacobian by the chain rule through the interpolation: the derivative along each state component of the
+ * interpolated state (a finite-difference quotient, path_lane_quot) times the P entry of each state row.
  */
 #ifndef GELATO_B200_MESH_ERROR_H_
 #define GELATO_B200_MESH_ERROR_H_
@@ -101,22 +105,88 @@ P_HD void mesh_point(const PlanView& P, int scen, const double* x, int sec, cons
   }
 }
 
-/* The path check (DESIGN.md section 11): one test point of an aero job.  The job's section is interpolated at test
- * point l with the chains of mesh_point (v = its xl[1..10]: position | velocity | quaternion), and the residual is the
- * expression aero_res gives objfunc's row at a node: pristine x, the time of the test point, the scenario's units and
- * wind table.  At a test point that is a node it is that row's value, bit for bit. */
-P_HD double mesh_path_point(const PlanView& P, int scen, const double* x, int job, const MeshTabs& tb, int l) {
-  const int32_t* ai = P.aero_i32 + job * GA_I32_COLS;
-  const int sec = ai[GA_SECTION];
+/* v[10] = position | velocity | quaternion of section `sec` interpolated at test point l with the chains of mesh_point
+ * (its xl[1..10]) */
+P_HD void mesh_path_state(const PlanView& P, const double* x, int sec, const MeshTabs& tb, int l, double* v) {
   const int32_t* si = P.sec_i32 + sec * GS_I32_COLS;
   const int n = si[GS_N], xa = si[GS_XA];
   const double* Prow = tb.P + (long long)l * (n + 1);
-  double v[10];
   dx_dot<3>(Prow, x + P.off_pos + 3 * xa, n + 1, v);
   dx_dot<3>(Prow, x + P.off_vel + 3 * xa, n + 1, v + 3);
   dx_dot<4>(Prow, x + P.off_quat + 4 * xa, n + 1, v + 6);
+}
+
+/* The path check (DESIGN.md section 11): one test point of an aero job.  The job's section is interpolated at test
+ * point l (mesh_path_state), and the residual is the expression aero_res gives objfunc's row at a node: pristine x,
+ * the time of the test point, the scenario's units and wind table.  At a test point that is a node it is that row's
+ * value, bit for bit. */
+P_HD double mesh_path_point(const PlanView& P, int scen, const double* x, int job, const MeshTabs& tb, int l) {
+  const int32_t* ai = P.aero_i32 + job * GA_I32_COLS;
+  const int sec = ai[GA_SECTION];
+  double v[10];
+  mesh_path_state(P, x, sec, tb, l, v);
   const double tn = time_node(tb.tau, l + 1, x[P.off_t + sec], x[P.off_t + sec + 1]);
   return 1.0 - aero_value(P, scen, ai[GA_KIND], v, tn, P.aero_f64[job * GA_F64_COLS + GA_LIMIT]);
+}
+
+/* ========================================================================= */
+/* Path rows (DESIGN.md section 11): the aero constraints as NLP rows at the  */
+/* test points of a grid of their own.  Per row 16 lanes:                     */
+/*   0 centre | 1-10 state component (position 3 | velocity 3 | quaternion 4)*/
+/*   | 11 to | 12 tf | 13-15 idle                                             */
+/* ========================================================================= */
+#define PATH_LANES 16
+enum { PR_POS = 0, PR_VEL, PR_QUAT, PR_T, PR_OFFS };
+/* one path row: aero job, test point of the job's section, and where each variable's entries start in the row values
+ * of one scenario (PR_QUAT: -1 for max-q, which has none); plan_host.h: build_path_rows */
+struct PathRow {
+  int32_t job, l;
+  int64_t off[PR_OFFS];
+};
+
+/* f / L of lane `lane` of a path row at step dx, v = mesh_path_state of the row's test point: lane 0 f(v, tn) (dx
+ * unused), lanes 1-10 f(v + dx e_(lane-1), tn), 11 and 12 f(v, tn) with to + dx and tf + dx.  The centre is the path
+ * check's f at that test point. */
+P_HD double path_lane_f(const PlanView& P, int scen, const double* x, int job, const MeshTabs& tb, int l, const double* v,
+                        int lane, double dx) {
+  const int32_t* ai = P.aero_i32 + job * GA_I32_COLS;
+  const int sec = ai[GA_SECTION];
+  double w[10];
+#pragma unroll
+  for (int k = 0; k < 10; k++) w[k] = k == lane - 1 ? v[k] + dx : v[k]; /* no dynamic index: w stays in registers */
+  double to = x[P.off_t + sec], tf = x[P.off_t + sec + 1];
+  if (lane == 11) to = to + dx;
+  else if (lane == 12) tf = tf + dx;
+  return aero_value(P, scen, ai[GA_KIND], w, time_node(tb.tau, l + 1, to, tf), P.aero_f64[job * GA_F64_COLS + GA_LIMIT]);
+}
+
+/* the derivative of the row 1 - f / L along lane `lane` (1-12), f0 = the centre: -fd_div(f(step) - f0, step); central
+ * differences (DESIGN.md H6) average that quotient at +step and at -step */
+P_HD double path_lane_quot(const PlanView& P, int scen, const double* x, int job, const MeshTabs& tb, int l, const double* v,
+                           int lane, double f0, int central, double step) {
+  /* one evaluation site for both steps: the device build of two inlined copies of the evaluation returned wrong -step
+   * quotients for the state lanes (the t lanes and forward mode were right) */
+  double q = 0.0;
+#pragma unroll 1
+  for (int s = 0; s <= central; s++) {
+    const double h = s ? -step : step;
+    const double qs = -fd_div(path_lane_f(P, scen, x, job, tb, l, v, lane, h) - f0, h);
+    q = s ? fd_central(q, qs) : qs;
+  }
+  return q;
+}
+
+/* the entries of lane `lane` (1-12) of path row `pr` into one scenario's row values: a state lane writes P[l][m] * q for
+ * the section's state rows m = 0..n at (m, component), lanes 11 / 12 write q itself */
+P_HD void path_lane_store(const PathRow& pr, const double* Prow, int n, int lane, double q, double* vals) {
+  if (lane >= 11) {
+    vals[pr.off[PR_T] + (lane - 11)] = q;
+    return;
+  }
+  const int var = lane <= 3 ? PR_POS : (lane <= 6 ? PR_VEL : PR_QUAT);
+  const int w = var == PR_QUAT ? 4 : 3, c = lane <= 3 ? lane - 1 : (lane <= 6 ? lane - 4 : lane - 7);
+  double* out = vals + pr.off[var] + c;
+  for (int m = 0; m <= n; m++) out[(long long)w * m] = Prow[m] * q;
 }
 
 /* min and argmin of r[0 .. m) as numpy.min / numpy.argmin give them: ties go to the first, a NaN wins (the first NaN);

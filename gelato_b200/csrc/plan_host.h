@@ -1,7 +1,7 @@
 /* plan_host.h -- host-side helpers shared by the CUDA library and the test
  * emulator: PlanView scalar fields from a GelatoPlanDesc, the node / row lists
- * and the block tables of the two kernels, and the test grid of the mesh error
- * estimate and of the path check. */
+ * and the block tables of the two kernels, the test grid of the mesh error
+ * estimate and of the path check, and the path rows. */
 #ifndef GELATO_B200_PLAN_HOST_H_
 #define GELATO_B200_PLAN_HOST_H_
 
@@ -359,6 +359,51 @@ static inline const char* build_path_points(const int32_t* aero_i32, int n_aero,
     }
     job0.push_back((int32_t)pts.size());
   }
+  return nullptr;
+}
+
+/* why the path-row entry points refuse a call before a grid is set */
+#define GELATO_NO_PATH_ROWS "no path rows set (gelato_plan_set_path_rows)"
+
+/* The path rows on the grid `secs` / `pool` (build_mesh_grid) of a plan whose sections have n[i] LGR nodes (DESIGN.md
+ * section 11): the aero jobs over a whole section (GA_NK > 1) in the plan's order, each job's test points l ascending,
+ * except a test point whose P row is exactly a unit vector -- a support point, where the node's own row holds the
+ * constraint.  The values of one scenario are laid out variable-major: position (3 (n + 1) per row, (m, c) order),
+ * velocity (the same), quaternion (4 (n + 1) per row of kinds alpha and Q-alpha only), t ((to, tf) per row); *n_vals of
+ * them.  Returns NULL or why the grid is refused. */
+static inline const char* build_path_rows(const int32_t* aero_i32, int n_aero, const int32_t* n, const std::vector<MeshSec>& secs,
+                                          const double* pool, std::vector<PathRow>& rows, long long* n_vals) {
+  rows.clear();
+  for (int k = 0; k < n_aero; k++) {
+    const int32_t* ai = aero_i32 + (size_t)k * GA_I32_COLS;
+    if (ai[GA_NK] <= 1) continue;
+    const int sec = ai[GA_SECTION], ni = n[sec];
+    const MeshTabs tb = mesh_tabs(pool, secs[sec], ni);
+    for (int l = 0; l < secs[sec].m; l++) {
+      const double* Prow = tb.P + (long long)l * (ni + 1);
+      int ones = 0, zeros = 0;
+      for (int m = 0; m <= ni; m++) {
+        ones += Prow[m] == 1.0;
+        zeros += Prow[m] == 0.0;
+      }
+      if (ones == 1 && zeros == ni) continue;
+      if ((long long)rows.size() * PATH_LANES >= 0x7fffffffLL) return "too many path rows";
+      PathRow r;
+      r.job = k;
+      r.l = l;
+      rows.push_back(r);
+    }
+  }
+  long long o = 0;
+  auto sec_n = [&](const PathRow& r) { return (long long)n[aero_i32[(size_t)r.job * GA_I32_COLS + GA_SECTION]]; };
+  for (PathRow& r : rows) { r.off[PR_POS] = o; o += 3 * (sec_n(r) + 1); }
+  for (PathRow& r : rows) { r.off[PR_VEL] = o; o += 3 * (sec_n(r) + 1); }
+  for (PathRow& r : rows) {
+    r.off[PR_QUAT] = -1;
+    if (aero_i32[(size_t)r.job * GA_I32_COLS + GA_KIND] != 1) { r.off[PR_QUAT] = o; o += 4 * (sec_n(r) + 1); }
+  }
+  for (PathRow& r : rows) { r.off[PR_T] = o; o += 2; }
+  *n_vals = o;
   return nullptr;
 }
 

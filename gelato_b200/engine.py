@@ -235,6 +235,10 @@ def load_library():
     L.gelato_eval_mesh_error_dev.argtypes = [vp, vp, vp, ctypes.c_int32, vp]
     L.gelato_eval_path_check.argtypes = [vp, _pd, _pd, _pi32, ctypes.c_int32]
     L.gelato_eval_path_check_dev.argtypes = [vp, vp, vp, vp, ctypes.c_int32, vp]
+    L.gelato_plan_set_path_rows.argtypes = [vp, ctypes.POINTER(MeshGridDesc)]
+    L.gelato_plan_path_rows.argtypes = [vp, _pi32, _pi64, _pi32, _pi32, _pi64]
+    L.gelato_eval_path_rows.argtypes = [vp, _pd, _pd, _pd, ctypes.c_int32]
+    L.gelato_eval_path_rows_dev.argtypes = [vp, vp, vp, vp, ctypes.c_int32, vp]
     L.gelato_eval_jacobian.argtypes = [vp, _pd, _pd, ctypes.c_int32]
     L.gelato_eval_residuals_ids.argtypes = [vp, _pd, _pd, ctypes.c_int32, _pi32]
     L.gelato_eval_jacobian_ids.argtypes = [vp, _pd, _pd, ctypes.c_int32, _pi32]
@@ -300,7 +304,8 @@ EXPORTS = (
     "gelato_leaf_atmosphere gelato_leaf_output_table gelato_init_rocket_simulation gelato_leaf_coordinate "
     "gelato_eval_pair_packed_range_dev gelato_plan_set_fd gelato_plan_get_fd "
     "gelato_plan_set_mesh_grid gelato_eval_mesh_error gelato_eval_mesh_error_dev "
-    "gelato_eval_path_check gelato_eval_path_check_dev"
+    "gelato_eval_path_check gelato_eval_path_check_dev "
+    "gelato_plan_set_path_rows gelato_plan_path_rows gelato_eval_path_rows gelato_eval_path_rows_dev"
 ).split()
 
 
@@ -349,6 +354,7 @@ class Engine:
         self.n_rows = L.gelato_plan_n_rows(h)
         self.n_vals = L.gelato_plan_n_vals(h)
         assert self.n_vars == plan.n_vars and self.n_rows == plan.n_rows and self.n_vals == plan.n_vals
+        self._prow = None  # the path-row layout (path_rows_layout), read once per grid
         ok = ctypes.c_int(0)
         _check(L, L.gelato_selftest_unfused(device, ctypes.byref(ok)), "gelato_selftest_unfused")
         if not ok.value:
@@ -422,6 +428,53 @@ class Engine:
     def path_check_dev(self, x_ptr, res_ptr, at_ptr, n_scen=1, stream=None):
         _check(self.L, self.L.gelato_eval_path_check_dev(self.h, x_ptr, res_ptr, at_ptr, n_scen, stream),
                "gelato_eval_path_check_dev")
+
+    # ---- path rows (DESIGN.md section 11) ----
+    def set_path_rows(self, tables):
+        """The grid of the path rows ({"m", "off", "pool"} as gelato_b200.mesh.grid_tables builds it), separate from the
+        mesh grid: the aero constraints become NLP rows at its test points (include/gelato_b200.h)."""
+        desc, _keep = make_mesh_grid_desc(tables)
+        _check(self.L, self.L.gelato_plan_set_path_rows(self.h, ctypes.byref(desc)), "gelato_plan_set_path_rows")
+        self._prow = None
+
+    def path_rows_layout(self):
+        """{"n_rows", "n_vals", "job" int32[n_rows], "l" int32[n_rows], "off" int64[n_rows][4]}: the rows (aero job,
+        test point) and where each row's position | velocity | quaternion (-1: none) | t entries start in the values of
+        one scenario (gelato_plan_path_rows; read once per grid)."""
+        if self._prow is None:
+            L, n, v = self.L, ctypes.c_int32(0), ctypes.c_int64(0)
+            _check(L, L.gelato_plan_path_rows(self.h, ctypes.byref(n), ctypes.byref(v), None, None, None),
+                   "gelato_plan_path_rows")
+            job, l = np.empty(n.value, dtype=np.int32), np.empty(n.value, dtype=np.int32)
+            off = np.empty((n.value, 4), dtype=np.int64)
+            _check(L, L.gelato_plan_path_rows(self.h, ctypes.byref(n), ctypes.byref(v), _ptr(job, _pi32), _ptr(l, _pi32),
+                                              _ptr(off, _pi64)), "gelato_plan_path_rows")
+            self._prow = {"n_rows": n.value, "n_vals": v.value, "job": job, "l": l, "off": off}
+        return self._prow
+
+    def eval_path_rows(self, x, n_scen=1, jacobian=True, out=None):
+        """(g [n_rows], vals [n_vals] or None) of the decision vectors x[n_scen][n_vars] (n_scen > 1: [n_scen][...]):
+        the path rows' values and, with `jacobian`, their Jacobian values in the current finite-difference mode.
+        out: (g, vals) float64 buffers to write into instead, page-locked ones DMA'd directly; a None entry is not
+        computed (`jacobian` is then not read)."""
+        x = self._x(x, n_scen)
+        self.calls += 1
+        lay = self.path_rows_layout()
+        nr, nv = lay["n_rows"], lay["n_vals"]
+        if out is not None:  # a None entry: that output is not computed
+            g = None if out[0] is None else _out(out[0], n_scen * nr, "out[0]")
+            v = None if out[1] is None else _out(out[1], n_scen * nv, "out[1]")
+        else:
+            g, v = np.empty(n_scen * nr), (np.empty(n_scen * nv) if jacobian else None)
+        _check(self.L, self.L.gelato_eval_path_rows(self.h, _ptr(x, _pd), _ptr(g, _pd), _ptr(v, _pd), n_scen),
+               "gelato_eval_path_rows")
+        if n_scen > 1:
+            g, v = (None if a is None else a.reshape(n_scen, -1) for a in (g, v))
+        return g, v
+
+    def eval_path_rows_dev(self, x_ptr, g_ptr, vals_ptr, n_scen=1, stream=None):
+        _check(self.L, self.L.gelato_eval_path_rows_dev(self.h, x_ptr, g_ptr, vals_ptr, n_scen, stream),
+               "gelato_eval_path_rows_dev")
 
     # ---- host-buffer calls (what objfunc / sens use) --------------------
     def _x(self, x, n_scen):

@@ -162,6 +162,8 @@ WRT = {
     "ineqcon_qalpha": ["position", "velocity", "quaternion", "t"], "ineqcon_mass": ["mass"], "ineqcon_kick": ["u"],
     "ineqcon_time": ["t"], "ineqcon_pos": ["position", "t"], "ineqcon_iip": ["position", "velocity", "t"],
     "ineqcon_antenna": ["position", "t"], "ineqcon_user": ["mass", "position", "velocity", "quaternion", "u", "t"],
+    # the aero constraints between the nodes (GelatoProblem(..., path_grid=...); DESIGN.md section 11)
+    "ineqcon_path": ["position", "velocity", "quaternion", "t"],
 }
 
 

@@ -1101,6 +1101,43 @@ class CompiledPlan:
         np.add.at(indptr, rows + 1, 1)
         return {"shape": (r0, o), "indptr": np.cumsum(indptr), "indices": cols, "src": src, "row0": row0}
 
+    PATH_VARS = ("position", "velocity", "quaternion", "t")
+
+    def path_rows_structure(self, layout):
+        """{variable: Block} of the path rows' Jacobian (DESIGN.md section 11) from the engine's path_rows_layout():
+        COO rows / cols and shape of each of position, velocity, quaternion and t, with `offset` the first of its entries
+        in the row values of one scenario -- each variable one contiguous range, entries in the order the C side writes
+        them (include/gelato_b200.h: gelato_plan_path_rows)."""
+        acc = {var: ([], []) for var in self.PATH_VARS}
+        first = {}
+        for k in range(layout["n_rows"]):
+            i = int(self.aero_i32[layout["job"][k], GA_SECTION])
+            xa, n = self._sec[i][2], self._sec[i][4]
+            off = layout["off"][k]
+            for c, (var, w) in enumerate((("position", 3), ("velocity", 3), ("quaternion", 4))):
+                if off[c] < 0:
+                    continue
+                first.setdefault(var, int(off[c]))
+                cols = (w * np.arange(xa, xa + n + 1)[:, None] + np.arange(w)).ravel()
+                acc[var][0].append(np.full(cols.size, k))
+                acc[var][1].append(cols)
+            first.setdefault("t", int(off[3]))
+            acc["t"][0].append([k, k])
+            acc["t"][1].append([i, i + 1])
+        nr = layout["n_rows"]
+        shapes = {"position": (nr, 3 * self.M), "velocity": (nr, 3 * self.M), "quaternion": (nr, 4 * self.M),
+                  "t": (nr, self.S + 1)}
+        out, o = {}, 0
+        for var in self.PATH_VARS:
+            blk = Block(o, _i4(acc[var][0]), _i4(acc[var][1]), shapes[var])
+            if var in first and first[var] != o:
+                raise ValueError("path-row layout is not variable-major")
+            out[var] = blk
+            o += blk.nnz
+        if o != layout["n_vals"]:
+            raise ValueError("path-row layout has %d values, the rows %d" % (layout["n_vals"], o))
+        return out
+
     def split_jacobian(self, vals, key_order=VAR_ORDER):
         """vals[n_vals] -> the reference's `funcsSens` dict; COO data arrays are
         views into `vals` (no copies)."""

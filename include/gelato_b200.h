@@ -336,6 +336,38 @@ int gelato_eval_path_check(GelatoPlan* plan, const double* x, double* res, int32
 int gelato_eval_path_check_dev(GelatoPlan* plan, const double* x_dev, double* res_dev, int32_t* at_dev, int32_t n_scen,
                                void* stream);
 
+/* Path rows (DESIGN.md section 11): the aero constraints as inequality rows of the NLP at the test points of a grid of
+ * their own, set per plan (separate from the grid of gelato_plan_set_mesh_grid, so re-gridding a diagnosis does not
+ * change the NLP).  Opt-in: a plan without path rows evaluates nothing new.
+ * Rows: the plan's aero jobs over a whole section (range "all"), in aero-job order, each job's test points l ascending,
+ * except a test point whose P row is exactly a unit vector (a support point: that node's own row already holds the
+ * constraint there; on the default grid of n + 1 flipped LGR points that drops +1).
+ * Value: r = 1 - f(v_l, tn_l) / L, exactly the path check's residual at that test point (same interpolation, time,
+ * units and wind table), bit for bit.
+ * Jacobian, by the chain rule through the interpolation (the NLP's node rows follow the reference's perturbation
+ * protocol; these rows have no reference counterpart):
+ *     gq_c = -fd_div(f(v_l + dx e_c, tn_l) - f(v_l, tn_l), dx)   for the 10 state components c (position 3 |
+ *            velocity 3 | quaternion 4; max-q rows have no quaternion entries); entry of state row xa + m: P[l][m] gq_c
+ *     gq_to / gq_tf: the same with tn_l at to + dx / tf + dx and v_l unchanged; one entry each
+ * with dx the plan's dx in forward mode; in central mode (gelato_plan_set_fd, DESIGN.md H6) every quotient is
+ * fd_central(gq(+h), gq(-h)).  The entries follow the mode at launch.
+ * Values of one scenario, variable-major (each funcsSens block a contiguous range): position, 3 (n + 1) per row in
+ * (m, c) order, rows in list order | velocity, the same | quaternion, 4 (n + 1) per row of kinds alpha and Q-alpha |
+ * t, (to, tf) per row.
+ * gelato_plan_set_path_rows: the grid as gelato_plan_set_mesh_grid takes it, with the same checks and reasons; a
+ * refused grid leaves the plan unchanged.
+ * gelato_plan_path_rows: *n_rows, *n_vals (values per scenario) and, per row, its aero job, test point and the offsets
+ * off[row][4] (position | velocity | quaternion (-1: none) | t) of its entries; job / l / off may be NULL.
+ * gelato_eval_path_rows: g_path[n_scen][n_rows] and vals_path[n_scen][n_vals] of x[n_scen][n_vars]; either may be NULL
+ * (g_path only: the centre evaluations alone).  Host buffers as gelato_eval_path_check; _dev: device pointers on
+ * `stream` (NULL = the plan's own), not synchronised.  Both use the scenario blocks and refuse an n_scen beyond them,
+ * refuse calls before path rows are set, and write nothing for a plan with zero rows.  One launch (k_path_rows). */
+int gelato_plan_set_path_rows(GelatoPlan* plan, const GelatoMeshGridDesc* grid);
+int gelato_plan_path_rows(const GelatoPlan* plan, int32_t* n_rows, int64_t* n_vals, int32_t* job, int32_t* l, int64_t* off);
+int gelato_eval_path_rows(GelatoPlan* plan, const double* x, double* g_path, double* vals_path, int32_t n_scen);
+int gelato_eval_path_rows_dev(GelatoPlan* plan, const double* x_dev, double* g_dev, double* vals_dev, int32_t n_scen,
+                              void* stream);
+
 int gelato_host_alloc(size_t bytes, void** out);
 int gelato_host_free(void* ptr);
 
