@@ -360,6 +360,12 @@ using gelato_host::GraphExec;
 using gelato_host::PinnedBuf;
 using gelato_host::Stream;
 
+// a test grid on the device (gelato_plan_set_mesh_grid, gelato_plan_set_path_rows): its sections and table pool
+struct TestGrid {
+  DeviceBuf<MeshSec> sec;
+  DeviceBuf<double> pool;
+};
+
 struct GelatoPlan {
   int device = 0;
   PlanView view{};         // device pointers
@@ -382,9 +388,11 @@ struct GelatoPlan {
   long long vals_template_sstride = 0;
   int n_scen_cfg = 1;
   // staging of every host-buffer entry point: x, g and the scenario ids of the batch slots, which hold either the
-  // caller's ids or 0, 1, 2 ... (ids_iota)
+  // caller's ids or 0, 1, 2 ... (ids_iota); the outputs of a diagnostic on a test grid (eval_diag), at most two a call
   DeviceBuf<double> d_x, d_g;
   PinnedBuf<double> h_x, h_g;
+  DeviceBuf<char> d_diag[2];
+  PinnedBuf<char> h_diag[2];
   DeviceBuf<int32_t> d_ids;
   bool ids_iota = false;
   // COO Jacobian of the host entry points: slot k of d_vals holds scenario k's constants for k < vals_filled (written
@@ -430,32 +438,27 @@ struct GelatoPlan {
   DeviceBuf<double> d_fd;
   const int64_t *d_pk_full = nullptr, *d_pk_src = nullptr;  // the packed map on the device (uploaded on first use)
   const double* d_pk_sgn = nullptr;
-  // mesh error estimate (gelato_plan_set_mesh_grid): the grid's sections, test points and table pool on the device,
-  // n_mesh_pts = 0 until a grid is set; d_mesh_pts is the per-point scratch, d_err / h_err the host entry's staging
+  // mesh error estimate (gelato_plan_set_mesh_grid): the grid and its test points on the device, n_mesh_pts = 0 until
+  // a grid is set; d_mesh_pts is the per-point scratch
   std::vector<int32_t> sec_n;  // LGR nodes of each section
-  DeviceBuf<MeshSec> d_mesh_sec;
+  TestGrid mesh_grid;
   DeviceBuf<MeshPt> d_mesh_pt;
-  DeviceBuf<double> d_mesh_pool, d_mesh_pts, d_err;
-  PinnedBuf<double> h_err;
+  DeviceBuf<double> d_mesh_pts;
   int n_mesh_pts = 0;
   // path check on the same grid: the test points of the aero jobs over a whole section and each job's first one
-  // (plan_host.h: build_path_points, rebuilt with the grid), the per-point scratch d_path_r, the host entry's staging
+  // (plan_host.h: build_path_points, rebuilt with the grid), the per-point scratch d_path_r
   std::vector<int32_t> aero_i32;  // the aero jobs, as the plan description gave them
   DeviceBuf<PathPt> d_path_pt;
-  DeviceBuf<int32_t> d_path_job0, d_at;
-  DeviceBuf<double> d_path_r, d_res;
-  PinnedBuf<double> h_res;
-  PinnedBuf<int32_t> h_at;
+  DeviceBuf<int32_t> d_path_job0;
+  DeviceBuf<double> d_path_r;
   int n_path_pts = 0;
-  // path rows (gelato_plan_set_path_rows) on a grid of their own: its sections and pool, the row list (plan_host.h:
-  // build_path_rows) on the host and the device, the values per scenario, and the host entry's staging
+  // path rows (gelato_plan_set_path_rows) on a grid of their own: the grid, the row list (plan_host.h: build_path_rows)
+  // on the host and the device, and the values per scenario
   bool prow_set = false;
   std::vector<PathRow> prow;
   long long prow_vals = 0;
-  DeviceBuf<MeshSec> d_prow_sec;
-  DeviceBuf<double> d_prow_pool, d_prow_g, d_prow_v;
+  TestGrid prow_grid;
   DeviceBuf<PathRow> d_prow;
-  PinnedBuf<double> h_prow_g, h_prow_v;
   long long launches = 0;
   Event ev0, ev1;
 };
@@ -955,6 +958,49 @@ template <typename T>
 static void land(T* out, const T* dst, size_t n) {
   if (dst != out) memcpy(out, dst, n * sizeof(T));
 }
+
+// d = src[0 .. n), copied on `st`
+template <typename T>
+static int upload_async(DeviceBuf<T>& d, const T* src, size_t n, cudaStream_t st) {
+  CU(d.reserve(n));
+  if (n) CU(cudaMemcpyAsync(d.get(), src, n * sizeof(T), cudaMemcpyHostToDevice, st));
+  return GELATO_OK;
+}
+
+// The host-buffer form of a diagnostic with outputs out0 / out1 of bytes0 / bytes1 (NULL: not computed), on lane 0:
+// x[n_scen][n_vars] staged and uploaded, launch(x_dev, out0_dev, out1_dev, stream) into the plan's output slots, and
+// each output downloaded into the caller's buffer, through the pinned slot when that buffer is pageable.
+template <typename Launch>
+static int eval_diag(GelatoPlan* p, const double* x, int32_t n_scen, void* out0, size_t bytes0, void* out1, size_t bytes1,
+                     Launch launch) {
+  CU(cudaSetDevice(p->device));
+  int rc = ensure_staging(p, n_scen);
+  if (rc) return rc;
+  const cudaStream_t st = p->lanes[0].stream;
+  const size_t nx = (size_t)n_scen * p->view.n_vars, bytes[2] = {bytes0, bytes1};
+  char *const out[2] = {(char*)out0, (char*)out1}, *dst[2];
+  for (int k = 0; k < 2; k++)
+    if (out[k]) CU(p->d_diag[k].reserve(bytes[k]));
+  CU(cudaMemcpyAsync(p->d_x.get(), host_src(x, p->h_x.get(), nx), nx * sizeof(double), cudaMemcpyHostToDevice, st));
+  if ((rc = launch(p->d_x.get(), out0 ? p->d_diag[0].get() : nullptr, out1 ? p->d_diag[1].get() : nullptr, st))) return rc;
+  for (int k = 0; k < 2; k++) {
+    if ((rc = host_dst(out[k], p->h_diag[k], bytes[k], &dst[k]))) return rc;
+    if (out[k]) CU(cudaMemcpyAsync(dst[k], p->d_diag[k].get(), bytes[k], cudaMemcpyDeviceToHost, st));
+  }
+  CU(cudaStreamSynchronize(st));
+  for (int k = 0; k < 2; k++) land(out[k], dst[k], bytes[k]);
+  return GELATO_OK;
+}
+}
+
+// The start of replacing a test grid once its lists are built: nothing in flight may still read the grid being
+// replaced, then the sections `secs` and the pool of g go to `tg` on lane 0's stream.  The caller uploads its own lists
+// on that stream and synchronises it.
+static int upload_grid(GelatoPlan* p, TestGrid& tg, const std::vector<MeshSec>& secs, const GelatoMeshGridDesc* g) {
+  CU(cudaSetDevice(p->device));
+  CU(cudaDeviceSynchronize());
+  const int rc = upload_async(tg.sec, secs.data(), secs.size(), p->lanes[0].stream);
+  return rc ? rc : upload_async(tg.pool, g->pool, (size_t)g->pool_len, p->lanes[0].stream);
 }
 
 static int eval_host(GelatoPlan* p, int which, const double* x, double* out, int32_t n_scen,
@@ -1051,20 +1097,12 @@ int gelato_plan_set_mesh_grid(GelatoPlan* p, const GelatoMeshGridDesc* g) {
   std::vector<int32_t> job0;
   if (const char* why = build_path_points(p->aero_i32.data(), p->view.n_aero, secs, path_pts, job0))
     return fail(GELATO_ERR_ARG, why);
-  CU(cudaSetDevice(p->device));
-  CU(cudaDeviceSynchronize());  // nothing in flight may still read the grid being replaced
-  CU(p->d_mesh_sec.reserve(secs.size()));
-  CU(p->d_mesh_pt.reserve(pts.size()));
-  CU(p->d_mesh_pool.reserve((size_t)g->pool_len));
-  CU(p->d_path_pt.reserve(path_pts.size()));
-  CU(p->d_path_job0.reserve(job0.size()));
   const cudaStream_t st = p->lanes[0].stream;
-  CU(cudaMemcpyAsync(p->d_mesh_sec.get(), secs.data(), secs.size() * sizeof(MeshSec), cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(p->d_mesh_pt.get(), pts.data(), pts.size() * sizeof(MeshPt), cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(p->d_mesh_pool.get(), g->pool, (size_t)g->pool_len * sizeof(double), cudaMemcpyHostToDevice, st));
-  if (!path_pts.empty())
-    CU(cudaMemcpyAsync(p->d_path_pt.get(), path_pts.data(), path_pts.size() * sizeof(PathPt), cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(p->d_path_job0.get(), job0.data(), job0.size() * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+  int rc;
+  if ((rc = upload_grid(p, p->mesh_grid, secs, g)) || (rc = upload_async(p->d_mesh_pt, pts.data(), pts.size(), st)) ||
+      (rc = upload_async(p->d_path_pt, path_pts.data(), path_pts.size(), st)) ||
+      (rc = upload_async(p->d_path_job0, job0.data(), job0.size(), st)))
+    return rc;
   CU(cudaStreamSynchronize(st));
   p->n_mesh_pts = (int)pts.size();
   p->n_path_pts = (int)path_pts.size();
@@ -1078,9 +1116,9 @@ static int launch_mesh_error(GelatoPlan* p, const double* x_dev, double* err_dev
     return fail(GELATO_ERR_ARG, "test points x n_scen exceeds the grid limit");
   CU(p->d_mesh_pts.reserve((size_t)n1 * MESH_PT));
   k_mesh_points<<<(unsigned)((n1 + GM_THREADS - 1) / GM_THREADS), GM_THREADS, 0, st>>>(
-      p->view, p->d_mesh_pt.get(), p->d_mesh_sec.get(), p->d_mesh_pool.get(), p->n_mesh_pts, n_scen, x_dev, p->d_mesh_pts.get());
+      p->view, p->d_mesh_pt.get(), p->mesh_grid.sec.get(), p->mesh_grid.pool.get(), p->n_mesh_pts, n_scen, x_dev, p->d_mesh_pts.get());
   k_mesh_error<<<(unsigned)((n2 + GM_THREADS - 1) / GM_THREADS), GM_THREADS, 0, st>>>(
-      p->view, p->d_mesh_sec.get(), p->d_mesh_pool.get(), p->n_mesh_pts, n_scen, x_dev, p->d_mesh_pts.get(), err_dev);
+      p->view, p->mesh_grid.sec.get(), p->mesh_grid.pool.get(), p->n_mesh_pts, n_scen, x_dev, p->d_mesh_pts.get(), err_dev);
   p->launches += 2;
   CU(cudaGetLastError());
   return GELATO_OK;
@@ -1100,19 +1138,11 @@ int gelato_eval_mesh_error(GelatoPlan* p, const double* x, double* err, int32_t 
   if (rc) return rc;
   if (!p->n_mesh_pts) return fail(GELATO_ERR_ARG, GELATO_NO_MESH_GRID);
   if (!x || !err) return fail(GELATO_ERR_ARG, "null buffer");
-  CU(cudaSetDevice(p->device));
-  if ((rc = ensure_staging(p, n_scen))) return rc;
-  const cudaStream_t st = p->lanes[0].stream;
-  const size_t nx = (size_t)n_scen * p->view.n_vars, ne = (size_t)n_scen * p->view.S * MESH_STATE;
-  CU(p->d_err.reserve(ne));
-  CU(cudaMemcpyAsync(p->d_x.get(), host_src(x, p->h_x.get(), nx), nx * sizeof(double), cudaMemcpyHostToDevice, st));
-  if ((rc = launch_mesh_error(p, p->d_x.get(), p->d_err.get(), n_scen, st))) return rc;
-  double* dst;
-  if ((rc = host_dst(err, p->h_err, ne, &dst))) return rc;
-  CU(cudaMemcpyAsync(dst, p->d_err.get(), ne * sizeof(double), cudaMemcpyDeviceToHost, st));
-  CU(cudaStreamSynchronize(st));
-  land(err, dst, ne);
-  return GELATO_OK;
+  const size_t ne = (size_t)n_scen * p->view.S * MESH_STATE;
+  return eval_diag(p, x, n_scen, err, ne * sizeof(double), nullptr, 0,
+                   [&](const double* xd, void* o0, void*, cudaStream_t st) {
+                     return launch_mesh_error(p, xd, (double*)o0, n_scen, st);
+                   });
 }
 
 // ---- path check (mesh_error.h) ----
@@ -1128,7 +1158,7 @@ static int launch_path_check(GelatoPlan* p, const double* x_dev, double* res_dev
   CU(p->d_path_r.reserve((size_t)n1));
   if (n1 > 0) {
     k_path_points<<<(unsigned)((n1 + GM_THREADS - 1) / GM_THREADS), GM_THREADS, 0, st>>>(
-        p->view, p->d_path_pt.get(), p->d_mesh_sec.get(), p->d_mesh_pool.get(), n_pts, n_scen, x_dev, p->d_path_r.get());
+        p->view, p->d_path_pt.get(), p->mesh_grid.sec.get(), p->mesh_grid.pool.get(), n_pts, n_scen, x_dev, p->d_path_r.get());
     p->launches++;
   }
   k_path_min<<<(unsigned)((n2 + GM_THREADS - 1) / GM_THREADS), GM_THREADS, 0, st>>>(
@@ -1154,23 +1184,11 @@ int gelato_eval_path_check(GelatoPlan* p, const double* x, double* res, int32_t*
   if (!p->n_mesh_pts) return fail(GELATO_ERR_ARG, GELATO_NO_MESH_GRID);
   if (!x || (p->view.n_aero && (!res || !at))) return fail(GELATO_ERR_ARG, "null buffer");
   if (!p->view.n_aero) return GELATO_OK;
-  CU(cudaSetDevice(p->device));
-  if ((rc = ensure_staging(p, n_scen))) return rc;
-  const cudaStream_t st = p->lanes[0].stream;
-  const size_t nx = (size_t)n_scen * p->view.n_vars, na = (size_t)n_scen * p->view.n_aero;
-  CU(p->d_res.reserve(na));
-  CU(p->d_at.reserve(na));
-  CU(cudaMemcpyAsync(p->d_x.get(), host_src(x, p->h_x.get(), nx), nx * sizeof(double), cudaMemcpyHostToDevice, st));
-  if ((rc = launch_path_check(p, p->d_x.get(), p->d_res.get(), p->d_at.get(), n_scen, st))) return rc;
-  double* res_dst;
-  int32_t* at_dst;
-  if ((rc = host_dst(res, p->h_res, na, &res_dst)) || (rc = host_dst(at, p->h_at, na, &at_dst))) return rc;
-  CU(cudaMemcpyAsync(res_dst, p->d_res.get(), na * sizeof(double), cudaMemcpyDeviceToHost, st));
-  CU(cudaMemcpyAsync(at_dst, p->d_at.get(), na * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
-  CU(cudaStreamSynchronize(st));
-  land(res, res_dst, na);
-  land(at, at_dst, na);
-  return GELATO_OK;
+  const size_t na = (size_t)n_scen * p->view.n_aero;
+  return eval_diag(p, x, n_scen, res, na * sizeof(double), at, na * sizeof(int32_t),
+                   [&](const double* xd, void* o0, void* o1, cudaStream_t st) {
+                     return launch_path_check(p, xd, (double*)o0, (int32_t*)o1, n_scen, st);
+                   });
 }
 
 // ---- path rows (mesh_error.h) ----
@@ -1183,16 +1201,10 @@ int gelato_plan_set_path_rows(GelatoPlan* p, const GelatoMeshGridDesc* g) {
   long long n_vals = 0;
   if (const char* why = build_path_rows(p->aero_i32.data(), p->view.n_aero, p->sec_n.data(), secs, g->pool, rows, &n_vals))
     return fail(GELATO_ERR_ARG, why);
-  CU(cudaSetDevice(p->device));
-  CU(cudaDeviceSynchronize());  // nothing in flight may still read the rows being replaced
-  CU(p->d_prow_sec.reserve(secs.size()));
-  CU(p->d_prow_pool.reserve((size_t)g->pool_len));
-  CU(p->d_prow.reserve(rows.size()));
   const cudaStream_t st = p->lanes[0].stream;
-  CU(cudaMemcpyAsync(p->d_prow_sec.get(), secs.data(), secs.size() * sizeof(MeshSec), cudaMemcpyHostToDevice, st));
-  CU(cudaMemcpyAsync(p->d_prow_pool.get(), g->pool, (size_t)g->pool_len * sizeof(double), cudaMemcpyHostToDevice, st));
-  if (!rows.empty())
-    CU(cudaMemcpyAsync(p->d_prow.get(), rows.data(), rows.size() * sizeof(PathRow), cudaMemcpyHostToDevice, st));
+  int rc;
+  if ((rc = upload_grid(p, p->prow_grid, secs, g)) || (rc = upload_async(p->d_prow, rows.data(), rows.size(), st)))
+    return rc;
   CU(cudaStreamSynchronize(st));
   p->prow.swap(rows);
   p->prow_vals = n_vals;
@@ -1224,7 +1236,7 @@ static int launch_path_rows(GelatoPlan* p, const double* x_dev, double* g_dev, d
   if ((nt + GP_THREADS - 1) / GP_THREADS > 0x7fffffffLL) return fail(GELATO_ERR_ARG, "path rows x n_scen exceeds the grid limit");
   const int central = p->fd_mode == GELATO_FD_CENTRAL;
   k_path_rows<<<(unsigned)((nt + GP_THREADS - 1) / GP_THREADS), GP_THREADS, 0, st>>>(
-      p->view, p->d_prow.get(), p->d_prow_sec.get(), p->d_prow_pool.get(), n_rows, p->prow_vals, n_scen, lanes, central,
+      p->view, p->d_prow.get(), p->prow_grid.sec.get(), p->prow_grid.pool.get(), n_rows, p->prow_vals, n_scen, lanes, central,
       central ? p->fd_step : p->view.un.dx, x_dev, g_dev, vals_dev);
   p->launches++;
   CU(cudaGetLastError());
@@ -1247,25 +1259,11 @@ int gelato_eval_path_rows(GelatoPlan* p, const double* x, double* g_path, double
   if (!p->prow_set) return fail(GELATO_ERR_ARG, GELATO_NO_PATH_ROWS);
   if (!x) return fail(GELATO_ERR_ARG, "null buffer");
   if (p->prow.empty() || (!g_path && !vals_path)) return GELATO_OK;
-  CU(cudaSetDevice(p->device));
-  if ((rc = ensure_staging(p, n_scen))) return rc;
-  const cudaStream_t st = p->lanes[0].stream;
-  const size_t nx = (size_t)n_scen * p->view.n_vars, ng = (size_t)n_scen * p->prow.size(),
-               nv = (size_t)n_scen * (size_t)p->prow_vals;
-  if (g_path) CU(p->d_prow_g.reserve(ng));
-  if (vals_path) CU(p->d_prow_v.reserve(nv));
-  CU(cudaMemcpyAsync(p->d_x.get(), host_src(x, p->h_x.get(), nx), nx * sizeof(double), cudaMemcpyHostToDevice, st));
-  if ((rc = launch_path_rows(p, p->d_x.get(), g_path ? p->d_prow_g.get() : nullptr, vals_path ? p->d_prow_v.get() : nullptr,
-                             n_scen, st)))
-    return rc;
-  double *g_dst, *v_dst;
-  if ((rc = host_dst(g_path, p->h_prow_g, ng, &g_dst)) || (rc = host_dst(vals_path, p->h_prow_v, nv, &v_dst))) return rc;
-  if (g_path) CU(cudaMemcpyAsync(g_dst, p->d_prow_g.get(), ng * sizeof(double), cudaMemcpyDeviceToHost, st));
-  if (vals_path) CU(cudaMemcpyAsync(v_dst, p->d_prow_v.get(), nv * sizeof(double), cudaMemcpyDeviceToHost, st));
-  CU(cudaStreamSynchronize(st));
-  if (g_path) land(g_path, g_dst, ng);
-  if (vals_path) land(vals_path, v_dst, nv);
-  return GELATO_OK;
+  const size_t ng = (size_t)n_scen * p->prow.size(), nv = (size_t)n_scen * (size_t)p->prow_vals;
+  return eval_diag(p, x, n_scen, g_path, ng * sizeof(double), vals_path, nv * sizeof(double),
+                   [&](const double* xd, void* o0, void* o1, cudaStream_t st) {
+                     return launch_path_rows(p, xd, (double*)o0, (double*)o1, n_scen, st);
+                   });
 }
 
 int gelato_pack_xdep_dev(GelatoPlan* p, const double* vals_dev, double* packed_dev, int32_t n_scen, void* stream) {

@@ -116,19 +116,6 @@ P_HD void mesh_path_state(const PlanView& P, const double* x, int sec, const Mes
   dx_dot<4>(Prow, x + P.off_quat + 4 * xa, n + 1, v + 6);
 }
 
-/* The path check (DESIGN.md section 11): one test point of an aero job.  The job's section is interpolated at test
- * point l (mesh_path_state), and the residual is the expression aero_res gives objfunc's row at a node: pristine x,
- * the time of the test point, the scenario's units and wind table.  At a test point that is a node it is that row's
- * value, bit for bit. */
-P_HD double mesh_path_point(const PlanView& P, int scen, const double* x, int job, const MeshTabs& tb, int l) {
-  const int32_t* ai = P.aero_i32 + job * GA_I32_COLS;
-  const int sec = ai[GA_SECTION];
-  double v[10];
-  mesh_path_state(P, x, sec, tb, l, v);
-  const double tn = time_node(tb.tau, l + 1, x[P.off_t + sec], x[P.off_t + sec + 1]);
-  return 1.0 - aero_value(P, scen, ai[GA_KIND], v, tn, P.aero_f64[job * GA_F64_COLS + GA_LIMIT]);
-}
-
 /* ========================================================================= */
 /* Path rows (DESIGN.md section 11): the aero constraints as NLP rows at the  */
 /* test points of a grid of their own.  Per row 16 lanes:                     */
@@ -158,6 +145,16 @@ P_HD double path_lane_f(const PlanView& P, int scen, const double* x, int job, c
   if (lane == 11) to = to + dx;
   else if (lane == 12) tf = tf + dx;
   return aero_value(P, scen, ai[GA_KIND], w, time_node(tb.tau, l + 1, to, tf), P.aero_f64[job * GA_F64_COLS + GA_LIMIT]);
+}
+
+/* The path check (DESIGN.md section 11): one test point of an aero job.  The job's section is interpolated at test
+ * point l (mesh_path_state), and the residual is the expression aero_res gives objfunc's row at a node: pristine x,
+ * the time of the test point, the scenario's units and wind table (path_lane_f's centre lane).  At a test point that is
+ * a node it is that row's value, bit for bit. */
+P_HD double mesh_path_point(const PlanView& P, int scen, const double* x, int job, const MeshTabs& tb, int l) {
+  double v[10];
+  mesh_path_state(P, x, P.aero_i32[job * GA_I32_COLS + GA_SECTION], tb, l, v);
+  return 1.0 - path_lane_f(P, scen, x, job, tb, l, v, 0, 0.0);
 }
 
 /* the derivative of the row 1 - f / L along lane `lane` (1-12), f0 = the centre: -fd_div(f(step) - f0, step); central

@@ -5,7 +5,7 @@
 // all threads of a block, then phase 2 -- the same order the block barrier
 // enforces on the GPU (the Jacobian kernel has GJ_PHASES phases, the residual kernel two).  It lets the CPU-only test tier check the plan compiler
 // and the kernels' index arithmetic against the oracle bit for bit, in both
-// finite-difference modes, and the mesh error estimate (mesh_error.h).  It is not
+// finite-difference modes, and the mesh error estimate, the path check and the path rows (mesh_error.h).  It is not
 // part of the product: libgelato_b200.so has no CPU path and bench.py never
 // loads this file.
 #include <cstring>
@@ -169,45 +169,135 @@ extern "C" void emu_block_counts(const GelatoPlanDesc* d, int* n_blocks_pair, in
   *n_vac = h.n_vac;
 }
 
-// ---- mesh error estimate (mesh_error.h; DESIGN.md section 11) ----
-static std::vector<int32_t> sec_nodes(const GelatoPlanDesc* d) {
-  std::vector<int32_t> n(d->n_sections);
-  for (int i = 0; i < d->n_sections; i++) n[i] = d->sec_i32[i * GS_I32_COLS + GS_N];
-  return n;
+// ---- test grids: mesh error estimate, path check and path rows (mesh_error.h; DESIGN.md section 11) ----
+// What every entry point on a test grid starts from: the plan's view with the scenario blocks sc, the LGR nodes of
+// each section and grid g's sections and test points (plan_host.h: build_mesh_grid, what the grid setters keep).
+struct GridCall {
+  PlanView P;
+  std::vector<int32_t> n;
+  std::vector<MeshSec> ms;
+  std::vector<MeshPt> mp;
+};
+// NULL or why the call is refused: the description fails validate_desc, g == NULL (no grid set: `no_grid`) or the grid
+// fails build_mesh_grid
+static const char* grid_call(const GelatoPlanDesc* d, const GelatoScenarioDesc* sc, const GelatoMeshGridDesc* g,
+                             const char* no_grid, GridCall& c) {
+  if (const char* why = validate_desc(d)) return why;
+  if (!g) return no_grid;
+  c.P = host_view(d);
+  apply_scen(c.P, sc);
+  c.n.resize(d->n_sections);
+  for (int i = 0; i < d->n_sections; i++) c.n[i] = d->sec_i32[i * GS_I32_COLS + GS_N];
+  return build_mesh_grid(g, c.n.data(), d->n_sections, c.ms, c.mp);
 }
 
-// NULL or why gelato_plan_set_mesh_grid refuses the grid (plan_host.h: build_mesh_grid)
+// NULL or why gelato_plan_set_mesh_grid refuses the grid
 extern "C" const char* emu_check_mesh_grid(const GelatoPlanDesc* d, const GelatoMeshGridDesc* g) {
-  std::vector<MeshSec> secs;
-  std::vector<MeshPt> pts;
-  return build_mesh_grid(g, sec_nodes(d).data(), d->n_sections, secs, pts);
+  GridCall c;
+  return grid_call(d, nullptr, g, GELATO_NO_MESH_GRID, c);
 }
 
 // err_all: [n_scen][S][11]; what k_mesh_points (every test point) and then k_mesh_error (every section and state
-// component) compute
-extern "C" int emu_eval_mesh_error(const GelatoPlanDesc* d, const GelatoScenarioDesc* sc, const GelatoMeshGridDesc* g,
-                                   const double* x_all, double* err_all, int n_scen) {
-  if (validate_desc(d)) return -1;
-  PlanView P = host_view(d);
-  apply_scen(P, sc);
-  const std::vector<int32_t> n = sec_nodes(d);
-  std::vector<MeshSec> ms;
-  std::vector<MeshPt> mp;
-  if (build_mesh_grid(g, n.data(), P.S, ms, mp)) return -1;
-  std::vector<double> pts(mp.size() * MESH_PT);
+// component) compute.  Returns NULL or why gelato_eval_mesh_error refuses the call (g == NULL: no grid set).
+extern "C" const char* emu_eval_mesh_error(const GelatoPlanDesc* d, const GelatoScenarioDesc* sc, const GelatoMeshGridDesc* g,
+                                           const double* x_all, double* err_all, int n_scen) {
+  GridCall c;
+  if (const char* why = grid_call(d, sc, g, GELATO_NO_MESH_GRID, c)) return why;
+  const PlanView& P = c.P;
+  std::vector<double> pts(c.mp.size() * MESH_PT);
   for (int scen = 0; scen < n_scen; scen++) {
     const double* x = x_all + (size_t)scen * P.n_vars;
-    for (size_t k = 0; k < mp.size(); k++) {
-      const MeshPt q = mp[k];
+    for (size_t k = 0; k < c.mp.size(); k++) {
+      const MeshPt q = c.mp[k];
       double* out = pts.data() + k * MESH_PT;
-      mesh_point(P, scen, x, q.sec, mesh_tabs(g->pool, ms[q.sec], n[q.sec]), q.l, out, out + MESH_STATE);
+      mesh_point(P, scen, x, q.sec, mesh_tabs(g->pool, c.ms[q.sec], c.n[q.sec]), q.l, out, out + MESH_STATE);
     }
     for (int i = 0; i < P.S; i++)
-      for (int c = 0; c < MESH_STATE; c++)
-        err_all[((size_t)scen * P.S + i) * MESH_STATE + c] = mesh_component(
-            P, x, i, mesh_tabs(g->pool, ms[i], n[i]), ms[i].m, pts.data() + (size_t)ms[i].pt0 * MESH_PT, c);
+      for (int k = 0; k < MESH_STATE; k++)
+        err_all[((size_t)scen * P.S + i) * MESH_STATE + k] = mesh_component(
+            P, x, i, mesh_tabs(g->pool, c.ms[i], c.n[i]), c.ms[i].m, pts.data() + (size_t)c.ms[i].pt0 * MESH_PT, k);
   }
-  return 0;
+  return nullptr;
+}
+
+// res_all / at_all: [n_scen][n_aero]; what k_path_points (every test point of the aero jobs over a whole section) and
+// then k_path_min (every aero job) compute.  Returns NULL or why gelato_eval_path_check refuses the call (g == NULL: no
+// grid set).
+extern "C" const char* emu_eval_path_check(const GelatoPlanDesc* d, const GelatoScenarioDesc* sc, const GelatoMeshGridDesc* g,
+                                           const double* x_all, double* res_all, int32_t* at_all, int n_scen) {
+  GridCall c;
+  if (const char* why = grid_call(d, sc, g, GELATO_NO_MESH_GRID, c)) return why;
+  std::vector<PathPt> pp;
+  std::vector<int32_t> job0;
+  if (const char* why = build_path_points(d->aero_i32, d->n_aero, c.ms, pp, job0)) return why;
+  std::vector<double> r(pp.size());
+  for (int scen = 0; scen < n_scen; scen++) {
+    const double* x = x_all + (size_t)scen * c.P.n_vars;
+    for (size_t k = 0; k < pp.size(); k++) {
+      const int sec = d->aero_i32[pp[k].job * GA_I32_COLS + GA_SECTION];
+      r[k] = mesh_path_point(c.P, scen, x, pp[k].job, mesh_tabs(g->pool, c.ms[sec], c.n[sec]), pp[k].l);
+    }
+    for (int j = 0; j < d->n_aero; j++)
+      mesh_path_min(r.data() + job0[j], job0[j + 1] - job0[j], res_all + (size_t)scen * d->n_aero + j,
+                    at_all + (size_t)scen * d->n_aero + j);
+  }
+  return nullptr;
+}
+
+// The path rows of grid g (plan_host.h: build_path_rows, what gelato_plan_set_path_rows keeps): *n_rows, *n_vals and,
+// where the arrays are not NULL, each row's job, test point and offsets [n_rows][PR_OFFS] (gelato_plan_path_rows).
+// Returns NULL or why gelato_plan_set_path_rows refuses the grid.
+extern "C" const char* emu_plan_path_rows(const GelatoPlanDesc* d, const GelatoMeshGridDesc* g, int32_t* n_rows,
+                                          int64_t* n_vals, int32_t* job, int32_t* l, int64_t* off) {
+  GridCall c;
+  std::vector<PathRow> rows;
+  long long nv = 0;
+  if (const char* why = grid_call(d, nullptr, g, GELATO_NO_PATH_ROWS, c)) return why;
+  if (const char* why = build_path_rows(d->aero_i32, d->n_aero, c.n.data(), c.ms, g->pool, rows, &nv)) return why;
+  *n_rows = (int32_t)rows.size();
+  *n_vals = nv;
+  for (size_t k = 0; k < rows.size(); k++) {
+    if (job) job[k] = rows[k].job;
+    if (l) l[k] = rows[k].l;
+    if (off)
+      for (int i = 0; i < PR_OFFS; i++) off[k * PR_OFFS + i] = rows[k].off[i];
+  }
+  return nullptr;
+}
+
+// g_all: [n_scen][n_rows], vals_all: [n_scen][n_vals], either may be NULL; what k_path_rows computes, lane by lane, in
+// finite-difference mode `fd_mode` (gelato_plan_set_fd) with step `step` (forward: the plan's dx).  Returns NULL or why
+// gelato_eval_path_rows refuses the call (g == NULL: no path rows set).
+extern "C" const char* emu_eval_path_rows(const GelatoPlanDesc* d, const GelatoScenarioDesc* sc, const GelatoMeshGridDesc* g,
+                                          const double* x_all, double* g_all, double* vals_all, int n_scen, int32_t fd_mode,
+                                          double step) {
+  GridCall c;
+  std::vector<PathRow> rows;
+  long long nv = 0;
+  if (const char* why = grid_call(d, sc, g, GELATO_NO_PATH_ROWS, c)) return why;
+  if (const char* why = build_path_rows(d->aero_i32, d->n_aero, c.n.data(), c.ms, g->pool, rows, &nv)) return why;
+  const PlanView& P = c.P;
+  const int central = fd_mode == GELATO_FD_CENTRAL;
+  const double dx = central ? step : P.un.dx;
+  for (int scen = 0; scen < n_scen; scen++) {
+    const double* x = x_all + (size_t)scen * P.n_vars;
+    for (size_t k = 0; k < rows.size(); k++) {
+      const PathRow& pr = rows[k];
+      const int sec = d->aero_i32[pr.job * GA_I32_COLS + GA_SECTION];
+      const MeshTabs tb = mesh_tabs(g->pool, c.ms[sec], c.n[sec]);
+      double v[10];
+      mesh_path_state(P, x, sec, tb, pr.l, v);
+      const double f0 = path_lane_f(P, scen, x, pr.job, tb, pr.l, v, 0, 0.0);
+      if (g_all) g_all[(size_t)scen * rows.size() + k] = 1.0 - f0;
+      if (!vals_all) continue;
+      for (int lane = 1; lane <= 12; lane++) {
+        if (pr.off[PR_QUAT] < 0 && lane >= 7 && lane <= 10) continue;
+        const double q = path_lane_quot(P, scen, x, pr.job, tb, pr.l, v, lane, f0, central, dx);
+        path_lane_store(pr, tb.P + (long long)pr.l * (c.n[sec] + 1), c.n[sec], lane, q, vals_all + (size_t)scen * nv);
+      }
+    }
+  }
+  return nullptr;
 }
 
 // packed layout of a plan: returns n_pack; with non-NULL arrays also the map of the n_xdep COO slots

@@ -2,7 +2,8 @@
 
 TEST HARNESS ONLY: lets the CPU test tier run the kernels' per-thread code
 (gelato_b200/csrc/jobs.h, mesh_error.h) through the same GelatoPlanDesc the GPU library gets, with the settings
-gelato_b200.engine.Engine has: the finite-difference mode (DESIGN.md H6) and the mesh grid (DESIGN.md section 11).
+gelato_b200.engine.Engine has: the finite-difference mode (DESIGN.md H6), the mesh grid and the grid of the path rows
+(DESIGN.md section 11).
 """
 import ctypes
 import os
@@ -55,14 +56,31 @@ class Emulator:
         L.emu_n_xdep.argtypes = [pdesc]
         L.emu_n_xdep.restype = ctypes.c_longlong
         L.emu_check_mesh_grid.argtypes = [pdesc, pgrid]
-        L.emu_check_mesh_grid.restype = ctypes.c_char_p
         L.emu_eval_mesh_error.argtypes = [pdesc, psc, pgrid, _pd, _pd, c_int]
+        L.emu_eval_path_check.argtypes = [pdesc, psc, pgrid, _pd, _pd, _pi32, c_int]
+        L.emu_plan_path_rows.argtypes = [pdesc, pgrid, _pi32, _pi64, _pi32, _pi32, _pi64]
+        L.emu_eval_path_rows.argtypes = [pdesc, psc, pgrid, _pd, _pd, _pd, c_int, ctypes.c_int32, ctypes.c_double]
+        for f in (L.emu_check_mesh_grid, L.emu_eval_mesh_error, L.emu_eval_path_check, L.emu_plan_path_rows,
+                  L.emu_eval_path_rows):
+            f.restype = ctypes.c_char_p  # NULL or the reason of a refusal
         self.n_pack = int(L.emu_packed_map(ctypes.byref(self.desc), None, None, None))
         self._fd = engine.fd_args("forward")  # (C mode code, step) as gelato_plan_set_fd takes them
-        self._grid = None
+        self._grid = None  # the mesh grid once set
+        self._prow = None  # (grid, layout) of the path rows once set
 
     def _sc(self):
         return ctypes.byref(self.sc) if self.sc is not None else None
+
+    @staticmethod
+    def _grid_ptr(grid):
+        return None if grid is None else ctypes.byref(grid[0])
+
+    @staticmethod
+    def _check(why, what):
+        """engine._check for the entry points that return NULL or the reason of a refusal: engine.GelatoError as the C
+        entry point `what` raises it."""
+        if why is not None:
+            raise engine.GelatoError("%s failed (-1): %s" % (what, why.decode()))
 
     @staticmethod
     def _ids(scen_ids):
@@ -83,13 +101,30 @@ class Emulator:
         return ("central", step) if code == engine.FD_MODES["central"] else ("forward", float(self.plan.units[5]))
 
     def set_mesh_grid(self, tables):
-        """engine.Engine.set_mesh_grid: a grid gelato_plan_set_mesh_grid refuses raises ValueError(<its reason>) and
-        the previous grid stays."""
+        """engine.Engine.set_mesh_grid: a grid gelato_plan_set_mesh_grid refuses raises engine.GelatoError with its
+        reason and the previous grid stays."""
         grid = engine.make_mesh_grid_desc(tables)
-        why = self.L.emu_check_mesh_grid(ctypes.byref(self.desc), ctypes.byref(grid[0]))
-        if why is not None:
-            raise ValueError(why.decode())
+        self._check(self.L.emu_check_mesh_grid(ctypes.byref(self.desc), ctypes.byref(grid[0])),
+                    "gelato_plan_set_mesh_grid")
         self._grid = grid
+
+    def set_path_rows(self, tables):
+        """engine.Engine.set_path_rows: a grid gelato_plan_set_path_rows refuses raises engine.GelatoError with its
+        reason and the previous rows stay."""
+        grid = engine.make_mesh_grid_desc(tables)
+        n, v = ctypes.c_int32(0), ctypes.c_int64(0)
+        args = (ctypes.byref(self.desc), ctypes.byref(grid[0]), ctypes.byref(n), ctypes.byref(v))
+        self._check(self.L.emu_plan_path_rows(*args, None, None, None), "gelato_plan_set_path_rows")
+        job, l = np.empty(n.value, dtype=np.int32), np.empty(n.value, dtype=np.int32)
+        off = np.empty((n.value, 4), dtype=np.int64)
+        self.L.emu_plan_path_rows(*args, job.ctypes.data_as(_pi32), l.ctypes.data_as(_pi32), off.ctypes.data_as(_pi64))
+        self._prow = (grid, {"n_rows": n.value, "n_vals": v.value, "job": job, "l": l, "off": off})
+
+    def path_rows_layout(self):
+        """engine.Engine.path_rows_layout."""
+        if self._prow is None:
+            raise engine.GelatoError("gelato_plan_path_rows failed (-1): no path rows set (gelato_plan_set_path_rows)")
+        return self._prow[1]
 
     # ---- evaluations ----
     def eval_residuals(self, x, n_scen=1, scen_ids=None):
@@ -135,14 +170,41 @@ class Emulator:
         return full, src, sgn
 
     def mesh_error(self, x, n_scen=1):
-        """engine.Engine.mesh_error."""
-        assert self._grid is not None, "no mesh grid set"
+        """engine.Engine.mesh_error: a call gelato_eval_mesh_error refuses raises engine.GelatoError with its reason."""
         x = np.ascontiguousarray(x, dtype=np.float64)
         err = np.full(n_scen * self.plan.S * 11, np.nan)
-        rc = self.L.emu_eval_mesh_error(ctypes.byref(self.desc), self._sc(), ctypes.byref(self._grid[0]),
-                                        x.ctypes.data_as(_pd), err.ctypes.data_as(_pd), n_scen)
-        assert rc == 0, "the plan description failed validate_desc (plan_host.h)"
+        self._check(self.L.emu_eval_mesh_error(ctypes.byref(self.desc), self._sc(), self._grid_ptr(self._grid),
+                                               x.ctypes.data_as(_pd), err.ctypes.data_as(_pd), n_scen),
+                    "gelato_eval_mesh_error")
         return err.reshape(self.plan.S, 11) if n_scen == 1 else err.reshape(n_scen, self.plan.S, 11)
+
+    def path_check(self, x, n_scen=1):
+        """engine.Engine.path_check: a call gelato_eval_path_check refuses raises engine.GelatoError with its reason."""
+        x = np.ascontiguousarray(x, dtype=np.float64)
+        n = n_scen * self.plan.n_aero
+        res, at = np.full(n, np.nan), np.full(n, -2, dtype=np.int32)
+        self._check(self.L.emu_eval_path_check(ctypes.byref(self.desc), self._sc(), self._grid_ptr(self._grid),
+                                               x.ctypes.data_as(_pd), res.ctypes.data_as(_pd), at.ctypes.data_as(_pi32),
+                                               n_scen), "gelato_eval_path_check")
+        return (res, at) if n_scen == 1 else (res.reshape(n_scen, -1), at.reshape(n_scen, -1))
+
+    def eval_path_rows(self, x, n_scen=1, jacobian=True, out=None):
+        """engine.Engine.eval_path_rows, in the emulator's finite-difference mode (set_fd)."""
+        x = np.ascontiguousarray(x, dtype=np.float64)
+        grid, lay = self._prow if self._prow is not None else (None, {"n_rows": 0, "n_vals": 0})
+        nr, nv = lay["n_rows"], lay["n_vals"]
+        if out is not None:
+            g = None if out[0] is None else engine._out(out[0], n_scen * nr, "out[0]")
+            v = None if out[1] is None else engine._out(out[1], n_scen * nv, "out[1]")
+        else:
+            g, v = np.full(n_scen * nr, np.nan), (np.full(n_scen * nv, np.nan) if jacobian else None)
+        self._check(self.L.emu_eval_path_rows(ctypes.byref(self.desc), self._sc(), self._grid_ptr(grid),
+                                              x.ctypes.data_as(_pd), None if g is None else g.ctypes.data_as(_pd),
+                                              None if v is None else v.ctypes.data_as(_pd), n_scen, *self._fd),
+                    "gelato_eval_path_rows")
+        if n_scen > 1:
+            g, v = (None if a is None else a.reshape(n_scen, -1) for a in (g, v))
+        return g, v
 
     # ---- one problem sharded over ranks (gelato_b200/batch.py: ShardedProblem) ----
     def block_counts(self):
@@ -181,6 +243,10 @@ class EmuEngine(Emulator):
         self.launches += 1
         self.calls += 1
         return super().eval_jacobian(x, n_scen, scen_ids)
+
+    def eval_path_rows(self, x, n_scen=1, jacobian=True, out=None):
+        self.calls += 1
+        return super().eval_path_rows(x, n_scen, jacobian, out)
 
     # update mode as the drop-in's default `sens` uses it: one output buffer kept across calls
     class _HostArray:

@@ -19,7 +19,6 @@ import pytest
 
 import central_oracle
 import emu_binding
-import emu_path
 import helpers
 import mesh_oracle
 import path_oracle
@@ -440,7 +439,7 @@ def test_mesh_error_and_path_check_on_edge_states(variant, case):
     """The mesh error estimate and the path check of the kernels' code against tests/mesh_oracle.py and
     tests/path_oracle.py, NaN propagation and the first NaN's index included."""
     p, u, c, x0, O, P = _setup(variant)
-    E = emu_path.PathEmuEngine(P)
+    E = emu_binding.EmuEngine(P)
     tabs = mesh.grid_tables(P.ps)
     E.set_mesh_grid(tabs)
     x = CATALOGUE[case][0](x0, P)

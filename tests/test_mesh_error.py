@@ -325,7 +325,7 @@ def test_emulator_refused_grids_keep_the_previous_grid_and_fd_mode_is_irrelevant
     E.set_mesh_grid(tabs)
     ref = E.mesh_error(x)
     for t, why in _malformed_grids(tabs):
-        with pytest.raises(ValueError, match=why):
+        with pytest.raises(engine.GelatoError, match=why):
             E.set_mesh_grid(t)
         assert _same_bits(E.mesh_error(x), ref)
     E.set_fd("central")

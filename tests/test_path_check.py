@@ -11,7 +11,7 @@ import ctypes
 import numpy as np
 import pytest
 
-import emu_path
+import emu_binding
 import helpers
 import mesh_oracle
 import path_oracle
@@ -80,7 +80,7 @@ def _job(P, kind, name):
 @pytest.mark.parametrize("variant,factor", VARIANTS)
 def test_emulator_equals_oracle_bit_for_bit(variant, factor):
     p, u, c, x0, O, P = _setup(variant, factor)
-    E = emu_path.PathEmuEngine(P)
+    E = emu_binding.EmuEngine(P)
     assert P.n_aero > 0
     for tabs in (mesh.grid_tables(O.ps), _square_grid(O.ps)):
         E.set_mesh_grid(tabs)
@@ -95,7 +95,7 @@ def test_all_aero_has_every_kind_and_both_ranges():
     assert {int(k) for k in P.aero_i32[:, 0]} == {0, 1, 2}
     assert {int(k) for k, _, nk, _ in P.aero_i32 if nk == 1} == {0, 1, 2}  # "initial" jobs
     assert {int(k) for k, _, nk, _ in P.aero_i32 if nk > 1} == {0, 1, 2}  # "all" jobs
-    E = emu_path.PathEmuEngine(P)
+    E = emu_binding.EmuEngine(P)
     E.set_mesh_grid(mesh.grid_tables(O.ps))
     res, at = E.path_check(problem.xdict_to_vector(helpers.perturbed(x0)))
     initial = P.aero_i32[:, 2] == 1
@@ -106,7 +106,7 @@ def test_all_aero_has_every_kind_and_both_ranges():
 def test_bare_plan_has_no_aero_jobs_and_an_empty_result():
     p, u, c, x0, O, P = _setup("bare")
     assert P.n_aero == 0
-    E = emu_path.PathEmuEngine(P)
+    E = emu_binding.EmuEngine(P)
     E.set_mesh_grid(mesh.grid_tables(O.ps))
     res, at = E.path_check(problem.xdict_to_vector(x0))
     assert res.shape == (0,) and at.shape == (0,)
@@ -120,7 +120,7 @@ def test_test_points_at_nodes_are_objfunc_rows(variant):
     """A test point that is an LGR node gives objfunc's row there bit for bit: one node per section at a time, the square
     grid (the minimum of the job's node rows after the first) and the default grid's last point (the job's last row)."""
     p, u, c, x0, O, P = _setup(variant)
-    E = emu_path.PathEmuEngine(P)
+    E = emu_binding.EmuEngine(P)
     x = helpers.perturbed(x0)
     xv = problem.xdict_to_vector(x)
     g = E.eval_residuals(xv)
@@ -148,7 +148,7 @@ def test_test_points_at_nodes_are_objfunc_rows(variant):
 def test_example_solution_violates_q_alpha_between_the_nodes():
     """The converged example holds Q-alpha at ZEROLIFT_START's nodes and exceeds it by 6 % in between."""
     p, u, c, x0, O, P = _setup("example")
-    E = emu_path.PathEmuEngine(P)
+    E = emu_binding.EmuEngine(P)
     tabs = mesh.grid_tables(O.ps)
     E.set_mesh_grid(tabs)
     x = _solution(P)
@@ -167,9 +167,10 @@ def test_example_solution_violates_q_alpha_between_the_nodes():
 
 def test_emulator_refuses_a_call_before_a_grid_is_set():
     p, u, c, x0, O, P = _setup("example")
-    E = emu_path.PathEmuEngine(P)
-    with pytest.raises(engine.GelatoError, match="no mesh grid set"):
-        E.path_check(problem.xdict_to_vector(x0))
+    E = emu_binding.EmuEngine(P)
+    for call in (E.path_check, E.mesh_error):
+        with pytest.raises(engine.GelatoError, match="no mesh grid set"):
+            call(problem.xdict_to_vector(x0))
 
 
 def test_refine_nodes_with_path_rule_cap_and_unchanged_without_it():
@@ -213,7 +214,7 @@ def test_gelato_problem_path_check_on_the_emulator():
     Lg = leaves.get("gmath")
     p, u, c, x0 = helpers.example_problem(coord=Lg.coordinate_c)
     prob = callbacks.GelatoProblem(p, u, c, user_eq=callbacks.PerigeeAtEvent(helpers.USER_EVENT), coord=Lg.coordinate_c,
-                                   engine_factory=emu_path.PathEmuEngine)
+                                   engine_factory=emu_binding.EmuEngine)
     P = prob.plan
     x = _solution(P)
     got = prob.path_check(x)

@@ -10,7 +10,7 @@ import ctypes
 import numpy as np
 import pytest
 
-import emu_path_rows
+import emu_binding
 import helpers
 import mesh_oracle
 import path_rows_oracle
@@ -69,7 +69,7 @@ def _want_layout(O, P, tabs):
 @pytest.mark.parametrize("variant,factor", VARIANTS)
 def test_emulator_equals_oracle_bit_for_bit(variant, factor):
     p, u, c, x0, O, P = _setup(variant, factor)
-    E = emu_path_rows.PathRowsEmuEngine(P)
+    E = emu_binding.EmuEngine(P)
     for tabs in _grids(O.ps):
         E.set_path_rows(tabs)
         lay = E.path_rows_layout()
@@ -87,7 +87,7 @@ def test_row_counts_and_the_support_point_rule():
     counts = {("example", 1): (1, 16, 2752), ("all_aero", 1): (3, 37, 5694), ("example", 15): (12, 240, 50880)}
     for (variant, factor), (jobs, rows, vals) in counts.items():
         p, u, c, x0, O, P = _setup(variant, factor)
-        E = emu_path_rows.PathRowsEmuEngine(P)
+        E = emu_binding.EmuEngine(P)
         E.set_path_rows(mesh.grid_tables(O.ps))
         lay = E.path_rows_layout()
         assert (len(set(lay["job"])), lay["n_rows"], lay["n_vals"]) == (jobs, rows, vals), variant
@@ -104,7 +104,7 @@ def test_row_counts_and_the_support_point_rule():
         pool[o + M + 3 * (n + 1): o + M + 4 * (n + 1)] = mesh.lagrange_basis(np.hstack((-1.0, O.ps.tau(i))), pool[o + 3:o + 4])[0]
         assert np.array_equal(pool[o + M + 3 * (n + 1): o + M + 4 * (n + 1)], np.eye(n + 1)[3])
     forced = dict(tabs, pool=pool)
-    E = emu_path_rows.PathRowsEmuEngine(P)
+    E = emu_binding.EmuEngine(P)
     E.set_path_rows(forced)
     lay = E.path_rows_layout()
     lost = sum(1 for k, i, nk, _ in P.aero_i32 if nk > 1 and i in moved)
@@ -136,7 +136,7 @@ def test_rows_are_the_path_check_residuals(variant):
     """Row (j, l) is the path check's residual at test point l, and the minimum over job j's rows and its last node
     row (the dropped point +1) is path_check's res[j], bit for bit."""
     p, u, c, x0, O, P = _setup(variant)
-    E = emu_path_rows.PathRowsEmuEngine(P)
+    E = emu_binding.EmuEngine(P)
     tabs = mesh.grid_tables(O.ps)
     E.set_path_rows(tabs)
     E.set_mesh_grid(tabs)
@@ -194,7 +194,7 @@ def test_derivative_against_fourth_order_differences(variant, mode):
     the kinks of the piecewise-linear wind and CA tables, which neither quotient resolves, and the t blocks' true
     derivatives are at the quotients' noise level in both row sets."""
     p, u, c, x0, O, P = _setup(variant)
-    E = emu_path_rows.PathRowsEmuEngine(P)
+    E = emu_binding.EmuEngine(P)
     tabs = mesh.grid_tables(O.ps)
     E.set_path_rows(tabs)
     E.set_fd(mode)
@@ -236,7 +236,7 @@ def _problem(path_grid=None, **kw):
     Lg = leaves.get("gmath")
     p, u, c, x0 = helpers.example_problem(coord=Lg.coordinate_c)
     prob = callbacks.GelatoProblem(p, u, c, user_eq=callbacks.PerigeeAtEvent(helpers.USER_EVENT), coord=Lg.coordinate_c,
-                                   engine_factory=emu_path_rows.PathRowsEmuEngine, path_grid=path_grid, **kw)
+                                   engine_factory=emu_binding.EmuEngine, path_grid=path_grid, **kw)
     return prob, p, u, c, x0
 
 
@@ -328,7 +328,7 @@ def test_fused_pair_keeps_the_path_rows_jacobian():
 
 def test_refusals():
     p, u, c, x0, O, P = _setup("example")
-    E = emu_path_rows.PathRowsEmuEngine(P)
+    E = emu_binding.EmuEngine(P)
     xv = problem.xdict_to_vector(x0)
     with pytest.raises(engine.GelatoError, match="no path rows set"):
         E.eval_path_rows(xv)
@@ -347,7 +347,7 @@ def test_refusals():
     assert _eq(got[0], ref[0]) and _eq(got[1], ref[1])
     # a bare plan: zero rows, nothing written
     p, u, c, x0, O, P = _setup("bare")
-    E = emu_path_rows.PathRowsEmuEngine(P)
+    E = emu_binding.EmuEngine(P)
     E.set_path_rows(mesh.grid_tables(O.ps))
     lay = E.path_rows_layout()
     assert (lay["n_rows"], lay["n_vals"]) == (0, 0)
@@ -361,7 +361,7 @@ def test_refusals():
 def test_edge_states(variant, case):
     """The edge-state catalogue of test_edge_states: equal bits, or NaN on both sides."""
     p, u, c, x0, O, P = edge._setup(variant)
-    E = emu_path_rows.PathRowsEmuEngine(P)
+    E = emu_binding.EmuEngine(P)
     tabs = mesh.grid_tables(P.ps)
     E.set_path_rows(tabs)
     x = edge.CATALOGUE[case][0](x0, P)
