@@ -213,6 +213,18 @@ class GelatoProblem:
         err = self.engine.mesh_error(self.pack(xdict))
         return {prm["name"]: err[i] for i, prm in enumerate(self.plan.p["params"][: self.plan.S])}
 
+    def mesh_error_intervals(self, xdict):
+        """{event name: err[K][11]}: mesh_error per LGR interval of each section (K = 1 for a section of one interval;
+        a section's row of mesh_error is the max over its intervals).  refine_nodes takes it as it is."""
+        self._default_mesh_grid()
+        err = self.engine.mesh_error_intervals(self.pack(xdict))
+        out, k = {}, 0
+        for i, prm in enumerate(self.plan.p["params"][: self.plan.S]):
+            K = len(self.plan.ps.intervals(i)[0])
+            out[prm["name"]] = err[k:k + K]
+            k += K
+        return out
+
     _AERO_KEYS = ("ineqcon_alpha", "ineqcon_q", "ineqcon_qalpha")
 
     def path_check(self, xdict):

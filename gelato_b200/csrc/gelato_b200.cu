@@ -226,7 +226,11 @@ __global__ void k_fd_central(double* __restrict__ out_all, long long out_stride,
 
 // Mesh error estimate (mesh_error.h; DESIGN.md section 11), two launches.  First one thread per (scenario, test point):
 // the interpolated state and the right-hand side there, MESH_PT doubles per point into pts[n_scen][n_pts][MESH_PT].
-// Then one thread per (scenario, section, state component): the integral and the two maxima, err[n_scen][S][11].
+// Then one thread per (scenario, section, state component) over the section's intervals (ints[int0[sec] ..
+// int0[sec + 1])): per interval the integral and the two maxima into err_int[n_scen][n_int][11], their max into
+// err[n_scen][S][11]; either output may be NULL.  INTERVALS == false (a grid without interval tables): interval sec is
+// the whole section, and the kernel reads no interval list -- the loads before the first integral are those of the
+// estimate without intervals.
 #define GM_THREADS 128
 __global__ void __launch_bounds__(GM_THREADS)
 k_mesh_points(const __grid_constant__ PlanView P, const MeshPt* __restrict__ pt, const MeshSec* __restrict__ ms,
@@ -240,9 +244,12 @@ k_mesh_points(const __grid_constant__ PlanView P, const MeshPt* __restrict__ pt,
   double* out = pts_all + (size_t)i * MESH_PT;
   mesh_point(P, scen, x_all + (size_t)scen * P.n_vars, q.sec, tb, q.l, out, out + MESH_STATE);
 }
+template <bool INTERVALS>
 __global__ void __launch_bounds__(GM_THREADS)
-k_mesh_error(const __grid_constant__ PlanView P, const MeshSec* __restrict__ ms, const double* __restrict__ pool, int n_pts,
-             int n_scen, const double* __restrict__ x_all, const double* __restrict__ pts_all, double* __restrict__ err_all) {
+k_mesh_error(const __grid_constant__ PlanView P, const MeshSec* __restrict__ ms, const MeshInt* __restrict__ ints,
+             const int32_t* __restrict__ int0, const double* __restrict__ pool, int n_pts, int n_int, int n_scen,
+             const double* __restrict__ x_all, const double* __restrict__ pts_all, double* __restrict__ err_all,
+             double* __restrict__ err_int) {
   const long long i = (long long)blockIdx.x * GM_THREADS + threadIdx.x;
   const int per = P.S * MESH_STATE;
   if (i >= (long long)per * n_scen) return;
@@ -251,7 +258,15 @@ k_mesh_error(const __grid_constant__ PlanView P, const MeshSec* __restrict__ ms,
   const MeshSec s = ms[sec];
   const MeshTabs tb = mesh_tabs(pool, s, P.sec_i32[sec * GS_I32_COLS + GS_N]);
   const double* pts = pts_all + ((size_t)scen * n_pts + s.pt0) * MESH_PT;
-  err_all[i] = mesh_component(P, x_all + (size_t)scen * P.n_vars, sec, tb, s.m, pts, c);
+  const double* x = x_all + (size_t)scen * P.n_vars;
+  const int k0 = INTERVALS ? int0[sec] : sec, k1 = INTERVALS ? int0[sec + 1] : sec + 1;
+  double e = 0.0;
+  for (int k = k0; k < k1; k++) {
+    const double ek = mesh_component(P, x, sec, tb, s.m, pts, c, INTERVALS ? ints[k] : MeshInt{0, 0, s.m});
+    if (err_int) err_int[((size_t)scen * n_int + k) * MESH_STATE + c] = ek;
+    e = k == k0 ? ek : mesh_max(e, ek);
+  }
+  if (err_all) err_all[i] = e;
 }
 
 // Path check (mesh_error.h; DESIGN.md section 11), two launches on the same grid.  First one thread per (scenario, test
@@ -445,6 +460,12 @@ struct GelatoPlan {
   DeviceBuf<MeshPt> d_mesh_pt;
   DeviceBuf<double> d_mesh_pts;
   int n_mesh_pts = 0;
+  // its intervals, and each section's first one (d_mesh_int0[S + 1]); n_mesh_int intervals in all; mesh_intervals:
+  // the grid came with interval tables (else interval i is section i)
+  DeviceBuf<MeshInt> d_mesh_int;
+  DeviceBuf<int32_t> d_mesh_int0;
+  int n_mesh_int = 0;
+  bool mesh_intervals = false;
   // path check on the same grid: the test points of the aero jobs over a whole section and each job's first one
   // (plan_host.h: build_path_points, rebuilt with the grid), the per-point scratch d_path_r
   std::vector<int32_t> aero_i32;  // the aero jobs, as the plan description gave them
@@ -1092,7 +1113,10 @@ int gelato_plan_set_mesh_grid(GelatoPlan* p, const GelatoMeshGridDesc* g) {
   if (!p || !g || !g->m || !g->off || !g->pool) return fail(GELATO_ERR_ARG, "null argument");
   std::vector<MeshSec> secs;
   std::vector<MeshPt> pts;
-  if (const char* why = build_mesh_grid(g, p->sec_n.data(), p->view.S, secs, pts)) return fail(GELATO_ERR_ARG, why);
+  std::vector<MeshInt> ints;
+  std::vector<int32_t> int0;
+  if (const char* why = build_mesh_grid(g, p->sec_n.data(), p->view.S, secs, pts, ints, int0))
+    return fail(GELATO_ERR_ARG, why);
   std::vector<PathPt> path_pts;
   std::vector<int32_t> job0;
   if (const char* why = build_path_points(p->aero_i32.data(), p->view.n_aero, secs, path_pts, job0))
@@ -1100,25 +1124,33 @@ int gelato_plan_set_mesh_grid(GelatoPlan* p, const GelatoMeshGridDesc* g) {
   const cudaStream_t st = p->lanes[0].stream;
   int rc;
   if ((rc = upload_grid(p, p->mesh_grid, secs, g)) || (rc = upload_async(p->d_mesh_pt, pts.data(), pts.size(), st)) ||
+      (rc = upload_async(p->d_mesh_int, ints.data(), ints.size(), st)) ||
+      (rc = upload_async(p->d_mesh_int0, int0.data(), int0.size(), st)) ||
       (rc = upload_async(p->d_path_pt, path_pts.data(), path_pts.size(), st)) ||
       (rc = upload_async(p->d_path_job0, job0.data(), job0.size(), st)))
     return rc;
   CU(cudaStreamSynchronize(st));
   p->n_mesh_pts = (int)pts.size();
+  p->n_mesh_int = (int)ints.size();
+  p->mesh_intervals = g->n_int != nullptr;
   p->n_path_pts = (int)path_pts.size();
   return GELATO_OK;
 }
 
-// The two launches of one estimate on `st`; the point scratch grows to the batch (DeviceBuf::reserve synchronises).
-static int launch_mesh_error(GelatoPlan* p, const double* x_dev, double* err_dev, int n_scen, cudaStream_t st) {
+// The two launches of one estimate on `st` into err_dev [n_scen][S][11] and / or err_int_dev [n_scen][n_int][11]; the
+// point scratch grows to the batch (DeviceBuf::reserve synchronises).
+static int launch_mesh_error(GelatoPlan* p, const double* x_dev, double* err_dev, double* err_int_dev, int n_scen,
+                             cudaStream_t st) {
   const long long n1 = (long long)n_scen * p->n_mesh_pts, n2 = (long long)n_scen * p->view.S * MESH_STATE;
   if ((std::max(n1, n2) + GM_THREADS - 1) / GM_THREADS > 0x7fffffffLL)
     return fail(GELATO_ERR_ARG, "test points x n_scen exceeds the grid limit");
   CU(p->d_mesh_pts.reserve((size_t)n1 * MESH_PT));
   k_mesh_points<<<(unsigned)((n1 + GM_THREADS - 1) / GM_THREADS), GM_THREADS, 0, st>>>(
       p->view, p->d_mesh_pt.get(), p->mesh_grid.sec.get(), p->mesh_grid.pool.get(), p->n_mesh_pts, n_scen, x_dev, p->d_mesh_pts.get());
-  k_mesh_error<<<(unsigned)((n2 + GM_THREADS - 1) / GM_THREADS), GM_THREADS, 0, st>>>(
-      p->view, p->mesh_grid.sec.get(), p->mesh_grid.pool.get(), p->n_mesh_pts, n_scen, x_dev, p->d_mesh_pts.get(), err_dev);
+  (p->mesh_intervals ? k_mesh_error<true> : k_mesh_error<false>)<<<(unsigned)((n2 + GM_THREADS - 1) / GM_THREADS),
+                                                                   GM_THREADS, 0, st>>>(
+      p->view, p->mesh_grid.sec.get(), p->d_mesh_int.get(), p->d_mesh_int0.get(), p->mesh_grid.pool.get(), p->n_mesh_pts,
+      p->n_mesh_int, n_scen, x_dev, p->d_mesh_pts.get(), err_dev, err_int_dev);
   p->launches += 2;
   CU(cudaGetLastError());
   return GELATO_OK;
@@ -1130,7 +1162,7 @@ int gelato_eval_mesh_error_dev(GelatoPlan* p, const double* x_dev, double* err_d
   if (rc) return rc;
   if (!p->n_mesh_pts) return fail(GELATO_ERR_ARG, GELATO_NO_MESH_GRID);
   if (!x_dev || !err_dev) return fail(GELATO_ERR_ARG, "null buffer");
-  return launch_mesh_error(p, x_dev, err_dev, n_scen, st);
+  return launch_mesh_error(p, x_dev, err_dev, nullptr, n_scen, st);
 }
 
 int gelato_eval_mesh_error(GelatoPlan* p, const double* x, double* err, int32_t n_scen) {
@@ -1141,7 +1173,29 @@ int gelato_eval_mesh_error(GelatoPlan* p, const double* x, double* err, int32_t 
   const size_t ne = (size_t)n_scen * p->view.S * MESH_STATE;
   return eval_diag(p, x, n_scen, err, ne * sizeof(double), nullptr, 0,
                    [&](const double* xd, void* o0, void*, cudaStream_t st) {
-                     return launch_mesh_error(p, xd, (double*)o0, n_scen, st);
+                     return launch_mesh_error(p, xd, (double*)o0, nullptr, n_scen, st);
+                   });
+}
+
+int gelato_eval_mesh_error_intervals_dev(GelatoPlan* p, const double* x_dev, double* err_int_dev, int32_t n_scen,
+                                         void* stream) {
+  cudaStream_t st;
+  int rc = begin_dev(p, n_scen, stream, &st);
+  if (rc) return rc;
+  if (!p->n_mesh_pts) return fail(GELATO_ERR_ARG, GELATO_NO_MESH_GRID);
+  if (!x_dev || !err_int_dev) return fail(GELATO_ERR_ARG, "null buffer");
+  return launch_mesh_error(p, x_dev, nullptr, err_int_dev, n_scen, st);
+}
+
+int gelato_eval_mesh_error_intervals(GelatoPlan* p, const double* x, double* err_int, int32_t n_scen) {
+  int rc = check_scen(p, n_scen);
+  if (rc) return rc;
+  if (!p->n_mesh_pts) return fail(GELATO_ERR_ARG, GELATO_NO_MESH_GRID);
+  if (!x || !err_int) return fail(GELATO_ERR_ARG, "null buffer");
+  const size_t ne = (size_t)n_scen * p->n_mesh_int * MESH_STATE;
+  return eval_diag(p, x, n_scen, err_int, ne * sizeof(double), nullptr, 0,
+                   [&](const double* xd, void* o0, void*, cudaStream_t st) {
+                     return launch_mesh_error(p, xd, nullptr, (double*)o0, n_scen, st);
                    });
 }
 

@@ -7,7 +7,9 @@
  * test point l the state X_l and controls U_l are interpolated and rh_l, the right-hand-side term of dyn_res_finish,
  * is evaluated there (mesh_point).  Per state component c the estimate is then
  *     err = max_l |X_0 + sum_k I[l][k] rh_k - X_l| / (1 + max_l |X_l|)
- * with X_0 the section's first state row (mesh_component).  Every sum is a fused multiply-add chain with ascending
+ * with X_0 the section's first state row (mesh_component).  A section made of several LGR intervals has one estimate per
+ * interval, over the interval's own test points and block of I, from the state row where the interval starts; the
+ * section's is their max.  Every sum is a fused multiply-add chain with ascending
  * index from 0.0, and max and division are exact, so the result has one value: the kernels, the host emulator
  * (tests/emu/emu.cpp) and the oracle (tests/mesh_oracle.py) agree bit for bit.
  *
@@ -32,6 +34,11 @@
 struct MeshSec {
   int32_t m, pt0;
   int64_t off;
+};
+/* one LGR interval of a section's test grid (h-refinement): the support column it integrates from and its test points
+ * l0 .. l0 + m - 1 */
+struct MeshInt {
+  int32_t base, l0, m;
 };
 /* one test point: its section and its index inside the section */
 struct MeshPt {
@@ -205,20 +212,28 @@ P_HD void mesh_path_min(const double* r, int m, double* res, int32_t* at) {
 /* max as numpy's: a NaN operand makes the result NaN */
 P_HD double mesh_max(double a, double b) { return (b > a || b != b) ? b : a; }
 
-/* The estimate of state component c of section `sec`: pts = the section's M test points as mesh_point left them,
- * MESH_PT doubles each. */
-P_HD double mesh_component(const PlanView& P, const double* x, int sec, const MeshTabs& tb, int M, const double* pts, int c) {
-  const double x0 = mesh_state(P, x, P.sec_i32[sec * GS_I32_COLS + GS_XA], c);
+/* The estimate of state component c over interval `iv` of section `sec` (its test points l0 .. l0 + m - 1, integrated
+ * from state row xa + base): pts = the section's M test points as mesh_point left them, MESH_PT doubles each.  Only the
+ * interval's block of I is read, so a NaN in one interval cannot reach another; one interval {0, 0, M} is the
+ * estimate of the whole section. */
+P_HD double mesh_component(const PlanView& P, const double* x, int sec, const MeshTabs& tb, int M, const double* pts, int c,
+                           const MeshInt& iv) {
+  const double x0 = mesh_state(P, x, P.sec_i32[sec * GS_I32_COLS + GS_XA] + iv.base, c);
   double emax = 0.0, xmax = 0.0;
-  for (int l = 0; l < M; l++) {
+  for (int l = iv.l0; l < iv.l0 + iv.m; l++) {
     const double* Irow = tb.I + (long long)l * M;
     double acc = 0.0;
-    for (int k = 0; k < M; k++) acc = gm_fma(Irow[k], pts[(long long)k * MESH_PT + MESH_STATE + c], acc);
+    for (int k = iv.l0; k < iv.l0 + iv.m; k++) acc = gm_fma(Irow[k], pts[(long long)k * MESH_PT + MESH_STATE + c], acc);
     const double xl = pts[(long long)l * MESH_PT + c];
     emax = mesh_max(emax, gm_fabs((x0 + acc) - xl));
     xmax = mesh_max(xmax, gm_fabs(xl));
   }
   return gm_div(emax, 1.0 + xmax);
+}
+
+/* The estimate of state component c of section `sec` as one interval: its M test points from state row xa */
+P_HD double mesh_component(const PlanView& P, const double* x, int sec, const MeshTabs& tb, int M, const double* pts, int c) {
+  return mesh_component(P, x, sec, tb, M, pts, c, MeshInt{0, 0, M});
 }
 
 #endif /* GELATO_B200_MESH_ERROR_H_ */

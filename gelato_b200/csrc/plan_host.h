@@ -321,12 +321,16 @@ static inline void build_host_tables(const GelatoPlanDesc* d, HostTables& h) {
 #define GELATO_NO_MESH_GRID "no mesh grid set (gelato_plan_set_mesh_grid)"
 
 /* The test grid of the mesh error estimate (include/gelato_b200.h: GelatoMeshGridDesc) over S sections of n[i] LGR
- * nodes: its sections and the list of its test points.  Returns NULL or why the grid is refused.  The kernels trust
- * the grid, so one that fails here is not uploaded. */
+ * nodes: its sections, the list of its test points, its intervals and the first interval of each section (int0[S + 1];
+ * no interval tables: one interval per section from column 0).  Returns NULL or why the grid is refused.  The kernels
+ * trust the grid, so one that fails here is not uploaded. */
 static inline const char* build_mesh_grid(const GelatoMeshGridDesc* g, const int32_t* n, int S, std::vector<MeshSec>& secs,
-                                          std::vector<MeshPt>& pts) {
+                                          std::vector<MeshPt>& pts, std::vector<MeshInt>& ints, std::vector<int32_t>& int0) {
   secs.assign(S, MeshSec());
   pts.clear();
+  ints.clear();
+  int0.assign(1, 0);
+  if (g->n_int && (!g->int_m || !g->int_base)) return "interval counts without the interval tables";
   for (int i = 0; i < S; i++) {
     const long long m = g->m[i], ni = n[i], off = g->off[i];
     if (m < 1) return "every section needs at least one test point";
@@ -337,10 +341,36 @@ static inline const char* build_mesh_grid(const GelatoMeshGridDesc* g, const int
     secs[i].pt0 = (int32_t)pts.size();
     secs[i].off = off;
     for (int l = 0; l < m; l++) pts.push_back(MeshPt{i, l});
+    if (!g->n_int) {
+      ints.push_back(MeshInt{0, 0, (int32_t)m});
+    } else {
+      const long long K = g->n_int[i];
+      if (K < 1) return "every section needs at least one interval";
+      if (K > m) return "an interval without test points";
+      long long l0 = 0;
+      for (long long k = 0; k < K; k++) {
+        const long long j = int0.back() + k, mk = g->int_m[j], base = g->int_base[j];
+        if (mk < 1 || mk > m - l0) return "the intervals' test points do not add up to the section's";
+        if (base < 0 || base > ni || (k == 0 && base != 0) || (k > 0 && base <= ints.back().base))
+          return "an interval's base column is out of range, not increasing or not 0 for the first interval";
+        ints.push_back(MeshInt{(int32_t)base, (int32_t)l0, (int32_t)mk});
+        l0 += mk;
+      }
+      if (l0 != m) return "the intervals' test points do not add up to the section's";
+    }
+    int0.push_back((int32_t)ints.size());
   }
   for (int64_t k = 0; k < g->pool_len; k++)
     if (!std::isfinite(g->pool[k])) return "the table pool holds a value that is not finite";
   return nullptr;
+}
+
+/* build_mesh_grid without the interval lists (the same checks): for users of a grid's sections and test points only */
+static inline const char* build_mesh_grid(const GelatoMeshGridDesc* g, const int32_t* n, int S, std::vector<MeshSec>& secs,
+                                          std::vector<MeshPt>& pts) {
+  std::vector<MeshInt> ints;
+  std::vector<int32_t> int0;
+  return build_mesh_grid(g, n, S, secs, pts, ints, int0);
 }
 
 /* The test points of the path check on the grid `secs` (build_mesh_grid): every test point of the section of every aero

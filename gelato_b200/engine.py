@@ -69,7 +69,8 @@ class ScenarioDesc(ctypes.Structure):
 class MeshGridDesc(ctypes.Structure):
     """GelatoMeshGridDesc (include/gelato_b200.h)."""
 
-    _fields_ = [("m", _pi32), ("off", _pi64), ("pool", _pd), ("pool_len", ctypes.c_int64)]
+    _fields_ = [("m", _pi32), ("off", _pi64), ("pool", _pd), ("pool_len", ctypes.c_int64), ("n_int", _pi32),
+                ("int_m", _pi32), ("int_base", _pi32)]
 
 
 def _ptr(arr, typ):
@@ -174,13 +175,24 @@ def make_scenario_desc(plans):
 
 
 def make_mesh_grid_desc(tables):
-    """{"m", "off", "pool"} (gelato_b200/mesh.py: grid_tables) -> (MeshGridDesc, keepalive list)."""
+    """{"m", "off", "pool"} and optionally {"n_int", "int_m", "int_base"} (gelato_b200/mesh.py: grid_tables) ->
+    (MeshGridDesc, keepalive list)."""
     m = np.ascontiguousarray(tables["m"], dtype=np.int32)
     off = np.ascontiguousarray(tables["off"], dtype=np.int64)
     pool = np.ascontiguousarray(tables["pool"], dtype=np.float64)
     d = MeshGridDesc()
     d.m, d.off, d.pool, d.pool_len = _ptr(m, _pi32), _ptr(off, _pi64), _ptr(pool, _pd), pool.size
-    return d, [m, off, pool]
+    keep = [m, off, pool]
+    if "n_int" in tables:
+        iv = [np.ascontiguousarray(tables[k], dtype=np.int32) for k in ("n_int", "int_m", "int_base")]
+        d.n_int, d.int_m, d.int_base = (_ptr(a, _pi32) for a in iv)
+        keep += iv
+    return d, keep
+
+
+def grid_intervals(tables):
+    """The number of intervals of a mesh grid: sum(n_int), or one per section without interval tables."""
+    return int(np.sum(tables["n_int"])) if "n_int" in tables else len(tables["m"])
 
 
 def build_library(force=False, verbose=False, out=None, extra=()):
@@ -233,6 +245,8 @@ def load_library():
     L.gelato_plan_set_mesh_grid.argtypes = [vp, ctypes.POINTER(MeshGridDesc)]
     L.gelato_eval_mesh_error.argtypes = [vp, _pd, _pd, ctypes.c_int32]
     L.gelato_eval_mesh_error_dev.argtypes = [vp, vp, vp, ctypes.c_int32, vp]
+    L.gelato_eval_mesh_error_intervals.argtypes = [vp, _pd, _pd, ctypes.c_int32]
+    L.gelato_eval_mesh_error_intervals_dev.argtypes = [vp, vp, vp, ctypes.c_int32, vp]
     L.gelato_eval_path_check.argtypes = [vp, _pd, _pd, _pi32, ctypes.c_int32]
     L.gelato_eval_path_check_dev.argtypes = [vp, vp, vp, vp, ctypes.c_int32, vp]
     L.gelato_plan_set_path_rows.argtypes = [vp, ctypes.POINTER(MeshGridDesc)]
@@ -304,6 +318,7 @@ EXPORTS = (
     "gelato_leaf_atmosphere gelato_leaf_output_table gelato_init_rocket_simulation gelato_leaf_coordinate "
     "gelato_eval_pair_packed_range_dev gelato_plan_set_fd gelato_plan_get_fd "
     "gelato_plan_set_mesh_grid gelato_eval_mesh_error gelato_eval_mesh_error_dev "
+    "gelato_eval_mesh_error_intervals gelato_eval_mesh_error_intervals_dev "
     "gelato_eval_path_check gelato_eval_path_check_dev "
     "gelato_plan_set_path_rows gelato_plan_path_rows gelato_eval_path_rows gelato_eval_path_rows_dev"
 ).split()
@@ -355,6 +370,7 @@ class Engine:
         self.n_vals = L.gelato_plan_n_vals(h)
         assert self.n_vars == plan.n_vars and self.n_rows == plan.n_rows and self.n_vals == plan.n_vals
         self._prow = None  # the path-row layout (path_rows_layout), read once per grid
+        self.n_mesh_int = 0  # intervals of the mesh grid once set (mesh_error_intervals)
         ok = ctypes.c_int(0)
         _check(L, L.gelato_selftest_unfused(device, ctypes.byref(ok)), "gelato_selftest_unfused")
         if not ok.value:
@@ -393,6 +409,7 @@ class Engine:
         """The test grid of the mesh error estimate: {"m", "off", "pool"} as gelato_b200.mesh.grid_tables builds it."""
         desc, _keep = make_mesh_grid_desc(tables)
         _check(self.L, self.L.gelato_plan_set_mesh_grid(self.h, ctypes.byref(desc)), "gelato_plan_set_mesh_grid")
+        self.n_mesh_int = grid_intervals(tables)
 
     def mesh_error(self, x, n_scen=1, out=None):
         """err[S][11] (n_scen > 1: [n_scen][S][11]) of the decision vectors x[n_scen][n_vars]: per section and state
@@ -406,6 +423,21 @@ class Engine:
 
     def mesh_error_dev(self, x_ptr, err_ptr, n_scen=1, stream=None):
         _check(self.L, self.L.gelato_eval_mesh_error_dev(self.h, x_ptr, err_ptr, n_scen, stream), "gelato_eval_mesh_error_dev")
+
+    def mesh_error_intervals(self, x, n_scen=1, out=None):
+        """err_int[n_int][11] (n_scen > 1: [n_scen][n_int][11]): the estimate of every LGR interval of the mesh grid, the
+        intervals of section 0 first (one per section on a grid without interval tables)."""
+        x = self._x(x, n_scen)
+        self.calls += 1
+        n = n_scen * self.n_mesh_int * 11
+        err = _out(out, n, "out") if out is not None else np.empty(n)
+        _check(self.L, self.L.gelato_eval_mesh_error_intervals(self.h, _ptr(x, _pd), _ptr(err, _pd), n_scen),
+               "gelato_eval_mesh_error_intervals")
+        return err.reshape(self.n_mesh_int, 11) if n_scen == 1 else err.reshape(n_scen, self.n_mesh_int, 11)
+
+    def mesh_error_intervals_dev(self, x_ptr, err_ptr, n_scen=1, stream=None):
+        _check(self.L, self.L.gelato_eval_mesh_error_intervals_dev(self.h, x_ptr, err_ptr, n_scen, stream),
+               "gelato_eval_mesh_error_intervals_dev")
 
     def path_check(self, x, n_scen=1, out=None):
         """(res, at) of the decision vectors x[n_scen][n_vars], [n_aero] each (n_scen > 1: [n_scen][n_aero]), in the

@@ -20,7 +20,7 @@ import os
 import numpy as np
 
 from . import hostmath
-from .psparams import PSparams
+from .psparams import PSparams, check_intervals
 
 G0 = 9.80665
 
@@ -68,6 +68,11 @@ def read_events(path):
             "yawrate_init": float(d["yawrate_init"]),
             "num_nodes": int(d["num_nodes"]),
         }
+        # optional: the LGR intervals of a composite section, ';'-separated (DESIGN.md section 11)
+        if d.get("mesh_intervals", "") != "":
+            ev["mesh_intervals"] = [int(v) for v in d["mesh_intervals"].split(";")]
+        if d.get("mesh_breaks", "") != "":
+            ev["mesh_breaks"] = [float(v) for v in d["mesh_breaks"].split(";")]
         events.append(ev)
     return events
 
@@ -81,6 +86,19 @@ def read_trajectory(path):
         except ValueError:
             cols[h] = [r[j] for r in body]
     return cols
+
+
+def event_intervals(e):
+    """None or (counts, breaks) of an event record's optional `mesh_intervals` / `mesh_breaks` (PSparams), validated
+    against its `num_nodes`; ValueError names the event."""
+    if "mesh_intervals" not in e:
+        if "mesh_breaks" in e:
+            raise ValueError("event %s: mesh_breaks without mesh_intervals" % e["name"])
+        return None
+    try:
+        return check_intervals(int(e["num_nodes"]), e["mesh_intervals"], e.get("mesh_breaks"))
+    except (TypeError, ValueError) as exc:
+        raise ValueError("event %s: %s" % (e["name"], exc)) from None
 
 
 def build_problem(settings, events, wind_table, ca_table, coord=None):
@@ -121,7 +139,7 @@ def build_problem(settings, events, wind_table, ca_table, coord=None):
     pdict["event_index"] = {e["name"]: i for i, e in enumerate(events)}
     nodes = [e["num_nodes"] for e in events[:-1]]
     N = int(sum(nodes))
-    pdict["ps_params"] = PSparams(nodes)
+    pdict["ps_params"] = PSparams(nodes, [event_intervals(e) for e in events[:-1]])
     pdict["wind_table"] = np.ascontiguousarray(wind_table, dtype=np.float64)
     pdict["ca_table"] = np.ascontiguousarray(ca_table, dtype=np.float64)
     pdict["N"] = N

@@ -62,16 +62,80 @@ def mesh_tables(n):
     return _MESH[n]
 
 
+def lgr_points(n):
+    """lgr_nodes(n), with n = 1 allowed: the one flipped LGR point is +1."""
+    return lgr_nodes(n) if n > 1 else np.ones(1)
+
+
+def interval_points(pts, a, b):
+    """Points in [-1, 1] (the last one +1) mapped affinely onto [a, b], the last one exactly b."""
+    out = a + (np.asarray(pts, dtype=np.float64) + 1.0) * ((b - a) / 2.0)
+    out[-1] = b
+    return out
+
+
+def check_intervals(n, counts, breaks=None):
+    """(counts, breaks) of a section of n nodes made of K = len(counts) LGR intervals, validated: every count >= 1 and
+    their sum n, breaks the K - 1 interior breakpoints, strictly increasing inside (-1, 1) (None: equal widths).
+    ValueError otherwise."""
+    counts = [int(c) for c in counts]
+    K = len(counts)
+    if K < 1 or min(counts) < 1 or sum(counts) != n:
+        raise ValueError("interval node counts must be >= 1 and add up to the section's %d nodes, got %r" % (n, counts))
+    if breaks is None:
+        breaks = [-1.0 + 2.0 * k / K for k in range(1, K)]
+    breaks = np.array(breaks, dtype=np.float64).reshape(-1)
+    b = np.hstack((-1.0, breaks, 1.0))
+    if breaks.size != K - 1 or not np.all(np.isfinite(breaks)) or not np.all(b[1:] > b[:-1]):
+        raise ValueError("%d intervals need %d interior breakpoints, strictly increasing inside (-1, 1), got %r"
+                         % (K, K - 1, breaks.tolist()))
+    return counts, breaks
+
+
+def composite_tables(counts, breaks):
+    """(tau[n], D[n, n+1]) of a section made of LGR intervals (check_intervals): interval k over [b_k, b_k+1] has its
+    n_k flipped LGR points mapped into it (its last one exactly b_k+1), and its rows of D are lgr_diff_matrix(n_k) * 2 /
+    w_k in its support columns c_k .. c_k + n_k (c_k = n_0 + .. + n_k-1), every other entry exactly 0."""
+    n = sum(counts)
+    b = np.hstack((-1.0, breaks, 1.0))
+    tau, D = np.empty(n), np.zeros((n, n + 1))
+    c = 0
+    for k, nk in enumerate(counts):
+        pts = lgr_points(nk)
+        tau[c:c + nk] = interval_points(pts, b[k], b[k + 1])
+        D[c:c + nk, c:c + nk + 1] = lgr_diff_matrix(nk, pts) * (2.0 / (b[k + 1] - b[k]))
+        c += nk
+    return tau, D
+
+
 class PSparams:
     """Per-section node counts, LGR points, differentiation matrices and the
-    index arithmetic of the decision vector (reference: SectionParameters.py)."""
+    index arithmetic of the decision vector (reference: SectionParameters.py).
 
-    def __init__(self, num_nodes):
+    intervals[i] (optional): None, one LGR interval as the reference has it, or (counts, breaks) of a composite section
+    of several LGR intervals (check_intervals, composite_tables; DESIGN.md section 11).  Every user of tau and D reads a
+    composite section as it reads any other: only values change, never the layout."""
+
+    def __init__(self, num_nodes, intervals=None):
         self._num_nodes = [int(n) for n in num_nodes]
         self._num_sections = len(self._num_nodes)
-        self._tau, self._D = [], []
-        for n in self._num_nodes:
-            tau, D = mesh_tables(n)
+        if intervals is None:
+            intervals = [None] * self._num_sections
+        if len(intervals) != self._num_sections:
+            raise ValueError("one interval entry per section is needed")
+        self._tau, self._D, self._int = [], [], []
+        for n, iv in zip(self._num_nodes, intervals):
+            if iv is not None:
+                counts, breaks = check_intervals(n, *iv)
+                iv = None if len(counts) == 1 else (counts, breaks)
+            if iv is None:
+                tau, D = mesh_tables(n)
+                self._int.append(([n], np.empty(0), [0]))
+            else:
+                tau, D = composite_tables(*iv)
+                tau.setflags(write=False)
+                D.setflags(write=False)
+                self._int.append((iv[0], iv[1], [int(v) for v in np.concatenate(([0], np.cumsum(iv[0])[:-1]))]))
             self._tau.append(tau)
             self._D.append(D)
         self._index_start_u = [int(v) for v in np.concatenate(([0], np.cumsum(self._num_nodes)[:-1]))]
@@ -92,6 +156,12 @@ class PSparams:
     def nodes(self, i):
         self._check(i)
         return self._num_nodes[i]
+
+    def intervals(self, i):
+        """(counts, breaks, support columns) of section i: the node count of each LGR interval, the interior
+        breakpoints in section tau and the first support column c_k of each; ([n], [], [0]) for one interval."""
+        self._check(i)
+        return self._int[i]
 
     def index_start_u(self, i):
         return self._index_start_u[i]

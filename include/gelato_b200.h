@@ -304,16 +304,32 @@ int gelato_eval_pair_packed_ids(GelatoPlan* plan, const double* x, double* g, do
  * directly, others staged).  _dev: device pointers, enqueued on `stream` (NULL = the plan's own), not synchronised.
  * Both use the scenario blocks of gelato_plan_set_scenarios, refuse an n_scen beyond them as every entry point does, and
  * refuse calls before a grid is set.  Two launches per call (DESIGN.md section 11 gives the measured cost); the _dev call
- * uses plan-owned scratch (n_scen x sum(M) x 22 doubles): calls on one plan must not overlap on different streams. */
+ * uses plan-owned scratch (n_scen x sum(M) x 22 doubles): calls on one plan must not overlap on different streams.
+ * Intervals (a section made of several LGR intervals, h-refinement; optional, trailing): n_int[i] (>= 1) intervals of
+ * section i; per interval, in section order, int_m its test points (they partition the section's M, in order) and
+ * int_base the support column (0..n) it integrates from: strictly increasing in a section, 0 for its first interval.
+ * Interval k of a section has the estimate of the formula above over its own test points l, with X_0 the state row
+ * xa + int_base[k] and the sum over its own k only (its block of I; P and Q rows may be interval-local bases).  The
+ * section's err is the max over its intervals.  n_int == NULL: one interval per section from column 0, the estimate
+ * above.  n_int < 1, interval test points that do not add up to m, or a base out of range, not increasing or not 0 for
+ * a section's first interval returns GELATO_ERR_ARG and leaves the plan unchanged.
+ * gelato_eval_mesh_error_intervals: err_int [n_scen][sum n_int][11], each interval's estimate, with the buffers,
+ * scenario blocks, scratch and refusals of gelato_eval_mesh_error; _dev as gelato_eval_mesh_error_dev. */
 typedef struct GelatoMeshGridDesc {
   const int32_t* m;   /* [S] test points of each section */
   const int64_t* off; /* [S] offset (doubles) of each section's tables in pool */
   const double* pool;
   int64_t pool_len;
+  const int32_t* n_int;    /* [S] intervals of each section, or NULL: one each */
+  const int32_t* int_m;    /* [sum n_int] test points of each interval */
+  const int32_t* int_base; /* [sum n_int] support column each interval integrates from */
 } GelatoMeshGridDesc;
 int gelato_plan_set_mesh_grid(GelatoPlan* plan, const GelatoMeshGridDesc* grid);
 int gelato_eval_mesh_error(GelatoPlan* plan, const double* x, double* err, int32_t n_scen);
 int gelato_eval_mesh_error_dev(GelatoPlan* plan, const double* x_dev, double* err_dev, int32_t n_scen, void* stream);
+int gelato_eval_mesh_error_intervals(GelatoPlan* plan, const double* x, double* err_int, int32_t n_scen);
+int gelato_eval_mesh_error_intervals_dev(GelatoPlan* plan, const double* x_dev, double* err_int_dev, int32_t n_scen,
+                                         void* stream);
 
 /* Path check (DESIGN.md section 11): do the aero constraints (ineqcon_alpha, ineqcon_q, ineqcon_qalpha) hold BETWEEN the
  * nodes?  The NLP enforces them at the state nodes only.  On the grid of gelato_plan_set_mesh_grid, for scenario s and
