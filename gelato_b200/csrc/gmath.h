@@ -9,8 +9,8 @@
  * CPU oracle both call THESE functions.  They are built only from IEEE-754
  * correctly rounded primitives (+ - * / sqrt fma) and integer bit operations,
  * therefore g++ (-ffp-contract=off) and nvcc (-fmad=false) produce identical
- * bits.  Accuracy is <= ~1 ulp for sin/cos/exp/pow/atan and <= ~3 ulp for
- * atan2/asin/acos/tan (measured against mpmath in tests/test_gmath.py).
+ * bits.  Accuracy is <= 2 ulp for every function over the whole double range
+ * (measured against mpmath in tests/test_gmath_device.py; maxima in DESIGN.md H1).
  *
  * The polynomial tables in gmath_coeffs.inc are generated from first
  * principles by tools/gen_gmath_coeffs.py (mpmath Chebyshev fits).
@@ -35,11 +35,15 @@
  * (ncu r02a: moves were 27 % of the instructions the Jacobian kernel executed, as many as its FP64 arithmetic). */
 #if defined(__CUDACC__)
 static __constant__ double gm_tab[GM_TAB_N] = GM_TAB_INIT;
+static __constant__ uint64_t gm_2opi_dev[GM_2OPI_N] = GM_2OPI_INIT;
 #endif
+static const uint64_t gm_2opi_host[GM_2OPI_N] = GM_2OPI_INIT;
 #if defined(__CUDA_ARCH__)
 #define GMC(name) gm_tab[GMT_##name]
+#define GM_2OPI(j) gm_2opi_dev[j]
 #else
 #define GMC(name) GM_##name
+#define GM_2OPI(j) gm_2opi_host[j]
 #endif
 
 #if defined(__CUDACC__)
@@ -150,6 +154,22 @@ GM_HD double gm_div_by(double a, const GmRcp R) {
 #define GM_ABS_MASK 0x7fffffffffffffffull
 #define GM_INF_BITS 0x7ff0000000000000ull
 
+/* high word of the 128-bit product; leading zeros of a non-zero word */
+GM_HD uint64_t gm_umulhi(uint64_t a, uint64_t b) {
+#if defined(__CUDA_ARCH__)
+  return __umul64hi(a, b);
+#else
+  return (uint64_t)(((unsigned __int128)a * b) >> 64);
+#endif
+}
+GM_HD int gm_clz64(uint64_t a) {
+#if defined(__CUDA_ARCH__)
+  return __clzll((long long)a);
+#else
+  return __builtin_clzll(a);
+#endif
+}
+
 GM_HD double gm_fabs(double x) { return gm_u2d(gm_d2u(x) & GM_ABS_MASK); }
 GM_HD double gm_copysign(double mag, double sgn) {
   return gm_u2d((gm_d2u(mag) & GM_ABS_MASK) | (gm_d2u(sgn) & GM_SIGN_MASK));
@@ -167,10 +187,100 @@ GM_HD double gm_rint(double x) {
 
 /* ---- sin / cos / tan -------------------------------------------------- */
 
-/* x - k*pi/2 as a double-double (r, rl); returns k mod 4.  Three 53-bit pieces
- * of pi/2 (159 bits): accurate for |x| up to ~1e6, which is far beyond the
- * O(1) arguments on this path (Earth-rotation angle, latitude, longitude). */
-GM_HD int gm_rem_pio2(double x, double* r, double* rl) {
+/* |x| from which gm_rem_pio2 takes the Payne-Hanek reduction: 2^50.  Below it k = rint(x 2/pi) < 2^50 and the
+ * three pieces of pi/2 are accurate enough: measured against mpmath on [2^49, 2^50), the doubles nearest k pi/2
+ * included, sin 0.76, cos 0.72, tan 1.96 ulp.  Above it they are not (the same measurement on [2^50, 2^51): sin 16.7,
+ * tan 18.2 ulp), and from 2^51 pi/2 on the rint trick no longer rounds k to an integer. */
+#define GM_REM_PIO2_LARGE 0x4310000000000000ull
+
+/* x - k*pi/2 for |x| >= GM_REM_PIO2_LARGE (Payne-Hanek; correct for every finite x).  With x = m 2^E (m the 53-bit
+ * significand) the bits of 2/pi before b(E-1) contribute multiples of 4 to x 2/pi, so only the 192 bits from b(E-1)
+ * on are needed: m times that window, modulo 2^192, is x 2/pi modulo 4 as a fixed-point number with 190 fractional
+ * bits.  The bits of 2/pi after the window add less than 2^-137 to it; the fraction of a double is never smaller
+ * than 2^-62 (the worst case, 6381956970095103 2^797), so hi + lo -- the 53 + 53 bits taken from it -- is the
+ * fraction to a relative 2^-75, far below an ulp of the result.
+ * Integer arithmetic only up to the final product with pi/2, so host and device agree.  Returned by value, so that no
+ * local of the caller has to live in memory. */
+typedef struct GmRem {
+  double r, rl; /* x - k pi/2 as a double-double */
+  int q;        /* k mod 4 */
+} GmRem;
+GM_HD GmRem gm_rem_pio2_large(double x) {
+  const uint64_t ux = gm_d2u(x);
+  const uint64_t m = (ux & 0x000fffffffffffffull) | 0x0010000000000000ull;
+  const int g = (int)((ux >> 52) & 0x7ffu) - 1075 - 2 + 64; /* bit b(E-1) in the table, whose word 0 is zeros */
+  const int j = g >> 6, sh = g & 63;
+  uint64_t w0 = GM_2OPI(j), w1 = GM_2OPI(j + 1), w2 = GM_2OPI(j + 2);
+  if (sh) {
+    w0 = (w0 << sh) | (w1 >> (64 - sh));
+    w1 = (w1 << sh) | (w2 >> (64 - sh));
+    w2 = (w2 << sh) | (GM_2OPI(j + 3) >> (64 - sh));
+  }
+  /* (a0, a1, a2) = m (w0, w1, w2) mod 2^192 */
+  const uint64_t a2 = m * w2;
+  const uint64_t p1 = m * w1, c2 = gm_umulhi(m, w2);
+  uint64_t a1 = p1 + c2;
+  uint64_t a0 = m * w0 + gm_umulhi(m, w1) + (uint64_t)(a1 < p1);
+  int q = (int)(a0 >> 62);
+  a0 &= 0x3fffffffffffffffull;
+  uint64_t b2 = a2, b1 = a1;
+  int neg = 0;
+  if (a0 >> 61) { /* fraction >= 1/2: x 2/pi = (q + 1) - (1 - fraction) */
+    q += 1;
+    neg = 1;
+    b2 = ~a2 + 1;
+    b1 = ~a1 + (uint64_t)(b2 == 0);
+    a0 = (~a0 + (uint64_t)(b2 == 0 && b1 == 0)) & 0x3fffffffffffffffull;
+  }
+  /* normalise (a0, b1, b2) so that bit 191 is set; s = the shift */
+  int s = 0;
+  if (a0 == 0) {
+    a0 = b1;
+    b1 = b2;
+    b2 = 0;
+    s += 64;
+    if (a0 == 0) {
+      a0 = b1;
+      b1 = 0;
+      s += 64;
+    }
+  }
+  double hi = 0.0, lo = 0.0;
+  if (a0 != 0) {
+    const int z = gm_clz64(a0);
+    if (z) {
+      a0 = (a0 << z) | (b1 >> (64 - z));
+      b1 = (b1 << z) | (b2 >> (64 - z));
+    }
+    s += z;
+    /* fraction = hi + lo: the top 53 bits and the next 53, both exact doubles; s <= 190 keeps the scales normal */
+    hi = (double)(a0 >> 11) * gm_u2d((uint64_t)(1023 - 51 - s) << 52);
+    lo = (double)(((a0 & 0x7ffu) << 42) | (b1 >> 22)) * gm_u2d((uint64_t)(1023 - 104 - s) << 52);
+  }
+  /* (hi + lo) pi/2 in double-double */
+  const double ph = hi * GMC(PIO2_1);
+  const double tail = gm_fma(hi, GMC(PIO2_1), -ph) + gm_fma(hi, GMC(PIO2_2), lo * GMC(PIO2_1));
+  double r0 = ph + tail;
+  double r1 = (ph - r0) + tail;
+  if (neg) {
+    r0 = -r0;
+    r1 = -r1;
+  }
+  if (ux & GM_SIGN_MASK) {
+    r0 = -r0;
+    r1 = -r1;
+    q = -q;
+  }
+  GmRem R;
+  R.r = r0;
+  R.rl = r1;
+  R.q = q & 3;
+  return R;
+}
+
+/* x - k*pi/2 as a double-double (r, rl) for |x| < GM_REM_PIO2_LARGE: k = rint(x 2/pi) and three 53-bit pieces of
+ * pi/2 (159 bits); returns k mod 4. */
+GM_HD int gm_rem_pio2_small(double x, double* r, double* rl) {
   double kd = gm_rint(x * GMC(2_OVER_PI));
   double t = gm_fma(-kd, GMC(PIO2_1), x); /* exact (cancellation) */
   double ph = kd * GMC(PIO2_2);
@@ -183,7 +293,18 @@ GM_HD int gm_rem_pio2(double x, double* r, double* rl) {
   double r0 = rh + lo;
   *rl = (rh - r0) + lo;
   *r = r0;
-  return (int)((int64_t)kd & 3);
+  return (int)((int64_t)kd & 3); /* |kd| < 2^50: the conversion is in range */
+}
+
+/* x - k*pi/2 as a double-double (r, rl) for every finite x; returns k mod 4 */
+GM_HD int gm_rem_pio2(double x, double* r, double* rl) {
+  if ((gm_d2u(x) & GM_ABS_MASK) >= GM_REM_PIO2_LARGE) {
+    const GmRem R = gm_rem_pio2_large(x);
+    *r = R.r;
+    *rl = R.rl;
+    return R.q;
+  }
+  return gm_rem_pio2_small(x, r, rl);
 }
 
 /* sin(x + y), |x| <~ pi/4, y a tail */
@@ -214,17 +335,8 @@ GM_HD double gm_kcos(double x, double y) {
   return w + (((1.0 - w) - hz) + (z * (z * p) - x * y));
 }
 
-GM_HD_INL void gm_sincos_inl(double x, double* s, double* c) {
-  uint64_t ax = gm_d2u(x) & GM_ABS_MASK;
-  if (ax >= GM_INF_BITS) { /* inf or nan */
-    *s = gm_nan();
-    *c = gm_nan();
-    return;
-  }
-  double r = x, rl = 0.0;
-  int q = 0;
-  if (ax > 0x3fe921fb54442d18ull) /* |x| > pi/4 */
-    q = gm_rem_pio2(x, &r, &rl);
+/* sin and cos of x = k pi/2 + r + rl from the reduced argument and q = k mod 4 */
+GM_HD void gm_sincos_reduced(double r, double rl, int q, double* s, double* c) {
   double ks = gm_ksin(r, rl);
   double kc = gm_kcos(r, rl);
   /* quadrant: q = 0 (s, c) | 1 (c, -s) | 2 (-s, -c) | 3 (-c, s); selects instead of a four-way branch */
@@ -232,6 +344,61 @@ GM_HD_INL void gm_sincos_inl(double x, double* s, double* c) {
   double cc = (q & 1) ? ks : kc;
   *s = (q & 2) ? -ss : ss;
   *c = ((q + 1) & 2) ? -cc : cc;
+}
+
+/* sin and cos for |x| >= GM_REM_PIO2_LARGE.  Inline, not a call: in the hot path (rotq_part) a call made the NLP
+ * kernels spill more (-Xptxas -v: k_residuals 604 -> 636 bytes of spill loads) and the bench step slower than the
+ * inlined form.  Inlined, the branch still costs +0.45 % of the bench step and changes the spills (stores / loads,
+ * bytes): k_jacobian 308 / 552 -> 276 / 496 and k_residuals 508 / 604 -> 500 / 588 (fewer), the measurement-only
+ * k_jacobian_heavy 36 / 56 -> 40 / 60 and k_jacobian_light 304 / 544 -> 320 / 576 (more).
+ * profiles/r10_ptxas.txt, profiles/r10_bench.txt. */
+typedef struct GmSinCos {
+  double s, c;
+} GmSinCos;
+GM_HD GmSinCos gm_sincos_large(double x) {
+  const GmRem R = gm_rem_pio2_large(x);
+  GmSinCos v;
+  gm_sincos_reduced(R.r, R.rl, R.q, &v.s, &v.c);
+  return v;
+}
+
+/* gm_sincos_inl without the large-argument branch, for the hot-path callers whose argument is an atan2 result or
+ * half of one (|x| <= pi): one copy of the large path fewer in each, which the bench step measured
+ * (profiles/r10_bench.txt).  For |x| < GM_REM_PIO2_LARGE the same bits as gm_sincos_inl; from there on (and for inf
+ * and NaN) NaN -- the one test that caught inf / NaN before, with a lower bound, so that gm_rem_pio2_small never sees
+ * an argument whose k it cannot convert. */
+GM_HD_INL void gm_sincos_small_inl(double x, double* s, double* c) {
+  uint64_t ax = gm_d2u(x) & GM_ABS_MASK;
+  if (ax >= GM_REM_PIO2_LARGE) { /* outside the domain, inf or nan */
+    *s = gm_nan();
+    *c = gm_nan();
+    return;
+  }
+  double r = x, rl = 0.0;
+  int q = 0;
+  if (ax > 0x3fe921fb54442d18ull) /* |x| > pi/4 */
+    q = gm_rem_pio2_small(x, &r, &rl);
+  gm_sincos_reduced(r, rl, q, s, c);
+}
+
+GM_HD_INL void gm_sincos_inl(double x, double* s, double* c) {
+  uint64_t ax = gm_d2u(x) & GM_ABS_MASK;
+  if (ax >= GM_INF_BITS) { /* inf or nan */
+    *s = gm_nan();
+    *c = gm_nan();
+    return;
+  }
+  if (ax >= GM_REM_PIO2_LARGE) {
+    const GmSinCos v = gm_sincos_large(x);
+    *s = v.s;
+    *c = v.c;
+    return;
+  }
+  double r = x, rl = 0.0;
+  int q = 0;
+  if (ax > 0x3fe921fb54442d18ull) /* |x| > pi/4 */
+    q = gm_rem_pio2_small(x, &r, &rl);
+  gm_sincos_reduced(r, rl, q, s, c);
 }
 GM_HD_CALL void gm_sincos(double x, double* s, double* c) { gm_sincos_inl(x, s, c); }
 
@@ -450,7 +617,7 @@ GM_HD_INL double gm_exp_dd_inl(double x, double xl) {
   double p = (rr * rr) * q;
   double s = rr + (p + gm_fma(rl, rr, rl));
   double y = 1.0 + s;
-  return gm_scale2(y, (int)kd);
+  return gm_scale2(y, (int)kd); /* the guards above keep |kd| <= 1076: the conversion is in range */
 }
 
 GM_HD_CALL double gm_exp_dd(double x, double xl) { return gm_exp_dd_inl(x, xl); }
@@ -561,6 +728,11 @@ GM_HD_CALL double gm_pow_slow(double x, double y) {
       int odd = gm_is_odd_int(y);
       if (y > 0.0) return odd ? -0.0 : 0.0;
       return odd ? -gm_inf() : gm_inf();
+    }
+    if (ax == GM_INF_BITS) { /* C99 F.9.4.4: -inf to a power that is not an odd integer is +inf or +0, not NaN */
+      const int odd = gm_is_odd_int(y);
+      if (y > 0.0) return odd ? -gm_inf() : gm_inf();
+      return odd ? -0.0 : 0.0;
     }
     if (!gm_is_int(y)) return gm_nan();
     if (gm_is_odd_int(y)) sgn = -1.0;

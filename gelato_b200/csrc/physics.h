@@ -101,14 +101,15 @@ struct Geodetic {
   double lat, lon, alt; /* radians, radians, metres */
 };
 /* WANT: bit0 altitude, bit1 longitude (latitude is always produced).  HOT: the elementary functions inlined
- * (gmath.h: gm_xxx_inl) -- for the two callers that are the Jacobian kernel's long items. */
+ * (gmath.h: gm_xxx_inl) -- for the two callers that are the Jacobian kernel's long items.  The sines and cosines here
+ * are of atan2 results (|x| <= pi): gm_sincos_small_inl. */
 template <int WANT, bool HOT = false>
 P_HD Geodetic ecef2geodetic(Vec3 r) {
   Geodetic g;
   double p = gm_sqrt(r.x * r.x + r.y * r.y);
   double theta = HOT ? gm_atan2_inl(r.z * P_RA, p * P_RB) : gm_atan2(r.z * P_RA, p * P_RB);
   double st, ct;
-  if (HOT) gm_sincos_inl(theta, &st, &ct);
+  if (HOT) gm_sincos_small_inl(theta, &st, &ct);
   else gm_sincos(theta, &st, &ct);
   const double ny = r.z + P_EP2 * P_RB * (st * st * st), nx = p - P_E2 * P_RA * (ct * ct * ct);
   g.lat = HOT ? gm_atan2_inl(ny, nx) : gm_atan2(ny, nx);
@@ -117,7 +118,7 @@ P_HD Geodetic ecef2geodetic(Vec3 r) {
   if (WANT & 2) g.lon = HOT ? gm_atan2_inl(r.y, r.x) : gm_atan2(r.y, r.x);
   if (WANT & 1) {
     double sl, cl;
-    if (HOT) gm_sincos_inl(g.lat, &sl, &cl);
+    if (HOT) gm_sincos_small_inl(g.lat, &sl, &cl);
     else gm_sincos(g.lat, &sl, &cl);
     double N = gm_div(P_RA, gm_sqrt(1.0 - P_E2 * sl * sl));
     g.alt = gm_div(p, cl) - N;
@@ -147,8 +148,8 @@ template <bool HOT = false>
 P_HD Quat quat_ecef2ned_ll(double lat, double lon) {
   double s_hl, c_hl, s_hp, c_hp;
   if (HOT) {
-    gm_sincos_inl(lon / 2.0, &s_hl, &c_hl);
-    gm_sincos_inl(lat / 2.0, &s_hp, &c_hp);
+    gm_sincos_small_inl(lon / 2.0, &s_hl, &c_hl);
+    gm_sincos_small_inl(lat / 2.0, &s_hp, &c_hp);
   } else {
     gm_sincos(lon / 2.0, &s_hl, &c_hl);
     gm_sincos(lat / 2.0, &s_hp, &c_hp);

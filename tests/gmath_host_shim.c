@@ -1,19 +1,25 @@
-/* Host-side export of gmath.h for tests/test_gmath.py (accuracy vs mpmath).
- * Built by tests/conftest.py with: gcc -O2 -ffp-contract=off -mfma -shared -fPIC */
-#include "../gelato_b200/csrc/gmath.h"
-#define V1(name, fn) void name(const double* x, double* y, int n) { for (int i = 0; i < n; i++) y[i] = fn(x[i]); }
-#define V2(name, fn) void name(const double* a, const double* b, double* y, int n) { for (int i = 0; i < n; i++) y[i] = fn(a[i], b[i]); }
-V1(gmt_sin, gm_sin)
-V1(gmt_cos, gm_cos)
-V1(gmt_tan, gm_tan)
-V1(gmt_atan, gm_atan)
-V1(gmt_asin, gm_asin)
-V1(gmt_acos, gm_acos)
-V1(gmt_exp, gm_exp)
-V1(gmt_log, gm_log)
-V2(gmt_atan2, gm_atan2)
-V2(gmt_pow, gm_pow)
-V2(gmt_atan2_slow, gm_atan2_slow)
-V2(gmt_pow_slow, gm_pow_slow)
-double gmt_div_by_one(double a, double d) { return gm_div_by(a, gm_rcp(d)); }
-V2(gmt_div_by, gmt_div_by_one)
+/* Host-side export of gmath.h for tests/test_gmath.py and tests/test_gmath_device.py (accuracy vs mpmath, and the
+ * host side of device == host).  Built by those tests with: gcc -O2 -ffp-contract=off -mfma -shared -fPIC */
+#include "gmath_shim.h"
+
+#define U(name, expr) \
+  void gmt_##name(const double* x, double* y, int n) { for (int i = 0; i < n; i++) { const double a = x[i]; y[i] = expr; } }
+#define B(name, expr)                                                       \
+  void gmt_##name(const double* x, const double* w, double* y, int n) {     \
+    for (int i = 0; i < n; i++) { const double a = x[i], b = w[i]; y[i] = expr; } \
+  }
+#define T(name, expr)                                                                        \
+  void gmt_##name(const double* x, const double* w, const double* v, double* y, int n) {    \
+    for (int i = 0; i < n; i++) { const double a = x[i], b = w[i], c = v[i]; y[i] = expr; } \
+  }
+#define U2(name, stmt)                                              \
+  void gmt_##name(const double* x, double* y, double* z, int n) {   \
+    for (int i = 0; i < n; i++) {                                   \
+      const double a = x[i];                                        \
+      double y0, y1;                                                \
+      stmt;                                                         \
+      y[i] = y0;                                                    \
+      z[i] = y1;                                                    \
+    }                                                               \
+  }
+GMATH_SHIM_ENTRIES(U, B, T, U2)

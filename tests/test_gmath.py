@@ -10,6 +10,8 @@ import mpmath
 import numpy as np
 import pytest
 
+import gmath_corpus
+
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB = os.path.join(HERE, "_build", "libgmath_shim.so")
 _pd = ctypes.POINTER(ctypes.c_double)
@@ -111,36 +113,9 @@ def test_fast_paths_equal_the_complete_functions(shim):
 def test_shared_reciprocal_division_is_the_ieee_quotient(shim):
     """gm_div_by(a, gm_rcp(d)) -- one reciprocal shared by several quotients, Markstein's correction -- must give the
     bits of a / d: random operands over the whole exponent range (the guard sends the extreme ones to the plain
-    division), operands with significands next to 1 and next to 2, few-bit significands, zeros, infinities and NaN."""
-    rng = np.random.default_rng(9)
-    n = 2_000_000
-
-    def sig(kind):
-        m = rng.integers(0, 1 << 52, n, dtype=np.uint64)
-        if kind == 1:
-            m = (np.uint64((1 << 52) - 1) - (m & np.uint64(0xff)))
-        elif kind == 2:
-            m = m & np.uint64(0xff)
-        elif kind == 3:
-            m = m & np.uint64(0xfffff00000000)
-        return m
-
-    parts_a, parts_d = [], []
-    for ka in range(4):
-        for kd in range(4):
-            if (ka, kd) not in ((0, 0), (1, 1), (2, 2), (0, 1), (1, 0), (0, 2), (2, 0), (3, 3), (0, 3)):
-                continue
-            ea = rng.integers(1023 - 600, 1023 + 600, n).astype(np.uint64)
-            ed = rng.integers(1023 - 600, 1023 + 600, n).astype(np.uint64)
-            sa = rng.integers(0, 2, n).astype(np.uint64) << np.uint64(63)
-            sd = rng.integers(0, 2, n).astype(np.uint64) << np.uint64(63)
-            parts_a.append((sa | (ea << np.uint64(52)) | sig(ka)).view(np.float64))
-            parts_d.append((sd | (ed << np.uint64(52)) | sig(kd)).view(np.float64))
-    special = np.array([0.0, -0.0, 1.0, -1.0, np.inf, -np.inf, np.nan, 5e-324, 2.2250738585072014e-308, 1.7976931348623157e308,
-                        1e-8, 6378137.0, 1000.0, 3.0, 1.0 / 3.0])
-    parts_a.append(np.repeat(special, special.size))
-    parts_d.append(np.tile(special, special.size))
-    a, d = np.concatenate(parts_a), np.concatenate(parts_d)
+    division), operands with significands next to 1 and next to 2, few-bit significands, the edges of the guard's
+    exponent window, zeros, infinities and NaN (tests/gmath_corpus.py: division_operands)."""
+    a, d = gmath_corpus.division_operands(np.random.default_rng(9), 2_000_000)
     with np.errstate(all="ignore"):
         got, want = _call2(shim, "gmt_div_by", a, d), a / d
     same = (got.view(np.uint64) == want.view(np.uint64)) | (np.isnan(got) & np.isnan(want))

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """gmath_coeffs.inc -> gmath_table.inc: the coefficient literals as one table (device: __constant__ memory) and the
-index of each name.  Run after tools/gen_gmath_coeffs.py."""
+index of each name; the words of 2/pi as a second table.  Run after tools/gen_gmath_coeffs.py."""
 import os
 import re
 
@@ -20,6 +20,12 @@ def main():
         out.append("  " + ", ".join(names[i:i + 4]) + (", \\" if i + 4 < len(names) else " \\"))
     out.append("}")
     out += ["#define GMT_%s %d" % (nm[3:], i) for i, nm in enumerate(names)]
+    # the words of 2/pi (integers, not operands of the polynomials): a table of their own
+    words = [m.group(1) for m in re.finditer(r"#define (GM_2OPI_W[0-9]+) 0x", inc)]
+    out += ["#define GM_2OPI_N %d" % len(words), "#define GM_2OPI_INIT { \\"]
+    for i in range(0, len(words), 4):
+        out.append("  " + ", ".join(words[i:i + 4]) + (", \\" if i + 4 < len(words) else " \\"))
+    out.append("}")
     open(os.path.join(CSRC, "gmath_table.inc"), "w").write("\n".join(out) + "\n")
 
 
