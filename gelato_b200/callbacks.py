@@ -17,7 +17,8 @@ of the whole result, sliced into the reference's dictionaries as views.
 import numpy as np
 
 from . import engine as _engine
-from .plan import GROUPS, ORBIT_QUANTITIES, VAR_ORDER, CompiledPlan, OrbitAtEvent, PerigeeAtEvent  # noqa: F401
+from .plan import (GROUPS, ORBIT_QUANTITIES, TABLE_COLUMNS, VAR_ORDER, CompiledPlan, OrbitAtEvent,  # noqa: F401
+                   PerigeeAtEvent, TableAtEvent)
 
 
 class GelatoProblem:

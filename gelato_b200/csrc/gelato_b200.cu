@@ -26,6 +26,7 @@
 #include "host_pool.h"
 #include "mesh_error.h"
 #include "plan_host.h"
+#include "user_table.h"
 
 // ---------------------------------------------------------------------------
 // kernels
@@ -327,6 +328,34 @@ k_path_rows(const __grid_constant__ PlanView P, const PathRow* __restrict__ rows
   path_lane_store(pr, tb.P + (long long)pr.l * (n + 1), n, lane, q, vals_all + (size_t)scen * n_vals);
 }
 
+// Result-table user constraints (user_table.h): one warp per (scenario, table job), lane l evaluating output_row on
+// its state once; per constraint row the quotients against lane 0 come from a shuffle.  out_all == NULL: residual only
+// (the pristine lane alone); g_all == NULL: Jacobian only.  Every thread of a warp reaches the shuffles (a warp is one
+// job; the warps past the last job run job 0 with every lane idle).
+#define GT_THREADS 128
+__global__ void __launch_bounds__(GT_THREADS)
+k_user_table(const __grid_constant__ PlanView P, const __grid_constant__ TabView T, const int n_scen,
+             const int32_t* __restrict__ scen_ids, const double* __restrict__ x_all, double* __restrict__ out_all,
+             double* __restrict__ g_all) {
+  const long long w = ((long long)blockIdx.x * GT_THREADS + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  const bool live = w < (long long)T.n_tab * n_scen;
+  const int scen = live ? (int)(w / T.n_tab) : 0;
+  const int job = live ? (int)(w - (long long)scen * T.n_tab) : 0;
+  const bool active = live && (lane < GT_PRISTINE ? out_all != nullptr : (lane == GT_PRISTINE && g_all != nullptr));
+  const int sid = scen_ids ? scen_ids[scen] : scen;
+  double out[GO_COLS];
+  if (active) table_lane_eval(P, T, sid, x_all + (size_t)scen * P.n_vars, job, lane, out);
+  double* vals = out_all ? out_all + (size_t)scen * (size_t)(P.packed ? P.n_pack : P.n_vals) : nullptr;
+  double* g = g_all ? g_all + (size_t)scen * P.n_rows : nullptr;
+  const int nrow = T.i32[(long long)job * GT_I32_COLS + GT_NROW];
+  for (int r = 0; r < nrow; r++) {
+    const double v = active ? table_row_value(T, job, r, out) : 0.0;
+    const double v0 = __shfl_sync(0xffffffffu, v, 0);
+    if (active) table_lane_store(P, T, job, r, lane, v, v0, vals, g);
+  }
+}
+
 // probe: is a*b+c left unfused?  (1 + 2^-30)(1 - 2^-30) - 1 is 0 unfused, -2^-60 fused
 __global__ void k_unfused_probe(double a, double b, double c, double* out) { *out = a * b + c; }
 
@@ -480,6 +509,8 @@ struct GelatoPlan {
   long long prow_vals = 0;
   TestGrid prow_grid;
   DeviceBuf<PathRow> d_prow;
+  // result-table user constraints (user_table.h; tab.n_tab = 0: none, and nothing is launched for them)
+  TabView tab{};
   long long launches = 0;
   Event ev0, ev1;
 };
@@ -521,7 +552,21 @@ static int add_lane(GelatoPlan* p) {
 struct JacRange {
   int b0 = 0, nb = -1, v0 = 0, nv = 0;
 };
+// The table jobs of n_scen batch slots on `st` (nothing for a plan without them): view v's layout and step, out_dev
+// NULL for a residual evaluation, g_dev NULL for a Jacobian-only one.
+static int launch_table(GelatoPlan* p, const PlanView& v, const double* x_dev, double* out_dev, double* g_dev, int n_scen,
+                        const int32_t* ids_dev, cudaStream_t st) {
+  if (p->tab.n_tab == 0) return GELATO_OK;
+  const long long threads = (long long)p->tab.n_tab * n_scen * 32;
+  k_user_table<<<(unsigned)((threads + GT_THREADS - 1) / GT_THREADS), GT_THREADS, 0, st>>>(v, p->tab, n_scen, ids_dev, x_dev,
+                                                                                          out_dev, g_dev);
+  p->launches++;
+  CU(cudaGetLastError());
+  return GELATO_OK;
+}
+
 // dx: the step of the finite-difference protocol (the plan's dx for forward differences).
+// The table jobs go on the pair stream next to the block kernel; a sub-range evaluates them when it starts at block 0.
 static int launch_jacobian_pass(GelatoPlan* p, double dx, const double* x_dev, double* out_dev, double* g_dev, int n_scen,
                                 cudaStream_t st, const Lane& L, const int32_t* ids_dev, bool packed, JacRange rg = JacRange()) {
   PlanView v = p->view;
@@ -533,7 +578,8 @@ static int launch_jacobian_pass(GelatoPlan* p, double dx, const double* x_dev, d
   const int v_first = p->vac_first + (all ? 0 : rg.v0);
   const int32_t* table = p->jac_blocks + (size_t)(all ? 0 : rg.b0) * BT_COLS;
   const cudaStream_t aux = L.pair_stream;
-  const bool side = nv > 0 && nb > 0 && aux != st;
+  const bool tab = p->tab.n_tab > 0 && (all || (rg.b0 == 0 && rg.nb > 0));
+  const bool side = (nv > 0 || tab) && nb > 0 && aux != st;
   if (side) {
     CU(cudaEventRecord(L.ev_fork, st));
     CU(cudaStreamWaitEvent(aux, L.ev_fork, 0));
@@ -543,6 +589,10 @@ static int launch_jacobian_pass(GelatoPlan* p, double dx, const double* x_dev, d
     k_jacobian_noair<<<(unsigned)per * n_scen, GV_THREADS, 0, side ? aux : st>>>(v, v_first, nv, n_scen, ids_dev, x_dev, out_dev,
                                                                                 g_dev);
     p->launches++;
+  }
+  if (tab) {
+    int rc = launch_table(p, v, x_dev, out_dev, g_dev, n_scen, ids_dev, side ? aux : st);
+    if (rc) return rc;
   }
   if (nb > 0) {
     k_jacobian<<<(unsigned)nb * n_scen, GJ_THREADS, 0, st>>>(v, table, n_scen, ids_dev, x_dev, out_dev, g_dev);
@@ -603,7 +653,7 @@ static int launch_residuals(GelatoPlan* p, const double* x_dev, double* g_dev, i
   k_residuals<<<(unsigned)p->n_res_blocks * n_scen, GR_THREADS, 0, st>>>(p->view, p->res_blocks, n_scen, ids_dev, x_dev, g_dev);
   p->launches++;
   CU(cudaGetLastError());
-  return GELATO_OK;
+  return launch_table(p, p->view, x_dev, nullptr, g_dev, n_scen, ids_dev, st);
 }
 
 static void drop_graph(GelatoPlan* p) {
@@ -678,6 +728,14 @@ int gelato_plan_create(const GelatoPlanDesc* d, int device, GelatoPlan** out) {
   }
   UP(p->vals_template, d->vals_template, d->n_vals)
   p->shared_template = p->vals_template;
+  p->tab.n_tab = d->n_tab;
+  if (d->n_tab > 0) {
+    UP(p->tab.i32, d->tab_i32, (size_t)d->n_tab * GT_I32_COLS)
+    UP(p->tab.f64, d->tab_f64, (size_t)d->n_tab * GT_F64_COLS)
+    UP(p->tab.col, d->tab_col, d->n_tab_rows)
+    UP(p->tab.aux, d->tab_aux, d->n_tab_rows)
+    UP(p->tab.sf, d->tab_sf, (size_t)d->n_tab_rows * GT_SF_COLS)
+  }
 
   // block tables
   HostTables ht;
@@ -705,6 +763,7 @@ int gelato_plan_create(const GelatoPlanDesc* d, int device, GelatoPlan** out) {
     UP(v.sec_pk, L.sec_pk.data(), L.sec_pk.size())
     UP(v.aero_pk, L.aero_pk.data(), L.aero_pk.size())
     UP(v.evt_pk, L.evt_pk.data(), L.evt_pk.size())
+    UP(p->tab.pk, L.tab_pk.data(), L.tab_pk.size())
     p->pk_full.swap(L.full_slot);
     p->pk_src.swap(L.src);
     p->pk_sgn.swap(L.sgn);
@@ -1046,6 +1105,9 @@ static int eval_host(GelatoPlan* p, int which, const double* x, double* out, int
       cudaMemcpyAsync(p->d_x.get(), p->h_x.get(), nx * sizeof(double), cudaMemcpyHostToDevice, L.stream);
       k_residuals<<<(unsigned)p->n_res_blocks * n_scen, GR_THREADS, 0, L.stream>>>(p->view, p->res_blocks, n_scen, nullptr,
                                                                                   p->d_x.get(), p->d_g.get());
+      if (p->tab.n_tab > 0)
+        k_user_table<<<(unsigned)(((long long)p->tab.n_tab * n_scen * 32 + GT_THREADS - 1) / GT_THREADS), GT_THREADS, 0,
+                       L.stream>>>(p->view, p->tab, n_scen, nullptr, p->d_x.get(), nullptr, p->d_g.get());
       cudaMemcpyAsync(p->h_g.get(), p->d_g.get(), no * sizeof(double), cudaMemcpyDeviceToHost, L.stream);
       CU(cudaStreamEndCapture(L.stream, &graph));
       cudaGraphExec_t exec = nullptr;

@@ -118,6 +118,23 @@ static inline const char* validate_desc(const GelatoPlanDesc* d) {
     else ok = GELATO_RANGE(ej[GE_J_POS], 3) && GELATO_RANGE(ej[GE_J_T], 1) && (type != GE_IIP || GELATO_RANGE(ej[GE_J_VEL], 3));
     if (!ok) return "an event job's Jacobian block is outside vals";
   }
+  if (d->n_tab < 0 || d->n_tab_rows < 0) return "negative table length";
+  if (d->n_tab > 0 && (!d->tab_i32 || !d->tab_f64 || !d->tab_col || !d->tab_aux || !d->tab_sf))
+    return "missing result-table job tables";
+  for (long long k = 0; k < d->n_tab; k++) {
+    const int32_t* ti = d->tab_i32 + k * GT_I32_COLS;
+    if (ti[GT_TIDX] < 0 || ti[GT_TIDX] >= S) return "result-table job event index out of range";
+    if (ti[GT_SROW] < 0 || ti[GT_SROW] >= M) return "result-table job state row out of range";
+    if (ti[GT_NROW] < 1 || ti[GT_ROW] < 1 || (long long)ti[GT_ROW] + ti[GT_NROW] > d->n_rows)
+      return "result-table job rows out of range";
+    if (ti[GT_R0] < 0 || (long long)ti[GT_R0] + ti[GT_NROW] > d->n_tab_rows) return "result-table job row list out of range";
+    for (int c = 0; c < 12; c++)
+      if (ti[GT_RC0 + c] < 0) return "negative residue count of a result-table job";
+  }
+  for (long long r = 0; r < d->n_tab_rows; r++) {
+    if (d->tab_col[r] < 0 || d->tab_col[r] >= GT_COLUMNS) return "unknown result-table column code";
+    if (!GELATO_RANGE(d->tab_aux[r], GT_AUX)) return "a result-table row's values are outside vals";
+  }
 #undef GELATO_RANGE
   return nullptr;
 }
@@ -142,10 +159,11 @@ struct HostTables {
  *                 node-diagonal [4n][4], u 8n, t 4n (tf = -to)
  *   per aero job  position 3nk | velocity 3nk | quaternion 4nk (not for max-q) | t 2nk
  *   per event job as in COO order
+ *   per result-table row  its GT_AUX values, after all of the above
  * `full_slot` (ascending) lists every x-dependent COO slot, `src` / `sgn` say which packed value it holds and
  * with what sign:  vals[full_slot[i]] = sgn[i] * packed[src[i]]. */
 struct PackedLayout {
-  std::vector<int64_t> sec_pk, aero_pk, evt_pk;
+  std::vector<int64_t> sec_pk, aero_pk, evt_pk, tab_pk;
   long long n_pack = 0;
   std::vector<int64_t> full_slot, src;
   std::vector<double> sgn;
@@ -232,6 +250,9 @@ static inline void build_packed_layout(const GelatoPlanDesc* d, PackedLayout& L)
       pk[GE_J_T] = direct(ej[GE_J_T], 1);
     }
   }
+  /* result-table rows (after everything else: plans without them keep this layout) */
+  L.tab_pk.assign((size_t)d->n_tab_rows, -1);
+  for (int r = 0; r < d->n_tab_rows; r++) L.tab_pk[r] = direct(d->tab_aux[r], GT_AUX);
   L.n_pack = c;
   std::sort(ents.begin(), ents.end(), [](const Ent& a, const Ent& b) { return a.full < b.full; });
   L.full_slot.resize(ents.size());

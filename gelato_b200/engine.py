@@ -56,6 +56,8 @@ class PlanDesc(ctypes.Structure):
         ("n_evt", ctypes.c_int32), ("evt_i32", _pi32), ("evt_i64", _pi64), ("evt_f64", _pd),
         ("vals_template", _pd),
         ("xdep_idx", _pi64), ("n_xdep", ctypes.c_int64),
+        ("n_tab", ctypes.c_int32), ("tab_i32", _pi32), ("tab_f64", _pd), ("n_tab_rows", ctypes.c_int32),
+        ("tab_col", _pi32), ("tab_aux", _pi64), ("tab_sf", _pd),
     ]
 
 
@@ -130,6 +132,12 @@ def make_desc(plan):
     xdep = c(plan.xdep_index(), np.int64)
     d.xdep_idx = _ptr(xdep, _pi64)
     d.n_xdep = xdep.size
+    d.n_tab, d.n_tab_rows = plan.n_tab, plan.n_tab_rows
+    d.tab_i32 = _ptr(c(plan.tab_i32, np.int32), _pi32)
+    d.tab_f64 = _ptr(c(plan.tab_f64, np.float64), _pd)
+    d.tab_col = _ptr(c(plan.tab_col, np.int32), _pi32)
+    d.tab_aux = _ptr(c(plan.tab_aux, np.int64), _pi64)
+    d.tab_sf = _ptr(c(plan.tab_sf, np.float64), _pd)
     return d, keep
 
 
@@ -144,7 +152,7 @@ def make_scenario_desc(plans):
             raise ValueError("scenario plans must share the problem structure")
         # what is NOT carried per scenario is evaluated with the base plan's copy: it must be the same everywhere
         shared = ("sec_i32", "sec_i64", "d_pool", "tau_pool", "ca", "lin_i32", "aero_i32", "aero_i64", "aero_f64",
-                  "rc_aero", "evt_i32", "evt_i64", "evt_f64")
+                  "rc_aero", "evt_i32", "evt_i64", "evt_f64", "tab_i32", "tab_f64", "tab_col", "tab_aux", "tab_sf")
         for name in shared:
             a, b = getattr(base, name, None), getattr(p, name, None)
             if a is None and b is None:

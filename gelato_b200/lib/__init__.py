@@ -34,7 +34,8 @@ _problems = {}  # id(pdict) -> _Cached
 
 
 def configure(user_eq=None, user_ineq=None, device=0, coord=None, engine_factory=None):
-    """Built-in user constraints (e.g. PerigeeAtEvent("IIP_END")) and the CUDA device used
+    """Built-in user constraints (e.g. PerigeeAtEvent("IIP_END"), TableAtEvent("FAIRING", [("altitude", 1e5, 1.0)]), or
+    a list of them) and the CUDA device used
     by problems created from now on.  Arbitrary Python user constraints stay on the host:
     evaluate them with the reference's own con_user / jac_fd (jac_fd below accepts them)."""
     _config.update(user_eq=user_eq, user_ineq=user_ineq, device=device, coord=coord, engine_factory=engine_factory)

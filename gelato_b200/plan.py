@@ -27,6 +27,7 @@ import math
 import numpy as np
 
 from . import hostmath
+from .output import KERNEL_COLUMNS
 
 EQ_GROUPS = (
     "eqcon_init eqcon_time eqcon_dyn_mass eqcon_dyn_pos eqcon_dyn_vel eqcon_dyn_quat eqcon_knot "
@@ -60,6 +61,13 @@ GE_J_POS, GE_J_VEL, GE_J_T, GE_I64_COLS = range(4)
 GE_REF, GE_DEN, GE_A0, GE_A1, GE_A2, GE_A3, GE_A4, GE_A5, GE_F64_COLS = range(9)
 
 AUX_PER_USER = 12  # per row: 6 finite differences + 6 "background" quotients (jobs.h, GE_USER_ORBIT)
+# include/gelato_b200.h: result-table jobs (GT_*)
+GT_SROW, GT_TIDX, GT_ROW, GT_NROW, GT_R0, GT_RC0 = range(6)
+GT_I32_COLS = GT_RC0 + 12
+AUX_PER_TABLE = 18  # per row: 12 finite differences + background quotients after 1, 4, 7, 11, 12 and 0 restores
+TABLE_COLUMNS = {name: k for k, name in enumerate(KERNEL_COLUMNS)}  # column codes: output.h / gelato_leaf_output_table
+# the slot of a table row's aux values holding the background quotient after k restores (user_table.h)
+_TABLE_BG_SLOT = {1: 12, 4: 13, 7: 14, 11: 15, 12: 16, 0: 17}
 
 # quantity codes of the user built-ins (include/gelato_b200.h: GEQ_*)
 ORBIT_QUANTITIES = {"perigee_radius": 0, "apogee_radius": 1, "semi_major_axis": 2, "eccentricity": 3,
@@ -103,6 +111,43 @@ class PerigeeAtEvent(OrbitAtEvent):
 
     def __init__(self, event_name):
         super().__init__(event_name, [("perigee_radius", 6378137.0, 1.0)])
+
+
+class TableAtEvent:
+    """GPU-resident built-in user constraint on the result table: rows
+
+        g_r = column_r(state at the first node of `event_name`) / scale_r - offset_r
+
+    with column_r one of output.KERNEL_COLUMNS -- the per-node quantities of the reference's result table
+    (output_result.py), in its units (deg, m, Pa, m/s, N): altitude, downrange, dynamic_pressure, AOA_total,
+    flightpath_vel_inertial_geocentric, ...  The node is the one OrbitAtEvent uses; its inputs are those the result table
+    gives that node: mass, position, velocity, quaternion, time t[i] * unit_t, section i's thrust / reference_area /
+    nozzle_area, the wind and CA tables and the launch site.  One row returns a scalar; several return a vector.
+    A user group may also be a list of built-ins (OrbitAtEvent and TableAtEvent mixed): their rows in list order."""
+
+    def __init__(self, event_name, rows):
+        self.event_name = event_name
+        self.rows = [(str(col), float(scale), float(offset)) for col, scale, offset in rows]
+        if not self.rows:
+            raise ValueError("a built-in user constraint has at least one row")
+        for col, scale, _ in self.rows:
+            if col not in TABLE_COLUMNS:
+                raise ValueError("unknown result-table column %r (known: %s)" % (col, ", ".join(KERNEL_COLUMNS)))
+            if scale == 0.0:
+                raise ValueError("scale must be non-zero")
+
+
+def _builtins(fn):
+    """The built-ins of a user group: [] for None, the list for a list / tuple, else [fn]; TypeError for anything that
+    is not a registered built-in."""
+    if fn is None:
+        return []
+    items = list(fn) if isinstance(fn, (list, tuple)) else [fn]
+    if not items or not all(isinstance(b, (OrbitAtEvent, TableAtEvent)) for b in items):
+        raise TypeError(
+            "user constraints evaluated on the GPU must be registered built-ins (OrbitAtEvent / PerigeeAtEvent, "
+            "TableAtEvent) or a non-empty list of them; arbitrary Python callables cannot run inside the CUDA kernels")
+    return items
 
 
 class Block:
@@ -154,19 +199,18 @@ class CompiledPlan:
             o += self.sizes[k]
         self.n_vars = o
         for fn in (user_eq, user_ineq):
-            if fn is not None and not isinstance(fn, OrbitAtEvent):
-                raise TypeError(
-                    "user constraints evaluated on the GPU must be registered built-ins (OrbitAtEvent / "
-                    "PerigeeAtEvent); arbitrary Python callables cannot run inside the CUDA kernels")
+            _builtins(fn)
         self.user_eq, self.user_ineq = user_eq, user_ineq
 
         self._sec = [self.ps.get_index(i) for i in range(S)]
         self._names = [prm["name"] for prm in pdict["params"]]
         self._lin = []  # (row, ip, im, sp, sm, c)
         self._evt = []  # dict per job
+        self._tab = []  # dict per result-table job
+        self._tab_rows = []  # (column code, scale, offset, aux offset) per result-table row
         self._aero = []
         self.group_rows = {}  # key -> (row0, nrow) | None
-        self.blocks = {}  # key -> {var: Block} | None | "dense-user"
+        self.blocks = {}  # key -> {var: Block} | None | ("dense-user", ...) (_g_user)
         self._tmpl = []  # (offset, values) constant segments
         self._nvals = 0
         self._row = 1  # g[0] = objective
@@ -829,21 +873,51 @@ class CompiledPlan:
 
     # ---- user constraints (con_user.py + jac_fd.py) ---------------------
     def _g_user(self, key, fn):
-        if fn is None:
+        """One user group: ONE jac_fd pass of the reference over every built-in of the group.  Each built-in's rows see
+        the same base state (the residue of the groups before) and depend on its own read variables only; the
+        group's pass leaves one residue on every variable."""
+        items = _builtins(fn)
+        if not items:
             self._absent(key)
             return
-        index = self.p["event_index"][fn.event_name]
-        srow = self.ps.index_start_u(index) + index
-        k = len(fn.rows)
-        g0 = self._begin(key, k)
-        codes = sum(ORBIT_QUANTITIES[q] << (8 * r) for r, (q, _, _) in enumerate(fn.rows))
-        a = [1.0, 0.0] * 3
-        for r, (_, scale, offset) in enumerate(fn.rows):
-            a[2 * r], a[2 * r + 1] = scale, offset
-        job = self._evt_job(GE_USER_ORBIT, -1, srow, codes, 0, g0, k, 0.0, 1.0, a=a)
-        self.blocks[key] = ("dense-user", job, srow)
+        r = self._begin(key, sum(len(b.rows) for b in items))
+        parts = []  # (job, srow, event index, first row of the part inside the group)
+        for b in items:
+            index = self.p["event_index"].get(b.event_name)
+            if index is None:
+                raise KeyError("unknown event %r (events: %s)" % (b.event_name, ", ".join(self.p["event_index"])))
+            if isinstance(b, TableAtEvent) and not 0 <= index < self.S:
+                raise ValueError("event %r starts no section: it has no first node" % b.event_name)
+            srow = self.ps.index_start_u(index) + index
+            k = len(b.rows)
+            if isinstance(b, OrbitAtEvent):
+                codes = sum(ORBIT_QUANTITIES[q] << (8 * j) for j, (q, _, _) in enumerate(b.rows))
+                a = [1.0, 0.0] * 3
+                for j, (_, scale, offset) in enumerate(b.rows):
+                    a[2 * j], a[2 * j + 1] = scale, offset
+                job = self._evt_job(GE_USER_ORBIT, -1, srow, codes, 0, r, k, 0.0, 1.0, a=a)
+            else:
+                job = self._tab_job(index, srow, r, b)
+            parts.append((job, srow, index, r - self.group_rows[key][0]))
+            r += k
+        # ("dense-user", first job, its state row, every part): the first two as a group of one OrbitAtEvent has them
+        self.blocks[key] = ("dense-user", parts[0][0], parts[0][1], parts)
         # jac_fd perturbs and restores EVERY variable in place (jac_fd.py:54-60)
         self._rc += 1
+
+    def _tab_job(self, index, srow, row, fn):
+        """Register a result-table job (include/gelato_b200.h: GT_*) with the residue counts of its 12 read variables."""
+        reads = ([self.off["mass"] + srow] + [self.off["position"] + 3 * srow + k for k in range(3)] +
+                 [self.off["velocity"] + 3 * srow + k for k in range(3)] +
+                 [self.off["quaternion"] + 4 * srow + k for k in range(4)] + [self.off["t"] + index])
+        lc = self.p["LaunchCondition"]
+        job = {"i32": [srow, index, row, len(fn.rows), len(self._tab_rows)] + [int(self._rc[j]) for j in reads],
+               "f64": [float(lc["lat"]), float(lc["lon"])], "rows": []}
+        for col, scale, offset in fn.rows:
+            job["rows"].append(len(self._tab_rows))
+            self._tab_rows.append([TABLE_COLUMNS[col], scale, offset, -1])
+        self._tab.append(job)
+        return job
 
     # ------------------------------------------------------------------
     def _finish(self):
@@ -853,8 +927,14 @@ class CompiledPlan:
         for key in ("eqcon_user", "ineqcon_user"):
             b = self.blocks.get(key)
             if isinstance(b, tuple):
-                b[1]["i64"][GE_J_POS] = self._nvals
-                self._nvals += AUX_PER_USER * b[1]["i32"][GE_NROW]
+                for job, _, _, _ in b[3]:
+                    if "rows" in job:  # result-table job: each row's values
+                        for k in job["rows"]:
+                            self._tab_rows[k][3] = self._nvals
+                            self._nvals += AUX_PER_TABLE
+                    else:
+                        job["i64"][GE_J_POS] = self._nvals
+                        self._nvals += AUX_PER_USER * job["i32"][GE_NROW]
         self.n_vals = self._nvals
         tmpl = np.zeros(self.n_vals, dtype=np.float64)
         for off, vals in self._tmpl:
@@ -873,6 +953,12 @@ class CompiledPlan:
         self.evt_i32 = np.array([j["i32"] for j in self._evt], dtype=np.int32).reshape(-1, GE_I32_COLS)
         self.evt_i64 = np.array([j["i64"] for j in self._evt], dtype=np.int64).reshape(-1, GE_I64_COLS)
         self.evt_f64 = np.array([j["f64"] for j in self._evt], dtype=np.float64).reshape(-1, GE_F64_COLS)
+        self.n_tab, self.n_tab_rows = len(self._tab), len(self._tab_rows)
+        self.tab_i32 = np.array([j["i32"] for j in self._tab], dtype=np.int32).reshape(-1, GT_I32_COLS)
+        self.tab_f64 = np.array([j["f64"] for j in self._tab], dtype=np.float64).reshape(-1, 2)
+        self.tab_col = np.array([t[0] for t in self._tab_rows], dtype=np.int32)
+        self.tab_sf = np.array([t[1:3] for t in self._tab_rows], dtype=np.float64).reshape(-1, 2)
+        self.tab_aux = np.array([t[3] for t in self._tab_rows], dtype=np.int64)
         self.wind = np.ascontiguousarray(self.p["wind_table"], dtype=np.float64)
         self.ca = np.ascontiguousarray(self.p["ca_table"], dtype=np.float64)
         self.units = (float(self.u["mass"]), float(self.u["position"]), float(self.u["velocity"]), float(self.u["u"]),
@@ -897,8 +983,9 @@ class CompiledPlan:
         lanes = {GE_LLH: 5, GE_IIP: 8, GE_ANT: 5, GE_TERM: 7, GE_USER_ORBIT: 13}
         evt_jac = sum(lanes[j["i32"][0]] for j in self._evt)
         aero_jac = 13 * aero_rows[0] + 9 * aero_rows[1] + 13 * aero_rows[2]
-        obj = self.N + n_free + sum(aero_rows.values()) + len(self._evt)
-        sens = 14 * n_air_fd + 9 * (self.N - n_air_fd) + 7 * n_free + aero_jac + evt_jac
+        # result-table jobs: one output_row per job in objfunc, 18 in sens (user_table.h: lanes 0-17)
+        obj = self.N + n_free + sum(aero_rows.values()) + len(self._evt) + len(self._tab)
+        sens = 14 * n_air_fd + 9 * (self.N - n_air_fd) + 7 * n_free + aero_jac + evt_jac + 18 * len(self._tab)
         return {"objfunc": obj, "sens": sens, "air_nodes": n_air, "air_fd_nodes": n_air_fd,
                 "noair_nodes": self.N - n_air, "free_nodes": n_free, "air_free_nodes": n_air_free,
                 "aero_rows": sum(aero_rows.values()),
@@ -955,6 +1042,8 @@ class CompiledPlan:
                 if typ == GE_IIP:
                     run(job["i64"][GE_J_VEL], 3)
                 run(job["i64"][GE_J_T], 1)
+        for aux in self.tab_aux:
+            run(aux, AUX_PER_TABLE)
         idx = np.sort(np.concatenate(parts)) if parts else np.zeros(0, dtype=np.int64)
         assert idx.size == np.unique(idx).size, "an x-dependent Jacobian slot is listed twice"
         self._xdep = idx
@@ -1005,15 +1094,30 @@ class CompiledPlan:
         return {"t": gvec}
 
     def _user_dense(self, vals, spec, key_order, out=None):
-        """Expand the 12 auxiliary quotients of every row into jac_fd's dense blocks
+        """Expand the auxiliary quotients of every row of a user group into jac_fd's dense blocks
         (jac_fd.py:54-60): a variable the function does not read still gets
-        (g(x after k restores) - g_base)/dx, k = how many of the six read
-        variables were visited before it -- for k = 0 that is (g_base - g_base)/dx, +0 or NaN where g_base is not
-        finite.  `out`: the dictionary of an earlier call to refill in place (its arrays
-        are column slices of one (rows, n_vars) buffer, filled by one gather per row)."""
-        _, job, srow = spec
-        nrow = job["i32"][GE_NROW]
+        (g(x after k restores) - g_base)/dx, k = how many of the variables its built-in reads were visited before it
+        -- for k = 0 that is (g_base - g_base)/dx, +0 or NaN where g_base is not finite.  `out`: the dictionary of an
+        earlier call to refill in place (its arrays are column slices of one (rows, n_vars) buffer, filled by one
+        gather per row)."""
         order = tuple(key_order)
+        nrow = sum(job["i32"][GE_NROW] if "rows" not in job else len(job["rows"]) for job, _, _, _ in spec[3])
+        if out is None:
+            buf = np.empty((nrow, self.n_vars))
+            out, o = _UserBlocks(buf), 0
+            for key in order:
+                out[key] = buf[:, o: o + self.sizes[key]]
+                o += self.sizes[key]
+        buf = out.buffer
+        for job, srow, index, r0 in spec[3]:
+            if "rows" in job:
+                self._table_dense(vals, job, srow, index, order, buf[r0: r0 + len(job["rows"])])
+            else:
+                self._orbit_dense(vals, job, srow, order, buf[r0: r0 + job["i32"][GE_NROW]])
+        return out
+
+    def _orbit_dense(self, vals, job, srow, order, buf):
+        """The rows of an OrbitAtEvent job: 12 auxiliary quotients each (jobs.h: GE_USER_ORBIT)."""
         maps = self.__dict__.setdefault("_user_maps", {})
         idx = maps.get((order, srow))
         if idx is None:
@@ -1032,23 +1136,46 @@ class CompiledPlan:
                     ix[3 * srow + 3:] = k
                 parts.append(ix)
             idx = maps[(order, srow)] = np.concatenate(parts)
-        if out is None:
-            buf = np.empty((nrow, idx.size))
-            out, o = _UserBlocks(buf), 0
-            for key in order:
-                out[key] = buf[:, o: o + self.sizes[key]]
-                o += self.sizes[key]
-        buf = out.buffer
         q = np.full(13, np.nan)  # q[1] (k = 1) is never indexed
         a0 = job["i64"][GE_J_POS]
-        for r in range(nrow):
+        for r in range(buf.shape[0]):
             # background slot 0 holds k = 0 (jobs.h: evt_jac_phase1, lane 7), slots 1..5 k = 2..6
             q[0] = 0.0 * vals[a0 + 6]  # the same +0 / NaN; 0 for csr_map's probe, whose entries here stay structural zeros
             q[2:7] = vals[a0 + 7: a0 + 12]
             q[7:13] = vals[a0: a0 + 6]
             np.take(q, idx, out=buf[r])
             a0 += AUX_PER_USER
-        return out
+
+    def _table_dense(self, vals, job, srow, index, order, buf):
+        """The rows of a TableAtEvent job: 18 auxiliary values each (user_table.h), taken by an index built once per
+        (state row, event index, key order)."""
+        maps = self.__dict__.setdefault("_user_maps", {})
+        idx = maps.get((order, "table", srow, index))
+        if idx is None:
+            if order != tuple(VAR_ORDER):  # the device visits the read variables in the reference's key order
+                raise NotImplementedError("xdict key order %s: result-table constraints follow the reference's %s"
+                                          % (list(order), list(VAR_ORDER)))
+            reads = {"mass": [srow], "position": [3 * srow + k for k in range(3)],
+                     "velocity": [3 * srow + k for k in range(3)], "quaternion": [4 * srow + k for k in range(4)],
+                     "t": [index]}
+            parts, k = [], 0  # k: read variables visited so far = the next one's finite-difference slot
+            for key in order:
+                ix = np.empty(self.sizes[key], dtype=np.intp)
+                at = 0
+                for j in reads.get(key, []):
+                    if j > at:
+                        ix[at: j] = _TABLE_BG_SLOT[k]
+                    ix[j] = k
+                    k += 1
+                    at = j + 1
+                ix[at:] = _TABLE_BG_SLOT[k]
+                parts.append(ix)
+            idx = maps[(order, "table", srow, index)] = np.concatenate(parts)
+        for r, row in enumerate(job["rows"]):
+            a0 = self._tab_rows[row][3]
+            q = np.array(vals[a0: a0 + AUX_PER_TABLE], dtype=np.float64)
+            q[17] = 0.0 * q[17]  # +0 / NaN; 0 for csr_map's probe, whose entries here stay structural zeros
+            np.take(q, idx, out=buf[r])
 
     def refresh_user_blocks(self, vals, sens_dict, key_order):
         """Refill the dense user-constraint blocks of a `funcsSens` dictionary made by split_jacobian from the SAME

@@ -126,6 +126,35 @@ enum {
 enum { GE_J_POS = 0, GE_J_VEL, GE_J_T, GE_I64_COLS };
 enum { GE_REF = 0, GE_DEN, GE_A0, GE_A1, GE_A2, GE_A3, GE_A4, GE_A5, GE_F64_COLS };
 
+/* ---- result-table user constraints (gelato_b200.plan.TableAtEvent) -------------------------------------------
+ * A built-in user constraint on columns of the reference's result table (the 34 outputs of gelato_leaf_output_table)
+ * at the first node of event i (state row srow = index_start_u(i) + i, time t[i] * unit_t, section i's thrust /
+ * reference_area / nozzle_area, the scenario's wind table, the plan's CA table, the launch site's lat / lon):
+ *     g[row + r] = column_r / scale_r - offset_r.
+ * The reference applies jac_fd (jac_fd.py:29-62) to it.  The function reads 12 variables, in xdict order: mass[srow],
+ * position[3 srow + 0..2], velocity[3 srow + 0..2], quaternion[4 srow + 0..3], t[i].  Each of its rows leaves GT_AUX
+ * values in vals, at its own offset:
+ *     0..11   the finite-difference quotient of each read variable (the variables visited before it restored, itself
+ *             perturbed by +dx)
+ *     12..16  the "background" quotients jac_fd gives the variables the function does not read: k = 1, 4, 7, 11, 12 of
+ *             the read variables restored, nothing perturbed
+ *     17      k = 0: (base - base) / dx, +0 or NaN where the base value is not finite
+ * all from the base state r^rc(x) (the 12 residue counts GT_RC0.. of the groups evaluated earlier).  One kernel of its
+ * own (k_user_table: a warp per scenario and job) evaluates them next to the Jacobian kernel. */
+#define GT_AUX 18
+#define GT_COLUMNS 34 /* column codes: the order of gelato_leaf_output_table's outputs */
+enum {
+  GT_SROW = 0, /* state row of the event's first node */
+  GT_TIDX,     /* event index i: t[i], section i's parameters; 0 <= i < S */
+  GT_ROW,      /* first residual row */
+  GT_NROW,     /* rows of the job (>= 1) */
+  GT_R0,       /* its first row in the row tables tab_col / tab_aux / tab_sf */
+  GT_RC0,      /* 12 residue counts: mass, position[3], velocity[3], quaternion[4], t */
+  GT_I32_COLS = GT_RC0 + 12
+};
+enum { GT_LAT0 = 0, GT_LON0, GT_F64_COLS }; /* LaunchCondition lat / lon (deg), for downrange */
+enum { GT_SCALE = 0, GT_OFFSET, GT_SF_COLS };
+
 typedef struct GelatoPlanDesc {
   /* sizes */
   int32_t n_sections, n_nodes; /* S, N;  M = N + S */
@@ -168,6 +197,14 @@ typedef struct GelatoPlanDesc {
    * every call); may be NULL, then the update-mode entry points are unavailable */
   const int64_t* xdep_idx;
   int64_t n_xdep;
+  /* result-table user constraints (GT_* above); n_tab = 0 / NULL tables: none */
+  int32_t n_tab;
+  const int32_t* tab_i32; /* [n_tab][GT_I32_COLS] */
+  const double* tab_f64;  /* [n_tab][GT_F64_COLS] */
+  int32_t n_tab_rows;
+  const int32_t* tab_col; /* [n_tab_rows] column code, 0 <= code < GT_COLUMNS */
+  const int64_t* tab_aux; /* [n_tab_rows] first of the row's GT_AUX slots in vals */
+  const double* tab_sf;   /* [n_tab_rows][GT_SF_COLS] */
 } GelatoPlanDesc;
 
 /* per-scenario overrides for batched evaluation (NULL members = shared) */
@@ -409,8 +446,9 @@ int gelato_eval_pair_packed_dev(GelatoPlan* plan, const double* x_dev, double* g
  * linear rows) and vacuum dynamics nodes [vac_first, vac_first + vac_count) (gelato_plan_n_blocks(plan, 5) nodes).
  * Every packed slot and residual row is written by exactly one block or node: ranks with disjoint covering ranges
  * fill disjoint parts of packed[] and g[] (gelato_b200/batch.py: ShardedProblem finds each rank's part once and
- * gathers).  Device pointers, caller's stream, not synchronised.  Forward differences only: in central mode it returns
- * GELATO_ERR_ARG. */
+ * gathers).  The result-table user constraints (GT_*) are evaluated by the range that starts at block 0 (block_first ==
+ * 0, block_count > 0), in full.  Device pointers, caller's stream, not synchronised.  Forward differences only: in
+ * central mode it returns GELATO_ERR_ARG. */
 int gelato_eval_pair_packed_range_dev(GelatoPlan* plan, const double* x_dev, double* g_dev, double* packed_dev, int32_t n_scen,
                                       int32_t block_first, int32_t block_count, int32_t vac_first, int32_t vac_count,
                                       void* stream);
